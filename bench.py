@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the CABiNet forward hot path (BASELINE.json: images/sec at 1024x1024, MNv3-Large).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4] [--dump-outputs DIR]
 
 ``--config`` picks a BASELINE.json workload: 2 (default, the one the metric is quoted on) = Large 16x3x1024x1024, 8
 classes; 3 = Large 1024x2048, 19 classes (Cityscapes shape, batch 8 per GPU); 4 = Small 2160x3840, 8 classes (UAVid 4K,
@@ -23,6 +23,10 @@ synthetic images per GPU.  Prints ONE JSON line on rank 0.
                 channels_last, same batch): what a user of the reference gets from cuDNN/cuBLAS today (the "practical
                 bar", BASELINE.md).
 * ``--impl reference`` times that same CPU implementation as the reference arm.
+
+``--dump-outputs DIR`` writes, on rank 0, what the timed path returned in its last timed step as float32
+``DIR/<name>.npy``: the two logit tensors (and for ``--config 5`` the loss and the gradients).  The inputs are seeded,
+so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -151,6 +155,33 @@ class ClockSampler:
                 "source": "nvidia-smi -lms 200"}
 
 
+DUMP_SAMPLE = 1 << 22  # elements kept of a larger output: 16 MB in float32, so a run dumps at most 64 MB in all
+
+
+def output_sample(t, n=DUMP_SAMPLE):
+    """-> numpy float32 copy of ``t``: the whole tensor if it has at most ``n`` elements, else a 1-D array of the
+    elements at up to ``n`` sorted flat indices drawn by a fixed seed from the element count alone, so that runs with
+    the same arguments sample the same positions."""
+    import numpy as np
+    import torch
+
+    t = t.detach()
+    if t.numel() > n:
+        idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), size=n))
+        t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+    return t.float().cpu().numpy()
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes ``{name: numpy array}`` as ``out_dir/<name>.npy``."""
+    import numpy as np
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
 def cpu_forward_rate(mode, n_classes, hw, batch, iters, warmup):
     """Oracle port of the reference forward on the host cores -> (images/s, threads)."""
     import torch
@@ -181,8 +212,10 @@ def run_reference(args):
         return
     t0 = time.perf_counter()
     B = args.ref_batch or args.batch
-    rate, threads, times, _ = cpu_forward_rate(args.mode, args.classes, (args.height, args.width), B, args.steps,
-                                               max(1, min(args.warmup, 2)))
+    rate, threads, times, ref_out = cpu_forward_rate(args.mode, args.classes, (args.height, args.width), B, args.steps,
+                                                     max(1, min(args.warmup, 2)))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"final_logits": output_sample(ref_out[0]), "aux_logits": output_sample(ref_out[1])})
     ms = 1e3 * statistics.median(times)
     sample = (f"{args.steps} steps x {B} images {args.height}x{args.width}, fp32, oracle port of src/models/cabinet.py "
               f"forward")
@@ -455,6 +488,10 @@ def run_ours(args):
         value = world * B * K / (ms_total * 1e-3)
         clocks = clk.summary()
         gpu_img0 = (out[0][:1].float().cpu(), out[1][:1].float().cpu())  # image 0: compared with the oracle below
+        # the graph's static output buffers: sampled now, before the traced steps below overwrite them
+        dumped = None
+        if args.dump_outputs and rank == 0:
+            dumped = {"final_logits": output_sample(out[0]), "aux_logits": output_sample(out[1])}
         del out
 
         # ---------------- per-kernel roofline: same K steps, every launch bracketed by CUDA events on its stream
@@ -591,6 +628,8 @@ def run_ours(args):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
 
     # whole-forward roofline: SURVEY 8(d)'s per-layer-fusion algorithmic bytes per image (two bf16 logit tensors returned)
     # x the batch / the step time; the engine's own per-launch byte count (block-fused kernels move less) alongside
@@ -671,10 +710,13 @@ def run_train(args):
     lb_host = make_labels(B, H, W, C, seed=11 + rank).pin_memory()
     x, lb = x_host.to(dev), lb_host.to(dev)
     eng = model.train_engine()
+    last = {}  # logits of the last timed step (--dump-outputs)
 
-    def step(xd, ld):
+    def step(xd, ld, keep=False):
         gb.zero_()
         out, out16 = model(xd)
+        if keep:
+            last.update(final_logits=out, aux_logits=out16)
         loss = crit_p(out, ld) + crit_16(out16, ld)
         loss.backward()
         if not os.environ.get("CABINET_BENCH_NO_GRAD_SYNC"):  # diagnostic: independent replicas (max over ranks without NCCL)
@@ -702,13 +744,19 @@ def run_train(args):
     launches = 0
     with ClockSampler(gpu_id) as clk:
         e0.record()
-        for _ in range(K):
-            loss = step(x, lb)
+        for i in range(K):
+            loss = step(x, lb, keep=bool(args.dump_outputs) and i == K - 1)
             launches += eng.launches
         e1.record()
         barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
     value = world * B * K / (ms * 1e-3)
+    dumped = None
+    if args.dump_outputs and rank == 0:  # before the steps below overwrite the gradients
+        grads = torch.cat([p.grad.reshape(-1) for p in model.parameters() if p.grad is not None])
+        dumped = {"loss": output_sample(loss), **{k: output_sample(v) for k, v in last.items()},
+                  "gradients": output_sample(grads)}
+        del grads
     # end to end: host batch in, loss out, every step
     from cabinet_b200.prefetch import DevicePrefetcher
 
@@ -781,6 +829,8 @@ def run_train(args):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     n_grad = sum(b.numel() for b in gb.buckets)
     print(json.dumps({
         "metric": "training images/sec at 1024x1024 (MNv3-L), fwd+bwd" if (H, W, args.mode) == (1024, 1024, "large")
@@ -822,7 +872,11 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--msflip", type=int, default=4, help="batch of the multi-scale + flip evaluation leg (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (at most 64 MB, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     cfg = CONFIGS[args.config]
     if args.size:
         args.height = args.height or args.size

@@ -17,8 +17,7 @@ plain numpy, which is what the CUDA kernels implement.
 Pinning: the reference's own tests hold no golden values for this path (SURVEY §8c), so the
 oracle is pinned against outputs of the *imported, unmodified reference* generated in the
 build container by ``oracle/make_golden.py`` and committed under ``tests/golden/``
-(``tests/test_oracle_golden.py``), plus a live comparison whenever ``/root/reference``
-is present (``tests/test_oracle_vs_reference.py``).
+(``tests/test_oracle_golden.py``).
 """
 
 from __future__ import annotations
