@@ -14,7 +14,7 @@ PKG = Path(__file__).resolve().parent
 LIB_PATH = PKG / "libcabinet_b200.so"
 CSRC = PKG / "csrc"
 
-F32, BF16 = 0, 1
+F32, BF16, F16 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_HSWISH, ACT_HSIGMOID, ACT_SIGMOID = 0, 1, 2, 3, 4
 
 _p, _i, _ll, _f = C.c_void_p, C.c_int, C.c_longlong, C.c_float
@@ -29,12 +29,17 @@ SIGNATURES = {
     "cabinet_conv2d_simt": ([_p, _i, _ll, _ll, _ll, _ll, _ll, _p, _i, _ll, _ll, _ll, _p, _p, _ll, _p, _i, _ll, _ll,
                              _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _p], _i),
     "cabinet_conv_tc": ([_p, _ll, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _p, _p, _ll, _p, _i, _ll, _i, _i, _i, _p], _i),
+    "cabinet_conv_tc_dt": ([_p, _ll, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _p, _p, _ll, _p, _i, _ll, _i, _i, _i, _i, _p],
+                           _i),
     "cabinet_conv_tc_view": ([_p, _ll, _i, _i, _i, _i, _p, _i, _i, _i, _i, _p, _p, _ll, _i, _i, _ll, _ll, _ll, _p], _i),
+    "cabinet_conv_tc_view_dt": ([_p, _ll, _i, _i, _i, _i, _p, _i, _i, _i, _i, _p, _p, _ll, _i, _i, _ll, _ll, _ll, _i, _p], _i),
     "cabinet_conv_tc_se": ([_p, _ll, _i, _i, _i, _i, _p, _i, _p, _i, _i, _i, _i, _i, _p, _p, _ll, _p, _i, _ll, _i, _i, _i,
                             _p], _i),
     "cabinet_conv_tc_split_act": ([_p, _ll, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _p, _p, _i, _ll, _i, _i, _i, _i, _p], _i),
     "cabinet_conv_tc_imgw": ([_p, _ll, _i, _i, _i, _i, _p, _ll, _i, _i, _i, _i, _i, _p, _p, _ll, _p, _i, _ll, _i, _i, _i,
                               _p], _i),
+    "cabinet_conv_tc_imgw_dt": ([_p, _ll, _i, _i, _i, _i, _p, _ll, _i, _i, _i, _i, _i, _p, _p, _ll, _p, _i, _ll, _i, _i, _i,
+                                 _i, _p], _i),
     "cabinet_conv_tc_up": ([_p, _ll, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _p, _p, _i, _i, _p, _ll, _i, _i, _i, _p], _i),
     "cabinet_gate_scale_weights": ([_p, _i, _f, _p, _p, _p, _p, _i, _i, _i, _p, _p, _i, _i, _i, _i, _i, _p], _i),
     "cabinet_scale_weights": ([_p, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
@@ -42,6 +47,7 @@ SIGNATURES = {
     "cabinet_stem_tc2": ([_p, _i, _i, _i, _p, _p, _ll, _p, _ll, _i, _i, _p], _i),
     "cabinet_dwconv": ([_p, _ll, _p, _p, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p], _i),
     "cabinet_dwconv_tma": ([_p, _ll, _p, _p, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p], _i),
+    "cabinet_dwconv_tma_dt": ([_p, _ll, _p, _p, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _i, _p], _i),
     "cabinet_mbconv_noexpand_fused": ([_p, _ll, _p, _p, _p, _p, _p, _ll, _i, _i, _i, _i, _i, _p], _i),
     "cabinet_mbconv_fused": ([_p, _ll, _i, _i, _i, _i, _p, _p, _i, _i, _i, _i, _i, _p, _p, _i, _i, _p, _ll, _i, _i, _p,
                               _p], _i),
@@ -70,8 +76,10 @@ SIGNATURES = {
     "cabinet_train_scratch_floats": ([_ll, _i, _i], _ll),
     "cabinet_pack_conv_weight": ([_p, _i, _i, _i, _i, _p, _i, _i, _i, _i, _p], _i),
     "cabinet_pack_conv_weight_parity": ([_p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _i, _i, _p], _i),
+    "cabinet_pack_conv_weight_parity_dt": ([_p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _i, _i, _i, _p], _i),
     "cabinet_pack_dw_weight": ([_p, _i, _i, _i, _p, _p], _i),
     "cabinet_im2col_nchw": ([_p, _i, _i, _i, _i, _i, _i, _i, _p, _ll, _p], _i),
+    "cabinet_im2col_nchw_dt": ([_p, _i, _i, _i, _i, _i, _i, _i, _p, _ll, _i, _p], _i),
     "cabinet_embed_filter": ([_p, _i, _i, _i, _i, _p, _ll, _i, _p], _i),
     "cabinet_bn_train_stats": ([_p, _ll, _i, _ll, _i, _p, _p, _f, _f, _p, _p, _p, _p, _p], _i),
     "cabinet_affine_act": ([_p, _ll, _i, _p, _p, _p, _f, _p, _ll, _p, _ll, _i, _ll, _ll, _i, _i, _p], _i),
@@ -86,15 +94,20 @@ SIGNATURES = {
                             _p], _i),
     "cabinet_conv_wgrad_tc_scratch_floats": ([_i, _i, _i, _i, _i, _i, _i, _i, _i], _ll),
     "cabinet_conv_wgrad_tc": ([_p, _ll, _p, _ll, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p], _i),
+    "cabinet_conv_wgrad_tc_dt": ([_p, _ll, _p, _ll, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _i, _p], _i),
     "cabinet_conv_wgrad_tc_batched": ([_p, _ll, _p, _ll, _p, _i, _i, _i, _i, _i, _p], _i),
+    "cabinet_conv_wgrad_tc_batched_dt": ([_p, _ll, _p, _ll, _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "cabinet_dwconv_dgrad": ([_p, _ll, _i, _p, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "cabinet_dwconv_wgrad": ([_p, _ll, _p, _ll, _i, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p], _i),
     "cabinet_resample_sep": ([_p, _i, _ll, _ll, _ll, _ll, _p, _i, _ll, _ll, _ll, _ll, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p,
                               _i, _p], _i),
     "cabinet_softmax_backward": ([_p, _p, _p, _ll, _i, _f, _p], _i),
     "cabinet_attn_softmax": ([_p, _f, _p, _p, _ll, _i, _p], _i),
+    "cabinet_attn_softmax_dt": ([_p, _f, _p, _p, _ll, _i, _i, _p], _i),
     "cabinet_attn_softmax_backward": ([_p, _p, _p, _ll, _i, _f, _p], _i),
+    "cabinet_attn_softmax_backward_dt": ([_p, _p, _p, _ll, _i, _f, _i, _p], _i),
     "cabinet_transpose_tokens": ([_p, _ll, _p, _i, _i, _i, _p], _i),
+    "cabinet_transpose_tokens_dt": ([_p, _ll, _p, _i, _i, _i, _i, _p], _i),
     "cabinet_cab_combine_backward": ([_p, _ll, _p, _p, _p, _p, _i, _p, _p, _p, _p, _ll, _i, _i, _p, _p], _i),
     "cabinet_add": ([_p, _ll, _p, _ll, _p, _ll, _i, _ll, _i, _p], _i),
     "cabinet_ohem_ce_forward": ([_p, _i, _p, _i, _i, _i, _ll, _p, _i, _f, _ll, _p, _p, _p, _p], _i),

@@ -1,6 +1,7 @@
 // Shared device/host helpers for libcabinet_b200.so (sm_100a only).
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -32,11 +33,61 @@ void cabinet_set_error(const char* fmt, ...);
 
 #define CAB_LAUNCH_CHECK() CAB_CUDA(cudaGetLastError())
 
+// ----------------------------------------------------------------------------- element types
+// Every entry point that takes an element type checks it against the set it implements BEFORE any CUDA call, and the
+// dispatch macros below decode exactly the three known codes: an unknown or unimplemented type is an error, never a
+// silent reinterpretation of the bits as one of the other types.
+#define CAB_DT_F32 (1 << CABINET_F32)
+#define CAB_DT_BF16 (1 << CABINET_BF16)
+#define CAB_DT_F16 (1 << CABINET_F16)
+#define CAB_DT_ALL (CAB_DT_F32 | CAB_DT_BF16 | CAB_DT_F16)
+static inline bool cab_dtype_ok(int dt, int mask) { return dt >= 0 && dt < 30 && ((mask >> dt) & 1); }
+static inline const char* cab_dtype_name(int dt) {
+    return dt == CABINET_F32 ? "fp32" : dt == CABINET_BF16 ? "bf16" : dt == CABINET_F16 ? "fp16" : "unknown";
+}
+#define CAB_REQUIRE_DTYPE(what, dt, mask)                                                                          \
+    CAB_REQUIRE(cab_dtype_ok((dt), (mask)), "%s: element type %d (%s) is not implemented by this entry point", what, \
+                static_cast<int>(dt), cab_dtype_name(dt))
 static inline int cab_dtype_size(int dt) { return dt == CABINET_F32 ? 4 : 2; }
 static inline long long cab_ceil_div(long long a, long long b) { return (a + b - 1) / b; }
 
 // ----------------------------------------------------------------------------- device helpers
 typedef __nv_bfloat16 bf16;
+typedef __half f16;
+
+// Host dispatch on one element type: runs the statement list with `T` = float / bf16 / f16.  The caller has
+// validated `dt` (CAB_REQUIRE_DTYPE); anything else is still rejected here.
+#define CAB_DISPATCH_DT(dt, T, ...)                                                                   \
+    do {                                                                                              \
+        if ((dt) == CABINET_F32) { typedef float T; __VA_ARGS__; }                                    \
+        else if ((dt) == CABINET_BF16) { typedef bf16 T; __VA_ARGS__; }                               \
+        else if ((dt) == CABINET_F16) { typedef f16 T; __VA_ARGS__; }                                 \
+        else CAB_REQUIRE(false, "unsupported element type %d", static_cast<int>(dt));                 \
+    } while (0)
+
+// The same for the 2-byte types only (kernels that exist for bf16 and fp16 operands alone).
+#define CAB_DISPATCH_DT_HALF(dt, T, ...)                                                              \
+    do {                                                                                              \
+        if ((dt) == CABINET_BF16) { typedef bf16 T; __VA_ARGS__; }                                    \
+        else if ((dt) == CABINET_F16) { typedef f16 T; __VA_ARGS__; }                                 \
+        else CAB_REQUIRE(false, "unsupported 2-byte element type %d", static_cast<int>(dt));          \
+    } while (0)
+
+// Host dispatch on two operands, each fp32 or the call's ONE 2-byte type (bf16 and fp16 never mix in a call):
+// M(TA, TB) with the matching C++ types.
+#define CAB_DISPATCH_DT_PAIR(da, db, M)                                                                             \
+    do {                                                                                                            \
+        const int _da = (da), _db = (db), _dh = _da != CABINET_F32 ? _da : _db;                                     \
+        CAB_REQUIRE(cab_dtype_ok(_dh, CAB_DT_ALL) && (_da == CABINET_F32 || _da == _dh) &&                          \
+                        (_db == CABINET_F32 || _db == _dh),                                                         \
+                    "unsupported element type pair %d / %d", _da, _db);                                             \
+        if (_dh == CABINET_F32) M(float, float);                                                                    \
+        else if (_dh == CABINET_BF16) {                                                                             \
+            if (_da == CABINET_F32) M(float, bf16); else if (_db == CABINET_F32) M(bf16, float); else M(bf16, bf16); \
+        } else {                                                                                                    \
+            if (_da == CABINET_F32) M(float, f16); else if (_db == CABINET_F32) M(f16, float); else M(f16, f16);     \
+        }                                                                                                           \
+    } while (0)
 
 __device__ __forceinline__ float cab_act(float v, int act) {
     // reference: src/models/mobilenetv3.py:38-65 (relu6(x+3)/6, x*hsig(x)); nn.ReLU; nn.Sigmoid
@@ -84,8 +135,32 @@ template <> __device__ __forceinline__ float to_f32<bf16>(bf16 v) { return __bfl
 template <typename T> __device__ __forceinline__ T from_f32(float v);
 template <> __device__ __forceinline__ float from_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ bf16 from_f32<bf16>(float v) { return __float2bfloat16_rn(v); }
+// fp16: round to nearest, overflow -> inf (never saturating: a loss-scale overflow must reach the gradients as inf)
+template <> __device__ __forceinline__ float to_f32<f16>(f16 v) { return __half2float(v); }
+template <> __device__ __forceinline__ f16 from_f32<f16>(float v) { return __float2half_rn(v); }
 
-// 16-byte vector of T: 4 floats or 8 bf16
+// Two packed 2-byte elements (one 32-bit word: element 0 in the low half) -> fp32
+template <typename T> __device__ __forceinline__ float2 cab_unpack2(uint32_t w);
+template <> __device__ __forceinline__ float2 cab_unpack2<bf16>(uint32_t w) {  // bf16 -> f32 is a 16-bit shift
+    return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
+}
+template <> __device__ __forceinline__ float2 cab_unpack2<f16>(uint32_t w) {
+    __half2 h;
+    *reinterpret_cast<uint32_t*>(&h) = w;
+    return __half22float2(h);
+}
+// fp32 pair -> two packed 2-byte elements (round to nearest; fp16 overflow -> inf)
+template <typename T> __device__ __forceinline__ uint32_t cab_pack2(float lo, float hi);
+template <> __device__ __forceinline__ uint32_t cab_pack2<bf16>(float lo, float hi) {
+    __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&h);
+}
+template <> __device__ __forceinline__ uint32_t cab_pack2<f16>(float lo, float hi) {
+    __half2 h = __floats2half2_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&h);
+}
+
+// 16-byte vector of T: 4 floats or 8 bf16 / fp16
 template <typename T> struct Vec16;
 template <> struct Vec16<float> {
     static constexpr int N = 4;
@@ -95,29 +170,26 @@ template <> struct Vec16<float> {
     __device__ __forceinline__ void unpack(float* f) const { f[0] = raw.x; f[1] = raw.y; f[2] = raw.z; f[3] = raw.w; }
     __device__ __forceinline__ void pack(const float* f) { raw = make_float4(f[0], f[1], f[2], f[3]); }
 };
-template <> struct Vec16<bf16> {
+template <typename T> struct Vec16Half {  // T = bf16 or f16
     static constexpr int N = 8;
     uint4 raw;
-    __device__ __forceinline__ void load(const bf16* p) { raw = *reinterpret_cast<const uint4*>(p); }
-    __device__ __forceinline__ void store(bf16* p) const { *reinterpret_cast<uint4*>(p) = raw; }
+    __device__ __forceinline__ void load(const T* p) { raw = *reinterpret_cast<const uint4*>(p); }
+    __device__ __forceinline__ void store(T* p) const { *reinterpret_cast<uint4*>(p) = raw; }
     __device__ __forceinline__ void unpack(float* f) const {
         const uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {  // bf16 -> f32 is a 16-bit shift
-            f[2 * i] = __uint_as_float(w[i] << 16);
-            f[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
+        for (int i = 0; i < 4; ++i) {
+            const float2 v = cab_unpack2<T>(w[i]);
+            f[2 * i] = v.x;
+            f[2 * i + 1] = v.y;
         }
     }
     __device__ __forceinline__ void pack(const float* f) {
-        uint32_t w[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            __nv_bfloat162 h = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
-            w[i] = *reinterpret_cast<uint32_t*>(&h);
-        }
-        raw = make_uint4(w[0], w[1], w[2], w[3]);
+        raw = make_uint4(cab_pack2<T>(f[0], f[1]), cab_pack2<T>(f[2], f[3]), cab_pack2<T>(f[4], f[5]), cab_pack2<T>(f[6], f[7]));
     }
 };
+template <> struct Vec16<bf16> : Vec16Half<bf16> {};
+template <> struct Vec16<f16> : Vec16Half<f16> {};
 
 // Bilinear source taps, align_corners=False (ATen area_pixel_compute_source_index; reference call sites
 // src/models/cabinet.py:228-245, src/models/cab.py:70-72). scale = in/out as float.

@@ -137,6 +137,9 @@ extern "C" int cabinet_conv2d_simt(const void* x, int x_dtype, long long sxn, lo
                                    long long y_batch_stride, int batches, int N, int H, int W, int Cin, int Cout,
                                    int KH, int KW, int stride, int pad, int OH, int OW, int act, float alpha,
                                    cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("conv2d_simt", x_dtype, CAB_DT_ALL);
+    CAB_REQUIRE_DTYPE("conv2d_simt", w_dtype, CAB_DT_ALL);
+    CAB_REQUIRE_DTYPE("conv2d_simt", y_dtype, CAB_DT_ALL);
     CAB_REQUIRE(x && w && y, "conv2d_simt: null pointer");
     CAB_REQUIRE(batches >= 1 && N >= 0 && H > 0 && W > 0 && Cin > 0 && Cout > 0 && KH > 0 && KW > 0,
                 "conv2d_simt: bad sizes");
@@ -152,6 +155,20 @@ extern "C" int cabinet_conv2d_simt(const void* x, int x_dtype, long long sxn, lo
     a.K = KH * KW * Cin;
     if (a.M == 0) return CABINET_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const bool has_f16 = x_dtype == CABINET_F16 || w_dtype == CABINET_F16 || y_dtype == CABINET_F16;
+    if (has_f16) {  // fp16 training mode: each operand fp32 or fp16
+        CAB_REQUIRE(x_dtype != CABINET_BF16 && w_dtype != CABINET_BF16 && y_dtype != CABINET_BF16,
+                    "conv2d_simt: bf16 and fp16 operands do not mix");
+        switch ((x_dtype == CABINET_F16) * 4 + (w_dtype == CABINET_F16) * 2 + (y_dtype == CABINET_F16)) {
+            case 1: return launch<float, float, f16>(a, batches, s);
+            case 2: return launch<float, f16, float>(a, batches, s);
+            case 3: return launch<float, f16, f16>(a, batches, s);
+            case 4: return launch<f16, float, float>(a, batches, s);
+            case 5: return launch<f16, float, f16>(a, batches, s);
+            case 6: return launch<f16, f16, float>(a, batches, s);
+            case 7: return launch<f16, f16, f16>(a, batches, s);
+        }
+    }
     const int key = x_dtype * 4 + w_dtype * 2 + y_dtype;
     switch (key) {
         case 0: return launch<float, float, float>(a, batches, s);

@@ -1,4 +1,5 @@
-// Implicit-GEMM convolution on the 5th-gen tensor cores (tcgen05.mma, fp32 accumulators in TMEM), bf16 NHWC.
+// Implicit-GEMM convolution on the 5th-gen tensor cores (tcgen05.mma, fp32 accumulators in TMEM), bf16 NHWC (fp16 for
+// the plain convolution forms of the fp16 training mode: same tiles, only the operand format bits and the map type change).
 //
 //   D[128 pixels x block_n couts] = sum over (tap, 64-channel block)  A_tap[128 x 64] * W_tap[block_n x 64]^T
 //
@@ -19,6 +20,8 @@
 //   (full-line writes, image-border and channel clipping by the tensor map); fp32 outputs (class logits) are
 //   stored directly.
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "tc_common.cuh"
 
@@ -50,7 +53,7 @@ struct TcConvParams {
     int a_act, hw;            // A-operand prologue: x <- act(x * a_scale[image][channel]); hw = pixels per image
     const float* a_scale;     // [N][Cin] fp32 or nullptr
     const float* bias;
-    const bf16* res;
+    const void* res;          // residual: the operand type (bf16 / fp16)
     long long ldres;
     void* y;
     long long ldy;
@@ -79,7 +82,7 @@ __device__ __forceinline__ TileCoord decode_tile(const TcConvParams& p, int tile
     return c;
 }
 
-template <int ACT, bool HAS_RES, bool OUT_F32, bool PRO, bool UP4 = false>
+template <int ACT, bool HAS_RES, bool OUT_F32, bool PRO, bool UP4 = false, typename T = bf16>
 __global__ void __launch_bounds__(PRO ? NUM_THREADS + PRO_THREADS : NUM_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
                const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmA3,
@@ -178,7 +181,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
     } else if (warp == 1) {
         // ================= MMA issuer: warp-uniform control flow, one elected lane issues =================
         const uint32_t leader = tc::elect_one();
-        const uint32_t idesc = tc::make_idesc_bf16(BLOCK_M, p.block_n);
+        const uint32_t idesc = tc::make_idesc<T>(BLOCK_M, p.block_n);
         const uint64_t a_desc0 = tc::make_desc_sw128(tc::smem_u32(sA));
         const uint64_t b_desc0 = tc::make_desc_sw128(tc::smem_u32(sB));
         const uint32_t a_step = A_STAGE_BYTES >> 4, b_step = static_cast<uint32_t>(b_stage_bytes) >> 4;
@@ -275,7 +278,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                     const int j = l ^ (r & 7);
                     const int c = cb * BLOCK_K + (l << 3);
                     if (c < p.Cin) {
-                        Vec16<bf16> v;
+                        Vec16<T> v;
                         v.raw = raw[jj];
                         float f[8];
                         v.unpack(f);
@@ -395,7 +398,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                             }
                         }
                     }
-                    constexpr bool RELU_ON_CVT = ACT == CABINET_ACT_RELU && !HAS_RES && !OUT_F32;  // cvt.rn.relu.bf16x2
+                    constexpr bool RELU_ON_CVT = ACT == CABINET_ACT_RELU && !HAS_RES && !OUT_F32;  // cvt.rn.relu.{bf16,f16}x2
                     const bool do_act = co0 < p.act_cols;  // uniform per 16-column chunk (act_cols % 16 == 0)
                     if constexpr (ACT == CABINET_ACT_RELU && !RELU_ON_CVT) {
                         if (do_act) {
@@ -410,11 +413,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                     }
                     if constexpr (HAS_RES) {
                         if (valid && co0 < p.Cout) {
-                            const bf16* rp = p.res + pix * p.ldres + co0;
+                            const T* rp = reinterpret_cast<const T*>(p.res) + pix * p.ldres + co0;
 #pragma unroll
                             for (int h = 0; h < 2; ++h) {
                                 if (co0 + 8 * h + 8 <= p.Cout) {
-                                    Vec16<bf16> rv;
+                                    Vec16<T> rv;
                                     rv.load(rp + 8 * h);
                                     float rf[8];
                                     rv.unpack(rf);
@@ -422,18 +425,23 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                                     for (int j = 0; j < 8; ++j) v[8 * h + j] += rf[j];
                                 } else {
                                     for (int j = 0; j < 8; ++j)
-                                        if (co0 + 8 * h + j < p.Cout) v[8 * h + j] += __bfloat162float(rp[8 * h + j]);
+                                        if (co0 + 8 * h + j < p.Cout) v[8 * h + j] += to_f32<T>(rp[8 * h + j]);
                                 }
                             }
                         }
                     }
                     if constexpr (!OUT_F32) {
-                        Vec16<bf16> o0, o1;
+                        Vec16<T> o0, o1;
                         if (RELU_ON_CVT && do_act) {
+                            // never .satfinite: an fp16 overflow stays inf (a loss-scale overflow must reach the gradients)
                             uint32_t w[8];
 #pragma unroll
-                            for (int j = 0; j < 8; ++j)
-                                asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(w[j]) : "f"(v[2 * j + 1]), "f"(v[2 * j]));
+                            for (int j = 0; j < 8; ++j) {
+                                if constexpr (std::is_same<T, f16>::value)
+                                    asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(w[j]) : "f"(v[2 * j + 1]), "f"(v[2 * j]));
+                                else
+                                    asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(w[j]) : "f"(v[2 * j + 1]), "f"(v[2 * j]));
+                            }
                             o0.raw = make_uint4(w[0], w[1], w[2], w[3]);
                             o1.raw = make_uint4(w[4], w[5], w[6], w[7]);
                         } else {
@@ -487,8 +495,10 @@ cab_encode_tiled_fn cab_get_encode_tiled() {
     return fn;
 }
 
-int cab_make_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                       const uint32_t* box, CUtensorMapL2promotion promo, CUtensorMapSwizzle swizzle) {
+int cab_make_tmap_2b(CUtensorMap* map, int elem_dtype, const void* base, int rank, const uint64_t* dims,
+                     const uint64_t* strides_bytes, const uint32_t* box, CUtensorMapL2promotion promo,
+                     CUtensorMapSwizzle swizzle) {
+    CAB_REQUIRE_DTYPE("tensor map", elem_dtype, CAB_DT_BF16 | CAB_DT_F16);
     cab_encode_tiled_fn enc = cab_get_encode_tiled();
     if (!enc) {
         cabinet_set_error("cuTensorMapEncodeTiled is unavailable (driver too old or no driver)");
@@ -502,7 +512,7 @@ int cab_make_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint6
         estr[i] = 1;
         if (i > 0) gstr[i - 1] = strides_bytes[i - 1];
     }
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(base), gdim, gstr, bdim, estr,
+    CUresult r = enc(map, elem_dtype == CABINET_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(base), gdim, gstr, bdim, estr,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
         cabinet_set_error("cuTensorMapEncodeTiled failed with CUresult %d (rank %d dims %llu,%llu,%llu,%llu box %u,%u,%u,%u)",
@@ -528,15 +538,23 @@ extern "C" int cabinet_debug_flags(int flags) {
 static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int Cin, const float* a_scale, int a_act,
                         const void* w_packed, long long w_image_stride, int Cout, int KH, int KW, int stride, int pad,
                         const float* bias, const void* res, long long ldres, void* y, int y_dtype, long long ldy,
-                        int OH, int OW, int act, cabinet_stream_t stream, int act_cols = 1 << 30,
+                        int OH, int OW, int act, int op_dtype, cabinet_stream_t stream, int act_cols = 1 << 30,
                         const float* up = nullptr, int up_h = 0, int up_w = 0, long long y_sw = 1, long long y_sh = 0,
                         long long y_sn = 0);
 
 extern "C" int cabinet_conv_tc_view(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed,
                                     int Cout, int KH, int KW, int pad, const float* bias, void* y, long long ldy, int OH,
                                     int OW, long long y_sw, long long y_sh, long long y_sn, cabinet_stream_t stream) {
+    return cabinet_conv_tc_view_dt(x, ldx, N, H, W, Cin, w_packed, Cout, KH, KW, pad, bias, y, ldy, OH, OW, y_sw, y_sh, y_sn,
+                                   CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_conv_tc_view_dt(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed,
+                                       int Cout, int KH, int KW, int pad, const float* bias, void* y, long long ldy, int OH,
+                                       int OW, long long y_sw, long long y_sh, long long y_sn, int op_dtype,
+                                       cabinet_stream_t stream) {
     return conv_tc_impl(x, ldx, N, H, W, Cin, nullptr, CABINET_ACT_NONE, w_packed, 0, Cout, KH, KW, 1, pad, bias, nullptr, 0,
-                        y, CABINET_BF16, ldy, OH, OW, CABINET_ACT_NONE, stream, 1 << 30, nullptr, 0, 0, y_sw, y_sh, y_sn);
+                        y, op_dtype, ldy, OH, OW, CABINET_ACT_NONE, op_dtype, stream, 1 << 30, nullptr, 0, 0, y_sw, y_sh, y_sn);
 }
 
 extern "C" int cabinet_conv_tc_se(const void* x, long long ldx, int N, int H, int W, int Cin, const float* a_scale,
@@ -544,18 +562,27 @@ extern "C" int cabinet_conv_tc_se(const void* x, long long ldx, int N, int H, in
                                   const float* bias, const void* res, long long ldres, void* y, int y_dtype,
                                   long long ldy, int OH, int OW, int act, cabinet_stream_t stream) {
     return conv_tc_impl(x, ldx, N, H, W, Cin, a_scale, a_act, w_packed, 0, Cout, KH, KW, stride, pad, bias, res, ldres, y,
-                        y_dtype, ldy, OH, OW, act, stream);
+                        y_dtype, ldy, OH, OW, act, CABINET_BF16, stream);
 }
 
 extern "C" int cabinet_conv_tc_imgw(const void* x, long long ldx, int N, int H, int W, int Cin,
                                     const void* w_packed_per_image, long long w_image_stride, int Cout, int KH, int KW,
                                     int stride, int pad, const float* bias, const void* res, long long ldres, void* y,
                                     int y_dtype, long long ldy, int OH, int OW, int act, cabinet_stream_t stream) {
+    return cabinet_conv_tc_imgw_dt(x, ldx, N, H, W, Cin, w_packed_per_image, w_image_stride, Cout, KH, KW, stride, pad, bias,
+                                   res, ldres, y, y_dtype, ldy, OH, OW, act, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_conv_tc_imgw_dt(const void* x, long long ldx, int N, int H, int W, int Cin,
+                                       const void* w_packed_per_image, long long w_image_stride, int Cout, int KH, int KW,
+                                       int stride, int pad, const float* bias, const void* res, long long ldres, void* y,
+                                       int y_dtype, long long ldy, int OH, int OW, int act, int op_dtype,
+                                       cabinet_stream_t stream) {
     CAB_REQUIRE(w_image_stride > 0 && w_image_stride % 8 == 0, "conv_tc_imgw: weight image stride must be a positive multiple of 8");
     CAB_REQUIRE(!(KH == 1 && KW == 1 && stride == 1 && pad == 0) || (static_cast<long long>(H) * W) % 128 == 0,
                 "conv_tc_imgw: a 1x1 convolution needs H * W %% 128 == 0 (a 128-pixel tile must not straddle two images)");
     return conv_tc_impl(x, ldx, N, H, W, Cin, nullptr, CABINET_ACT_NONE, w_packed_per_image, w_image_stride, Cout, KH, KW,
-                        stride, pad, bias, res, ldres, y, y_dtype, ldy, OH, OW, act, stream);
+                        stride, pad, bias, res, ldres, y, y_dtype, ldy, OH, OW, act, op_dtype, stream);
 }
 
 extern "C" int cabinet_conv_tc_split_act(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed,
@@ -564,15 +591,23 @@ extern "C" int cabinet_conv_tc_split_act(const void* x, long long ldx, int N, in
                                          cabinet_stream_t stream) {
     CAB_REQUIRE(act_cols >= 0 && act_cols % 16 == 0, "conv_tc_split_act: act_cols must be a multiple of 16");
     return conv_tc_impl(x, ldx, N, H, W, Cin, nullptr, CABINET_ACT_NONE, w_packed, 0, Cout, KH, KW, stride, pad, bias,
-                        nullptr, 0, y, y_dtype, ldy, OH, OW, act, stream, act_cols);
+                        nullptr, 0, y, y_dtype, ldy, OH, OW, act, CABINET_BF16, stream, act_cols);
 }
 
 extern "C" int cabinet_conv_tc(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed,
                                int Cout, int KH, int KW, int stride, int pad, const float* bias, const void* res,
                                long long ldres, void* y, int y_dtype, long long ldy, int OH, int OW, int act,
                                cabinet_stream_t stream) {
-    return cabinet_conv_tc_se(x, ldx, N, H, W, Cin, nullptr, CABINET_ACT_NONE, w_packed, Cout, KH, KW, stride, pad, bias,
-                              res, ldres, y, y_dtype, ldy, OH, OW, act, stream);
+    return cabinet_conv_tc_dt(x, ldx, N, H, W, Cin, w_packed, Cout, KH, KW, stride, pad, bias, res, ldres, y, y_dtype, ldy,
+                              OH, OW, act, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_conv_tc_dt(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed,
+                                  int Cout, int KH, int KW, int stride, int pad, const float* bias, const void* res,
+                                  long long ldres, void* y, int y_dtype, long long ldy, int OH, int OW, int act, int op_dtype,
+                                  cabinet_stream_t stream) {
+    return conv_tc_impl(x, ldx, N, H, W, Cin, nullptr, CABINET_ACT_NONE, w_packed, 0, Cout, KH, KW, stride, pad, bias, res,
+                        ldres, y, y_dtype, ldy, OH, OW, act, op_dtype, stream);
 }
 
 extern "C" int cabinet_conv_tc_up(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed,
@@ -581,20 +616,24 @@ extern "C" int cabinet_conv_tc_up(const void* x, long long ldx, int N, int H, in
                                   cabinet_stream_t stream) {
     CAB_REQUIRE(up != nullptr, "conv_tc_up: null low-resolution map");
     return conv_tc_impl(x, ldx, N, H, W, Cin, nullptr, CABINET_ACT_NONE, w_packed, 0, Cout, KH, KW, stride, pad, bias,
-                        nullptr, 0, y, CABINET_BF16, ldy, OH, OW, act, stream, 1 << 30, up, up_h, up_w);
+                        nullptr, 0, y, CABINET_BF16, ldy, OH, OW, act, CABINET_BF16, stream, 1 << 30, up, up_h, up_w);
 }
 
 static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int Cin, const float* a_scale, int a_act,
                         const void* w_packed, long long w_image_stride, int Cout, int KH, int KW, int stride, int pad,
                         const float* bias, const void* res, long long ldres, void* y, int y_dtype, long long ldy,
-                        int OH, int OW, int act, cabinet_stream_t stream, int act_cols, const float* up, int up_h,
+                        int OH, int OW, int act, int op_dtype, cabinet_stream_t stream, int act_cols, const float* up, int up_h,
                         int up_w, long long y_sw, long long y_sh, long long y_sn) {
     // y_sw / y_sh / y_sn (pixels): the output is a strided VIEW (pixel, row, image pitch) of a larger NHWC tensor -- e.g.
     // one input-parity class of the data gradient of a stride-2 convolution.  Defaults: a dense [N][OH][OW] tensor.
+    // op_dtype: the 2-byte type of x, w_packed, res and a 2-byte y (bf16, or fp16 for the plain convolution forms)
+    CAB_REQUIRE_DTYPE("conv_tc", op_dtype, CAB_DT_BF16 | CAB_DT_F16);
+    CAB_REQUIRE_DTYPE("conv_tc (output)", y_dtype, CAB_DT_F32 | (1 << op_dtype));
+    CAB_REQUIRE(op_dtype == CABINET_BF16 || (!a_scale && !up), "conv_tc: the prologue / upsample epilogues are built for bf16");
     CAB_REQUIRE(x && w_packed && bias && y, "conv_tc: null pointer");
     const bool out_view = y_sw != 1 || y_sh != 0 || y_sn != 0;
-    CAB_REQUIRE(!out_view || (y_dtype == CABINET_BF16 && !res && !up && y_sw >= 1 && y_sh >= OW && y_sn >= OH),
-                "conv_tc: a strided output view needs bf16 output and no residual");
+    CAB_REQUIRE(!out_view || (y_dtype == op_dtype && !res && !up && y_sw >= 1 && y_sh >= OW && y_sn >= OH),
+                "conv_tc: a strided output view needs a 2-byte output and no residual");
     const int reverse = (act & CABINET_CONV_REVERSE_TILES) ? 1 : 0;
     act &= ~CABINET_CONV_REVERSE_TILES;
     CAB_REQUIRE(!up || (up_h > 0 && up_w > 0 && Cout % 16 == 0 && (reinterpret_cast<uintptr_t>(up) & 15) == 0 && !res &&
@@ -609,7 +648,7 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
     CAB_REQUIRE(ldx % 8 == 0 && ldx >= Cin && (reinterpret_cast<uintptr_t>(x) & 15) == 0,
                 "conv_tc: input needs 16-byte aligned pixels (ldx %% 8 == 0)");
     CAB_REQUIRE(ldy >= Cout && (y_dtype == CABINET_F32 || (ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0)),
-                "conv_tc: bf16 output needs 16-byte aligned pixels");
+                "conv_tc: a 2-byte output needs 16-byte aligned pixels");
     CAB_REQUIRE(!res || (ldres % 8 == 0 && (reinterpret_cast<uintptr_t>(res) & 15) == 0), "conv_tc: residual alignment");
     CAB_REQUIRE((reinterpret_cast<uintptr_t>(w_packed) & 15) == 0, "conv_tc: weight alignment");
     if (N == 0) return CABINET_OK;
@@ -632,7 +671,7 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
     p.reverse = reverse;
     p.b_per_image = w_image_stride > 0 ? 1 : 0;
     p.b_resident = (!p.b_per_image && p.n_tiles == 1 && p.num_k_blocks * b_stage_bytes <= B_RESIDENT_MAX) ? 1 : 0;
-    p.c_bufs = (y_dtype == CABINET_BF16 && p.block_n > 64) ? 2 : 1;
+    p.c_bufs = (y_dtype != CABINET_F32 && p.block_n > 64) ? 2 : 1;
     const int fixed = 2 * p.c_bufs * C_STAGE_BYTES + (p.b_resident ? p.num_k_blocks * b_stage_bytes : 0) + 1024;
     const int stage_bytes = A_STAGE_BYTES + (p.b_resident ? 0 : b_stage_bytes);
     // experiment hook: CAB_SMEM_CAP_KB caps the dynamic smem of kernels whose accumulators need <= 256 TMEM columns, so
@@ -641,7 +680,7 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
     const int limit = (cap_kb > 0 && p.tmem_cols <= 256) ? std::max(cap_kb * 1024, fixed + 2 * stage_bytes) : SMEM_LIMIT;
     // the prologue variants keep a 4 KB scale row in static shared memory: leave room for it under the 227 KB CTA limit
     p.stages = std::max(2, std::min(MAX_STAGES, (std::min(limit, SMEM_LIMIT) - (a_scale ? 4096 : 0) - fixed) / stage_bytes));
-    p.act = act; p.y_dtype = y_dtype; p.bias = bias; p.res = reinterpret_cast<const bf16*>(res); p.ldres = ldres;
+    p.act = act; p.y_dtype = y_dtype; p.bias = bias; p.res = res; p.ldres = ldres;
     p.y = y; p.ldy = ldy; p.debug = g_debug;
     p.a_scale = a_scale; p.a_act = a_act; p.hw = H * W;
     p.up = up; p.up_h = up_h; p.up_w = up_w; p.img_h = OH; p.img_w = OW; p.up_flat = 0;
@@ -657,7 +696,7 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
         const uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)P, 1, 1};
         const uint64_t strides[3] = {(uint64_t)ldx * es, (uint64_t)ldx * es * P, (uint64_t)ldx * es * P};
         const uint32_t box[4] = {BLOCK_K, BLOCK_M, 1, 1};
-        int rc = cab_make_tmap_bf16(&tmA[0], x, 4, dims, strides, box);
+        int rc = cab_make_tmap_2b(&tmA[0], op_dtype, x, 4, dims, strides, box);
         if (rc) return rc;
         tmA[1] = tmA[2] = tmA[3] = tmA[0];
     } else {
@@ -672,14 +711,14 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
         p.tiles_w = static_cast<int>(cab_ceil_div(OW, p.TW));
         p.tiles_h = static_cast<int>(cab_ceil_div(OH, p.TH));
         const uint32_t box[4] = {BLOCK_K, (uint32_t)p.TW, (uint32_t)p.TH, 1};
-        const bf16* xb = reinterpret_cast<const bf16*>(x);
+        const uint16_t* xb = reinterpret_cast<const uint16_t*>(x);  // 2-byte elements of either type
         for (int py = 0; py < stride; ++py)
             for (int px = 0; px < stride; ++px) {
                 const uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)((W - px + stride - 1) / stride),
                                           (uint64_t)((H - py + stride - 1) / stride), (uint64_t)N};
                 const uint64_t strides[3] = {(uint64_t)ldx * es * stride, (uint64_t)ldx * es * W * stride,
                                              (uint64_t)ldx * es * W * H};
-                int rc = cab_make_tmap_bf16(&tmA[py * stride + px], xb + (static_cast<long long>(py) * W + px) * ldx, 4,
+                int rc = cab_make_tmap_2b(&tmA[py * stride + px], op_dtype, xb + (static_cast<long long>(py) * W + px) * ldx, 4,
                                             dims, strides, box);
                 if (rc) return rc;
             }
@@ -691,16 +730,16 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
         const uint64_t dims[3] = {ktot, (uint64_t)n16, (uint64_t)(p.b_per_image ? N : 1)};
         const uint64_t strides[2] = {ktot * es, (p.b_per_image ? static_cast<uint64_t>(w_image_stride) : ktot * n16) * es};
         const uint32_t box[3] = {BLOCK_K, (uint32_t)p.block_n, 1};
-        int rc = cab_make_tmap_bf16(&tmB, w_packed, 3, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+        int rc = cab_make_tmap_2b(&tmB, op_dtype, w_packed, 3, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
         if (rc) return rc;
     }
-    if (y_dtype == CABINET_BF16) {
+    if (y_dtype != CABINET_F32) {
         // store map: {Cout (true extent: clips padded / foreign channels), OW, OH, N}, 64-channel boxes
         const uint64_t dims[4] = {(uint64_t)Cout, (uint64_t)p.OW, (uint64_t)p.OH, (uint64_t)Ng};
         const uint64_t strides[3] = {(uint64_t)ldy * es * (uint64_t)y_sw, (uint64_t)ldy * es * (uint64_t)(y_sh ? y_sh : p.OW),
                                      (uint64_t)ldy * es * (uint64_t)(y_sn ? y_sn : (long long)p.OW * p.OH)};
         const uint32_t box[4] = {64, (uint32_t)p.TW, (uint32_t)p.TH, 1};
-        int rc = cab_make_tmap_bf16(&tmY, y, 4, dims, strides, box);
+        int rc = cab_make_tmap_2b(&tmY, op_dtype, y, 4, dims, strides, box);
         if (rc) return rc;
     } else {
         tmY = tmB;  // unused
@@ -718,17 +757,22 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
     static const int max_ctas = getenv("CAB_TC_MAX_CTAS") ? atoi(getenv("CAB_TC_MAX_CTAS")) : 0;
     const int grid = static_cast<int>(std::min<long long>(tiles, max_ctas > 0 ? std::min(max_ctas, sms) : sms));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-#define CAB_TC_LAUNCH(ACT_, RES_, F32_, PRO_)                                                                        \
+#define CAB_TC_LAUNCH_T(ACT_, RES_, F32_, PRO_, T_)                                                                  \
     do {                                                                                                             \
         static bool attr_done = false;                                                                               \
         if (!attr_done) {                                                                                            \
-            CAB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<ACT_, RES_, F32_, PRO_>,                                    \
+            CAB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<ACT_, RES_, F32_, PRO_, false, T_>,                         \
                                           cudaFuncAttributeMaxDynamicSharedMemorySize,                               \
                                           SMEM_LIMIT + 1024 - ((PRO_) ? 4096 : 0)));                                 \
             attr_done = true;                                                                                        \
         }                                                                                                            \
-        conv_tc_kernel<ACT_, RES_, F32_, PRO_><<<grid, (PRO_) ? NUM_THREADS + PRO_THREADS : NUM_THREADS, smem, st>>>( \
-            tmA[0], tmA[1], tmA[2], tmA[3], tmB, tmY, p);                                                            \
+        conv_tc_kernel<ACT_, RES_, F32_, PRO_, false, T_>                                                            \
+            <<<grid, (PRO_) ? NUM_THREADS + PRO_THREADS : NUM_THREADS, smem, st>>>(tmA[0], tmA[1], tmA[2], tmA[3], tmB, tmY, p); \
+    } while (0)
+#define CAB_TC_LAUNCH(ACT_, RES_, F32_, PRO_)                                                                        \
+    do {                                                                                                             \
+        if (op_dtype == CABINET_F16) CAB_TC_LAUNCH_T(ACT_, RES_, F32_, PRO_, f16);                                   \
+        else CAB_TC_LAUNCH_T(ACT_, RES_, F32_, PRO_, bf16);                                                          \
     } while (0)
 #define CAB_TC_LAUNCH_UP(ACT_)                                                                                       \
     do {                                                                                                             \
@@ -751,8 +795,8 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
         }
     } else if (a_scale) {
         CAB_REQUIRE(!f32 && act == CABINET_ACT_NONE, "conv_tc: the A-operand prologue is built for the linear project conv");
-        if (res) CAB_TC_LAUNCH(CABINET_ACT_NONE, true, false, true);
-        else CAB_TC_LAUNCH(CABINET_ACT_NONE, false, false, true);
+        if (res) CAB_TC_LAUNCH_T(CABINET_ACT_NONE, true, false, true, bf16);
+        else CAB_TC_LAUNCH_T(CABINET_ACT_NONE, false, false, true, bf16);
     } else if (f32 && !res && act == CABINET_ACT_NONE) CAB_TC_LAUNCH(CABINET_ACT_NONE, false, true, false);
     else if (!f32 && !res && act == CABINET_ACT_NONE) CAB_TC_LAUNCH(CABINET_ACT_NONE, false, false, false);
     else if (!f32 && !res && act == CABINET_ACT_RELU) CAB_TC_LAUNCH(CABINET_ACT_RELU, false, false, false);
@@ -764,6 +808,7 @@ static int conv_tc_impl(const void* x, long long ldx, int N, int H, int W, int C
         return CABINET_ERR_INVALID;
     }
 #undef CAB_TC_LAUNCH
+#undef CAB_TC_LAUNCH_T
 #undef CAB_TC_LAUNCH_UP
     CAB_LAUNCH_CHECK();
     return CABINET_OK;

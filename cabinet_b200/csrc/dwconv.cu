@@ -131,6 +131,7 @@ int launch(const void* x, long long ldx, const float* w, const float* bias, void
 extern "C" int cabinet_dwconv(const void* x, long long ldx, const float* w, const float* bias, void* y,
                               long long ldy, int dtype, int N, int H, int W, int C, int k, int stride, int OH, int OW,
                               int act, float* gap_sum, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("dwconv", dtype, CAB_DT_F32 | CAB_DT_BF16);
     CAB_REQUIRE(x && w && bias && y, "dwconv: null pointer");
     CAB_REQUIRE((k == 3 || k == 5) && (stride == 1 || stride == 2), "dwconv: k must be 3|5 and stride 1|2 (got %d,%d)",
                 k, stride);

@@ -1,4 +1,4 @@
-// Depthwise k x k convolution, bf16 NHWC, shared-memory halo staging by TMA.
+// Depthwise k x k convolution, bf16 (or fp16) NHWC, shared-memory halo staging by TMA.
 //
 // One CTA = one 8 x 16 output patch of one image for one chunk of <= 64 channels.  A single 4-D TMA box
 // {CB channels, (16-1)*S+K cols, (8-1)*S+K rows, 1} brings the input patch INCLUDING its halo into shared memory;
@@ -18,7 +18,7 @@ struct DwParams {
     int C, OH, OW, CB, act, reverse;  // reverse: blocks walk (tile, image) back to front (CABINET_CONV_REVERSE_TILES)
     const float* w;
     const float* bias;
-    bf16* y;
+    void* y;                 // the operand type T of the kernel (bf16 / f16)
     long long ldy;
     long long* gap_sum;      // [N][C] fixed-point (2^-24) pooling sums of the written values (SE consumers), or nullptr
 };
@@ -29,7 +29,7 @@ struct DwParams {
 // The thread keeps all K*K taps of its two channels in registers for its whole lifetime (loaded while the TMA is in
 // flight) and slides over its COLS output columns: ((COLS-1)*S + K) loads per filter row feed COLS*K*2 FMAs, no weight
 // traffic and no bounds checks in the loop.
-template <int K, int S, int COLS>
+template <int K, int S, int COLS, typename T>
 __device__ __forceinline__ void dw_row(const DwParams& p, const uint8_t* tile, uint64_t* bar, float* s_gap, int cw,
                                        int chunk, int n, int oh0, int ow0) {
     constexpr int IWT = (TW - 1) * S + K;
@@ -80,7 +80,7 @@ __device__ __forceinline__ void dw_row(const DwParams& p, const uint8_t* tile, u
             for (int sx = 0; sx < SPAN; ++sx) {
                 uint32_t raw;
                 asm volatile("ld.shared.u32 %0, [%1];" : "=r"(raw) : "r"(rowp + sx * pitch));
-                const float2 xv = make_float2(__uint_as_float(raw << 16), __uint_as_float(raw & 0xffff0000u));
+                const float2 xv = cab_unpack2<T>(raw);
 #pragma unroll
                 for (int r = 0; r < COLS; ++r) {
                     const int kx = sx - r * S;  // compile-time after unrolling
@@ -92,14 +92,13 @@ __device__ __forceinline__ void dw_row(const DwParams& p, const uint8_t* tile, u
         const int oh = oh0 + row;
         float g0 = 0.f, g1 = 0.f;
         if (oh < p.OH) {
-            bf16* yout = p.y + ((static_cast<long long>(n) * p.OH + oh) * p.OW + ow0 + col0) * p.ldy + c0;
+            T* yout = reinterpret_cast<T*>(p.y) + ((static_cast<long long>(n) * p.OH + oh) * p.OW + ow0 + col0) * p.ldy + c0;
 #pragma unroll
             for (int r = 0; r < COLS; ++r) {
                 if (ow0 + col0 + r < p.OW) {
                     g0 += acc[r].x;
                     g1 += acc[r].y;
-                    *reinterpret_cast<__nv_bfloat162*>(yout + static_cast<long long>(r) * p.ldy) =
-                        __floats2bfloat162_rn(acc[r].x, acc[r].y);
+                    *reinterpret_cast<uint32_t*>(yout + static_cast<long long>(r) * p.ldy) = cab_pack2<T>(acc[r].x, acc[r].y);
                 }
             }
         }
@@ -110,7 +109,7 @@ __device__ __forceinline__ void dw_row(const DwParams& p, const uint8_t* tile, u
     }
 }
 
-template <int K, int S>
+template <int K, int S, typename T>
 __global__ void __launch_bounds__(256, K > 3 ? 3 : 4)
 dwconv_tma_kernel(const __grid_constant__ CUtensorMap tmX, const DwParams p) {
     constexpr int PAD = (K - 1) / 2;
@@ -140,10 +139,10 @@ dwconv_tma_kernel(const __grid_constant__ CUtensorMap tmX, const DwParams p) {
 
     const int cw = min(p.CB, p.C - chunk * p.CB);  // channels of this chunk (multiple of 8)
     // columns per lane: as many column groups as fit into the 32 lanes (power of two)
-    if (cw > 32) dw_row<K, S, 16>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
-    else if (cw > 16) dw_row<K, S, 8>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
-    else if (cw > 8) dw_row<K, S, 4>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
-    else dw_row<K, S, 2>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
+    if (cw > 32) dw_row<K, S, 16, T>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
+    else if (cw > 16) dw_row<K, S, 8, T>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
+    else if (cw > 8) dw_row<K, S, 4, T>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
+    else dw_row<K, S, 2, T>(p, tile, &bar, s_gap, cw, chunk, n, oh0, ow0);
 
     if (p.gap_sum) {
         // Deterministic pooling sums: fixed-order fp32 sum over the rows / column groups of this CTA, then ONE 64-bit
@@ -235,7 +234,7 @@ mbconv1_fused_kernel(const __grid_constant__ CUtensorMap tmX, const Mb1Params p)
                 for (int kx = 0; kx < K; ++kx) {
                     uint32_t raw;
                     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(raw) : "r"(base + (sy * IWT + kx) * PITCH));
-                    const float2 xv = make_float2(__uint_as_float(raw << 16), __uint_as_float(raw & 0xffff0000u));
+                    const float2 xv = cab_unpack2<bf16>(raw);
 #pragma unroll
                     for (int r = 0; r < ROWS; ++r) {
                         const int ky = sy - r;
@@ -315,8 +314,9 @@ mbconv1_fused_kernel(const __grid_constant__ CUtensorMap tmX, const Mb1Params p)
                 for (int nt = 0; nt < NT; ++nt) {
                     uint32_t raw;  // residual: the block input at the same pixel (centre of the staged patch)
                     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(raw) : "r"(res + nt * 16));
-                    const float o0 = acc[nt][2 * hh] + __uint_as_float(raw << 16);
-                    const float o1 = acc[nt][2 * hh + 1] + __uint_as_float(raw & 0xffff0000u);
+                    const float2 rv = cab_unpack2<bf16>(raw);
+                    const float o0 = acc[nt][2 * hh] + rv.x;
+                    const float o1 = acc[nt][2 * hh + 1] + rv.y;
                     *reinterpret_cast<__nv_bfloat162*>(yp + nt * 8) = __floats2bfloat162_rn(o0, o1);
                 }
             }
@@ -351,26 +351,27 @@ mbconv1_fused_kernel(const __grid_constant__ CUtensorMap tmX, const Mb1Params p)
             asm volatile("ld.shared.u32 %0, [%1];"
                          : "=r"(raw)
                          : "r"(tc::smem_u32(tile) + ((row + PAD) * IWT + col + PAD) * PITCH + co * 2));
-            o0 += __uint_as_float(raw << 16);
-            o1 += __uint_as_float(raw & 0xffff0000u);
+            const float2 rv = cab_unpack2<bf16>(raw);
+            o0 += rv.x;
+            o1 += rv.y;
             *reinterpret_cast<__nv_bfloat162*>(p.y + ((static_cast<long long>(n) * p.OH + oh) * p.OW + ow) * p.ldy + co) =
                 __floats2bfloat162_rn(o0, o1);
         }
     }
 }
 
-template <int K, int S>
+template <int K, int S, typename T>
 int launch(const CUtensorMap& tm, const DwParams& p, int N, int n_chunks, cudaStream_t s) {
     constexpr int IWT = (TW - 1) * S + K, IHT = (TH - 1) * S + K;
     const size_t smem = static_cast<size_t>(IWT) * IHT * 128 + 128;
     static bool attr_set = false;
     if (!attr_set) {
-        CAB_CUDA(cudaFuncSetAttribute(dwconv_tma_kernel<K, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+        CAB_CUDA(cudaFuncSetAttribute(dwconv_tma_kernel<K, S, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         attr_set = true;
     }
     const int tiles = ((p.OW + TW - 1) / TW) * ((p.OH + TH - 1) / TH);
     dim3 grid(tiles, n_chunks, N);
-    dwconv_tma_kernel<K, S><<<grid, 32 * TH, smem, s>>>(tm, p);
+    dwconv_tma_kernel<K, S, T><<<grid, 32 * TH, smem, s>>>(tm, p);
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -418,6 +419,13 @@ extern "C" int cabinet_mbconv_noexpand_fused(const void* x, long long ldx, const
 extern "C" int cabinet_dwconv_tma(const void* x, long long ldx, const float* w, const float* bias, void* y,
                                   long long ldy, int N, int H, int W, int C, int k, int stride, int OH, int OW, int act,
                                   long long* gap_sum, cabinet_stream_t stream) {
+    return cabinet_dwconv_tma_dt(x, ldx, w, bias, y, ldy, N, H, W, C, k, stride, OH, OW, act, gap_sum, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_dwconv_tma_dt(const void* x, long long ldx, const float* w, const float* bias, void* y,
+                                     long long ldy, int N, int H, int W, int C, int k, int stride, int OH, int OW, int act,
+                                     long long* gap_sum, int op_dtype, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("dwconv_tma", op_dtype, CAB_DT_BF16 | CAB_DT_F16);
     CAB_REQUIRE(x && w && bias && y, "dwconv_tma: null pointer");
     const int reverse = (act & CABINET_CONV_REVERSE_TILES) ? 1 : 0;
     act &= ~CABINET_CONV_REVERSE_TILES;
@@ -437,18 +445,20 @@ extern "C" int cabinet_dwconv_tma(const void* x, long long ldx, const float* w, 
     // tail would pack 8 column groups into a warp whose rows sit a multiple of 128 B apart: an 8-way bank conflict
     // that makes the tail cost more than a full chunk.  The TMA box stays 64 channels wide.
     p.CB = ((C + n_chunks - 1) / n_chunks + 7) / 8 * 8;
-    p.y = reinterpret_cast<bf16*>(y); p.ldy = ldy; p.gap_sum = gap_sum;
+    p.y = y; p.ldy = ldy; p.gap_sum = gap_sum;
     const int IWT = (TW - 1) * stride + k, IHT = (TH - 1) * stride + k;
     CUtensorMap tm;
     const uint64_t dims[4] = {(uint64_t)C, (uint64_t)W, (uint64_t)H, (uint64_t)N};
     const uint64_t strides[3] = {(uint64_t)ldx * 2, (uint64_t)ldx * 2 * W, (uint64_t)ldx * 2 * W * H};
     const uint32_t box[4] = {64, (uint32_t)IWT, (uint32_t)IHT, 1};
-    int rc = cab_make_tmap_bf16(&tm, x, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_SWIZZLE_NONE);
+    int rc = cab_make_tmap_2b(&tm, op_dtype, x, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                              CU_TENSOR_MAP_SWIZZLE_NONE);
     if (rc) return rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (k == 3 && stride == 1) return launch<3, 1>(tm, p, N, n_chunks, s);
-    if (k == 3 && stride == 2) return launch<3, 2>(tm, p, N, n_chunks, s);
-    if (k == 5 && stride == 1) return launch<5, 1>(tm, p, N, n_chunks, s);
-    return launch<5, 2>(tm, p, N, n_chunks, s);
+    CAB_DISPATCH_DT_HALF(op_dtype, T,
+                         if (k == 3 && stride == 1) return launch<3, 1, T>(tm, p, N, n_chunks, s);
+                         if (k == 3 && stride == 2) return launch<3, 2, T>(tm, p, N, n_chunks, s);
+                         if (k == 5 && stride == 1) return launch<5, 1, T>(tm, p, N, n_chunks, s);
+                         return launch<5, 2, T>(tm, p, N, n_chunks, s));
+    return CABINET_OK;
 }

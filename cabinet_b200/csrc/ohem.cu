@@ -407,6 +407,7 @@ extern "C" int cabinet_ohem_ce_forward(const void* logits, int dtype, const void
                                        long long HW, const float* weight, int ignore_label, float thresh,
                                        long long n_min, float* loss_px, void* workspace, float* loss_out,
                                        cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("ohem_ce_forward", dtype, CAB_DT_F32 | CAB_DT_BF16);
     CAB_REQUIRE(logits && labels && loss_px && workspace && loss_out && C > 0 && HW > 0 && N >= 0 && N <= 65535 &&
                     n_min >= 1,
                 "ohem_ce_forward: bad arguments");
@@ -441,6 +442,7 @@ extern "C" int cabinet_ohem_ce_forward(const void* logits, int dtype, const void
 extern "C" int cabinet_ohem_ce_backward(const void* logits, int dtype, const void* labels, int label_dtype, int N, int C,
                                         long long HW, const float* weight, const float* loss_px, const void* workspace,
                                         const float* grad_out, void* grad_logits, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("ohem_ce_backward", dtype, CAB_DT_F32 | CAB_DT_BF16);
     CAB_REQUIRE(logits && labels && loss_px && workspace && grad_out && grad_logits && C > 0 && HW > 0 && N >= 0 &&
                     N <= 65535,
                 "ohem_ce_backward: bad arguments");

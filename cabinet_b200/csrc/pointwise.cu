@@ -282,6 +282,7 @@ channel_sum_kernel(const T* __restrict__ x, long long ldx, long long HW, int C, 
 
 extern "C" int cabinet_channel_sum(const void* x, long long ldx, int dtype, int N, long long HW, int C, float* out,
                                    float* scratch, long long scratch_bytes, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("channel_sum", dtype, CAB_DT_ALL);
     CAB_REQUIRE(x && out && scratch, "channel_sum: null pointer");
     const int V = dtype == CABINET_F32 ? 4 : 8;
     CAB_REQUIRE(C > 0 && C % V == 0 && ldx % V == 0 && ldx >= C && C / V <= 256 && N <= 65535 && HW * ldx < (1LL << 31),
@@ -302,12 +303,9 @@ extern "C" int cabinet_channel_sum(const void* x, long long ldx, int dtype, int 
     float* partial = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(scratch) + off);
     dim3 grid(nb, N);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (dtype == CABINET_BF16)
-        channel_sum_kernel<bf16><<<grid, 256, smem, s>>>(reinterpret_cast<const bf16*>(x), ldx, HW, C, out, pix_per_block,
-                                                         partial, tickets);
-    else
-        channel_sum_kernel<float><<<grid, 256, smem, s>>>(reinterpret_cast<const float*>(x), ldx, HW, C, out,
-                                                          pix_per_block, partial, tickets);
+    CAB_DISPATCH_DT(dtype, T,
+                    channel_sum_kernel<T><<<grid, 256, smem, s>>>(reinterpret_cast<const T*>(x), ldx, HW, C, out, pix_per_block,
+                                                                  partial, tickets));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -340,6 +338,7 @@ extern "C" int cabinet_gate_fc(const float* in, float in_scale, const float* W, 
 
 extern "C" int cabinet_scale_act(void* x, long long ldx, int dtype, const float* scale, int N, long long HW, int C,
                                  int act, int plus_one, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("scale_act", dtype, CAB_DT_F32 | CAB_DT_BF16);
     CAB_REQUIRE(x && scale, "scale_act: null pointer");
     const int V = dtype == CABINET_F32 ? 4 : 8;
     CAB_REQUIRE(C > 0 && C % V == 0 && ldx % V == 0 && ldx >= C && C / V <= 256 && HW < (1LL << 31) && N <= 65535,
@@ -501,6 +500,7 @@ extern "C" int cabinet_scale_weights(const void* w_packed, const float* scale, v
 
 extern "C" int cabinet_softmax_rows(const float* s, void* p, int p_dtype, long long rows, int cols,
                                     cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("softmax_rows", p_dtype, CAB_DT_F32 | CAB_DT_BF16);
     CAB_REQUIRE(s && p && cols > 0, "softmax_rows: bad arguments");
     if (rows == 0) return CABINET_OK;
     dim3 grid(static_cast<unsigned>(cab_ceil_div(rows, 8)));
@@ -516,6 +516,7 @@ extern "C" int cabinet_softmax_rows(const float* s, void* p, int p_dtype, long l
 extern "C" int cabinet_cab_combine(const void* g, const void* x, const void* r, void* out, long long ldo,
                                    const float* gamma, int dtype, long long n_pixels, int C,
                                    cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("cab_combine", dtype, CAB_DT_ALL);
     CAB_REQUIRE(g && x && r && out && gamma, "cab_combine: null pointer");
     const int V = dtype == CABINET_F32 ? 4 : 8;
     CAB_REQUIRE(C > 0 && C % V == 0 && ldo % V == 0 && ldo >= C, "cab_combine: C/ldo must be multiples of %d", V);
@@ -524,15 +525,10 @@ extern "C" int cabinet_cab_combine(const void* g, const void* x, const void* r, 
     const long long nvec = n_pixels * CG;
     dim3 grid(static_cast<unsigned>(std::min<long long>(cab_ceil_div(nvec, 256), 148 * 16)));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (dtype == CABINET_BF16)
-        cab_combine_kernel<bf16><<<grid, 256, 0, s>>>(reinterpret_cast<const bf16*>(g), reinterpret_cast<const bf16*>(x),
-                                                     reinterpret_cast<const bf16*>(r), reinterpret_cast<bf16*>(out),
-                                                     ldo, CG, gamma, nvec);
-    else
-        cab_combine_kernel<float><<<grid, 256, 0, s>>>(reinterpret_cast<const float*>(g),
-                                                      reinterpret_cast<const float*>(x),
-                                                      reinterpret_cast<const float*>(r), reinterpret_cast<float*>(out),
-                                                      ldo, CG, gamma, nvec);
+    CAB_DISPATCH_DT(dtype, T,
+                    cab_combine_kernel<T><<<grid, 256, 0, s>>>(reinterpret_cast<const T*>(g), reinterpret_cast<const T*>(x),
+                                                               reinterpret_cast<const T*>(r), reinterpret_cast<T*>(out), ldo, CG,
+                                                               gamma, nvec));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }

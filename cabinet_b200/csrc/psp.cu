@@ -171,6 +171,7 @@ psp_concat_kernel(const T* __restrict__ x, long long ldx, const float* __restric
 
 extern "C" int cabinet_psp_pool(const void* x, long long ldx, int dtype, float* pooled, int N, int H, int W, int C,
                                 float* scratch, long long scratch_bytes, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("psp_pool", dtype, CAB_DT_F32 | CAB_DT_BF16);
     const int vpt = dtype == CABINET_BF16 ? 8 : 4;
     CAB_REQUIRE(x && pooled && H > 0 && W > 0 && C > 0 && ldx >= C && C % vpt == 0 && C <= 1024 && ldx % vpt == 0 &&
                     (reinterpret_cast<uintptr_t>(x) & 15) == 0,
@@ -218,6 +219,7 @@ extern "C" int cabinet_psp_pool(const void* x, long long ldx, int dtype, float* 
 
 extern "C" int cabinet_psp_concat(const void* x, long long ldx, const float* pooled, void* out, long long ldo,
                                   int dtype, int N, int H, int W, int C, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("psp_concat", dtype, CAB_DT_F32 | CAB_DT_BF16);
     const int vpt = dtype == CABINET_BF16 ? 8 : 4;
     CAB_REQUIRE(x && pooled && out && H > 0 && W > 0 && C > 0 && ldx >= C && ldo >= 5LL * C, "psp_concat: bad arguments");
     CAB_REQUIRE(C % vpt == 0 && ldx % vpt == 0 && ldo % vpt == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&

@@ -712,6 +712,8 @@ extern "C" int cabinet_normalize_u8(const uint8_t* x, float* y, int N, int H, in
 
 extern "C" int cabinet_bilinear_nhwc(const void* x, long long ldx, int x_dtype, void* y, long long ldy, int y_dtype,
                                      int N, int IH, int IW, int C, int OH, int OW, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("bilinear_nhwc", x_dtype, CAB_DT_F32 | CAB_DT_BF16);
+    CAB_REQUIRE_DTYPE("bilinear_nhwc", y_dtype, CAB_DT_F32 | CAB_DT_BF16);
     CAB_REQUIRE(x && y && IH > 0 && IW > 0 && OH > 0 && OW > 0 && C > 0 && ldx >= C && ldy >= C,
                 "bilinear_nhwc: bad arguments");
     if (N == 0) return CABINET_OK;
@@ -749,6 +751,7 @@ extern "C" int cabinet_bilinear_nhwc(const void* x, long long ldx, int x_dtype, 
 
 extern "C" int cabinet_upsample_logits_nchw(const float* x, int N, int IH, int IW, int C, void* y, int y_dtype, int OH,
                                             int OW, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("upsample_logits_nchw", y_dtype, CAB_DT_F32 | CAB_DT_BF16);
     CAB_REQUIRE(x && y && IH > 0 && IW > 0 && OH > 0 && OW > 0 && C > 0, "upsample_logits_nchw: bad arguments");
     CAB_REQUIRE(OH <= 65535 && N <= 65535, "upsample_logits_nchw: OH/N exceed grid limits");
     if (N == 0) return CABINET_OK;

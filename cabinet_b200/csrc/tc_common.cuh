@@ -126,6 +126,14 @@ __host__ __device__ __forceinline__ uint32_t make_idesc_bf16(int M, int N) {
     return (1u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(N >> 3) << 17) |
            (static_cast<uint32_t>(M >> 4) << 24);
 }
+// The same with fp16 operands: A/B format 0 = f16 (fp32 accumulation either way).
+__host__ __device__ __forceinline__ uint32_t make_idesc_f16(int M, int N) {
+    return (1u << 4) | (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
+}
+// Instruction descriptor for operand type T (bf16 or f16)
+template <typename T> __host__ __device__ __forceinline__ uint32_t make_idesc(int M, int N);
+template <> __host__ __device__ __forceinline__ uint32_t make_idesc<bf16>(int M, int N) { return make_idesc_bf16(M, N); }
+template <> __host__ __device__ __forceinline__ uint32_t make_idesc<f16>(int M, int N) { return make_idesc_f16(M, N); }
 
 }  // namespace tc
 
@@ -137,11 +145,18 @@ typedef CUresult (*cab_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuin
                                         CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 cab_encode_tiled_fn cab_get_encode_tiled();
 
-// bf16 tensor map, rank <= 5, 128B swizzle, zero OOB fill.  dims/strides innermost first; strides in BYTES for
-// dims 1..rank-1 (dim 0 is contiguous).
-int cab_make_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                       const uint32_t* box, CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                       CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B);
+// Tensor map of 2-byte elements (elem_dtype CABINET_BF16 or CABINET_F16), rank <= 5, 128B swizzle, zero OOB fill.
+// dims/strides innermost first; strides in BYTES for dims 1..rank-1 (dim 0 is contiguous).
+int cab_make_tmap_2b(CUtensorMap* map, int elem_dtype, const void* base, int rank, const uint64_t* dims,
+                     const uint64_t* strides_bytes, const uint32_t* box,
+                     CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B);
+static inline int cab_make_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
+                                     const uint64_t* strides_bytes, const uint32_t* box,
+                                     CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                                     CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
+    return cab_make_tmap_2b(map, CABINET_BF16, base, rank, dims, strides_bytes, box, promo, swizzle);
+}
 
 namespace tc {
 // ----------------------------------------------------------------------------- TMA stores (smem -> global, bulk group)

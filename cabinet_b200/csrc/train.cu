@@ -7,7 +7,7 @@
 //   * squeeze-excite / FFM gate backward, CAB combine backward, softmax backward, the adjoints of every bilinear
 //     resize / adaptive average pool as ONE separable sparse resampling kernel, small helpers.
 // All reductions have a fixed summation order (no floating-point atomics): a training step is bit-reproducible.
-// Activations are NHWC (fp32 or bf16), statistics / gradients of parameters fp32.
+// Activations are NHWC (fp32, bf16 or fp16), statistics / gradients of parameters fp32.
 #include <type_traits>
 
 #include "tc_common.cuh"
@@ -242,12 +242,12 @@ __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_
                  : "memory");
 }
 
-// f(row0, row1, acc): row0 / row1 = this thread's 8 channels of one row of source 0 / 1 as fp32
-template <int NQ, int NSRC, typename F>
-__device__ __forceinline__ void col_reduce_tma(const bf16* __restrict__ src0, const bf16* __restrict__ src1, long long M, int C,
+// f(row0, row1, acc): row0 / row1 = this thread's 8 channels of one row of source 0 / 1 as fp32 (T = bf16 or f16)
+template <int NQ, int NSRC, typename T, typename F>
+__device__ __forceinline__ void col_reduce_tma(const T* __restrict__ src0, const T* __restrict__ src1, long long M, int C,
                                                long long rows_per_block, int chunk_rows, float* __restrict__ partial, F f) {
     constexpr int V = 8;
-    extern __shared__ __align__(128) uint8_t s_ring[];  // [RT_STAGES][NSRC][chunk_rows * C] bf16; reused for the block sum
+    extern __shared__ __align__(128) uint8_t s_ring[];  // [RT_STAGES][NSRC][chunk_rows * C] T; reused for the block sum
     __shared__ __align__(8) uint64_t full_bar[RT_STAGES], empty_bar[RT_STAGES];
     const int warp = threadIdx.x >> 5;
     const long long m0 = static_cast<long long>(blockIdx.x) * rows_per_block;
@@ -287,8 +287,8 @@ __device__ __forceinline__ void col_reduce_tma(const bf16* __restrict__ src0, co
             const int st = i % RT_STAGES;
             tc::mbar_wait(&full_bar[st], (i / RT_STAGES) & 1);
             const int rows = static_cast<int>(min(static_cast<long long>(chunk_rows), m1 - (m0 + static_cast<long long>(i) * chunk_rows)));
-            const bf16* c0 = reinterpret_cast<const bf16*>(s_ring + static_cast<size_t>(st) * NSRC * src_bytes) + cv * V;
-            const bf16* c1 = reinterpret_cast<const bf16*>(s_ring + static_cast<size_t>(st) * NSRC * src_bytes + src_bytes) + cv * V;
+            const T* c0 = reinterpret_cast<const T*>(s_ring + static_cast<size_t>(st) * NSRC * src_bytes) + cv * V;
+            const T* c1 = reinterpret_cast<const T*>(s_ring + static_cast<size_t>(st) * NSRC * src_bytes + src_bytes) + cv * V;
             if (lane < lanes) {
                 for (int r = lane; r < rows; r += lanes) {
                     float a[V], b[V];
@@ -319,11 +319,12 @@ __device__ __forceinline__ void col_reduce_tma(const bf16* __restrict__ src0, co
     }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(RT_THREADS)
-bn_stats_tma_kernel(const bf16* __restrict__ x, long long M, int C, long long rpb, int chunk_rows, float* __restrict__ partial) {
+bn_stats_tma_kernel(const T* __restrict__ x, long long M, int C, long long rpb, int chunk_rows, float* __restrict__ partial) {
     float kv[8];  // the shift (row 0) of this thread's channel vector
     ldv(x + (threadIdx.x % (C / 8)) * 8, kv);
-    col_reduce_tma<2, 1>(x, nullptr, M, C, rpb, chunk_rows, partial, [&](const float* xv, const float*, float* acc) {
+    col_reduce_tma<2, 1, T>(x, nullptr, M, C, rpb, chunk_rows, partial, [&](const float* xv, const float*, float* acc) {
 #pragma unroll
         for (int v = 0; v < 8; ++v) {
             const float d = xv[v] - kv[v];
@@ -333,8 +334,9 @@ bn_stats_tma_kernel(const bf16* __restrict__ x, long long M, int C, long long rp
     });
 }
 
+template <typename T>
 __global__ void __launch_bounds__(RT_THREADS)
-bn_bwd_reduce_tma_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ z, const float* __restrict__ stats, int act,
+bn_bwd_reduce_tma_kernel(const T* __restrict__ dy, const T* __restrict__ z, const float* __restrict__ stats, int act,
                          long long M, int C, long long rpb, int chunk_rows, float* __restrict__ partial) {
     float mean[8], invstd[8], scale[8], shift[8];
     const int c0 = (threadIdx.x % (C / 8)) * 8;
@@ -342,7 +344,7 @@ bn_bwd_reduce_tma_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ z
     for (int v = 0; v < 8; ++v) {
         mean[v] = stats[c0 + v]; invstd[v] = stats[C + c0 + v]; scale[v] = stats[2 * C + c0 + v]; shift[v] = stats[3 * C + c0 + v];
     }
-    col_reduce_tma<2, 2>(dy, z, M, C, rpb, chunk_rows, partial, [&](const float* dv, const float* zv, float* acc) {
+    col_reduce_tma<2, 2, T>(dy, z, M, C, rpb, chunk_rows, partial, [&](const float* dv, const float* zv, float* acc) {
         float u[8], ag[8];
 #pragma unroll
         for (int v = 0; v < 8; ++v) u[v] = fmaf(zv[v], scale[v], shift[v]);
@@ -732,9 +734,10 @@ __global__ void pack_conv_weight_kernel(const float* __restrict__ w, int Cout, i
 // Sub-filter of one input-parity class (py, px) of a stride-2 convolution's data gradient, transposed for cabinet_conv_tc:
 //   dx[2a+py][2b+px][ci] = sum_{jy, jx, co} dy[a - pad2 + jy][b - pad2 + jx][co] * w[co][ci][ky(jy)][kx(jx)],
 //   ky(j) = py + pad - 2 (j - pad2)   (taps outside [0, K) are zero)
-// out [rows_pad >= Cin][KH2 * KW2][k_pad >= Cout] bf16, zero padded.
+// out [rows_pad >= Cin][KH2 * KW2][k_pad >= Cout] bf16 / fp16, zero padded.
+template <typename T>
 __global__ void pack_conv_weight_parity_kernel(const float* __restrict__ w, int Cout, int Cin, int K, int pad, int py, int px,
-                                               int KH2, int KW2, int pad2, int rows_pad, int k_pad, bf16* __restrict__ out) {
+                                               int KH2, int KW2, int pad2, int rows_pad, int k_pad, T* __restrict__ out) {
     const long long total = static_cast<long long>(rows_pad) * KH2 * KW2 * k_pad;
     for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
          i += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -745,7 +748,7 @@ __global__ void pack_conv_weight_parity_kernel(const float* __restrict__ w, int 
         const int ky = py + pad - 2 * (jy - pad2), kx = px + pad - 2 * (jx - pad2);
         float v = 0.f;
         if (co < Cout && ci < Cin && ky >= 0 && ky < K && kx >= 0 && kx < K) v = w[((static_cast<long long>(co) * Cin + ci) * K + ky) * K + kx];
-        out[i] = __float2bfloat16_rn(v);
+        out[i] = from_f32<T>(v);
     }
 }
 
@@ -758,12 +761,13 @@ __global__ void pack_dw_weight_kernel(const float* __restrict__ w, int C, int ta
 
 // ---------------------------------------------------------------------------------------------------------------
 // im2col of the fp32 NCHW network input for the two stem convolutions (7x7 s2 p3 and, embedded in its centre, 3x3 s2 p1):
-// out[n*OH*OW + oy*OW + ox][ci*K*K + ky*K + kx] = bf16(x[n][ci][oy*S - P + ky][ox*S - P + kx]) (0 outside the image and in
+// out[n*OH*OW + oy*OW + ox][ci*K*K + ky*K + kx] = T(x[n][ci][oy*S - P + ky][ox*S - P + kx]) (0 outside the image and in
 // the padding columns >= Cin*K*K).  The column order is the OIHW flattening of the filter, so the stem convolutions and
 // their weight gradients become plain 1x1 GEMMs on the tensor cores with the parameter / gradient tensors used in place.
+template <typename T>
 __global__ void __launch_bounds__(256)
 im2col_nchw_kernel(const float* __restrict__ x, int N, int Cin, int H, int W, int K, int S, int P, int OH, int OW,
-                   bf16* __restrict__ out, int ld) {
+                   T* __restrict__ out, int ld) {
     // one thread = one output pixel x one 16-byte chunk (8 columns): consecutive threads write consecutive chunks of a row
     const unsigned chunks = ld / 8, cols = Cin * K * K, KK = K * K;
     const long long total = static_cast<long long>(N) * OH * OW * chunks;
@@ -786,7 +790,7 @@ im2col_nchw_kernel(const float* __restrict__ x, int N, int Cin, int H, int W, in
                 if (iy >= 0 && iy < H && ix >= 0 && ix < W) v[j] = __ldg(x + ((static_cast<long long>(n) * Cin + ci) * H + iy) * W + ix);
             }
         }
-        Vec16<bf16> o;
+        Vec16<T> o;
         o.pack(v);
         o.store(out + static_cast<long long>(pix) * ld + ch * 8);
     }
@@ -798,9 +802,10 @@ im2col_nchw_kernel(const float* __restrict__ x, int N, int Cin, int H, int W, in
 // global memory once per block instead of once per (pixel, tap) (the per-element kernel above ran at 0.7 TB/s of its
 // output bytes: 0.94 ms for the 1024 x 1024 stem of batch 8).
 constexpr int IM2COL_PX = 64;
+template <typename T>
 __global__ void __launch_bounds__(256)
 im2col_nchw_row_kernel(const float* __restrict__ x, int Cin, int H, int W, int K, int S, int P, int OH, int OW,
-                       bf16* __restrict__ out, int ld, int segs) {
+                       T* __restrict__ out, int ld, int segs) {
     extern __shared__ float s_win[];  // [Cin * K][winw] | int table[ld]
     const int winw = IM2COL_PX * S + K - S, rows = Cin * K, cols = Cin * K * K;
     int* s_tab = reinterpret_cast<int*>(s_win + rows * winw);
@@ -821,7 +826,7 @@ im2col_nchw_row_kernel(const float* __restrict__ x, int Cin, int H, int W, int K
     }
     __syncthreads();
     const int chunks = ld / 8;
-    bf16* orow = out + ((static_cast<long long>(n) * OH + oy) * OW + ox0) * ld;
+    T* orow = out + ((static_cast<long long>(n) * OH + oy) * OW + ox0) * ld;
     for (int i = threadIdx.x; i < npx * chunks; i += 256) {
         const int px = i / chunks, ch = i - px * chunks;
         float v[8];
@@ -830,7 +835,7 @@ im2col_nchw_row_kernel(const float* __restrict__ x, int Cin, int H, int W, int K
             const int o = s_tab[ch * 8 + j];
             v[j] = o >= 0 ? s_win[o + px * S] : 0.f;
         }
-        Vec16<bf16> o;
+        Vec16<T> o;
         o.pack(v);
         o.store(orow + static_cast<long long>(px) * ld + ch * 8);
     }
@@ -1263,10 +1268,8 @@ dw_wgrad_kernel(const T* __restrict__ dy, long long lddy, const T* __restrict__ 
 // channel-pair variant (4-byte bf16x2 / 8-byte float2 accesses: a warp reads 128 / 256 contiguous bytes per tap)
 template <typename T> __device__ __forceinline__ float2 ld2(const T* p);
 template <> __device__ __forceinline__ float2 ld2<float>(const float* p) { return *reinterpret_cast<const float2*>(p); }
-template <> __device__ __forceinline__ float2 ld2<bf16>(const bf16* p) {
-    const uint32_t r = *reinterpret_cast<const uint32_t*>(p);
-    return make_float2(__uint_as_float(r << 16), __uint_as_float(r & 0xffff0000u));
-}
+template <> __device__ __forceinline__ float2 ld2<bf16>(const bf16* p) { return cab_unpack2<bf16>(*reinterpret_cast<const uint32_t*>(p)); }
+template <> __device__ __forceinline__ float2 ld2<f16>(const f16* p) { return cab_unpack2<f16>(*reinterpret_cast<const uint32_t*>(p)); }
 
 template <typename T, int KK>
 __global__ void __launch_bounds__(RED_THREADS)
@@ -1369,12 +1372,14 @@ template <> struct Raw2<float> {
     static __device__ __forceinline__ float2 load(const float* p) { return *reinterpret_cast<const float2*>(p); }
     static __device__ __forceinline__ float2 cvt(float2 r) { return r; }
 };
-template <> struct Raw2<bf16> {
+template <typename T> struct Raw2Half {  // T = bf16 or f16: two packed elements in one 32-bit word
     typedef uint32_t type;
     static __device__ __forceinline__ uint32_t zero() { return 0u; }
-    static __device__ __forceinline__ uint32_t load(const bf16* p) { return *reinterpret_cast<const uint32_t*>(p); }
-    static __device__ __forceinline__ float2 cvt(uint32_t r) { return make_float2(__uint_as_float(r << 16), __uint_as_float(r & 0xffff0000u)); }
+    static __device__ __forceinline__ uint32_t load(const T* p) { return *reinterpret_cast<const uint32_t*>(p); }
+    static __device__ __forceinline__ float2 cvt(uint32_t r) { return cab_unpack2<T>(r); }
 };
+template <> struct Raw2<bf16> : Raw2Half<bf16> {};
+template <> struct Raw2<f16> : Raw2Half<f16> {};
 
 constexpr int DWR_SL = 2;  // segment lanes (warps per filter row) of a block
 
@@ -1658,11 +1663,12 @@ softmax_bwd_kernel(const float* __restrict__ p, const float* __restrict__ dp, fl
     for (int c = lane; c < cols; c += 32) out[c] = pr[c] * (dr[c] - dot) * alpha;
 }
 
-// Attention on the tensor cores (training, bf16 mode): the GEMMs run as cabinet_conv_tc_imgw / cabinet_conv_wgrad_tc calls
-// on bf16 operands; these three passes sit between them.
-// p = softmax(scale * s) over rows, written as fp32 (kept for the backward) AND as bf16 (the operand of P V and P^T dO)
+// Attention on the tensor cores (training, bf16 / fp16 mode): the GEMMs run as cabinet_conv_tc_imgw / cabinet_conv_wgrad_tc
+// calls on 2-byte operands (T); these three passes sit between them.
+// p = softmax(scale * s) over rows, written as fp32 (kept for the backward) AND as T (the operand of P V and P^T dO)
+template <typename T>
 __global__ void __launch_bounds__(256)
-attn_softmax_kernel(const float* __restrict__ s, float scale, float* __restrict__ p, bf16* __restrict__ p16, long long rows,
+attn_softmax_kernel(const float* __restrict__ s, float scale, float* __restrict__ p, T* __restrict__ p16, long long rows,
                     int cols) {
     const long long row = static_cast<long long>(blockIdx.x) * (blockDim.x / 32) + threadIdx.x / 32;
     const int lane = threadIdx.x % 32;
@@ -1680,13 +1686,14 @@ attn_softmax_kernel(const float* __restrict__ s, float scale, float* __restrict_
     for (int c = lane; c < cols; c += 32) {
         const float v = expf(in[c] * scale - m) * inv;
         p[row * cols + c] = v;
-        p16[row * cols + c] = __float2bfloat16_rn(v);
+        p16[row * cols + c] = from_f32<T>(v);
     }
 }
 
-// ds = p * (dp - sum_j dp_j p_j) * alpha as bf16 (the operand of dS K and dS^T Q)
+// ds = p * (dp - sum_j dp_j p_j) * alpha as T (the operand of dS K and dS^T Q)
+template <typename T>
 __global__ void __launch_bounds__(256)
-attn_softmax_bwd_kernel(const float* __restrict__ p, const float* __restrict__ dp, bf16* __restrict__ ds, long long rows,
+attn_softmax_bwd_kernel(const float* __restrict__ p, const float* __restrict__ dp, T* __restrict__ ds, long long rows,
                         int cols, float alpha) {
     const long long row = static_cast<long long>(blockIdx.x) * (blockDim.x / 32) + threadIdx.x / 32;
     const int lane = threadIdx.x % 32;
@@ -1697,21 +1704,22 @@ attn_softmax_bwd_kernel(const float* __restrict__ p, const float* __restrict__ d
     for (int c = lane; c < cols; c += 32) dot = fmaf(pr[c], dr[c], dot);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
-    for (int c = lane; c < cols; c += 32) ds[row * cols + c] = __float2bfloat16_rn(pr[c] * (dr[c] - dot) * alpha);
+    for (int c = lane; c < cols; c += 32) ds[row * cols + c] = from_f32<T>(pr[c] * (dr[c] - dot) * alpha);
 }
 
-// out[n][c][l] = x[n][l][c] (bf16): per-image K^T / V^T as cabinet_conv_tc weight matrices ([rows = channels][k = tokens])
+// out[n][c][l] = x[n][l][c] (2-byte T): per-image K^T / V^T as cabinet_conv_tc weight matrices ([rows = channels][k = tokens])
+template <typename T>
 __global__ void __launch_bounds__(256)
-transpose_tokens_kernel(const bf16* __restrict__ x, long long ldx, bf16* __restrict__ out, int L, int C) {
-    __shared__ bf16 tile[32][34];
+transpose_tokens_kernel(const T* __restrict__ x, long long ldx, T* __restrict__ out, int L, int C) {
+    __shared__ T tile[32][34];
     const int n = blockIdx.z, l0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
-    const bf16* xin = x + static_cast<long long>(n) * L * ldx;
+    const T* xin = x + static_cast<long long>(n) * L * ldx;
 #pragma unroll
     for (int r = ty; r < 32; r += 8)
         if (l0 + r < L && c0 + tx < C) tile[r][tx] = xin[static_cast<long long>(l0 + r) * ldx + c0 + tx];
     __syncthreads();
-    bf16* o = out + static_cast<long long>(n) * C * L;
+    T* o = out + static_cast<long long>(n) * C * L;
 #pragma unroll
     for (int r = ty; r < 32; r += 8)
         if (c0 + r < C && l0 + tx < L) o[static_cast<long long>(c0 + r) * L + l0 + tx] = tile[tx][r];
@@ -1848,37 +1856,38 @@ inline unsigned ew_grid(long long total) { return static_cast<unsigned>(std::min
 
 }  // namespace
 
-#define CAB_DT2(dt, CALL_F, CALL_B)          \
-    do {                                     \
-        if ((dt) == CABINET_F32) { CALL_F; } \
-        else { CALL_B; }                     \
-    } while (0)
-
 extern "C" int cabinet_pack_conv_weight(const float* w_oihw, int Cout, int Cin, int KH, int KW, void* out, int out_dtype,
                                         int rows_pad, int k_pad, int transpose_flip, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("pack_conv_weight", out_dtype, CAB_DT_ALL);
     CAB_REQUIRE(w_oihw && out && Cout > 0 && Cin > 0 && KH > 0 && KW > 0 && rows_pad >= (transpose_flip ? Cin : Cout) &&
                     k_pad >= (transpose_flip ? Cout : Cin),
                 "pack_conv_weight: bad arguments");
     const long long total = static_cast<long long>(rows_pad) * KH * KW * k_pad;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (out_dtype == CABINET_F32)
-        pack_conv_weight_kernel<float><<<ew_grid(total), 256, 0, s>>>(w_oihw, Cout, Cin, KH * KW, rows_pad, k_pad, transpose_flip,
-                                                                       reinterpret_cast<float*>(out));
-    else
-        pack_conv_weight_kernel<bf16><<<ew_grid(total), 256, 0, s>>>(w_oihw, Cout, Cin, KH * KW, rows_pad, k_pad, transpose_flip,
-                                                                      reinterpret_cast<bf16*>(out));
+    CAB_DISPATCH_DT(out_dtype, T,
+                    pack_conv_weight_kernel<T><<<ew_grid(total), 256, 0, s>>>(w_oihw, Cout, Cin, KH * KW, rows_pad, k_pad,
+                                                                             transpose_flip, reinterpret_cast<T*>(out)));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
 
 extern "C" int cabinet_pack_conv_weight_parity(const float* w_oihw, int Cout, int Cin, int K, int pad, int py, int px, int KH2,
                                                int KW2, int pad2, void* out, int rows_pad, int k_pad, cabinet_stream_t stream) {
+    return cabinet_pack_conv_weight_parity_dt(w_oihw, Cout, Cin, K, pad, py, px, KH2, KW2, pad2, out, rows_pad, k_pad, CABINET_BF16,
+                                              stream);
+}
+
+extern "C" int cabinet_pack_conv_weight_parity_dt(const float* w_oihw, int Cout, int Cin, int K, int pad, int py, int px, int KH2,
+                                                  int KW2, int pad2, void* out, int rows_pad, int k_pad, int out_dtype,
+                                                  cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("pack_conv_weight_parity", out_dtype, CAB_DT_BF16 | CAB_DT_F16);
     CAB_REQUIRE(w_oihw && out && Cout > 0 && Cin > 0 && K > 0 && KH2 > 0 && KW2 > 0 && rows_pad >= Cin && k_pad >= Cout &&
                     (py == 0 || py == 1) && (px == 0 || px == 1),
                 "pack_conv_weight_parity: bad arguments");
     const long long total = static_cast<long long>(rows_pad) * KH2 * KW2 * k_pad;
-    pack_conv_weight_parity_kernel<<<ew_grid(total), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        w_oihw, Cout, Cin, K, pad, py, px, KH2, KW2, pad2, rows_pad, k_pad, reinterpret_cast<bf16*>(out));
+    CAB_DISPATCH_DT_HALF(out_dtype, T,
+                    pack_conv_weight_parity_kernel<T><<<ew_grid(total), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+                        w_oihw, Cout, Cin, K, pad, py, px, KH2, KW2, pad2, rows_pad, k_pad, reinterpret_cast<T*>(out)));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -1893,6 +1902,12 @@ extern "C" int cabinet_pack_dw_weight(const float* w, int C, int k, int flip, fl
 
 extern "C" int cabinet_im2col_nchw(const float* x, int N, int Cin, int H, int W, int k, int stride, int pad, void* out,
                                    long long ld, cabinet_stream_t stream) {
+    return cabinet_im2col_nchw_dt(x, N, Cin, H, W, k, stride, pad, out, ld, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_im2col_nchw_dt(const float* x, int N, int Cin, int H, int W, int k, int stride, int pad, void* out,
+                                      long long ld, int out_dtype, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("im2col_nchw", out_dtype, CAB_DT_BF16 | CAB_DT_F16);
     CAB_REQUIRE(x && out && N >= 0 && Cin > 0 && H > 0 && W > 0 && k > 0 && stride > 0 && ld >= static_cast<long long>(Cin) * k * k &&
                     ld % 8 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0,
                 "im2col_nchw: bad arguments (ld must be a multiple of 8 >= Cin*k*k, out 16-byte aligned)");
@@ -1902,12 +1917,13 @@ extern "C" int cabinet_im2col_nchw(const float* x, int N, int Cin, int H, int W,
     CAB_REQUIRE(total * (ld / 8) < (1LL << 31), "im2col_nchw: too many pixels");
     const size_t smem = (static_cast<size_t>(Cin) * k * (IM2COL_PX * stride + k - stride) + static_cast<size_t>(ld)) * 4;
     const int segs = (OW + IM2COL_PX - 1) / IM2COL_PX;
-    if (smem <= 48 * 1024 && static_cast<long long>(N) * OH * segs < (1LL << 31))
-        im2col_nchw_row_kernel<<<static_cast<unsigned>(static_cast<long long>(N) * OH * segs), 256, smem, static_cast<cudaStream_t>(stream)>>>(
-            x, Cin, H, W, k, stride, pad, OH, OW, reinterpret_cast<bf16*>(out), static_cast<int>(ld), segs);
-    else
-        im2col_nchw_kernel<<<ew_grid(total * (ld / 8)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-            x, N, Cin, H, W, k, stride, pad, OH, OW, reinterpret_cast<bf16*>(out), static_cast<int>(ld));
+    CAB_DISPATCH_DT_HALF(out_dtype, T,
+        if (smem <= 48 * 1024 && static_cast<long long>(N) * OH * segs < (1LL << 31))
+            im2col_nchw_row_kernel<T><<<static_cast<unsigned>(static_cast<long long>(N) * OH * segs), 256, smem, static_cast<cudaStream_t>(stream)>>>(
+                x, Cin, H, W, k, stride, pad, OH, OW, reinterpret_cast<T*>(out), static_cast<int>(ld), segs);
+        else
+            im2col_nchw_kernel<T><<<ew_grid(total * (ld / 8)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+                x, N, Cin, H, W, k, stride, pad, OH, OW, reinterpret_cast<T*>(out), static_cast<int>(ld)));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -1945,7 +1961,7 @@ struct RtPlan {
 };
 static RtPlan rt_plan(int dtype, long long M, int C, bool dense, int nsrc, int nb_max) {
     RtPlan p = {false, 0, 0, 0};
-    if (dtype != CABINET_BF16 || !dense || C % 8 != 0 || C / 8 > RED_THREADS || M * C < (1LL << 20) || (cabinet_debug_flags_value() & 128))
+    if ((dtype != CABINET_BF16 && dtype != CABINET_F16) || !dense || C % 8 != 0 || C / 8 > RED_THREADS || M * C < (1LL << 20) || (cabinet_debug_flags_value() & 128))
         return p;
     const int lanes = RED_THREADS / (C / 8);
     p.chunk_rows = (RT_STAGE_BYTES / nsrc) / (C * 2) / lanes * lanes;
@@ -1960,6 +1976,7 @@ static RtPlan rt_plan(int dtype, long long M, int C, bool dense, int nsrc, int n
 extern "C" int cabinet_bn_train_stats(const void* x, long long ldx, int dtype, long long M, int C, const float* gamma,
                                       const float* beta, float eps, float momentum, float* running_mean,
                                       float* running_var, float* stats, float* scratch, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("bn_train_stats", dtype, CAB_DT_ALL);
     CAB_REQUIRE(x && stats && scratch && M > 0 && C > 0 && ldx >= C, "bn_train_stats: bad arguments");
     long long rpb;
     const int nb = red_blocks(M, &rpb);
@@ -1969,32 +1986,32 @@ extern "C" int cabinet_bn_train_stats(const void* x, long long ldx, int dtype, l
     if (tp.ok) {
         static bool attr_done = false;
         if (!attr_done) {
-            CAB_CUDA(cudaFuncSetAttribute(bn_stats_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_STAGES * RT_STAGE_BYTES));
+            CAB_CUDA(cudaFuncSetAttribute(bn_stats_tma_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_STAGES * RT_STAGE_BYTES));
+            CAB_CUDA(cudaFuncSetAttribute(bn_stats_tma_kernel<f16>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_STAGES * RT_STAGE_BYTES));
             attr_done = true;
         }
-        bn_stats_tma_kernel<<<tp.nb, RT_THREADS, RT_STAGES * RT_STAGE_BYTES, s>>>(reinterpret_cast<const bf16*>(x), M, C, tp.rpb, tp.chunk_rows, scratch);
-        CAB_LAUNCH_CHECK();
-        bn_finalize_kernel<bf16><<<static_cast<unsigned>(cab_ceil_div(C, 4)), 128, 0, s>>>(scratch, tp.nb, M, C, reinterpret_cast<const bf16*>(x), gamma, beta, eps,
-                                                                                         momentum, running_mean, running_var, stats);
+        CAB_DISPATCH_DT_HALF(dtype, T,
+                        bn_stats_tma_kernel<T><<<tp.nb, RT_THREADS, RT_STAGES * RT_STAGE_BYTES, s>>>(reinterpret_cast<const T*>(x), M, C, tp.rpb,
+                                                                                                     tp.chunk_rows, scratch);
+                        CAB_LAUNCH_CHECK();
+                        bn_finalize_kernel<T><<<static_cast<unsigned>(cab_ceil_div(C, 4)), 128, 0, s>>>(scratch, tp.nb, M, C, reinterpret_cast<const T*>(x),
+                                                                                                      gamma, beta, eps, momentum, running_mean,
+                                                                                                      running_var, stats));
         CAB_LAUNCH_CHECK();
         return CABINET_OK;
     }
     if (C % V == 0 && ldx % V == 0 && al16(x)) {
-        CAB_DT2(dtype,
-                (bn_stats_v_kernel<float><<<nb, RED_THREADS, red_smem_v<float>(2), s>>>(reinterpret_cast<const float*>(x), ldx, M, C, rpb, scratch)),
-                (bn_stats_v_kernel<bf16><<<nb, RED_THREADS, red_smem_v<bf16>(2), s>>>(reinterpret_cast<const bf16*>(x), ldx, M, C, rpb, scratch)));
+        CAB_DISPATCH_DT(dtype, T,
+                bn_stats_v_kernel<T><<<nb, RED_THREADS, red_smem_v<T>(2), s>>>(reinterpret_cast<const T*>(x), ldx, M, C, rpb, scratch));
     } else {
-        CAB_DT2(dtype,
-                (bn_stats_kernel<float><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const float*>(x), ldx, M, C, rpb, scratch)),
-                (bn_stats_kernel<bf16><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const bf16*>(x), ldx, M, C, rpb, scratch)));
+        CAB_DISPATCH_DT(dtype, T,
+                bn_stats_kernel<T><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const T*>(x), ldx, M, C, rpb, scratch));
     }
     CAB_LAUNCH_CHECK();
     const unsigned g = static_cast<unsigned>(cab_ceil_div(C, 4));  // 4 warps = 4 channels per block
-    CAB_DT2(dtype,
-            (bn_finalize_kernel<float><<<g, 128, 0, s>>>(scratch, nb, M, C, reinterpret_cast<const float*>(x), gamma, beta, eps,
-                                                        momentum, running_mean, running_var, stats)),
-            (bn_finalize_kernel<bf16><<<g, 128, 0, s>>>(scratch, nb, M, C, reinterpret_cast<const bf16*>(x), gamma, beta, eps,
-                                                       momentum, running_mean, running_var, stats)));
+    CAB_DISPATCH_DT(dtype, T,
+                bn_finalize_kernel<T><<<g, 128, 0, s>>>(scratch, nb, M, C, reinterpret_cast<const T*>(x), gamma, beta, eps,
+                                                       momentum, running_mean, running_var, stats));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -2003,6 +2020,8 @@ extern "C" int cabinet_affine_act(const void* z, long long ldz, int z_dtype, con
                                   const float* gate, float gate_plus, const void* res, long long ldres, void* y,
                                   long long ldy, int y_dtype, long long M, long long HW, int C, int act,
                                   cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("affine_act", z_dtype, CAB_DT_ALL);
+    CAB_REQUIRE_DTYPE("affine_act", y_dtype, CAB_DT_ALL);
     CAB_REQUIRE(z && y && M >= 0 && C > 0 && HW > 0 && (!scale || shift), "affine_act: bad arguments");
     if (M == 0) return CABINET_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -2013,10 +2032,7 @@ extern "C" int cabinet_affine_act(const void* z, long long ldz, int z_dtype, con
     affine_act_v_kernel<TZ, TY><<<gv, 256, 0, s>>>(reinterpret_cast<const TZ*>(z), ldz, scale, shift, gate, gate_plus,   \
                                                    reinterpret_cast<const TY*>(res), ldres, reinterpret_cast<TY*>(y), ldy, \
                                                    M, HW, C, act)
-        if (z_dtype == CABINET_F32 && y_dtype == CABINET_F32) CAB_AAV(float, float);
-        else if (z_dtype == CABINET_F32) CAB_AAV(float, bf16);
-        else if (y_dtype == CABINET_F32) CAB_AAV(bf16, float);
-        else CAB_AAV(bf16, bf16);
+        CAB_DISPATCH_DT_PAIR(z_dtype, y_dtype, CAB_AAV);
 #undef CAB_AAV
         CAB_LAUNCH_CHECK();
         return CABINET_OK;
@@ -2026,10 +2042,7 @@ extern "C" int cabinet_affine_act(const void* z, long long ldz, int z_dtype, con
     affine_act_kernel<TZ, TY><<<g, 256, 0, s>>>(reinterpret_cast<const TZ*>(z), ldz, scale, shift, gate, gate_plus,   \
                                                 reinterpret_cast<const TY*>(res), ldres, reinterpret_cast<TY*>(y), ldy, \
                                                 M, HW, C, act)
-    if (z_dtype == CABINET_F32 && y_dtype == CABINET_F32) CAB_AA(float, float);
-    else if (z_dtype == CABINET_F32) CAB_AA(float, bf16);
-    else if (y_dtype == CABINET_F32) CAB_AA(bf16, float);
-    else CAB_AA(bf16, bf16);
+    CAB_DISPATCH_DT_PAIR(z_dtype, y_dtype, CAB_AA);
 #undef CAB_AA
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
@@ -2039,6 +2052,7 @@ extern "C" int cabinet_bn_train_backward(const void* dy, long long lddy, const v
                                          const float* stats, int act, float* dgamma, float* dbeta, void* dz,
                                          long long lddz, long long M, int C, int accumulate, float* scratch,
                                          cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("bn_train_backward", dtype, CAB_DT_ALL);
     CAB_REQUIRE(dy && z && stats && dz && scratch && M > 0 && C > 0, "bn_train_backward: bad arguments");
     long long rpb;
     const int nb = red_blocks(M, &rpb);
@@ -2051,42 +2065,37 @@ extern "C" int cabinet_bn_train_backward(const void* dy, long long lddy, const v
     if (tp.ok) {
         static bool attr_done = false;
         if (!attr_done) {
-            CAB_CUDA(cudaFuncSetAttribute(bn_bwd_reduce_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_STAGES * RT_STAGE_BYTES));
+            CAB_CUDA(cudaFuncSetAttribute(bn_bwd_reduce_tma_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_STAGES * RT_STAGE_BYTES));
+            CAB_CUDA(cudaFuncSetAttribute(bn_bwd_reduce_tma_kernel<f16>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_STAGES * RT_STAGE_BYTES));
             attr_done = true;
         }
-        bn_bwd_reduce_tma_kernel<<<tp.nb, RT_THREADS, RT_STAGES * RT_STAGE_BYTES, s>>>(reinterpret_cast<const bf16*>(dy), reinterpret_cast<const bf16*>(z), stats, act,
-                                                                                      M, C, tp.rpb, tp.chunk_rows, scratch);
+        CAB_DISPATCH_DT_HALF(dtype, T,
+                        bn_bwd_reduce_tma_kernel<T><<<tp.nb, RT_THREADS, RT_STAGES * RT_STAGE_BYTES, s>>>(reinterpret_cast<const T*>(dy),
+                                                                                                          reinterpret_cast<const T*>(z), stats, act, M, C,
+                                                                                                          tp.rpb, tp.chunk_rows, scratch));
         nb_red = tp.nb;
     } else if (vec) {
-        CAB_DT2(dtype,
-                (bn_bwd_reduce_v_kernel<float><<<nb, RED_THREADS, red_smem_v<float>(2), s>>>(reinterpret_cast<const float*>(dy), lddy,
-                                                                                          reinterpret_cast<const float*>(z), ldz, stats, act, M, C, rpb, scratch)),
-                (bn_bwd_reduce_v_kernel<bf16><<<nb, RED_THREADS, red_smem_v<bf16>(2), s>>>(reinterpret_cast<const bf16*>(dy), lddy,
-                                                                                        reinterpret_cast<const bf16*>(z), ldz, stats, act, M, C, rpb, scratch)));
+        CAB_DISPATCH_DT(dtype, T,
+                bn_bwd_reduce_v_kernel<T><<<nb, RED_THREADS, red_smem_v<T>(2), s>>>(reinterpret_cast<const T*>(dy), lddy,
+                                                                                        reinterpret_cast<const T*>(z), ldz, stats, act, M, C, rpb, scratch));
     } else {
-        CAB_DT2(dtype,
-                (bn_bwd_reduce_kernel<float><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const float*>(dy), lddy,
-                                                                             reinterpret_cast<const float*>(z), ldz, stats, act, M, C, rpb, scratch)),
-                (bn_bwd_reduce_kernel<bf16><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const bf16*>(dy), lddy,
-                                                                            reinterpret_cast<const bf16*>(z), ldz, stats, act, M, C, rpb, scratch)));
+        CAB_DISPATCH_DT(dtype, T,
+                bn_bwd_reduce_kernel<T><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const T*>(dy), lddy,
+                                                                            reinterpret_cast<const T*>(z), ldz, stats, act, M, C, rpb, scratch));
     }
     CAB_LAUNCH_CHECK();
     bn_bwd_finalize_kernel<<<static_cast<unsigned>(cab_ceil_div(C, 4)), 128, 0, s>>>(scratch, nb_red, M, C, dgamma, dbeta, coef);
     CAB_LAUNCH_CHECK();
     if (vec) {
         const unsigned gv = row_grid(M, 256 / (C / V));
-        CAB_DT2(dtype,
-                (bn_bwd_apply_v_kernel<float><<<gv, 256, 0, s>>>(reinterpret_cast<const float*>(dy), lddy, reinterpret_cast<const float*>(z), ldz,
-                                                                stats, coef, act, reinterpret_cast<float*>(dz), lddz, M, C, accumulate)),
-                (bn_bwd_apply_v_kernel<bf16><<<gv, 256, 0, s>>>(reinterpret_cast<const bf16*>(dy), lddy, reinterpret_cast<const bf16*>(z), ldz,
-                                                               stats, coef, act, reinterpret_cast<bf16*>(dz), lddz, M, C, accumulate)));
+        CAB_DISPATCH_DT(dtype, T,
+                bn_bwd_apply_v_kernel<T><<<gv, 256, 0, s>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(z), ldz,
+                                                               stats, coef, act, reinterpret_cast<T*>(dz), lddz, M, C, accumulate));
     } else {
         const unsigned g = ew_grid(M * C);
-        CAB_DT2(dtype,
-                (bn_bwd_apply_kernel<float><<<g, 256, 0, s>>>(reinterpret_cast<const float*>(dy), lddy, reinterpret_cast<const float*>(z), ldz,
-                                                             stats, coef, act, reinterpret_cast<float*>(dz), lddz, M, C, accumulate)),
-                (bn_bwd_apply_kernel<bf16><<<g, 256, 0, s>>>(reinterpret_cast<const bf16*>(dy), lddy, reinterpret_cast<const bf16*>(z), ldz,
-                                                            stats, coef, act, reinterpret_cast<bf16*>(dz), lddz, M, C, accumulate)));
+        CAB_DISPATCH_DT(dtype, T,
+                bn_bwd_apply_kernel<T><<<g, 256, 0, s>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(z), ldz,
+                                                            stats, coef, act, reinterpret_cast<T*>(dz), lddz, M, C, accumulate));
     }
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
@@ -2096,6 +2105,7 @@ extern "C" int cabinet_gate_apply_backward(const void* dy, long long lddy, const
                                            const float* s, float plus, const float* dm, float inv_hw, int act, void* dv,
                                            long long lddv, int N, long long HW, int C, int accumulate,
                                            cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("gate_apply_backward", dtype, CAB_DT_ALL);
     CAB_REQUIRE(dy && v && dv && N >= 0 && HW > 0 && C > 0, "gate_apply_backward: bad arguments");
     if (N == 0) return CABINET_OK;
     const long long M = static_cast<long long>(N) * HW;
@@ -2105,19 +2115,15 @@ extern "C" int cabinet_gate_apply_backward(const void* dy, long long lddy, const
         const int lanes = 256 / (C / V);
         const unsigned gx = static_cast<unsigned>(std::max<long long>(1, std::min<long long>(cab_ceil_div(HW, 4LL * lanes), 148LL * 16 / N + 1)));
         dim3 grid(gx, N);
-        CAB_DT2(dtype,
-                (gate_bwd_apply_v_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(dy), lddy, reinterpret_cast<const float*>(v), ldv, s, plus, dm,
-                                                                     inv_hw, act, reinterpret_cast<float*>(dv), lddv, HW, C, accumulate)),
-                (gate_bwd_apply_v_kernel<bf16><<<grid, 256, 0, st>>>(reinterpret_cast<const bf16*>(dy), lddy, reinterpret_cast<const bf16*>(v), ldv, s, plus, dm,
-                                                                    inv_hw, act, reinterpret_cast<bf16*>(dv), lddv, HW, C, accumulate)));
+        CAB_DISPATCH_DT(dtype, T,
+                gate_bwd_apply_v_kernel<T><<<grid, 256, 0, st>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(v), ldv, s, plus, dm,
+                                                                    inv_hw, act, reinterpret_cast<T*>(dv), lddv, HW, C, accumulate));
         CAB_LAUNCH_CHECK();
         return CABINET_OK;
     }
-    CAB_DT2(dtype,
-            (gate_bwd_apply_kernel<float><<<ew_grid(M * C), 256, 0, st>>>(reinterpret_cast<const float*>(dy), lddy, reinterpret_cast<const float*>(v), ldv, s, plus,
-                                                                         dm, inv_hw, act, reinterpret_cast<float*>(dv), lddv, M, HW, C, accumulate)),
-            (gate_bwd_apply_kernel<bf16><<<ew_grid(M * C), 256, 0, st>>>(reinterpret_cast<const bf16*>(dy), lddy, reinterpret_cast<const bf16*>(v), ldv, s, plus,
-                                                                        dm, inv_hw, act, reinterpret_cast<bf16*>(dv), lddv, M, HW, C, accumulate)));
+    CAB_DISPATCH_DT(dtype, T,
+                gate_bwd_apply_kernel<T><<<ew_grid(M * C), 256, 0, st>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(v), ldv, s, plus,
+                                                                        dm, inv_hw, act, reinterpret_cast<T*>(dv), lddv, M, HW, C, accumulate));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -2125,6 +2131,7 @@ extern "C" int cabinet_gate_apply_backward(const void* dy, long long lddy, const
 extern "C" int cabinet_gate_scale_backward(const void* dy, long long lddy, const void* v, long long ldv, int dtype,
                                            const float* s, float plus, int act, float* ds, int N, long long HW, int C,
                                            float* scratch, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("gate_scale_backward", dtype, CAB_DT_ALL);
     CAB_REQUIRE(dy && v && s && ds && scratch && N > 0 && HW > 0 && C > 0 && N <= 65535, "gate_scale_backward: bad arguments");
     long long rpb;
     const int nb = red_blocks(HW, &rpb);
@@ -2132,22 +2139,18 @@ extern "C" int cabinet_gate_scale_backward(const void* dy, long long lddy, const
     dim3 grid(nb, N);
     const int V = dtype == CABINET_F32 ? 4 : 8;
     if (C % V == 0 && lddy % V == 0 && ldv % V == 0 && al16(dy) && al16(v)) {
-        CAB_DT2(dtype,
-                (gate_bwd_reduce_v_kernel<float><<<grid, RED_THREADS, red_smem_v<float>(1), st>>>(reinterpret_cast<const float*>(dy), lddy,
-                                                                                                 reinterpret_cast<const float*>(v), ldv, s, plus, act, HW, C, rpb, scratch)),
-                (gate_bwd_reduce_v_kernel<bf16><<<grid, RED_THREADS, red_smem_v<bf16>(1), st>>>(reinterpret_cast<const bf16*>(dy), lddy,
-                                                                                               reinterpret_cast<const bf16*>(v), ldv, s, plus, act, HW, C, rpb, scratch)));
+        CAB_DISPATCH_DT(dtype, T,
+                gate_bwd_reduce_v_kernel<T><<<grid, RED_THREADS, red_smem_v<T>(1), st>>>(reinterpret_cast<const T*>(dy), lddy,
+                                                                                               reinterpret_cast<const T*>(v), ldv, s, plus, act, HW, C, rpb, scratch));
         CAB_LAUNCH_CHECK();
         sum_partials_kernel<<<dim3(static_cast<unsigned>(cab_ceil_div(C, 128)), N), 128, 0, st>>>(scratch, nb, C, static_cast<long long>(nb) * C, ds,
                                                                                                    1.f, 0);
         CAB_LAUNCH_CHECK();
         return CABINET_OK;
     }
-    CAB_DT2(dtype,
-            (gate_bwd_reduce_kernel<float><<<grid, RED_THREADS, RED_SMEM, st>>>(reinterpret_cast<const float*>(dy), lddy, reinterpret_cast<const float*>(v), ldv,
-                                                                               s, plus, act, HW, C, rpb, scratch)),
-            (gate_bwd_reduce_kernel<bf16><<<grid, RED_THREADS, RED_SMEM, st>>>(reinterpret_cast<const bf16*>(dy), lddy, reinterpret_cast<const bf16*>(v), ldv,
-                                                                              s, plus, act, HW, C, rpb, scratch)));
+    CAB_DISPATCH_DT(dtype, T,
+                gate_bwd_reduce_kernel<T><<<grid, RED_THREADS, RED_SMEM, st>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(v), ldv,
+                                                                              s, plus, act, HW, C, rpb, scratch));
     CAB_LAUNCH_CHECK();
     sum_partials_kernel<<<dim3(static_cast<unsigned>(cab_ceil_div(C, 128)), N), 128, 0, st>>>(scratch, nb, C, static_cast<long long>(nb) * C, ds,
                                                                                                1.f, 0);
@@ -2157,13 +2160,13 @@ extern "C" int cabinet_gate_scale_backward(const void* dy, long long lddy, const
 
 extern "C" int cabinet_col_sum(const void* x, long long ldx, int dtype, long long M, int C, float* out, int accumulate,
                                float* scratch, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("col_sum", dtype, CAB_DT_ALL);
     CAB_REQUIRE(x && out && scratch && M > 0 && C > 0, "col_sum: bad arguments");
     long long rpb;
     const int nb = red_blocks(M, &rpb);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    CAB_DT2(dtype,
-            (col_sum_kernel<float><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const float*>(x), ldx, M, C, rpb, scratch)),
-            (col_sum_kernel<bf16><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const bf16*>(x), ldx, M, C, rpb, scratch)));
+    CAB_DISPATCH_DT(dtype, T,
+                col_sum_kernel<T><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const T*>(x), ldx, M, C, rpb, scratch));
     CAB_LAUNCH_CHECK();
     sum_partials_kernel<<<dim3(static_cast<unsigned>(cab_ceil_div(C, 128)), 1), 128, 0, s>>>(scratch, nb, C, 0, out, 1.f, accumulate);
     CAB_LAUNCH_CHECK();
@@ -2174,6 +2177,8 @@ extern "C" int cabinet_conv_dgrad(const void* dy, long long lddy, int dtype, con
                                   long long w_sco, long long w_stap, void* dx, long long lddx, int N, int H, int W, int Cin,
                                   int Cout, int KH, int KW, int stride, int pad, int OH, int OW, int accumulate,
                                   cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("conv_dgrad", dtype, CAB_DT_ALL);
+    CAB_REQUIRE_DTYPE("conv_dgrad", w_dtype, CAB_DT_ALL);
     CAB_REQUIRE(dy && w_packed && dx && N >= 0 && H > 0 && W > 0 && Cin > 0 && Cout > 0 && stride >= 1, "conv_dgrad: bad arguments");
     if (N == 0) return CABINET_OK;
     DgradArgs a;
@@ -2191,10 +2196,7 @@ extern "C" int cabinet_conv_dgrad(const void* dy, long long lddy, int dtype, con
         if (s2) conv_dgrad_kernel<T, TW, true><<<grid, 256, 0, s>>>(a);    \
         else conv_dgrad_kernel<T, TW, false><<<grid, 256, 0, s>>>(a);      \
     } while (0)
-    if (dtype == CABINET_F32 && w_dtype == CABINET_F32) CAB_DG(float, float);
-    else if (dtype == CABINET_F32) CAB_DG(float, bf16);
-    else if (w_dtype == CABINET_F32) CAB_DG(bf16, float);
-    else CAB_DG(bf16, bf16);
+    CAB_DISPATCH_DT_PAIR(dtype, w_dtype, CAB_DG);
 #undef CAB_DG
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
@@ -2212,6 +2214,8 @@ extern "C" int cabinet_conv_wgrad(const void* dy, long long lddy, int dtype, con
                                   long long sxh, long long sxw, long long sxc, float* dw_oihw, int N, int H, int W, int Cin,
                                   int Cout, int KH, int KW, int stride, int pad, int OH, int OW, float* scratch,
                                   cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("conv_wgrad", dtype, CAB_DT_ALL);
+    CAB_REQUIRE_DTYPE("conv_wgrad", x_dtype, CAB_DT_ALL);
     CAB_REQUIRE(dy && x && dw_oihw && scratch && N > 0 && Cin > 0 && Cout > 0, "conv_wgrad: bad arguments");
     WgradArgs a;
     a.dy = dy; a.lddy = lddy; a.x = x; a.sxn = sxn; a.sxh = sxh; a.sxw = sxw; a.sxc = sxc; a.partial = scratch;
@@ -2225,10 +2229,9 @@ extern "C" int cabinet_conv_wgrad(const void* dy, long long lddy, int dtype, con
     const int nz = static_cast<int>(cab_ceil_div(a.M, a.rows_per_split));
     dim3 grid(static_cast<unsigned>(cab_ceil_div(Cout, GBM)), static_cast<unsigned>(cab_ceil_div(a.Kn, GBN)), nz);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (dtype == CABINET_F32 && x_dtype == CABINET_F32) conv_wgrad_kernel<float, float><<<grid, 256, 0, s>>>(a);
-    else if (dtype == CABINET_F32) conv_wgrad_kernel<float, bf16><<<grid, 256, 0, s>>>(a);
-    else if (x_dtype == CABINET_F32) conv_wgrad_kernel<bf16, float><<<grid, 256, 0, s>>>(a);
-    else conv_wgrad_kernel<bf16, bf16><<<grid, 256, 0, s>>>(a);
+#define CAB_WG(T, TX) conv_wgrad_kernel<T, TX><<<grid, 256, 0, s>>>(a)
+    CAB_DISPATCH_DT_PAIR(dtype, x_dtype, CAB_WG);
+#undef CAB_WG
     CAB_LAUNCH_CHECK();
     wgrad_finalize_kernel<<<static_cast<unsigned>(cab_ceil_div(total, 256)), 256, 0, s>>>(scratch, nz, Cout, Cin, KH * KW, dw_oihw);
     CAB_LAUNCH_CHECK();
@@ -2238,6 +2241,7 @@ extern "C" int cabinet_conv_wgrad(const void* dy, long long lddy, int dtype, con
 extern "C" int cabinet_dwconv_dgrad(const void* dy, long long lddy, int dtype, const float* w_packed, void* dx,
                                     long long lddx, int N, int H, int W, int C, int k, int stride, int OH, int OW,
                                     int accumulate, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("dwconv_dgrad", dtype, CAB_DT_ALL);
     CAB_REQUIRE(dy && w_packed && dx && C > 0 && (k == 3 || k == 5) && stride >= 1, "dwconv_dgrad: bad arguments");
     if (N == 0) return CABINET_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -2250,26 +2254,21 @@ extern "C" int cabinet_dwconv_dgrad(const void* dy, long long lddy, int dtype, c
 #define CAB_DG2(T, KK)                                                                                                          \
     dw_dgrad_s2_kernel<T, KK><<<g2, 256, 0, s>>>(reinterpret_cast<const T*>(dy), lddy, w_packed, reinterpret_cast<T*>(dx), lddx, N, H, W, \
                                                  C, OH, OW, accumulate)
-            if (dtype == CABINET_F32) { if (k == 3) CAB_DG2(float, 3); else CAB_DG2(float, 5); }
-            else { if (k == 3) CAB_DG2(bf16, 3); else CAB_DG2(bf16, 5); }
+            CAB_DISPATCH_DT(dtype, T, if (k == 3) CAB_DG2(T, 3); else CAB_DG2(T, 5));
 #undef CAB_DG2
             CAB_LAUNCH_CHECK();
             return CABINET_OK;
         }
-        CAB_DT2(dtype,
-                (dw_dgrad_v_kernel<float><<<ew_grid(tv), 256, 0, s>>>(reinterpret_cast<const float*>(dy), lddy, w_packed, reinterpret_cast<float*>(dx), lddx, N, H,
-                                                                     W, C, k, stride, OH, OW, accumulate)),
-                (dw_dgrad_v_kernel<bf16><<<ew_grid(tv), 256, 0, s>>>(reinterpret_cast<const bf16*>(dy), lddy, w_packed, reinterpret_cast<bf16*>(dx), lddx, N, H,
-                                                                    W, C, k, stride, OH, OW, accumulate)));
+        CAB_DISPATCH_DT(dtype, T,
+                dw_dgrad_v_kernel<T><<<ew_grid(tv), 256, 0, s>>>(reinterpret_cast<const T*>(dy), lddy, w_packed, reinterpret_cast<T*>(dx), lddx, N, H,
+                                                                    W, C, k, stride, OH, OW, accumulate));
         CAB_LAUNCH_CHECK();
         return CABINET_OK;
     }
     const long long total = static_cast<long long>(N) * H * W * C;
-    CAB_DT2(dtype,
-            (dw_dgrad_kernel<float><<<ew_grid(total), 256, 0, s>>>(reinterpret_cast<const float*>(dy), lddy, w_packed, reinterpret_cast<float*>(dx), lddx, N, H, W,
-                                                                  C, k, stride, OH, OW, accumulate)),
-            (dw_dgrad_kernel<bf16><<<ew_grid(total), 256, 0, s>>>(reinterpret_cast<const bf16*>(dy), lddy, w_packed, reinterpret_cast<bf16*>(dx), lddx, N, H, W,
-                                                                 C, k, stride, OH, OW, accumulate)));
+    CAB_DISPATCH_DT(dtype, T,
+                dw_dgrad_kernel<T><<<ew_grid(total), 256, 0, s>>>(reinterpret_cast<const T*>(dy), lddy, w_packed, reinterpret_cast<T*>(dx), lddx, N, H, W,
+                                                                 C, k, stride, OH, OW, accumulate));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -2277,6 +2276,7 @@ extern "C" int cabinet_dwconv_dgrad(const void* dy, long long lddy, int dtype, c
 extern "C" int cabinet_dwconv_wgrad(const void* dy, long long lddy, const void* x, long long ldx, int dtype, float* dw,
                                     int N, int H, int W, int C, int k, int stride, int OH, int OW, float* scratch,
                                     cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("dwconv_wgrad", dtype, CAB_DT_ALL);
     CAB_REQUIRE(dy && x && dw && scratch && N > 0 && C > 0 && (k == 3 || k == 5), "dwconv_wgrad: bad arguments");
     const long long M = static_cast<long long>(N) * OH * OW;
     CAB_REQUIRE(M < (1LL << 31), "dwconv_wgrad: too many pixels");
@@ -2310,7 +2310,7 @@ extern "C" int cabinet_dwconv_wgrad(const void* dy, long long lddy, const void* 
         if (k == 3 && stride == 1) CAB_DWR(T, 3, 1); else if (k == 3) CAB_DWR(T, 3, 2);             \
         else if (stride == 1) CAB_DWR(T, 5, 1); else CAB_DWR(T, 5, 2);                              \
     } while (0)
-        if (dtype == CABINET_F32) CAB_DWR2(float); else CAB_DWR2(bf16);
+        CAB_DISPATCH_DT(dtype, T, CAB_DWR2(T));
 #undef CAB_DWR2
 #undef CAB_DWR
         CAB_LAUNCH_CHECK();
@@ -2338,6 +2338,8 @@ extern "C" int cabinet_dwconv_wgrad(const void* dy, long long lddy, const void* 
             CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_line_kernel<float, 5, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
             CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_line_kernel<bf16, 5, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
             CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_line_kernel<bf16, 5, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+            CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_line_kernel<f16, 5, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+            CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_line_kernel<f16, 5, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
             attr_done = true;
         }
 #define CAB_DWL(T, KK, SS)                                                                                                     \
@@ -2348,7 +2350,7 @@ extern "C" int cabinet_dwconv_wgrad(const void* dy, long long lddy, const void* 
         if (k == 3 && stride == 1) CAB_DWL(T, 3, 1); else if (k == 3) CAB_DWL(T, 3, 2);             \
         else if (stride == 1) CAB_DWL(T, 5, 1); else CAB_DWL(T, 5, 2);                              \
     } while (0)
-        if (dtype == CABINET_F32) CAB_DWL2(float); else CAB_DWL2(bf16);
+        CAB_DISPATCH_DT(dtype, T, CAB_DWL2(T));
 #undef CAB_DWL2
 #undef CAB_DWL
         CAB_LAUNCH_CHECK();
@@ -2362,13 +2364,13 @@ extern "C" int cabinet_dwconv_wgrad(const void* dy, long long lddy, const void* 
         if (!attr_done) {
             CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_v2_kernel<float, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
             CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_v2_kernel<bf16, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+            CAB_CUDA(cudaFuncSetAttribute(dw_wgrad_v2_kernel<f16, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
             attr_done = true;
         }
 #define CAB_DWV(T, KK)                                                                                                       \
     dw_wgrad_v2_kernel<T, KK><<<nb, RED_THREADS, smem2, s>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(x), \
                                                             ldx, H, W, C, stride, OH, OW, M, rpb, scratch)
-        if (dtype == CABINET_F32) { if (k == 3) CAB_DWV(float, 3); else CAB_DWV(float, 5); }
-        else { if (k == 3) CAB_DWV(bf16, 3); else CAB_DWV(bf16, 5); }
+        CAB_DISPATCH_DT(dtype, T, if (k == 3) CAB_DWV(T, 3); else CAB_DWV(T, 5));
 #undef CAB_DWV
         CAB_LAUNCH_CHECK();
         dw_wgrad_finalize_kernel<<<static_cast<unsigned>(cab_ceil_div(C * k * k, 8)), 256, 0, s>>>(scratch, nb, C, k * k, dw);
@@ -2379,8 +2381,7 @@ extern "C" int cabinet_dwconv_wgrad(const void* dy, long long lddy, const void* 
 #define CAB_DWW(T, KK)                                                                                                   \
     dw_wgrad_kernel<T, KK><<<nb, RED_THREADS, smem, s>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(x), \
                                                          ldx, H, W, C, stride, OH, OW, M, rpb, scratch)
-    if (dtype == CABINET_F32) { if (k == 3) CAB_DWW(float, 3); else CAB_DWW(float, 5); }
-    else { if (k == 3) CAB_DWW(bf16, 3); else CAB_DWW(bf16, 5); }
+    CAB_DISPATCH_DT(dtype, T, if (k == 3) CAB_DWW(T, 3); else CAB_DWW(T, 5));
 #undef CAB_DWW
     CAB_LAUNCH_CHECK();
     dw_wgrad_finalize_kernel<<<static_cast<unsigned>(cab_ceil_div(C * k * k, 8)), 256, 0, s>>>(scratch, nb, C, k * k, dw);
@@ -2393,6 +2394,8 @@ extern "C" int cabinet_resample_sep(const void* in, int in_dtype, long long isn,
                                     long long osc, int N, int OH, int OW, int C, const int* y_start, const int* y_index,
                                     const float* y_weight, const int* x_start, const int* x_index, const float* x_weight,
                                     int accumulate, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("resample_sep", in_dtype, CAB_DT_ALL);
+    CAB_REQUIRE_DTYPE("resample_sep", out_dtype, CAB_DT_ALL);
     CAB_REQUIRE(in && out && y_start && y_index && y_weight && x_start && x_index && x_weight && OH > 0 && OW > 0 && C > 0,
                 "resample_sep: bad arguments");
     if (N == 0) return CABINET_OK;
@@ -2414,10 +2417,7 @@ extern "C" int cabinet_resample_sep(const void* in, int in_dtype, long long isn,
                                                          y_weight, x_start, x_index, x_weight, accumulate & 1, vec)
         const int vw = in_dtype == CABINET_F32 ? 4 : 8;  // columns per 16-byte load
         const int vec = (W_in % vw == 0 && isn % vw == 0 && isc % vw == 0 && al16(in)) ? 1 : 0;
-        if (in_dtype == CABINET_F32 && out_dtype == CABINET_F32) CAB_RB(float, float);
-        else if (in_dtype == CABINET_F32) CAB_RB(float, bf16);
-        else if (out_dtype == CABINET_F32) CAB_RB(bf16, float);
-        else CAB_RB(bf16, bf16);
+        CAB_DISPATCH_DT_PAIR(in_dtype, out_dtype, CAB_RB);
 #undef CAB_RB
         CAB_LAUNCH_CHECK();
         return CABINET_OK;
@@ -2428,10 +2428,7 @@ extern "C" int cabinet_resample_sep(const void* in, int in_dtype, long long isn,
     resample_sep_v_kernel<TI, TO><<<ew_grid(total / 8), 256, 0, s>>>(reinterpret_cast<const TI*>(in), isn, isy, isx,             \
                                                                      reinterpret_cast<TO*>(out), osn, osy, osx, N, OH, OW, C,    \
                                                                      y_start, y_index, y_weight, x_start, x_index, x_weight, accumulate)
-        if (in_dtype == CABINET_F32 && out_dtype == CABINET_F32) CAB_RSV(float, float);
-        else if (in_dtype == CABINET_F32) CAB_RSV(float, bf16);
-        else if (out_dtype == CABINET_F32) CAB_RSV(bf16, float);
-        else CAB_RSV(bf16, bf16);
+        CAB_DISPATCH_DT_PAIR(in_dtype, out_dtype, CAB_RSV);
 #undef CAB_RSV
         CAB_LAUNCH_CHECK();
         return CABINET_OK;
@@ -2440,10 +2437,7 @@ extern "C" int cabinet_resample_sep(const void* in, int in_dtype, long long isn,
     resample_sep_kernel<TI, TO><<<ew_grid(total), 256, 0, s>>>(reinterpret_cast<const TI*>(in), isn, isy, isx, isc,      \
                                                                reinterpret_cast<TO*>(out), osn, osy, osx, osc, N, OH, OW, C, \
                                                                y_start, y_index, y_weight, x_start, x_index, x_weight, accumulate)
-    if (in_dtype == CABINET_F32 && out_dtype == CABINET_F32) CAB_RS(float, float);
-    else if (in_dtype == CABINET_F32) CAB_RS(float, bf16);
-    else if (out_dtype == CABINET_F32) CAB_RS(bf16, float);
-    else CAB_RS(bf16, bf16);
+    CAB_DISPATCH_DT_PAIR(in_dtype, out_dtype, CAB_RS);
 #undef CAB_RS
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
@@ -2460,31 +2454,52 @@ extern "C" int cabinet_softmax_backward(const float* p, const float* dp, float* 
 
 extern "C" int cabinet_attn_softmax(const float* s, float scale, float* p, void* p_bf16, long long rows, int cols,
                                     cabinet_stream_t stream) {
-    CAB_REQUIRE(s && p && p_bf16 && cols > 0, "attn_softmax: bad arguments");
+    return cabinet_attn_softmax_dt(s, scale, p, p_bf16, rows, cols, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_attn_softmax_dt(const float* s, float scale, float* p, void* p_half, long long rows, int cols,
+                                       int op_dtype, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("attn_softmax", op_dtype, CAB_DT_BF16 | CAB_DT_F16);
+    CAB_REQUIRE(s && p && p_half && cols > 0, "attn_softmax: bad arguments");
     if (rows == 0) return CABINET_OK;
-    attn_softmax_kernel<<<static_cast<unsigned>(cab_ceil_div(rows, 8)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        s, scale, p, reinterpret_cast<bf16*>(p_bf16), rows, cols);
+    CAB_DISPATCH_DT_HALF(op_dtype, T,
+                    attn_softmax_kernel<T><<<static_cast<unsigned>(cab_ceil_div(rows, 8)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+                        s, scale, p, reinterpret_cast<T*>(p_half), rows, cols));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
 
 extern "C" int cabinet_attn_softmax_backward(const float* p, const float* dp, void* ds_bf16, long long rows, int cols,
                                              float alpha, cabinet_stream_t stream) {
-    CAB_REQUIRE(p && dp && ds_bf16 && cols > 0, "attn_softmax_backward: bad arguments");
+    return cabinet_attn_softmax_backward_dt(p, dp, ds_bf16, rows, cols, alpha, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_attn_softmax_backward_dt(const float* p, const float* dp, void* ds_half, long long rows, int cols,
+                                                float alpha, int op_dtype, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("attn_softmax_backward", op_dtype, CAB_DT_BF16 | CAB_DT_F16);
+    CAB_REQUIRE(p && dp && ds_half && cols > 0, "attn_softmax_backward: bad arguments");
     if (rows == 0) return CABINET_OK;
-    attn_softmax_bwd_kernel<<<static_cast<unsigned>(cab_ceil_div(rows, 8)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        p, dp, reinterpret_cast<bf16*>(ds_bf16), rows, cols, alpha);
+    CAB_DISPATCH_DT_HALF(op_dtype, T,
+                    attn_softmax_bwd_kernel<T><<<static_cast<unsigned>(cab_ceil_div(rows, 8)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+                        p, dp, reinterpret_cast<T*>(ds_half), rows, cols, alpha));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
 
 extern "C" int cabinet_transpose_tokens(const void* x, long long ldx, void* out, int N, int L, int C,
                                         cabinet_stream_t stream) {
+    return cabinet_transpose_tokens_dt(x, ldx, out, N, L, C, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_transpose_tokens_dt(const void* x, long long ldx, void* out, int N, int L, int C, int op_dtype,
+                                           cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("transpose_tokens", op_dtype, CAB_DT_BF16 | CAB_DT_F16);
     CAB_REQUIRE(x && out && N >= 0 && L > 0 && C > 0 && ldx >= C && N <= 65535, "transpose_tokens: bad arguments");
     if (N == 0) return CABINET_OK;
     dim3 grid(static_cast<unsigned>(cab_ceil_div(L, 32)), static_cast<unsigned>(cab_ceil_div(C, 32)), N);
-    transpose_tokens_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const bf16*>(x), ldx,
-                                                                               reinterpret_cast<bf16*>(out), L, C);
+    CAB_DISPATCH_DT_HALF(op_dtype, T,
+                    transpose_tokens_kernel<T><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const T*>(x), ldx,
+                                                                                                  reinterpret_cast<T*>(out), L, C));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
@@ -2493,20 +2508,17 @@ extern "C" int cabinet_cab_combine_backward(const void* dout, long long ldo, con
                                             const float* gamma, int dtype, void* dg, void* dx, void* dr, float* dgamma,
                                             long long n_pixels, int C, int accumulate_dx, float* scratch,
                                             cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("cab_combine_backward", dtype, CAB_DT_ALL);
     CAB_REQUIRE(dout && g && x && r && gamma && dg && dx && dr && dgamma && scratch && n_pixels > 0 && C > 0,
                 "cab_combine_backward: bad arguments");
     long long rpb;
     const int nb = red_blocks(n_pixels, &rpb);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    CAB_DT2(dtype,
-            (cab_combine_bwd_kernel<float><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const float*>(dout), ldo, reinterpret_cast<const float*>(g),
-                                                                           reinterpret_cast<const float*>(x), reinterpret_cast<const float*>(r), gamma,
-                                                                           reinterpret_cast<float*>(dg), reinterpret_cast<float*>(dx), reinterpret_cast<float*>(dr),
-                                                                           n_pixels, C, rpb, scratch, accumulate_dx)),
-            (cab_combine_bwd_kernel<bf16><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const bf16*>(dout), ldo, reinterpret_cast<const bf16*>(g),
-                                                                          reinterpret_cast<const bf16*>(x), reinterpret_cast<const bf16*>(r), gamma,
-                                                                          reinterpret_cast<bf16*>(dg), reinterpret_cast<bf16*>(dx), reinterpret_cast<bf16*>(dr),
-                                                                          n_pixels, C, rpb, scratch, accumulate_dx)));
+    CAB_DISPATCH_DT(dtype, T,
+                cab_combine_bwd_kernel<T><<<nb, RED_THREADS, RED_SMEM, s>>>(reinterpret_cast<const T*>(dout), ldo, reinterpret_cast<const T*>(g),
+                                                                          reinterpret_cast<const T*>(x), reinterpret_cast<const T*>(r), gamma,
+                                                                          reinterpret_cast<T*>(dg), reinterpret_cast<T*>(dx), reinterpret_cast<T*>(dr),
+                                                                          n_pixels, C, rpb, scratch, accumulate_dx));
     CAB_LAUNCH_CHECK();
     sum_all_kernel<<<1, 256, 0, s>>>(scratch, static_cast<long long>(nb) * C, dgamma);
     CAB_LAUNCH_CHECK();
@@ -2515,14 +2527,13 @@ extern "C" int cabinet_cab_combine_backward(const void* dout, long long ldo, con
 
 extern "C" int cabinet_add(const void* a, long long lda, const void* b, long long ldb, void* out, long long ldo, int dtype,
                            long long M, int C, cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("add", dtype, CAB_DT_ALL);
     CAB_REQUIRE(a && b && out && C > 0, "add: bad arguments");
     if (M == 0) return CABINET_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    CAB_DT2(dtype,
-            (add_kernel<float><<<ew_grid(M * C), 256, 0, s>>>(reinterpret_cast<const float*>(a), lda, reinterpret_cast<const float*>(b), ldb,
-                                                             reinterpret_cast<float*>(out), ldo, M, C)),
-            (add_kernel<bf16><<<ew_grid(M * C), 256, 0, s>>>(reinterpret_cast<const bf16*>(a), lda, reinterpret_cast<const bf16*>(b), ldb,
-                                                            reinterpret_cast<bf16*>(out), ldo, M, C)));
+    CAB_DISPATCH_DT(dtype, T,
+                add_kernel<T><<<ew_grid(M * C), 256, 0, s>>>(reinterpret_cast<const T*>(a), lda, reinterpret_cast<const T*>(b), ldb,
+                                                            reinterpret_cast<T*>(out), ldo, M, C));
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }

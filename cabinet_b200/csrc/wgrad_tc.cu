@@ -42,6 +42,7 @@ __device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t smem_addr, uint3
     return d;
 }
 
+template <typename T>  // operand type: bf16 or f16
 __global__ void __launch_bounds__(WG_THREADS, 2)
 conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constant__ CUtensorMap tmX,
                      const __grid_constant__ CUtensorMap tmX1, const __grid_constant__ CUtensorMap tmX2,
@@ -110,8 +111,8 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_cons
     } else if (warp == 1) {
         // ---------------- MMA issuer: D[128 x NB] += A^T B over the pixel tiles of this split
         const uint32_t leader = tc::elect_one();
-        // kind::f16, D fp32, A/B bf16, BOTH MN-major (bits 15, 16), N >> 3 at [17,23), M >> 4 at [24,29)
-        const uint32_t idesc = tc::make_idesc_bf16(128, p.NB) | (1u << 15) | (1u << 16);
+        // kind::f16, D fp32, A/B bf16 or f16, BOTH MN-major (bits 15, 16), N >> 3 at [17,23), M >> 4 at [24,29)
+        const uint32_t idesc = tc::make_idesc<T>(128, p.NB) | (1u << 15) | (1u << 16);
         for (int t = t0; t < t1; ++t) {
             const int it = t - t0, s = it % p.stages;
             tc::mbar_wait(&full_bar[s], (it / p.stages) & 1);
@@ -242,8 +243,9 @@ extern "C" long long cabinet_conv_wgrad_tc_scratch_floats(int N, int H, int W, i
 
 // per_image: 1x1 only; one pixel split per image and the "partials" ARE the result: out[n][co][ci] (no second level)
 static int wgrad_tc_impl(const void* dy, long long lddy, const void* x, long long ldx, float* dw_oihw, int N, int H, int W,
-                         int Cin, int Cout, int KH, int KW, int stride, int pad, float* scratch, cabinet_stream_t stream,
-                         bool per_image) {
+                         int Cin, int Cout, int KH, int KW, int stride, int pad, float* scratch, int op_dtype,
+                         cabinet_stream_t stream, bool per_image) {
+    CAB_REQUIRE_DTYPE("conv_wgrad_tc", op_dtype, CAB_DT_BF16 | CAB_DT_F16);
     CAB_REQUIRE(dy && x && dw_oihw && scratch, "conv_wgrad_tc: null pointer");
     CAB_REQUIRE(N > 0 && H > 0 && W > 0 && Cin > 0 && Cout > 0 && KH > 0 && KW > 0 && KH == KW && pad >= 0 &&
                     ((stride == 1 && 2 * pad == KH - 1) || (stride == 2 && H >= 2 && W >= 2)),
@@ -277,7 +279,7 @@ static int wgrad_tc_impl(const void* dy, long long lddy, const void* x, long lon
             const long long ld = which ? ldx : lddy;
             const uint64_t dims[4] = {(uint64_t)(which ? Cin : Cout), P, 1, 1};
             const uint64_t strides[3] = {(uint64_t)ld * es, (uint64_t)ld * es * P, (uint64_t)ld * es * P};
-            int rc = cab_make_tmap_bf16(which ? &tmX[0] : &tmDY, which ? x : dy, 4, dims, strides, box);
+            int rc = cab_make_tmap_2b(which ? &tmX[0] : &tmDY, op_dtype, which ? x : dy, 4, dims, strides, box);
             if (rc) return rc;
         }
         tmX[1] = tmX[2] = tmX[3] = tmX[0];
@@ -286,17 +288,17 @@ static int wgrad_tc_impl(const void* dy, long long lddy, const void* x, long lon
         {
             const uint64_t dims[4] = {(uint64_t)Cout, (uint64_t)OW, (uint64_t)OH, (uint64_t)N};
             const uint64_t strides[3] = {(uint64_t)lddy * es, (uint64_t)lddy * es * OW, (uint64_t)lddy * es * OW * OH};
-            int rc = cab_make_tmap_bf16(&tmDY, dy, 4, dims, strides, box);
+            int rc = cab_make_tmap_2b(&tmDY, op_dtype, dy, 4, dims, strides, box);
             if (rc) return rc;
         }
-        const bf16* xb = reinterpret_cast<const bf16*>(x);
+        const uint16_t* xb = reinterpret_cast<const uint16_t*>(x);  // 2-byte elements of either type
         for (int py = 0; py < stride; ++py)
             for (int px = 0; px < stride; ++px) {
                 const uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)((W - px + stride - 1) / stride),
                                           (uint64_t)((H - py + stride - 1) / stride), (uint64_t)N};
                 const uint64_t strides[3] = {(uint64_t)ldx * es * stride, (uint64_t)ldx * es * W * stride,
                                              (uint64_t)ldx * es * W * H};
-                int rc = cab_make_tmap_bf16(&tmX[py * stride + px], xb + (static_cast<long long>(py) * W + px) * ldx, 4, dims,
+                int rc = cab_make_tmap_2b(&tmX[py * stride + px], op_dtype, xb + (static_cast<long long>(py) * W + px) * ldx, 4, dims,
                                             strides, box);
                 if (rc) return rc;
             }
@@ -305,12 +307,13 @@ static int wgrad_tc_impl(const void* dy, long long lddy, const void* x, long lon
     const size_t smem = static_cast<size_t>(p.stages) * p.stage_bytes + 1024;
     static bool attr_done = false;
     if (!attr_done) {
-        CAB_CUDA(cudaFuncSetAttribute(conv_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        CAB_CUDA(cudaFuncSetAttribute(conv_wgrad_tc_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        CAB_CUDA(cudaFuncSetAttribute(conv_wgrad_tc_kernel<f16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
         attr_done = true;
     }
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     dim3 grid(g.m_tiles, p.taps * g.n_tiles, g.splits);
-    conv_wgrad_tc_kernel<<<grid, WG_THREADS, smem, s>>>(tmDY, tmX[0], tmX[1], tmX[2], tmX[3], p);
+    CAB_DISPATCH_DT_HALF(op_dtype, T, conv_wgrad_tc_kernel<T><<<grid, WG_THREADS, smem, s>>>(tmDY, tmX[0], tmX[1], tmX[2], tmX[3], p));
     CAB_LAUNCH_CHECK();
     const long long total = static_cast<long long>(Cout) * Cin * p.taps;
     if (per_image) return CABINET_OK;
@@ -328,11 +331,23 @@ static int wgrad_tc_impl(const void* dy, long long lddy, const void* x, long lon
 extern "C" int cabinet_conv_wgrad_tc(const void* dy, long long lddy, const void* x, long long ldx, float* dw_oihw, int N,
                                      int H, int W, int Cin, int Cout, int KH, int KW, int stride, int pad, float* scratch,
                                      cabinet_stream_t stream) {
-    return wgrad_tc_impl(dy, lddy, x, ldx, dw_oihw, N, H, W, Cin, Cout, KH, KW, stride, pad, scratch, stream, false);
+    return cabinet_conv_wgrad_tc_dt(dy, lddy, x, ldx, dw_oihw, N, H, W, Cin, Cout, KH, KW, stride, pad, scratch, CABINET_BF16,
+                                    stream);
+}
+
+extern "C" int cabinet_conv_wgrad_tc_dt(const void* dy, long long lddy, const void* x, long long ldx, float* dw_oihw, int N,
+                                        int H, int W, int Cin, int Cout, int KH, int KW, int stride, int pad, float* scratch,
+                                        int op_dtype, cabinet_stream_t stream) {
+    return wgrad_tc_impl(dy, lddy, x, ldx, dw_oihw, N, H, W, Cin, Cout, KH, KW, stride, pad, scratch, op_dtype, stream, false);
 }
 
 extern "C" int cabinet_conv_wgrad_tc_batched(const void* a, long long lda, const void* x, long long ldx, float* out, int N,
                                              int H, int W, int Cin, int Cout, cabinet_stream_t stream) {
+    return cabinet_conv_wgrad_tc_batched_dt(a, lda, x, ldx, out, N, H, W, Cin, Cout, CABINET_BF16, stream);
+}
+
+extern "C" int cabinet_conv_wgrad_tc_batched_dt(const void* a, long long lda, const void* x, long long ldx, float* out, int N,
+                                                int H, int W, int Cin, int Cout, int op_dtype, cabinet_stream_t stream) {
     CAB_REQUIRE(out != nullptr, "conv_wgrad_tc_batched: null pointer");
-    return wgrad_tc_impl(a, lda, x, ldx, out, N, H, W, Cin, Cout, 1, 1, 1, 0, out, stream, true);
+    return wgrad_tc_impl(a, lda, x, ldx, out, N, H, W, Cin, Cout, 1, 1, 1, 0, out, op_dtype, stream, true);
 }

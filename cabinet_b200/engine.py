@@ -20,8 +20,19 @@ from typing import Optional
 import torch
 
 from . import _lib
-from ._lib import ACT_HSIGMOID, ACT_HSWISH, ACT_NONE, ACT_RELU, ACT_SIGMOID, BF16, F32, check
+from ._lib import ACT_HSIGMOID, ACT_HSWISH, ACT_NONE, ACT_RELU, ACT_SIGMOID, BF16, F16, F32, check
 from .constants import BN_EPS
+
+
+_DTYPE_CODES = {torch.float32: F32, torch.bfloat16: BF16, torch.float16: F16}
+
+
+def dtype_code(dtype: torch.dtype) -> int:
+    """C-ABI element-type code of a tensor dtype; any other dtype is an error, never passed on as fp32."""
+    code = _DTYPE_CODES.get(dtype)
+    if code is None:
+        raise TypeError(f"cabinet_b200 kernels take float32, bfloat16 or float16 tensors, got {dtype}")
+    return code
 
 
 @dataclass
@@ -38,7 +49,7 @@ class Map:
 
     @property
     def dt(self) -> int:
-        return BF16 if self.t.dtype == torch.bfloat16 else F32
+        return dtype_code(self.t.dtype)
 
     @property
     def ptr(self) -> int:

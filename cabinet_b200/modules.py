@@ -275,7 +275,7 @@ class CABiNet(nn.Module):
         self.conv_out = CABiNetOutput(256, 256, n_classes)
         self.precision = "bf16"
         self.logits_dtype = torch.float32
-        self.train_precision = "fp32"   # activation dtype of the training step: "fp32" | "bf16"
+        self.train_precision = "fp32"   # activation dtype of the training step: "fp32" | "bf16" | "fp16"
         self.use_cuda_graph = False  # replay a captured kernel schedule per input shape (static output buffers)
         self.sub_batch = 0           # > 0: run the schedule over chunks of this many images (L2-resident activations)
         self.__dict__["_engine"] = None

@@ -8,8 +8,10 @@ tensors and returns one fp32 gradient per parameter, so ``loss.backward()``, ``G
 the reference module.  PyTorch supplies memory, streams and the autograd hand-off only: every arithmetic step is a
 kernel of ``libcabinet_b200.so`` (``csrc/train.cu`` + the forward kernels of the inference path).
 
-Layout: NHWC activations (fp32 in ``precision='fp32'``, bf16 in ``'bf16'``), class-logit maps / statistics / parameter
-gradients fp32.  All reductions are deterministic (fixed summation order), so a step is bit-reproducible.
+Layout: NHWC activations (fp32 in ``precision='fp32'``, bf16 in ``'bf16'``, fp16 in ``'fp16'``), class-logit maps /
+statistics / parameter gradients fp32.  ``'fp16'`` is the ``'bf16'`` schedule with fp16 storage and fp16 tensor-core
+operands: the numerics of the reference's ``autocast`` + ``GradScaler`` recipe (an overflow reaches the parameter
+gradients as inf / NaN, so ``GradScaler`` skips the step).  All reductions are deterministic (fixed summation order), so a step is bit-reproducible.
 
 The step is ~660 C-ABI calls; enqueueing them from Python takes ~19 ms against ~21 ms of GPU work, and the small layers
 at the end of the network leave the GPU waiting for the host.  After ``graph_after`` eager steps with the same input
@@ -29,9 +31,9 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import ACT_HSIGMOID, ACT_HSWISH, ACT_NONE, ACT_RELU, ACT_SIGMOID, BF16, F32, check
+from ._lib import ACT_HSIGMOID, ACT_HSWISH, ACT_NONE, ACT_RELU, ACT_SIGMOID, BF16, F16, F32, check
 from .constants import BN_EPS
-from .engine import Map, _out_size
+from .engine import Map, _out_size, dtype_code
 
 BN_MOMENTUM = 0.1  # nn.BatchNorm2d default (the reference never overrides it)
 PSP_SIZES = (1, 3, 6, 8)  # reference: src/models/cab.py:49
@@ -124,15 +126,16 @@ class _Grads:
 
 class TrainEngine:
     def __init__(self, model, precision: str = "fp32"):
-        if precision not in ("bf16", "fp32"):
-            raise ValueError(f"precision must be 'bf16' or 'fp32', got {precision!r}")
+        if precision not in ("bf16", "fp16", "fp32"):
+            raise ValueError(f"precision must be 'bf16', 'fp16' or 'fp32', got {precision!r}")
         p0 = next(model.parameters())
         if not p0.is_cuda:
             raise RuntimeError("cabinet_b200 training needs the model on a CUDA device (no CPU path)")
         self.lib = _lib.load()
         self.model, self.dev, self.precision = model, p0.device, precision
-        self.tdt = torch.bfloat16 if precision == "bf16" else torch.float32
-        self.dt = BF16 if precision == "bf16" else F32
+        # the activation dtype, in one place: every 2-byte buffer and operand of the schedule follows it
+        self.tdt = {"bf16": torch.bfloat16, "fp16": torch.float16, "fp32": torch.float32}[precision]
+        self.dt = dtype_code(self.tdt)
         self.n_classes = model.n_classes
         self.tables = _Tables(self.dev)
         self.tape: List = []
@@ -142,7 +145,7 @@ class TrainEngine:
         self._bn_seen: List[torch.Tensor] = []
         self.launches = 0
         self.trace, self.phase = None, "fwd"
-        self.use_tc = precision == "bf16"   # tcgen05 / TMA kernels for the GEMM-shaped and depthwise layers
+        self.use_tc = precision != "fp32"   # tcgen05 / TMA kernels for the GEMM-shaped and depthwise layers
         self.wgrad_tc = True                # tcgen05 weight gradients (stride-1 "same" and stride-2 convolutions)
         self.stem_gemm = True               # both stems as 1x1 GEMMs on one bf16 im2col of the input
         self.dgrad_s2_tc = True             # stride-2 data gradients as four parity-class conv_tc calls
@@ -177,6 +180,14 @@ class TrainEngine:
             rc = getattr(self.lib, name)(*args, self.stream)
         check(rc, name)
         self.launches += 1
+
+    def _call_tc(self, name: str, *args):
+        """A tensor-core / staging entry point with 2-byte operands: the bf16 schedule calls ``name`` itself, the fp16
+        schedule its ``name + '_dt'`` variant with the operand type appended."""
+        if self.dt == F16:
+            self._call(name + "_dt", *args, F16)
+        else:
+            self._call(name, *args)
 
     def start_trace(self):
         self.trace = []
@@ -231,7 +242,7 @@ class TrainEngine:
 
     @staticmethod
     def _dt(t: torch.Tensor) -> int:
-        return BF16 if t.dtype == torch.bfloat16 else F32
+        return dtype_code(t.dtype)
 
     # ------------------------------------------------------------------ ops (forward + tape entry)
     def _zeros(self, n: int) -> torch.Tensor:
@@ -242,11 +253,11 @@ class TrainEngine:
 
     @staticmethod
     def _tc_ok(m: Map) -> bool:
-        return m.dt == BF16 and m.ld % 8 == 0 and m.off % 8 == 0 and m.t.data_ptr() % 16 == 0
+        return m.dt in (BF16, F16) and m.ld % 8 == 0 and m.off % 8 == 0 and m.t.data_ptr() % 16 == 0
 
     def conv(self, x: Optional[Map], conv, out: Optional[Map] = None, out_dtype=None, nchw: Optional[torch.Tensor] = None,
              need_dx: bool = True) -> Map:
-        """nn.Conv2d (bias optional) on an NHWC map or the fp32 NCHW network input.  bf16 mode: forward and the stride-1
+        """nn.Conv2d (bias optional) on an NHWC map or the fp32 NCHW network input.  bf16 / fp16 mode: forward and the stride-1
         data gradient run on the tensor cores (cabinet_conv_tc; the data gradient of a stride-1 convolution is the
         convolution of dy with the transposed, mirrored weights); fp32 mode and the remaining cases: CUDA-core kernels."""
         w, b = conv.weight, conv.bias
@@ -268,12 +279,12 @@ class TrainEngine:
               and (out.dt == F32 or self._tc_ok(out)))
         if tc:
             r16, k64 = -(-cout // 16) * 16, -(-cin // 64) * 64
-            wp = torch.empty((r16, taps, k64), dtype=torch.bfloat16, device=self.dev)
-            self._call("cabinet_pack_conv_weight", w.data_ptr(), cout, cin, kh, kw, wp.data_ptr(), BF16, r16, k64, 0)
-            self._call("cabinet_conv_tc", x.ptr, x.ld, N, H, W, cin, wp.data_ptr(), cout, kh, kw, stride, pad,
-                       (bias if bias is not None else self._zeros(cout)).data_ptr(), None, 0, out.ptr, out.dt, out.ld, OH, OW,
-                       ACT_NONE)
-            wdt, w_sco, w_stap = BF16, taps * k64, k64
+            wp = torch.empty((r16, taps, k64), dtype=self.tdt, device=self.dev)
+            self._call("cabinet_pack_conv_weight", w.data_ptr(), cout, cin, kh, kw, wp.data_ptr(), self.dt, r16, k64, 0)
+            self._call_tc("cabinet_conv_tc", x.ptr, x.ld, N, H, W, cin, wp.data_ptr(), cout, kh, kw, stride, pad,
+                          (bias if bias is not None else self._zeros(cout)).data_ptr(), None, 0, out.ptr, out.dt, out.ld, OH, OW,
+                          ACT_NONE)
+            wdt, w_sco, w_stap = self.dt, taps * k64, k64
         else:
             wp = torch.empty((cout, taps, cin), dtype=torch.float32, device=self.dev)
             self._call("cabinet_pack_conv_weight", w.data_ptr(), cout, cin, kh, kw, wp.data_ptr(), F32, cout, cin, 0)
@@ -295,8 +306,8 @@ class TrainEngine:
                         and ((stride == 1 and 2 * pad == kh - 1) or (stride == 2 and H >= 2 and W >= 2))):
                     n = int(self.lib.cabinet_conv_wgrad_tc_scratch_floats(N, H, W, cin, cout, kh, kw, stride, pad))
                     sc = torch.empty(n, dtype=torch.float32, device=self.dev)
-                    self._call("cabinet_conv_wgrad_tc", dy.ptr, dy.ld, x.ptr, x.ld, self.pgrad(w).data_ptr(), N, H, W, cin,
-                               cout, kh, kw, stride, pad, sc.data_ptr())
+                    self._call_tc("cabinet_conv_wgrad_tc", dy.ptr, dy.ld, x.ptr, x.ld, self.pgrad(w).data_ptr(), N, H, W, cin,
+                                  cout, kh, kw, stride, pad, sc.data_ptr())
                 else:
                     n = int(self.lib.cabinet_conv_wgrad_scratch_floats(N, OH, OW, cin, cout, kh, kw))
                     sc = torch.empty(n, dtype=torch.float32, device=self.dev)
@@ -304,7 +315,7 @@ class TrainEngine:
                                H, W, cin, cout, kh, kw, stride, pad, OH, OW, sc.data_ptr())
             if nchw is not None or not need_dx:
                 return
-            if dy.dt != x.dt:  # fp32 class-logit gradients into a bf16 activation gradient (pixel stride padded to 8)
+            if dy.dt != x.dt:  # fp32 class-logit gradients into a 2-byte activation gradient (pixel stride padded to 8)
                 dyc = Map(torch.empty((N, OH, OW, -(-cout // 8) * 8), dtype=x.t.dtype, device=self.dev), N, OH, OW, cout,
                           -(-cout // 8) * 8)
                 self._call("cabinet_affine_act", dy.ptr, dy.ld, dy.dt, None, None, None, 0.0, None, 0, dyc.ptr, dyc.ld,
@@ -313,11 +324,11 @@ class TrainEngine:
             dx, acc = g.out(x)
             if self.use_tc and stride == 1 and self._tc_ok(dy) and self._tc_ok(dx) and (OH, OW) == (H, W):
                 r16, k64 = -(-cin // 16) * 16, -(-cout // 64) * 64
-                wt = torch.empty((r16, taps, k64), dtype=torch.bfloat16, device=self.dev)
-                self._call("cabinet_pack_conv_weight", w.data_ptr(), cout, cin, kh, kw, wt.data_ptr(), BF16, r16, k64, 1)
-                self._call("cabinet_conv_tc", dy.ptr, dy.ld, N, H, W, cout, wt.data_ptr(), cin, kh, kw, 1, kh - 1 - pad,
-                           self._zeros(cin).data_ptr(), dx.ptr if acc else None, dx.ld if acc else 0, dx.ptr, dx.dt, dx.ld,
-                           H, W, ACT_NONE)
+                wt = torch.empty((r16, taps, k64), dtype=self.tdt, device=self.dev)
+                self._call("cabinet_pack_conv_weight", w.data_ptr(), cout, cin, kh, kw, wt.data_ptr(), self.dt, r16, k64, 1)
+                self._call_tc("cabinet_conv_tc", dy.ptr, dy.ld, N, H, W, cout, wt.data_ptr(), cin, kh, kw, 1, kh - 1 - pad,
+                              self._zeros(cin).data_ptr(), dx.ptr if acc else None, dx.ld if acc else 0, dx.ptr, dx.dt, dx.ld,
+                              H, W, ACT_NONE)
                 return
             if (self.use_tc and self.dgrad_s2_tc and stride == 2 and kh == kw and not acc and self._tc_ok(dy)
                     and self._tc_ok(dx) and H >= 2 and W >= 2 and self._parity_pads(kh, pad) is not None):
@@ -330,12 +341,12 @@ class TrainEngine:
                         hc, wc = (H - py + 1) // 2, (W - px + 1) // 2
                         if hc == 0 or wc == 0:
                             continue
-                        wt = torch.empty((r16, kh2 * kw2, k64), dtype=torch.bfloat16, device=self.dev)
-                        self._call("cabinet_pack_conv_weight_parity", w.data_ptr(), cout, cin, kh, pad, py, px, kh2, kw2, pad2,
-                                   wt.data_ptr(), r16, k64)
+                        wt = torch.empty((r16, kh2 * kw2, k64), dtype=self.tdt, device=self.dev)
+                        self._call_tc("cabinet_pack_conv_weight_parity", w.data_ptr(), cout, cin, kh, pad, py, px, kh2, kw2,
+                                      pad2, wt.data_ptr(), r16, k64)
                         view = dx.ptr + (py * W + px) * dx.ld * 2
-                        self._call("cabinet_conv_tc_view", dy.ptr, dy.ld, N, OH, OW, cout, wt.data_ptr(), cin, kh2, kw2, pad2,
-                                   self._zeros(cin).data_ptr(), view, dx.ld, hc, wc, 2, 2 * W, H * W)
+                        self._call_tc("cabinet_conv_tc_view", dy.ptr, dy.ld, N, OH, OW, cout, wt.data_ptr(), cin, kh2, kw2,
+                                      pad2, self._zeros(cin).data_ptr(), view, dx.ld, hc, wc, 2, 2 * W, H * W)
                 return
             self._call("cabinet_conv_dgrad", dy.ptr, dy.ld, dy.dt, wp.data_ptr(), wdt, w_sco, w_stap, dx.ptr, dx.ld, N, H, W,
                        cin, cout, kh, kw, stride, pad, OH, OW, acc)
@@ -362,14 +373,14 @@ class TrainEngine:
     STEM_K, STEM_LD = 7, 152   # im2col footprint of the stems: 3 x 7 x 7 = 147 columns, pixel stride padded to 8
 
     def stem_im2col(self, x: torch.Tensor) -> Map:
-        """bf16 im2col [N, H/2, W/2, 152] of the fp32 NCHW input over the 7x7 / stride-2 / pad-3 footprint shared by both
+        """2-byte (bf16 / fp16) im2col [N, H/2, W/2, 152] of the fp32 NCHW input over the 7x7 / stride-2 / pad-3 footprint shared by both
         stem convolutions (the 3x3 / pad-1 backbone stem is its centre): read once, used by two forward GEMMs and two
         weight-gradient GEMMs on the tensor cores."""
         N, _, H, W = x.shape
         OH, OW = _out_size(H, 7, 2, 3), _out_size(W, 7, 2, 3)
-        xcol = Map(torch.empty((N, OH, OW, self.STEM_LD), dtype=torch.bfloat16, device=self.dev), N, OH, OW, self.STEM_LD,
+        xcol = Map(torch.empty((N, OH, OW, self.STEM_LD), dtype=self.tdt, device=self.dev), N, OH, OW, self.STEM_LD,
                    self.STEM_LD)
-        self._call("cabinet_im2col_nchw", x.data_ptr(), N, 3, H, W, 7, 2, 3, xcol.ptr, xcol.ld)
+        self._call_tc("cabinet_im2col_nchw", x.data_ptr(), N, 3, H, W, 7, 2, 3, xcol.ptr, xcol.ld)
         return xcol
 
     def conv_stem(self, xcol: Map, conv) -> Map:
@@ -382,11 +393,11 @@ class TrainEngine:
         r16, k64 = -(-cout // 16) * 16, -(-LD // 64) * 64
         wbig = torch.zeros((cout, LD), dtype=torch.float32, device=self.dev)
         self.launches += 1
-        wp = torch.empty((r16, 1, k64), dtype=torch.bfloat16, device=self.dev)
+        wp = torch.empty((r16, 1, k64), dtype=self.tdt, device=self.dev)
         self._call("cabinet_embed_filter", w.data_ptr(), cout, 3, k, self.STEM_K, wbig.data_ptr(), LD, 0)
-        self._call("cabinet_pack_conv_weight", wbig.data_ptr(), cout, LD, 1, 1, wp.data_ptr(), BF16, r16, k64, 0)
-        self._call("cabinet_conv_tc", xcol.ptr, xcol.ld, N, OH, OW, LD, wp.data_ptr(), cout, 1, 1, 1, 0,
-                   self._zeros(cout).data_ptr(), None, 0, out.ptr, out.dt, out.ld, OH, OW, ACT_NONE)
+        self._call("cabinet_pack_conv_weight", wbig.data_ptr(), cout, LD, 1, 1, wp.data_ptr(), self.dt, r16, k64, 0)
+        self._call_tc("cabinet_conv_tc", xcol.ptr, xcol.ld, N, OH, OW, LD, wp.data_ptr(), cout, 1, 1, 1, 0,
+                      self._zeros(cout).data_ptr(), None, 0, out.ptr, out.dt, out.ld, OH, OW, ACT_NONE)
 
         def backward(g: _Grads):
             dy = g.get(out)
@@ -397,15 +408,15 @@ class TrainEngine:
                 self.launches += 1
                 n = int(self.lib.cabinet_conv_wgrad_tc_scratch_floats(N, OH, OW, LD, cout, 1, 1, 1, 0))
                 sc = torch.empty(n, dtype=torch.float32, device=self.dev)
-                self._call("cabinet_conv_wgrad_tc", dy.ptr, dy.ld, xcol.ptr, xcol.ld, dwbig.data_ptr(), N, OH, OW, LD, cout, 1, 1,
-                           1, 0, sc.data_ptr())
+                self._call_tc("cabinet_conv_wgrad_tc", dy.ptr, dy.ld, xcol.ptr, xcol.ld, dwbig.data_ptr(), N, OH, OW, LD, cout,
+                              1, 1, 1, 0, sc.data_ptr())
                 self._call("cabinet_embed_filter", self.pgrad(w).data_ptr(), cout, 3, k, self.STEM_K, dwbig.data_ptr(), LD, 1)
 
         self.tape.append(backward)
         return out
 
     def dwconv(self, x: Map, conv) -> Map:
-        """Depthwise nn.Conv2d (groups = C, no bias).  bf16 mode: the TMA-staged kernel forward, and for stride 1 also
+        """Depthwise nn.Conv2d (groups = C, no bias).  bf16 / fp16 mode: the TMA-staged kernel forward, and for stride 1 also
         backward (the data gradient is the depthwise convolution of dy with the mirrored filter)."""
         w = conv.weight
         C, k, stride = w.shape[0], w.shape[2], conv.stride[0]
@@ -416,8 +427,8 @@ class TrainEngine:
         self._call("cabinet_pack_dw_weight", w.data_ptr(), C, k, 0, wp.data_ptr())
         tma = self.use_tc and self._tc_ok(x) and self._tc_ok(out) and C % 8 == 0
         if tma:
-            self._call("cabinet_dwconv_tma", x.ptr, x.ld, wp.data_ptr(), self._zeros(C).data_ptr(), out.ptr, out.ld, x.N, x.H,
-                       x.W, C, k, stride, OH, OW, ACT_NONE, None)
+            self._call_tc("cabinet_dwconv_tma", x.ptr, x.ld, wp.data_ptr(), self._zeros(C).data_ptr(), out.ptr, out.ld, x.N,
+                          x.H, x.W, C, k, stride, OH, OW, ACT_NONE, None)
         else:
             self._call("cabinet_dwconv", x.ptr, x.ld, wp.data_ptr(), self._zeros(C).data_ptr(), out.ptr, out.ld, x.dt, x.N, x.H,
                        x.W, C, k, stride, OH, OW, ACT_NONE, None)
@@ -435,8 +446,8 @@ class TrainEngine:
                 wf = torch.empty((k * k, C), dtype=torch.float32, device=self.dev)
                 self._call("cabinet_pack_dw_weight", w.data_ptr(), C, k, 1, wf.data_ptr())
                 tgt = self.new(x.N, x.H, x.W, C) if acc else dx
-                self._call("cabinet_dwconv_tma", dy.ptr, dy.ld, wf.data_ptr(), self._zeros(C).data_ptr(), tgt.ptr, tgt.ld, x.N,
-                           x.H, x.W, C, k, 1, x.H, x.W, ACT_NONE, None)
+                self._call_tc("cabinet_dwconv_tma", dy.ptr, dy.ld, wf.data_ptr(), self._zeros(C).data_ptr(), tgt.ptr, tgt.ld,
+                              x.N, x.H, x.W, C, k, 1, x.H, x.W, ACT_NONE, None)
                 if acc:
                     self._call("cabinet_add", dx.ptr, dx.ld, tgt.ptr, tgt.ld, dx.ptr, dx.ld, dx.dt, x.N * x.H * x.W, C)
                 return
@@ -634,12 +645,12 @@ class TrainEngine:
         return ctx
 
     def _attention_tc(self, q: Map, k: Map, v: Map, alpha: float) -> Map:
-        """The same attention with all six GEMMs on the tensor cores (bf16 operands, fp32 accumulation): a dense [L][d] map
+        """The same attention with all six GEMMs on the tensor cores (bf16 / fp16 operands, fp32 accumulation): a dense [L][d] map
         of an image IS a cabinet_conv_tc weight matrix (rows = tokens, k = channels), so S = Q K^T and dP = dO V^T are 1x1
         convolutions with per-image weights K / V, P V and dQ = dS K the same with K^T / V^T ([d][L], one small transpose
         each), and dV = P^T dO, dK = dS^T Q reduce over the token ("pixel") index: the weight-gradient GEMM, batched per image."""
         N, L, d, H, W = q.N, q.H * q.W, q.C, q.H, q.W
-        dev, bf = self.dev, torch.bfloat16
+        dev, bf = self.dev, self.tdt
         s = torch.empty((N, L, L), dtype=torch.float32, device=dev)
         p = torch.empty((N, L, L), dtype=torch.float32, device=dev)
         p16 = torch.empty((N, L, L), dtype=bf, device=dev)
@@ -648,13 +659,13 @@ class TrainEngine:
         zL, zd = self._zeros(L), self._zeros(d)
 
         def gemm(x_ptr, ldx, cin, w_ptr, cout, bias, y_ptr, ydt, ldy):
-            # y[n][l][co] = sum_k x[n][l][k] w[n][co][k]   (w: [N][cout][cin] bf16, dense)
-            self._call("cabinet_conv_tc_imgw", x_ptr, ldx, N, H, W, cin, w_ptr, cout * cin, cout, 1, 1, 1, 0, bias.data_ptr(),
-                       None, 0, y_ptr, ydt, ldy, H, W, ACT_NONE)
+            # y[n][l][co] = sum_k x[n][l][k] w[n][co][k]   (w: [N][cout][cin] 2-byte, dense)
+            self._call_tc("cabinet_conv_tc_imgw", x_ptr, ldx, N, H, W, cin, w_ptr, cout * cin, cout, 1, 1, 1, 0,
+                          bias.data_ptr(), None, 0, y_ptr, ydt, ldy, H, W, ACT_NONE)
 
         gemm(q.ptr, q.ld, d, k.ptr, L, zL, s.data_ptr(), F32, L)
-        self._call("cabinet_attn_softmax", s.data_ptr(), alpha, p.data_ptr(), p16.data_ptr(), N * L, L)
-        self._call("cabinet_transpose_tokens", v.ptr, v.ld, vt.data_ptr(), N, L, d)
+        self._call_tc("cabinet_attn_softmax", s.data_ptr(), alpha, p.data_ptr(), p16.data_ptr(), N * L, L)
+        self._call_tc("cabinet_transpose_tokens", v.ptr, v.ld, vt.data_ptr(), N, L, d)
         gemm(p16.data_ptr(), L, L, vt.data_ptr(), d, zd, ctx.ptr, ctx.dt, ctx.ld)
 
         def backward(g: _Grads):
@@ -668,12 +679,12 @@ class TrainEngine:
             dkv = torch.empty((2, N, L, d), dtype=torch.float32, device=dev)
 
             def wgrad(a, x_map, out):  # out[n][j][c] = sum_i a[n][i][j] x[n][i][c]
-                self._call("cabinet_conv_wgrad_tc_batched", a.data_ptr(), L, x_map.ptr, x_map.ld, out.data_ptr(), N, H, W, d, L)
+                self._call_tc("cabinet_conv_wgrad_tc_batched", a.data_ptr(), L, x_map.ptr, x_map.ld, out.data_ptr(), N, H, W, d, L)
 
             wgrad(p16, do, dkv[1])                                                # dV[j][c] = sum_i P[i][j] dO[i][c]
             gemm(do.ptr, do.ld, d, v.ptr, L, zL, dp.data_ptr(), F32, L)           # dP[i][j] = sum_c dO[i][c] V[j][c]
-            self._call("cabinet_attn_softmax_backward", p.data_ptr(), dp.data_ptr(), ds16.data_ptr(), N * L, L, alpha)
-            self._call("cabinet_transpose_tokens", k.ptr, k.ld, kt.data_ptr(), N, L, d)
+            self._call_tc("cabinet_attn_softmax_backward", p.data_ptr(), dp.data_ptr(), ds16.data_ptr(), N * L, L, alpha)
+            self._call_tc("cabinet_transpose_tokens", k.ptr, k.ld, kt.data_ptr(), N, L, d)
             gemm(ds16.data_ptr(), L, L, kt.data_ptr(), d, zd, dq.ptr, dq.dt, dq.ld)  # dQ[i][c] = sum_j dS[i][j] K[j][c]
             wgrad(ds16, q, dkv[0])                                                # dK[j][c] = sum_i dS[i][j] Q[i][c]
             dk, dv = self.new(N, H, W, d), self.new(N, H, W, d)

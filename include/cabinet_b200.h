@@ -9,7 +9,10 @@
  *
  * Activations are NHWC; `ld*` arguments are the PIXEL stride in elements (>= channels), which is
  * how channel-concatenation (reference torch.cat) is expressed without a copy.  Element types are
- * CABINET_F32 or CABINET_BF16.  The reference is pure PyTorch (SURVEY F1): each entry point cites
+ * CABINET_F32, CABINET_BF16 and, in the training entry points the fp16 training mode calls, CABINET_F16; an entry point
+ * given a type it does not implement returns CABINET_ERR_INVALID before it launches anything.  The `*_dt` variants of
+ * the tensor-core and staging entry points take the 2-byte operand type (CABINET_BF16 or CABINET_F16) as their last
+ * argument before `stream`; the names without the suffix are the CABINET_BF16 case.  The reference is pure PyTorch (SURVEY F1): each entry point cites
  * the reference Python it replaces (paths relative to the reference repo root); there is no
  * pre-existing FFI in the reference, INTEGRATION.md shows the binding a maintainer would add.
  */
@@ -25,7 +28,7 @@ extern "C" {
 #define CABINET_ABI_VERSION 2
 
 enum { CABINET_OK = 0, CABINET_ERR_INVALID = 1, CABINET_ERR_CUDA = 2 };
-enum { CABINET_F32 = 0, CABINET_BF16 = 1 };
+enum { CABINET_F32 = 0, CABINET_BF16 = 1, CABINET_F16 = 2 };
 enum {
     CABINET_ACT_NONE = 0,
     CABINET_ACT_RELU = 1,     /* nn.ReLU */
@@ -84,6 +87,10 @@ int cabinet_conv2d_simt(const void* x, int x_dtype, long long sxn, long long sxh
 int cabinet_conv_tc(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed, int Cout,
                     int KH, int KW, int stride, int pad, const float* bias, const void* res, long long ldres,
                     void* y, int y_dtype, long long ldy, int OH, int OW, int act, cabinet_stream_t stream);
+/* The same with bf16 or fp16 operands (op_dtype; x, w_packed and a 2-byte y all of that type). */
+int cabinet_conv_tc_dt(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed, int Cout,
+                       int KH, int KW, int stride, int pad, const float* bias, const void* res, long long ldres,
+                       void* y, int y_dtype, long long ldy, int OH, int OW, int act, int op_dtype, cabinet_stream_t stream);
 
 /* cabinet_conv_tc (stride 1, no activation / residual, bf16) writing a strided VIEW of a larger NHWC tensor: output pixel
  * (n, oh, ow) lands at y + ((n * y_sn) + oh * y_sh + ow * y_sw) * ldy (pitches in pixels).  With the sub-filters of
@@ -92,6 +99,9 @@ int cabinet_conv_tc(const void* x, long long ldx, int N, int H, int W, int Cin, 
 int cabinet_conv_tc_view(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed, int Cout, int KH,
                          int KW, int pad, const float* bias, void* y, long long ldy, int OH, int OW, long long y_sw,
                          long long y_sh, long long y_sn, cabinet_stream_t stream);
+int cabinet_conv_tc_view_dt(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed, int Cout, int KH,
+                            int KW, int pad, const float* bias, void* y, long long ldy, int OH, int OW, long long y_sw,
+                            long long y_sh, long long y_sn, int op_dtype, cabinet_stream_t stream);
 
 /* cabinet_conv_tc with the squeeze-excite apply fused in front (A-operand prologue): the GEMM consumes
  * act(x[n][p][c] * a_scale[n][c]) (a_scale fp32 [N][Cin]) without that tensor ever being written:
@@ -138,6 +148,9 @@ int cabinet_dwconv(const void* x, long long ldx, const float* w, const float* bi
 int cabinet_dwconv_tma(const void* x, long long ldx, const float* w, const float* bias, void* y, long long ldy, int N,
                        int H, int W, int C, int k, int stride, int OH, int OW, int act, long long* gap_sum,
                        cabinet_stream_t stream);
+int cabinet_dwconv_tma_dt(const void* x, long long ldx, const float* w, const float* bias, void* y, long long ldy, int N,
+                          int H, int W, int C, int k, int stride, int OH, int OW, int act, long long* gap_sum, int op_dtype,
+                          cabinet_stream_t stream);
 
 /* Whole no-expand inverted-residual block in one kernel (inp == hidden, no SE, stride 1, identity):
  *   y = x + W_pw * act(dw3x3(x) + b_dw) + b_pw     (src/models/mobilenetv3.py:110-125,154-159; Large f1)
@@ -173,6 +186,10 @@ int cabinet_conv_tc_imgw(const void* x, long long ldx, int N, int H, int W, int 
                          long long w_image_stride, int Cout, int KH, int KW, int stride, int pad, const float* bias,
                          const void* res, long long ldres, void* y, int y_dtype, long long ldy, int OH, int OW, int act,
                          cabinet_stream_t stream);
+int cabinet_conv_tc_imgw_dt(const void* x, long long ldx, int N, int H, int W, int Cin, const void* w_packed_per_image,
+                            long long w_image_stride, int Cout, int KH, int KW, int stride, int pad, const float* bias,
+                            const void* res, long long ldres, void* y, int y_dtype, long long ldy, int OH, int OW, int act,
+                            int op_dtype, cabinet_stream_t stream);
 
 /* out[n][r][t][c] = bf16(w[r][t][c] * (scale[n][c] + plus_one)): per-image copies of a cabinet_conv_tc weight pack
  * ([rows][taps][cin_pad] bf16, cin_pad % 8 == 0; channels >= Cin stay 0); scale is fp32 [N][Cin]. */
@@ -373,7 +390,7 @@ int cabinet_ohem_ce_backward(const void* logits, int dtype, const void* labels, 
 
 /* ---------------------------------------------------------------------------------------------
  * Training step (BASELINE config 5; src/scripts/train.py:429-441: net(im) in .train() mode -> 2 x OhemCELoss ->
- * backward).  NHWC activations (fp32 or bf16), fp32 statistics and parameter gradients.  Every reduction has a fixed
+ * backward).  NHWC activations (fp32, bf16 or fp16), fp32 statistics and parameter gradients.  Every reduction has a fixed
  * summation order (two-level sums, no floating-point atomics).  Scratch buffers are uninitialised device memory of
  * cabinet_train_scratch_floats(rows, C, quantities) floats unless stated otherwise.
  */
@@ -394,6 +411,9 @@ int cabinet_pack_dw_weight(const float* w, int C, int k, int flip, float* out, c
  * (zero outside the filter): dx[2a+py][2b+px] = conv(dy, out, pad2)[a][b]. */
 int cabinet_pack_conv_weight_parity(const float* w_oihw, int Cout, int Cin, int K, int pad, int py, int px, int KH2, int KW2,
                                     int pad2, void* out, int rows_pad, int k_pad, cabinet_stream_t stream);
+int cabinet_pack_conv_weight_parity_dt(const float* w_oihw, int Cout, int Cin, int K, int pad, int py, int px, int KH2,
+                                       int KW2, int pad2, void* out, int rows_pad, int k_pad, int out_dtype,
+                                       cabinet_stream_t stream);
 
 /* im2col of the fp32 NCHW network input for the stem convolutions (sb.conv1 7x7 s2 p3, src/models/cabinet.py:111; backbone
  * stem 3x3 s2 p1 = the centre of the same footprint, src/models/mobilenetv3.py:86-91): out bf16 [N*OH*OW][ld], column
@@ -403,6 +423,8 @@ int cabinet_pack_conv_weight_parity(const float* w_oihw, int Cout, int Cin, int 
  * w_small += that slice of w_big (extract_add = 1: the gradient of the embedded filter). */
 int cabinet_im2col_nchw(const float* x, int N, int Cin, int H, int W, int k, int stride, int pad, void* out, long long ld,
                         cabinet_stream_t stream);
+int cabinet_im2col_nchw_dt(const float* x, int N, int Cin, int H, int W, int k, int stride, int pad, void* out, long long ld,
+                           int out_dtype, cabinet_stream_t stream);
 int cabinet_embed_filter(float* w_small, int Cout, int Cin, int k, int K, float* w_big, long long ld_big, int extract_add,
                          cabinet_stream_t stream);
 
@@ -466,12 +488,17 @@ int cabinet_conv_wgrad(const void* dy, long long lddy, int dtype, const void* x,
 long long cabinet_conv_wgrad_tc_scratch_floats(int N, int H, int W, int Cin, int Cout, int KH, int KW, int stride, int pad);
 int cabinet_conv_wgrad_tc(const void* dy, long long lddy, const void* x, long long ldx, float* dw_oihw, int N, int H, int W,
                           int Cin, int Cout, int KH, int KW, int stride, int pad, float* scratch, cabinet_stream_t stream);
+int cabinet_conv_wgrad_tc_dt(const void* dy, long long lddy, const void* x, long long ldx, float* dw_oihw, int N, int H,
+                             int W, int Cin, int Cout, int KH, int KW, int stride, int pad, float* scratch, int op_dtype,
+                             cabinet_stream_t stream);
 
 /* Batched form for per-image products (training-mode attention: dV = P^T dO, dK = dS^T Q, src/models/cab.py:149-153):
  * out[n][co][ci] = sum over the H * W pixels of image n of a[n][pix][co] * x[n][pix][ci]   (fp32, overwritten; one launch,
  * no second-level sum).  H * W must be a multiple of 64. */
 int cabinet_conv_wgrad_tc_batched(const void* a, long long lda, const void* x, long long ldx, float* out, int N, int H, int W,
                                   int Cin, int Cout, cabinet_stream_t stream);
+int cabinet_conv_wgrad_tc_batched_dt(const void* a, long long lda, const void* x, long long ldx, float* out, int N, int H,
+                                     int W, int Cin, int Cout, int op_dtype, cabinet_stream_t stream);
 
 /* Depthwise convolution gradients; w_packed [k*k][C] fp32; dw ([C][1][k][k] fp32) +=; scratch: (N*OH*OW, C, k*k). */
 int cabinet_dwconv_dgrad(const void* dy, long long lddy, int dtype, const float* w_packed, void* dx, long long lddx, int N,
@@ -508,6 +535,13 @@ int cabinet_attn_softmax(const float* s, float scale, float* p, void* p_bf16, lo
 int cabinet_attn_softmax_backward(const float* p, const float* dp, void* ds_bf16, long long rows, int cols, float alpha,
                                   cabinet_stream_t stream);
 int cabinet_transpose_tokens(const void* x, long long ldx, void* out, int N, int L, int C, cabinet_stream_t stream);
+/* The same with the 2-byte outputs / operands of type op_dtype (CABINET_BF16 or CABINET_F16). */
+int cabinet_attn_softmax_dt(const float* s, float scale, float* p, void* p_half, long long rows, int cols, int op_dtype,
+                            cabinet_stream_t stream);
+int cabinet_attn_softmax_backward_dt(const float* p, const float* dp, void* ds_half, long long rows, int cols, float alpha,
+                                     int op_dtype, cabinet_stream_t stream);
+int cabinet_transpose_tokens_dt(const void* x, long long ldx, void* out, int N, int L, int C, int op_dtype,
+                                cabinet_stream_t stream);
 
 /* Backward of out = gamma * g + x + x * sigmoid(r) (cab.py:175-184,213-216), dense [n_pixels][C] operands:
  * dg = gamma * dout, dx (+)= dout * (1 + sigmoid(r)), dr = dout * x * sigmoid'(r), *dgamma += sum dout * g.
