@@ -2,6 +2,7 @@
 // two OHEM losses, backward).  Everything the inference path does not have:
 //   * train-mode BatchNorm: batch statistics (shifted single pass, deterministic two-level sums), running-statistics
 //     update (momentum 0.1, unbiased variance), normalise + activation, and its backward (two reductions + apply);
+//   * eval-mode BatchNorm inside a training step (frozen BN): statistics from the running statistics, one-pass backward;
 //   * data gradients and weight gradients of the dense and depthwise convolutions (CUDA-core implicit GEMM with
 //     fp32 accumulation; split over the pixel dimension with a fixed-order second-level sum for the weight gradients);
 //   * squeeze-excite / FFM gate backward, CAB combine backward, softmax backward, the adjoints of every bilinear
@@ -529,8 +530,8 @@ affine_act_v_kernel(const TZ* __restrict__ z, long long ldz, const float* __rest
     }
 }
 
-// sums the block partials in order; dgamma / dbeta accumulate into the parameter gradients; coef[2][C] = the two
-// per-channel means the apply kernel subtracts
+// sums the block partials in order; dgamma / dbeta accumulate into the parameter gradients; coef[2][C] (may be NULL) =
+// the two per-channel means the apply kernel subtracts
 __global__ void bn_bwd_finalize_kernel(const float* __restrict__ partial, int nb, long long M, int C,
                                        float* __restrict__ dgamma, float* __restrict__ dbeta, float* __restrict__ coef) {
     const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;  // one warp per channel
@@ -560,6 +561,7 @@ __global__ void bn_bwd_finalize_kernel(const float* __restrict__ partial, int nb
     if (lane != 0) return;
     if (dbeta) dbeta[c] += s1;
     if (dgamma) dgamma[c] += s2;
+    if (!coef) return;  // eval-mode BN: its dz needs no means
     coef[c] = s1 / static_cast<float>(M);
     coef[C + c] = s2 / static_cast<float>(M);
 }
@@ -582,6 +584,106 @@ bn_bwd_apply_kernel(const T* __restrict__ dy, long long lddy, const T* __restric
         T* o = dz + m * lddz + c;
         if (accumulate) v += ldf(o);
         *o = from_f32<T>(v);
+    }
+}
+
+// ---- eval-mode BatchNorm: stats[4][C] from the running statistics (the layout bn_finalize_kernel writes), on the device
+// so that a replayed graph reads the running statistics of replay time
+__global__ void bn_frozen_stats_kernel(const float* __restrict__ gamma, const float* __restrict__ beta,
+                                       const float* __restrict__ run_mean, const float* __restrict__ run_var, float eps, int C,
+                                       float* __restrict__ stats) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    const float mean = run_mean[c];
+    const float invstd = static_cast<float>(1.0 / sqrt(static_cast<double>(run_var[c]) + static_cast<double>(eps)));
+    const float g = gamma ? gamma[c] : 1.f, bt = beta ? beta[c] : 0.f;
+    stats[c] = mean;
+    stats[C + c] = invstd;
+    stats[2 * C + c] = g * invstd;
+    stats[3 * C + c] = bt - mean * g * invstd;
+}
+
+// ---- eval-mode BatchNorm (+activation) backward.  The statistics do not depend on z, so dz (+)= scale * g needs no
+// column sum: ONE pass writes dz and (RED) the block partials of sum g and sum g * xhat (dbeta, dgamma; level 2 is
+// bn_bwd_finalize_kernel).  dz may be NULL (parameter gradients only).  RED = false: an elementwise grid-stride pass.
+template <typename T, bool RED>
+__global__ void __launch_bounds__(RED_THREADS)
+bn_frozen_bwd_kernel(const T* __restrict__ dy, long long lddy, const T* __restrict__ z, long long ldz,
+                     const float* __restrict__ stats, int act, T* __restrict__ dz, long long lddz, long long M, int C,
+                     int accumulate, long long rpb, float* __restrict__ partial) {
+    auto one = [&](long long m, int c, float* acc) {
+        const float zv = ldf(z + m * ldz + c);
+        const float sc = stats[2 * C + c];
+        const float g = ldf(dy + m * lddy + c) * act_grad(fmaf(zv, sc, stats[3 * C + c]), act);
+        if (dz) {
+            T* o = dz + m * lddz + c;
+            float r = __fmul_rn(sc, g);  // never fused into the add: every path rounds dz the same way
+            if (accumulate) r += ldf(o);
+            *o = from_f32<T>(r);
+        }
+        if (RED) {
+            acc[0] += g;
+            acc[1] = fmaf(g, (zv - stats[c]) * stats[C + c], acc[1]);
+        }
+    };
+    if constexpr (RED) {
+        col_reduce_block<2>(M, C, rpb, partial, one);
+    } else {
+        float acc[2];
+        const long long total = M * C;
+        for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
+             i += static_cast<long long>(gridDim.x) * blockDim.x) {
+            const long long m = i / C;
+            one(m, static_cast<int>(i - m * C), acc);
+        }
+    }
+}
+
+// 16-byte vectorised form (C / V <= RED_THREADS, C and every pixel stride a multiple of V, 16-byte aligned bases)
+template <typename T, bool RED>
+__global__ void __launch_bounds__(RED_THREADS)
+bn_frozen_bwd_v_kernel(const T* __restrict__ dy, long long lddy, const T* __restrict__ z, long long ldz,
+                       const float* __restrict__ stats, int act, T* __restrict__ dz, long long lddz, long long M, int C,
+                       int accumulate, long long rpb, float* __restrict__ partial) {
+    constexpr int V = vec_n<T>();
+    float mean[V], invstd[V], scale[V], shift[V];   // per-channel constants of this thread's vector, loaded once
+    int kc = -1;
+    auto one = [&](long long m, int c0, float* acc) {
+        if (c0 != kc) {
+#pragma unroll
+            for (int v = 0; v < V; ++v) {
+                mean[v] = stats[c0 + v]; invstd[v] = stats[C + c0 + v]; scale[v] = stats[2 * C + c0 + v]; shift[v] = stats[3 * C + c0 + v];
+            }
+            kc = c0;
+        }
+        float zv[V], dv[V], u[V], ag[V], o[V];
+        ldv(z + m * ldz + c0, zv);
+        ldv(dy + m * lddy + c0, dv);
+        if (dz && accumulate) ldv(dz + m * lddz + c0, o);
+#pragma unroll
+        for (int v = 0; v < V; ++v) u[v] = fmaf(zv[v], scale[v], shift[v]);
+        act_grad_vec<V>(u, act, ag);
+#pragma unroll
+        for (int v = 0; v < V; ++v) {
+            const float g = dv[v] * ag[v];
+            if (RED) {
+                acc[v] += g;
+                acc[V + v] = fmaf(g, (zv[v] - mean[v]) * invstd[v], acc[V + v]);
+            }
+            const float r = __fmul_rn(scale[v], g);
+            o[v] = accumulate ? o[v] + r : r;
+        }
+        if (dz) stv(dz + m * lddz + c0, o);
+    };
+    if constexpr (RED) {
+        col_reduce_block_v<2, V>(M, C, rpb, partial, one);
+    } else {
+        const int CV = C / V;
+        const int cv = threadIdx.x % CV, lane = threadIdx.x / CV, lanes = blockDim.x / CV;
+        if (lane >= lanes) return;
+        float acc[2 * V];
+        for (long long m = static_cast<long long>(blockIdx.x) * lanes + lane; m < M; m += static_cast<long long>(gridDim.x) * lanes)
+            one(m, cv * V, acc);
     }
 }
 
@@ -2097,6 +2199,55 @@ extern "C" int cabinet_bn_train_backward(const void* dy, long long lddy, const v
                 bn_bwd_apply_kernel<T><<<g, 256, 0, s>>>(reinterpret_cast<const T*>(dy), lddy, reinterpret_cast<const T*>(z), ldz,
                                                             stats, coef, act, reinterpret_cast<T*>(dz), lddz, M, C, accumulate));
     }
+    CAB_LAUNCH_CHECK();
+    return CABINET_OK;
+}
+
+extern "C" int cabinet_bn_frozen_stats(const float* gamma, const float* beta, const float* running_mean,
+                                       const float* running_var, float eps, int C, float* stats, cabinet_stream_t stream) {
+    CAB_REQUIRE(running_mean && running_var && stats && C > 0 && eps >= 0.f, "bn_frozen_stats: bad arguments");
+    bn_frozen_stats_kernel<<<static_cast<unsigned>(cab_ceil_div(C, 256)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+            gamma, beta, running_mean, running_var, eps, C, stats);
+    CAB_LAUNCH_CHECK();
+    return CABINET_OK;
+}
+
+extern "C" int cabinet_bn_frozen_backward(const void* dy, long long lddy, const void* z, long long ldz, int dtype,
+                                          const float* stats, int act, float* dgamma, float* dbeta, void* dz,
+                                          long long lddz, long long M, int C, int accumulate, float* scratch,
+                                          cabinet_stream_t stream) {
+    CAB_REQUIRE_DTYPE("bn_frozen_backward", dtype, CAB_DT_ALL);
+    const bool red = dgamma || dbeta;
+    CAB_REQUIRE(dy && z && stats && (red || dz) && (!red || scratch) && M > 0 && C > 0 && lddy >= C && ldz >= C &&
+                        (!dz || lddz >= C),
+                "bn_frozen_backward: bad arguments");
+    long long rpb;
+    const int nb = red_blocks(M, &rpb);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int V = dtype == CABINET_F32 ? 4 : 8;
+    const bool vec = C % V == 0 && C / V <= RED_THREADS && lddy % V == 0 && ldz % V == 0 && al16(dy) && al16(z) &&
+                     (!dz || (lddz % V == 0 && al16(dz)));
+#define CAB_FB(KERNEL, RED, GRID, SMEM)                                                                                  \
+    CAB_DISPATCH_DT(dtype, T,                                                                                            \
+                    KERNEL<T, RED><<<GRID, RED_THREADS, SMEM, s>>>(reinterpret_cast<const T*>(dy), lddy,                 \
+                                                                   reinterpret_cast<const T*>(z), ldz, stats, act,       \
+                                                                   reinterpret_cast<T*>(dz), lddz, M, C, accumulate, rpb, \
+                                                                   scratch))
+    if (red) {
+        if (vec) {
+            CAB_FB(bn_frozen_bwd_v_kernel, true, nb, red_smem_v<T>(2));
+        } else {
+            CAB_FB(bn_frozen_bwd_kernel, true, nb, RED_SMEM);
+        }
+        CAB_LAUNCH_CHECK();
+        bn_bwd_finalize_kernel<<<static_cast<unsigned>(cab_ceil_div(C, 4)), 128, 0, s>>>(scratch, nb, M, C, dgamma, dbeta,
+                                                                                          nullptr);
+    } else if (vec) {
+        CAB_FB(bn_frozen_bwd_v_kernel, false, row_grid(M, RED_THREADS / (C / V)), 0);
+    } else {
+        CAB_FB(bn_frozen_bwd_kernel, false, ew_grid(M * C), 0);
+    }
+#undef CAB_FB
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }

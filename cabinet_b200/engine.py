@@ -46,6 +46,7 @@ class Map:
     C: int
     ld: int
     off: int = 0  # channel offset inside the pixel
+    needs_grad: bool = False  # training step: the map depends on a parameter that requires grad
 
     @property
     def dt(self) -> int:
@@ -56,7 +57,7 @@ class Map:
         return self.t.data_ptr() + self.off * self.t.element_size()
 
     def slice(self, c0: int, c: int) -> "Map":
-        return Map(self.t, self.N, self.H, self.W, c, self.ld, self.off + c0)
+        return Map(self.t, self.N, self.H, self.W, c, self.ld, self.off + c0, self.needs_grad)
 
     def nhwc(self) -> torch.Tensor:
         """Dense torch view (tests/debug)."""

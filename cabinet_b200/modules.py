@@ -351,7 +351,9 @@ class CABiNet(nn.Module):
         schedule (BN folded into the weights).  ``.train()``: batch-statistics BatchNorm (running statistics updated) and a
         differentiable result -- ``loss.backward()`` fills ``p.grad`` of every parameter on the forward path
         (reference: src/scripts/train.py:429-441); ``torch.no_grad()`` in train mode gives the same forward without a tape
-        kept alive (``val_step``, train.py:443-456).
+        kept alive (``val_step``, train.py:443-456).  Partial fine-tuning works as with an ``nn.Module``: a parameter with
+        ``requires_grad=False`` gets no gradient (and layers that lead to no trainable parameter run no backward), and
+        a BatchNorm put in ``.eval()`` uses and keeps its running statistics.
         """
         if self.training:
             self._check_input(x, inference_only=False)

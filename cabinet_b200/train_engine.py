@@ -13,6 +13,9 @@ statistics / parameter gradients fp32.  ``'fp16'`` is the ``'bf16'`` schedule wi
 operands: the numerics of the reference's ``autocast`` + ``GradScaler`` recipe (an overflow reaches the parameter
 gradients as inf / NaN, so ``GradScaler`` skips the step).  All reductions are deterministic (fixed summation order), so a step is bit-reproducible.
 
+Partial fine-tuning follows PyTorch per module: a parameter with ``requires_grad=False`` gets no gradient, a layer whose
+input and parameters need none runs no backward, and a BatchNorm in eval mode uses (and keeps) its running statistics.
+
 The step is ~660 C-ABI calls; enqueueing them from Python takes ~19 ms against ~21 ms of GPU work, and the small layers
 at the end of the network leave the GPU waiting for the host.  After ``graph_after`` eager steps with the same input
 geometry the engine therefore captures the forward and the backward schedule into two CUDA graphs that share one
@@ -24,6 +27,7 @@ shape or engine switch re-captures; tracing (``start_trace``) and steps inside s
 from __future__ import annotations
 
 import contextlib
+import gc
 import math
 from typing import Dict, List, Optional, Tuple
 
@@ -235,7 +239,10 @@ class TrainEngine:
     def _ensure_pflat(self):
         if self._pflat is None:  # one buffer, one fill kernel per backward instead of one per parameter
             off = 0
+            self._pslots = {}
             for q in self.model.parameters():
+                if not q.requires_grad:
+                    continue  # frozen: no slot, no gradient
                 self._pslots[id(q)] = (off, q.numel())
                 off += -(-q.numel() // 64) * 64  # 256-byte aligned slots
             self._pflat = torch.zeros(max(off, 1), dtype=torch.float32, device=self.dev)
@@ -255,12 +262,16 @@ class TrainEngine:
     def _tc_ok(m: Map) -> bool:
         return m.dt in (BF16, F16) and m.ld % 8 == 0 and m.off % 8 == 0 and m.t.data_ptr() % 16 == 0
 
-    def conv(self, x: Optional[Map], conv, out: Optional[Map] = None, out_dtype=None, nchw: Optional[torch.Tensor] = None,
-             need_dx: bool = True) -> Map:
+    def conv(self, x: Optional[Map], conv, out: Optional[Map] = None, out_dtype=None,
+             nchw: Optional[torch.Tensor] = None) -> Map:
         """nn.Conv2d (bias optional) on an NHWC map or the fp32 NCHW network input.  bf16 / fp16 mode: forward and the stride-1
         data gradient run on the tensor cores (cabinet_conv_tc; the data gradient of a stride-1 convolution is the
-        convolution of dy with the transposed, mirrored weights); fp32 mode and the remaining cases: CUDA-core kernels."""
+        convolution of dy with the transposed, mirrored weights); fp32 mode and the remaining cases: CUDA-core kernels.
+        The backward computes the gradient of each parameter that requires grad, and the data gradient only when the
+        input map needs one (the network input never does)."""
         w, b = conv.weight, conv.bias
+        w_rg, b_rg = w.requires_grad, b is not None and b.requires_grad
+        need_dx = nchw is None and x.needs_grad
         cout, cin, kh, kw = w.shape
         taps = kh * kw
         stride, pad = conv.stride[0], conv.padding[0]
@@ -292,28 +303,31 @@ class TrainEngine:
                        bias.data_ptr() if bias is not None else None, None, 0, out.ptr, out.dt, out.ld, 0, 1, N, H, W, cin,
                        cout, kh, kw, stride, pad, OH, OW, ACT_NONE, 1.0)
             wdt, w_sco, w_stap = F32, taps * cin, cin
+        out.needs_grad = need_dx or w_rg or b_rg
 
         def backward(g: _Grads):
-            dy = g.get(out)
+            dy = g.get(out) if out.needs_grad else None
             if dy is None:
                 return
-            with self._wgrad_stream():
-                if b is not None:
-                    sc = self.scratch(N * OH * OW, cout, 1)
-                    self._call("cabinet_col_sum", dy.ptr, dy.ld, dy.dt, N * OH * OW, cout, self.pgrad(b).data_ptr(), 1,
-                               sc.data_ptr())
-                if (self.use_tc and self.wgrad_tc and nchw is None and kh == kw and self._tc_ok(x) and self._tc_ok(dy)
-                        and ((stride == 1 and 2 * pad == kh - 1) or (stride == 2 and H >= 2 and W >= 2))):
-                    n = int(self.lib.cabinet_conv_wgrad_tc_scratch_floats(N, H, W, cin, cout, kh, kw, stride, pad))
-                    sc = torch.empty(n, dtype=torch.float32, device=self.dev)
-                    self._call_tc("cabinet_conv_wgrad_tc", dy.ptr, dy.ld, x.ptr, x.ld, self.pgrad(w).data_ptr(), N, H, W, cin,
-                                  cout, kh, kw, stride, pad, sc.data_ptr())
-                else:
-                    n = int(self.lib.cabinet_conv_wgrad_scratch_floats(N, OH, OW, cin, cout, kh, kw))
-                    sc = torch.empty(n, dtype=torch.float32, device=self.dev)
-                    self._call("cabinet_conv_wgrad", dy.ptr, dy.ld, dy.dt, xptr, xdt, *strides, self.pgrad(w).data_ptr(), N,
-                               H, W, cin, cout, kh, kw, stride, pad, OH, OW, sc.data_ptr())
-            if nchw is not None or not need_dx:
+            if w_rg or b_rg:
+                with self._wgrad_stream():
+                    if b_rg:
+                        sc = self.scratch(N * OH * OW, cout, 1)
+                        self._call("cabinet_col_sum", dy.ptr, dy.ld, dy.dt, N * OH * OW, cout, self.pgrad(b).data_ptr(), 1,
+                                   sc.data_ptr())
+                    if w_rg and (self.use_tc and self.wgrad_tc and nchw is None and kh == kw and self._tc_ok(x)
+                                 and self._tc_ok(dy)
+                                 and ((stride == 1 and 2 * pad == kh - 1) or (stride == 2 and H >= 2 and W >= 2))):
+                        n = int(self.lib.cabinet_conv_wgrad_tc_scratch_floats(N, H, W, cin, cout, kh, kw, stride, pad))
+                        sc = torch.empty(n, dtype=torch.float32, device=self.dev)
+                        self._call_tc("cabinet_conv_wgrad_tc", dy.ptr, dy.ld, x.ptr, x.ld, self.pgrad(w).data_ptr(), N, H, W,
+                                      cin, cout, kh, kw, stride, pad, sc.data_ptr())
+                    elif w_rg:
+                        n = int(self.lib.cabinet_conv_wgrad_scratch_floats(N, OH, OW, cin, cout, kh, kw))
+                        sc = torch.empty(n, dtype=torch.float32, device=self.dev)
+                        self._call("cabinet_conv_wgrad", dy.ptr, dy.ld, dy.dt, xptr, xdt, *strides, self.pgrad(w).data_ptr(),
+                                   N, H, W, cin, cout, kh, kw, stride, pad, OH, OW, sc.data_ptr())
+            if not need_dx:
                 return
             if dy.dt != x.dt:  # fp32 class-logit gradients into a 2-byte activation gradient (pixel stride padded to 8)
                 dyc = Map(torch.empty((N, OH, OW, -(-cout // 8) * 8), dtype=x.t.dtype, device=self.dev), N, OH, OW, cout,
@@ -398,9 +412,10 @@ class TrainEngine:
         self._call("cabinet_pack_conv_weight", wbig.data_ptr(), cout, LD, 1, 1, wp.data_ptr(), self.dt, r16, k64, 0)
         self._call_tc("cabinet_conv_tc", xcol.ptr, xcol.ld, N, OH, OW, LD, wp.data_ptr(), cout, 1, 1, 1, 0,
                       self._zeros(cout).data_ptr(), None, 0, out.ptr, out.dt, out.ld, OH, OW, ACT_NONE)
+        out.needs_grad = w.requires_grad  # the network input needs no gradient
 
         def backward(g: _Grads):
-            dy = g.get(out)
+            dy = g.get(out) if out.needs_grad else None
             if dy is None:
                 return
             with self._wgrad_stream():
@@ -433,14 +448,20 @@ class TrainEngine:
             self._call("cabinet_dwconv", x.ptr, x.ld, wp.data_ptr(), self._zeros(C).data_ptr(), out.ptr, out.ld, x.dt, x.N, x.H,
                        x.W, C, k, stride, OH, OW, ACT_NONE, None)
 
+        w_rg = w.requires_grad
+        out.needs_grad = x.needs_grad or w_rg
+
         def backward(g: _Grads):
-            dy = g.get(out)
+            dy = g.get(out) if out.needs_grad else None
             if dy is None:
                 return
-            with self._wgrad_stream():
-                sc = self.scratch(x.N * OH * OW, C, k * k)
-                self._call("cabinet_dwconv_wgrad", dy.ptr, dy.ld, x.ptr, x.ld, x.dt, self.pgrad(w).data_ptr(), x.N, x.H, x.W, C,
-                           k, stride, OH, OW, sc.data_ptr())
+            if w_rg:
+                with self._wgrad_stream():
+                    sc = self.scratch(x.N * OH * OW, C, k * k)
+                    self._call("cabinet_dwconv_wgrad", dy.ptr, dy.ld, x.ptr, x.ld, x.dt, self.pgrad(w).data_ptr(), x.N, x.H,
+                               x.W, C, k, stride, OH, OW, sc.data_ptr())
+            if not x.needs_grad:
+                return
             dx, acc = g.out(x)
             if tma and stride == 1 and self._tc_ok(dy):
                 wf = torch.empty((k * k, C), dtype=torch.float32, device=self.dev)
@@ -458,31 +479,51 @@ class TrainEngine:
         return out
 
     def bn(self, z: Map, bn, act: int, res: Optional[Map] = None, out: Optional[Map] = None) -> Map:
-        """Train-mode BatchNorm2d (+activation) (+ residual add)."""
+        """BatchNorm2d (+activation) (+ residual add), per module as PyTorch does it: a module in training mode normalises
+        with the batch statistics and updates its running statistics; one in eval mode (``bn.eval()`` inside a
+        ``.train()`` model) normalises with its running statistics and leaves them, and ``num_batches_tracked``, alone."""
         M, C = z.N * z.H * z.W, z.C
         stats = torch.empty((4, C), dtype=torch.float32, device=self.dev)
-        sc = self.scratch(M, C, 2)
-        self._call("cabinet_bn_train_stats", z.ptr, z.ld, z.dt, M, C, bn.weight.data_ptr(), bn.bias.data_ptr(), float(bn.eps),
-                   BN_MOMENTUM if bn.momentum is None else float(bn.momentum), bn.running_mean.data_ptr(),
-                   bn.running_var.data_ptr(), stats.data_ptr(), sc.data_ptr())
-        self._bn_seen.append(bn.num_batches_tracked)  # += 1 for all of them at the end of the forward (one kernel)
+        frozen = not bn.training
+        if frozen:
+            self._call("cabinet_bn_frozen_stats", bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(),
+                       bn.running_var.data_ptr(), float(bn.eps), C, stats.data_ptr())
+        else:
+            sc = self.scratch(M, C, 2)
+            self._call("cabinet_bn_train_stats", z.ptr, z.ld, z.dt, M, C, bn.weight.data_ptr(), bn.bias.data_ptr(),
+                       float(bn.eps), BN_MOMENTUM if bn.momentum is None else float(bn.momentum),
+                       bn.running_mean.data_ptr(), bn.running_var.data_ptr(), stats.data_ptr(), sc.data_ptr())
+            self._bn_seen.append(bn.num_batches_tracked)  # += 1 for all of them at the end of the forward (one kernel)
         if out is None:
             out = self.new(z.N, z.H, z.W, C)
         self._call("cabinet_affine_act", z.ptr, z.ld, z.dt, stats[2].data_ptr(), stats[3].data_ptr(), None, 0.0,
                    res.ptr if res is not None else None, res.ld if res is not None else 0, out.ptr, out.ld, out.dt, M,
                    z.H * z.W, C, act)
+        g_rg, b_rg = bn.weight.requires_grad, bn.bias.requires_grad
+        res_rg = res is not None and res.needs_grad
+        out.needs_grad = z.needs_grad or g_rg or b_rg or res_rg
 
         def backward(g: _Grads):
-            dy = g.get(out)
+            dy = g.get(out) if out.needs_grad else None
             if dy is None:
                 return
-            if res is not None:  # identity branch: d res += dy
+            if res_rg:  # identity branch: d res += dy
                 self.add_grad(g, res, dy)
-            dz, acc = g.out(z)
-            sc2 = self.scratch(M, C, 4)
-            self._call("cabinet_bn_train_backward", dy.ptr, dy.ld, z.ptr, z.ld, z.dt, stats.data_ptr(), act,
-                       self.pgrad(bn.weight).data_ptr(), self.pgrad(bn.bias).data_ptr(), dz.ptr, dz.ld, M, C, acc,
-                       sc2.data_ptr())
+            dgamma = self.pgrad(bn.weight).data_ptr() if g_rg else None
+            dbeta = self.pgrad(bn.bias).data_ptr() if b_rg else None
+            if z.needs_grad and not frozen:
+                dz, acc = g.out(z)
+                sc2 = self.scratch(M, C, 4)
+                self._call("cabinet_bn_train_backward", dy.ptr, dy.ld, z.ptr, z.ld, z.dt, stats.data_ptr(), act, dgamma, dbeta,
+                           dz.ptr, dz.ld, M, C, acc, sc2.data_ptr())
+            elif z.needs_grad or g_rg or b_rg:
+                # eval mode: dz = scale * g in the same pass as the reductions; or a training module whose input needs no
+                # gradient: its dgamma / dbeta are the same two sums over the batch statistics
+                dz, acc = g.out(z) if z.needs_grad else (None, 0)
+                sc2 = self.scratch(M, C, 2) if (g_rg or b_rg) else None
+                self._call("cabinet_bn_frozen_backward", dy.ptr, dy.ld, z.ptr, z.ld, z.dt, stats.data_ptr(), act, dgamma,
+                           dbeta, dz.ptr if dz is not None else None, dz.ld if dz is not None else 0, M, C, acc,
+                           sc2.data_ptr() if sc2 is not None else None)
 
         self.tape.append(backward)
         return out
@@ -523,9 +564,11 @@ class TrainEngine:
             out = self.new(v.N, v.H, v.W, C)
         self._call("cabinet_affine_act", v.ptr, v.ld, v.dt, None, None, s.data_ptr(), plus, None, 0, out.ptr, out.ld, out.dt,
                    N * HW, HW, C, act)
+        rg = [p is not None and p.requires_grad for p in (w1, b1, w2, b2)]
+        out.needs_grad = v.needs_grad or any(rg)
 
         def backward(g: _Grads):
-            dy = g.get(out)
+            dy = g.get(out) if out.needs_grad else None
             if dy is None:
                 return
             ds = torch.empty((N, C), dtype=torch.float32, device=self.dev)
@@ -534,10 +577,16 @@ class TrainEngine:
                        HW, C, sc.data_ptr())
             dm = torch.empty((N, C), dtype=torch.float32, device=self.dev)
             sc2 = torch.empty(N * (C + J), dtype=torch.float32, device=self.dev)
+            # the kernel writes both weight gradients on its way to dm: a frozen weight's goes to a scratch buffer
+            dw = [self.pgrad(p) if r else None for p, r in zip((w1, b1, w2, b2), rg)]
+            for i in (0, 2):
+                if dw[i] is None:
+                    dw[i] = torch.empty(J * C, dtype=torch.float32, device=self.dev)
             self._call("cabinet_gate_mlp_backward", sums.data_ptr(), 1.0 / HW, w1f.data_ptr(), w2f.data_ptr(), hidden.data_ptr(),
-                       s.data_ptr(), ds.data_ptr(), gate_act, N, C, J, self.pgrad(w1).data_ptr(),
-                       self.pgrad(b1).data_ptr() if b1 is not None else None, self.pgrad(w2).data_ptr(),
-                       self.pgrad(b2).data_ptr() if b2 is not None else None, dm.data_ptr(), sc2.data_ptr())
+                       s.data_ptr(), ds.data_ptr(), gate_act, N, C, J, *(t.data_ptr() if t is not None else None for t in dw),
+                       dm.data_ptr(), sc2.data_ptr())
+            if not v.needs_grad:
+                return
             dv, acc = g.out(v)
             self._call("cabinet_gate_apply_backward", dy.ptr, dy.ld, v.ptr, v.ld, v.dt, s.data_ptr(), plus, dm.data_ptr(), 1.0 / HW,
                        act, dv.ptr, dv.ld, N, HW, C, acc)
@@ -569,9 +618,10 @@ class TrainEngine:
             self._reduce_two_pass(src, out, ty, tx, 0)
         else:
             self._resample_call(src, out, ty, tx, 4 if up else 0)  # bit 2: few taps per output -> vector kernel
+        out.needs_grad = src.needs_grad
 
         def backward(g: _Grads):
-            dy = g.get(out)
+            dy = g.get(out) if out.needs_grad else None
             if dy is None:
                 return
             dx, acc = g.out(src)
@@ -592,9 +642,10 @@ class TrainEngine:
         ident = cat.slice(0, x.C)
         self._call("cabinet_affine_act", x.ptr, x.ld, x.dt, None, None, None, 0.0, None, 0, ident.ptr, ident.ld, ident.dt,
                    x.N * x.H * x.W, x.H * x.W, x.C, ACT_NONE)
+        cat.needs_grad = ident.needs_grad = x.needs_grad  # every slice of the concatenation is a function of x alone
 
         def ident_bwd(g: _Grads):
-            dy = g.get(ident)
+            dy = g.get(ident) if ident.needs_grad else None
             if dy is not None:
                 self.add_grad(g, x, dy)
 
@@ -622,9 +673,10 @@ class TrainEngine:
         gemm(q.ptr, q.dt, q.ld, 1, L * q.ld, k.ptr, k.dt, k.ld, 1, L * k.ld, s.data_ptr(), F32, L, L * L, L, d, L, alpha)
         self._call("cabinet_softmax_rows", s.data_ptr(), p.data_ptr(), F32, N * L, L)
         gemm(p.data_ptr(), F32, L, 1, L * L, v.ptr, v.dt, 1, v.ld, L * v.ld, ctx.ptr, ctx.dt, ctx.ld, L * ctx.ld, L, L, d)
+        ctx.needs_grad = q.needs_grad or k.needs_grad or v.needs_grad
 
         def backward(g: _Grads):
-            do = g.get(ctx)
+            do = g.get(ctx) if ctx.needs_grad else None
             if do is None:
                 return
             dp = s  # the raw scores are not needed any more: reuse their buffer
@@ -639,7 +691,8 @@ class TrainEngine:
             gemm(ds.data_ptr(), F32, L, 1, L * L, k.ptr, k.dt, 1, k.ld, L * k.ld, dq.ptr, dq.dt, d, L * d, L, L, d)
             gemm(ds.data_ptr(), F32, 1, L, L * L, q.ptr, q.dt, 1, q.ld, L * q.ld, dk.ptr, dk.dt, d, L * d, L, L, d)
             for tgt, src in ((q, dq), (k, dk), (v, dv)):
-                self.add_grad(g, tgt, src)
+                if tgt.needs_grad:
+                    self.add_grad(g, tgt, src)
 
         self.tape.append(backward)
         return ctx
@@ -667,9 +720,10 @@ class TrainEngine:
         self._call_tc("cabinet_attn_softmax", s.data_ptr(), alpha, p.data_ptr(), p16.data_ptr(), N * L, L)
         self._call_tc("cabinet_transpose_tokens", v.ptr, v.ld, vt.data_ptr(), N, L, d)
         gemm(p16.data_ptr(), L, L, vt.data_ptr(), d, zd, ctx.ptr, ctx.dt, ctx.ld)
+        ctx.needs_grad = q.needs_grad or k.needs_grad or v.needs_grad
 
         def backward(g: _Grads):
-            do = g.get(ctx)
+            do = g.get(ctx) if ctx.needs_grad else None
             if do is None:
                 return
             dp = s  # the raw scores are not needed any more: reuse their buffer
@@ -692,7 +746,8 @@ class TrainEngine:
                 self._call("cabinet_affine_act", src.data_ptr(), d, F32, None, None, None, 0.0, None, 0, dst.ptr, dst.ld,
                            dst.dt, N * L, L, d, ACT_NONE)
             for tgt, src in ((q, dq), (k, dk), (v, dv)):
-                self.add_grad(g, tgt, src)
+                if tgt.needs_grad:
+                    self.add_grad(g, tgt, src)
 
         self.tape.append(backward)
         return ctx
@@ -702,17 +757,21 @@ class TrainEngine:
         M = x.N * x.H * x.W
         gm = gamma.detach().float().contiguous()
         self._call("cabinet_cab_combine", gmap.ptr, x.ptr, r.ptr, out.ptr, out.ld, gm.data_ptr(), self.dt, M, x.C)
+        out.needs_grad = gmap.needs_grad or x.needs_grad or r.needs_grad or gamma.requires_grad
 
         def backward(g: _Grads):
-            dy = g.get(out)
+            dy = g.get(out) if out.needs_grad else None
             if dy is None:
                 return
+            # one elementwise pass writes all three data gradients and the gamma partials; the producers of the maps that
+            # need no gradient skip theirs, and a frozen gamma's sum goes to a scratch slot
             dg, _ = g.out(gmap)
             dr, _ = g.out(r)
             dx, acc = g.out(x)
             sc = self.scratch(M, x.C, 1)
+            dgamma = self.pgrad(gamma) if gamma.requires_grad else torch.empty(1, dtype=torch.float32, device=self.dev)
             self._call("cabinet_cab_combine_backward", dy.ptr, dy.ld, gmap.ptr, x.ptr, r.ptr, gm.data_ptr(), self.dt, dg.ptr,
-                       dx.ptr, dr.ptr, self.pgrad(gamma).data_ptr(), M, x.C, acc, sc.data_ptr())
+                       dx.ptr, dr.ptr, dgamma.data_ptr(), M, x.C, acc, sc.data_ptr())
 
         self.tape.append(backward)
 
@@ -723,6 +782,8 @@ class TrainEngine:
         self._call("cabinet_upsample_logits_nchw", src.ptr, N, src.H, src.W, C, y.data_ptr(), self._dt(y), H, W)
 
         def backward(g: _Grads, dy_nchw: torch.Tensor):
+            if not src.needs_grad:
+                return
             dy_nchw = dy_nchw.contiguous()
             dx, acc = g.out(src)
             ay, ax = self.tables.get("bilinear", src.H, H, True), self.tables.get("bilinear", src.W, W, True)
@@ -754,7 +815,7 @@ class TrainEngine:
         H8, W8 = s3.H, s3.W
         n_sb = sb.conv_out.conv.out_channels
         cat_ffm = self.new(N, H8, W8, n_sb + ab.convb.out_channels)
-        self.bn(self.conv(s3, sb.conv_out.conv), sb.conv_out.bn, ACT_RELU, out=cat_ffm.slice(0, n_sb))
+        sb_feat = self.bn(self.conv(s3, sb.conv_out.conv), sb.conv_out.bn, ACT_RELU, out=cat_ffm.slice(0, n_sb))
         sb_hi = len(self.tape)
 
         # ---- backbone (mobilenetv3.py:102-159,202-205)
@@ -798,7 +859,9 @@ class TrainEngine:
         feat2 = cat_b1.slice(n_mf, 256)
         self.cab_combine(gl, feat, r, cab.gamma, feat2)
         low = self.conv(feat2, ab.convb)
-        self.resample(low, "bilinear", H8, W8, out=cat_ffm.slice(n_sb, low.C))                  # cabinet.py:228-233
+        low_up = self.resample(low, "bilinear", H8, W8, out=cat_ffm.slice(n_sb, low.C))         # cabinet.py:228-233
+        cat_b1.needs_grad = mf.needs_grad or feat2.needs_grad
+        cat_ffm.needs_grad = sb_feat.needs_grad or low_up.needs_grad
         fused = self.bn(self.conv(cat_b1, ab.b1), ab.b2, ACT_RELU)
         high = self.conv(fused, ab.b4, out_dtype=torch.float32)
         aux8 = self.resample(high, "bilinear", H8, W8)                                          # cabinet.py:234-239
@@ -819,7 +882,7 @@ class TrainEngine:
         return final, aux
 
     def backward(self, d_final: Optional[torch.Tensor], d_aux: Optional[torch.Tensor]) -> Dict[int, torch.Tensor]:
-        """Gradients of the two logit tensors -> {id(parameter): fp32 gradient}."""
+        """Gradients of the two logit tensors -> {id(parameter): fp32 gradient} for the parameters that require grad."""
         g = _Grads(self)
         self.pgrads, self.phase, self._pflat, self._side_used = {}, "bwd", None, False
         self._ensure_pflat()  # zero-filled on THIS stream before any branch adds into it
@@ -850,9 +913,11 @@ class TrainEngine:
 
     # ------------------------------------------------------------------ the step as two CUDA graphs
     def _addresses(self) -> tuple:
-        """Everything a captured graph has baked in: parameter / buffer addresses and which parameters take a gradient."""
+        """Everything a captured graph has baked in: parameter / buffer addresses, which parameters take a gradient and
+        which BatchNorm modules use their batch statistics."""
         return (tuple((p.data_ptr(), p.requires_grad) for p in self.model.parameters()),
-                tuple(b.data_ptr() for b in self.model.buffers()))
+                tuple(b.data_ptr() for b in self.model.buffers()),
+                tuple(m.training for m in self.model.modules() if isinstance(m, torch.nn.BatchNorm2d)))
 
     def step_forward(self, x: torch.Tensor, logits_dtype=torch.float32):
         """``forward`` for the autograd hand-off: eager for the first ``graph_after`` steps of a geometry, graph replay after."""
@@ -911,13 +976,21 @@ class TrainEngine:
         st.x.copy_(x)
         fwd, bwd = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
         pool = torch.cuda.graph_pool_handle()
-        with torch.cuda.graph(fwd, pool=pool, capture_error_mode="thread_local"):
-            st.final, st.aux = self.forward(st.x, logits_dtype)
-        st.n_fwd = self.launches
-        st.tape, st.out_bwd, st.branch = self.tape, self._out_bwd, self._branch  # keeps every saved activation alive
-        st.d_final, st.d_aux = torch.empty_like(st.final), torch.empty_like(st.aux)
-        with torch.cuda.graph(bwd, pool=pool, capture_error_mode="thread_local"):
-            st.grads = dict(self.backward(st.d_final, st.d_aux))
+        # no cyclic garbage collection during the captures: a discarded model is a cycle (model <-> engine), and collecting
+        # it destroys its CUDA graphs, which invalidates a capture in progress
+        gc_enabled = gc.isenabled()
+        gc.disable()
+        try:
+            with torch.cuda.graph(fwd, pool=pool, capture_error_mode="thread_local"):
+                st.final, st.aux = self.forward(st.x, logits_dtype)
+            st.n_fwd = self.launches
+            st.tape, st.out_bwd, st.branch = self.tape, self._out_bwd, self._branch  # keeps every saved activation alive
+            st.d_final, st.d_aux = torch.empty_like(st.final), torch.empty_like(st.aux)
+            with torch.cuda.graph(bwd, pool=pool, capture_error_mode="thread_local"):
+                st.grads = dict(self.backward(st.d_final, st.d_aux))
+        finally:
+            if gc_enabled:
+                gc.enable()
         st.n_bwd = self.launches - st.n_fwd
         st.fwd, st.bwd, st.addr = fwd, bwd, addr
 

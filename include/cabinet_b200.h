@@ -448,6 +448,24 @@ int cabinet_bn_train_backward(const void* dy, long long lddy, const void* z, lon
                               int act, float* dgamma, float* dbeta, void* dz, long long lddz, long long M, int C,
                               int accumulate, float* scratch, cabinet_stream_t stream);
 
+/* Eval-mode BatchNorm2d inside a training step (bn.eval() in a .train() model, e.g. frozen BN for fine-tuning): stats[4][C]
+ * in the layout of cabinet_bn_train_stats, from the running statistics: mean = running_mean, invstd =
+ * 1/sqrt(running_var + eps), scale = gamma * invstd, shift = beta - mean * scale (gamma / beta may be NULL: 1 / 0).  Runs
+ * on the device, so a replayed graph reads the running statistics of replay time; they are never written.  The forward
+ * apply is cabinet_affine_act with stats[2] / stats[3]. */
+int cabinet_bn_frozen_stats(const float* gamma, const float* beta, const float* running_mean, const float* running_var,
+                            float eps, int C, float* stats, cabinet_stream_t stream);
+
+/* Backward of y = act(BN_eval(z)) with stats from cabinet_bn_frozen_stats: g = dy * act'(u), dz (+)= scale * g,
+ * dgamma += sum g * xhat, dbeta += sum g.  One pass over dy and z writes dz and the per-block column partials; a
+ * fixed-order second-level sum gives the parameter gradients (bit-reproducible).  dgamma and dbeta NULL: no reduction;
+ * dz NULL: no store (at least one output).  With the batch statistics of cabinet_bn_train_stats and dz NULL it gives the
+ * parameter gradients of a train-mode BN whose input needs no gradient.  scratch: (M, C, 2) (the block partials), unused
+ * without a reduction. */
+int cabinet_bn_frozen_backward(const void* dy, long long lddy, const void* z, long long ldz, int dtype, const float* stats,
+                               int act, float* dgamma, float* dbeta, void* dz, long long lddz, long long M, int C,
+                               int accumulate, float* scratch, cabinet_stream_t stream);
+
 /* Backward of y = act(v * (s[n][c] + plus)) (SE apply, mobilenetv3.py:83,143; FFM feat * atten + feat, cabinet.py:152):
  *   _scale_backward: ds[n][c] = sum_p dy * act'(v s') * v          (scratch: (HW, C, 1) * N floats)
  *   _apply_backward: dv (+)= dy * act'(v s') * s' + dm[n][c] * inv_hw  (dm = gradient of the pooled mean, may be NULL;
