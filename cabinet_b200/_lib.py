@@ -86,6 +86,7 @@ SIGNATURES = {
     "cabinet_bn_train_backward": ([_p, _ll, _p, _ll, _i, _p, _i, _p, _p, _p, _ll, _ll, _i, _i, _p, _p], _i),
     "cabinet_bn_frozen_stats": ([_p, _p, _p, _p, _f, _i, _p, _p], _i),
     "cabinet_bn_frozen_backward": ([_p, _ll, _p, _ll, _i, _p, _i, _p, _p, _p, _ll, _ll, _i, _i, _p, _p], _i),
+    "cabinet_stem_dgrad": ([_p, _ll, _p, _ll, _i, _p, _p, _p, _i, _i, _i, _i, _i, _p], _i),
     "cabinet_gate_scale_backward": ([_p, _ll, _p, _ll, _i, _p, _f, _i, _p, _i, _ll, _i, _p, _p], _i),
     "cabinet_gate_apply_backward": ([_p, _ll, _p, _ll, _i, _p, _f, _p, _f, _i, _p, _ll, _i, _ll, _i, _i, _p], _i),
     "cabinet_gate_mlp_backward": ([_p, _f, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p], _i),

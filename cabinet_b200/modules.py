@@ -354,8 +354,15 @@ class CABiNet(nn.Module):
         kept alive (``val_step``, train.py:443-456).  Partial fine-tuning works as with an ``nn.Module``: a parameter with
         ``requires_grad=False`` gets no gradient (and layers that lead to no trainable parameter run no backward), and
         a BatchNorm put in ``.eval()`` uses and keeps its running statistics.
+
+        Input gradients: an ``x`` that requires grad gets ``x.grad`` in both modes.  In ``.eval()`` with grad mode on and
+        ``x.requires_grad`` (adversarial attacks, saliency, a frozen segmenter as a loss), the call runs the
+        differentiable training schedule at ``train_precision`` with every BatchNorm in eval mode: running-statistics
+        normalisation, buffers untouched, gradients for the parameters that require grad and for ``x``.  Every other
+        eval-mode call (``x`` without grad, ``torch.no_grad()``, ``torch.inference_mode()``) stays on the inference
+        schedule and returns outputs without ``grad_fn``.
         """
-        if self.training:
+        if self.training or (torch.is_grad_enabled() and x.requires_grad):
             self._check_input(x, inference_only=False)
             from .train_engine import TrainStep
 

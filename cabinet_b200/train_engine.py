@@ -15,6 +15,8 @@ gradients as inf / NaN, so ``GradScaler`` skips the step).  All reductions are d
 
 Partial fine-tuning follows PyTorch per module: a parameter with ``requires_grad=False`` gets no gradient, a layer whose
 input and parameters need none runs no backward, and a BatchNorm in eval mode uses (and keeps) its running statistics.
+An input that requires grad gets its gradient: both stems' output gradients are then computed (even for frozen stem
+weights) and one ``cabinet_stem_dgrad`` call turns them into the fp32 NCHW ``dx``.
 
 The step is ~660 C-ABI calls; enqueueing them from Python takes ~19 ms against ~21 ms of GPU work, and the small layers
 at the end of the network leave the GPU waiting for the host.  After ``graph_after`` eager steps with the same input
@@ -166,6 +168,8 @@ class TrainEngine:
         self.max_graphs = 2                 # captured geometries kept (each pins a step's activations)
         self._gsteps: Dict[tuple, "_GraphedStep"] = {}
         self._active: Optional["_GraphedStep"] = None
+        self._stems: Optional[Tuple[Map, Map, tuple]] = None   # stem output maps + input shape when x needs a gradient
+        self.dx: Optional[torch.Tensor] = None                  # input gradient of the last backward (None: not needed)
 
     # ------------------------------------------------------------------ plumbing
     @property
@@ -268,7 +272,8 @@ class TrainEngine:
         data gradient run on the tensor cores (cabinet_conv_tc; the data gradient of a stride-1 convolution is the
         convolution of dy with the transposed, mirrored weights); fp32 mode and the remaining cases: CUDA-core kernels.
         The backward computes the gradient of each parameter that requires grad, and the data gradient only when the
-        input map needs one (the network input never does)."""
+        input map needs one.  The network input's gradient is cabinet_stem_dgrad's (``backward``): a stem on it keeps its
+        output gradient when the input requires grad."""
         w, b = conv.weight, conv.bias
         w_rg, b_rg = w.requires_grad, b is not None and b.requires_grad
         need_dx = nchw is None and x.needs_grad
@@ -303,7 +308,7 @@ class TrainEngine:
                        bias.data_ptr() if bias is not None else None, None, 0, out.ptr, out.dt, out.ld, 0, 1, N, H, W, cin,
                        cout, kh, kw, stride, pad, OH, OW, ACT_NONE, 1.0)
             wdt, w_sco, w_stap = F32, taps * cin, cin
-        out.needs_grad = need_dx or w_rg or b_rg
+        out.needs_grad = need_dx or w_rg or b_rg or (nchw is not None and self._stems is not None)
 
         def backward(g: _Grads):
             dy = g.get(out) if out.needs_grad else None
@@ -412,10 +417,10 @@ class TrainEngine:
         self._call("cabinet_pack_conv_weight", wbig.data_ptr(), cout, LD, 1, 1, wp.data_ptr(), self.dt, r16, k64, 0)
         self._call_tc("cabinet_conv_tc", xcol.ptr, xcol.ld, N, OH, OW, LD, wp.data_ptr(), cout, 1, 1, 1, 0,
                       self._zeros(cout).data_ptr(), None, 0, out.ptr, out.dt, out.ld, OH, OW, ACT_NONE)
-        out.needs_grad = w.requires_grad  # the network input needs no gradient
+        out.needs_grad = w.requires_grad or self._stems is not None  # the input's gradient: cabinet_stem_dgrad
 
         def backward(g: _Grads):
-            dy = g.get(out) if out.needs_grad else None
+            dy = g.get(out) if out.needs_grad and w.requires_grad else None
             if dy is None:
                 return
             with self._wgrad_stream():
@@ -794,22 +799,24 @@ class TrainEngine:
         return y, backward
 
     # ------------------------------------------------------------------ the step
-    def forward(self, x: torch.Tensor, logits_dtype=torch.float32):
-        """Train-mode ``CABiNet.forward`` (cabinet.py:207-247) -> (final_logit, high_res_logit_up), NCHW."""
+    def forward(self, x: torch.Tensor, logits_dtype=torch.float32, input_grad: bool = False):
+        """Train-mode ``CABiNet.forward`` (cabinet.py:207-247) -> (final_logit, high_res_logit_up), NCHW.  ``input_grad``:
+        the backward also computes the gradient of ``x`` (``self.dx``)."""
         m = self.model
         if x.dtype != torch.float32 or not x.is_contiguous():
             x = x.float().contiguous()
         N, _, H, W = x.shape
         self.tape, self.launches, self.pgrads, self.phase = [], 0, {}, "fwd"
         self._pflat, self._bn_seen = None, []
+        self._stems = (None, None, tuple(x.shape)) if input_grad else None
         mob, sb, ab, ffm, head = m.mobile, m.sb, m.ab, m.ffm, m.conv_out
         ga, cab = ab.a2block.global_attn, ab.a2block
 
         # ---- spatial branch (cabinet.py:108-129)
         xcol = self.stem_im2col(x) if (self.use_tc and self.stem_gemm) else None
         sb_lo = len(self.tape)
-        s1 = self.bn(self.conv_stem(xcol, sb.conv1.conv) if xcol is not None else self.conv(None, sb.conv1.conv, nchw=x),
-                     sb.conv1.bn, ACT_RELU)
+        stem7 = self.conv_stem(xcol, sb.conv1.conv) if xcol is not None else self.conv(None, sb.conv1.conv, nchw=x)
+        s1 = self.bn(stem7, sb.conv1.bn, ACT_RELU)
         s2 = self.bn(self.conv(s1, sb.conv2.conv), sb.conv2.bn, ACT_RELU)
         s3 = self.bn(self.conv(s2, sb.conv3.conv), sb.conv3.bn, ACT_RELU)
         H8, W8 = s3.H, s3.W
@@ -819,8 +826,11 @@ class TrainEngine:
         sb_hi = len(self.tape)
 
         # ---- backbone (mobilenetv3.py:102-159,202-205)
-        f = self.bn(self.conv_stem(xcol, mob.features[0][0]) if xcol is not None
-                    else self.conv(None, mob.features[0][0], nchw=x), mob.features[0][1], ACT_HSWISH)
+        stem3 = (self.conv_stem(xcol, mob.features[0][0]) if xcol is not None
+                 else self.conv(None, mob.features[0][0], nchw=x))
+        f = self.bn(stem3, mob.features[0][1], ACT_HSWISH)
+        if input_grad:
+            self._stems = (stem7, stem3, tuple(x.shape))
         for blk in list(mob.features)[1:]:
             s, c = blk.spec, blk.conv
             act = ACT_HSWISH if s["hs"] else ACT_RELU
@@ -882,7 +892,8 @@ class TrainEngine:
         return final, aux
 
     def backward(self, d_final: Optional[torch.Tensor], d_aux: Optional[torch.Tensor]) -> Dict[int, torch.Tensor]:
-        """Gradients of the two logit tensors -> {id(parameter): fp32 gradient} for the parameters that require grad."""
+        """Gradients of the two logit tensors -> {id(parameter): fp32 gradient} for the parameters that require grad, and
+        ``self.dx``: the fp32 NCHW gradient of the input when the forward was asked for it (else None)."""
         g = _Grads(self)
         self.pgrads, self.phase, self._pflat, self._side_used = {}, "bwd", None, False
         self._ensure_pflat()  # zero-filled on THIS stream before any branch adds into it
@@ -905,11 +916,26 @@ class TrainEngine:
                         self.tape[j](g)
         if hi > lo:
             main.wait_stream(self._side2)
+        self.dx = self._stem_dgrad(g) if self._stems is not None else None
         if self._side_used:  # join: the parameter gradients are complete when the caller's stream continues
             main.wait_stream(self._side)
         self.tape = []
         return self.pgrads
 
+    def _stem_dgrad(self, g: _Grads) -> Optional[torch.Tensor]:
+        """dx of the network input: both stems' data gradients in one cabinet_stem_dgrad call, on the main stream once the
+        spatial branch (sb.conv1's output gradient) has joined it.  None when neither stem received a gradient."""
+        stem7, stem3, (N, _, H, W) = self._stems
+        dy7, dy3 = g.get(stem7), g.get(stem3)
+        if dy7 is None and dy3 is None:
+            return None
+        dx = torch.empty((N, 3, H, W), dtype=torch.float32, device=self.dev)
+        w7, w3 = self.model.sb.conv1.conv.weight, self.model.mobile.features[0][0].weight
+        dt = (dy7 if dy7 is not None else dy3).dt
+        self._call("cabinet_stem_dgrad", dy7.ptr if dy7 is not None else None, dy7.ld if dy7 is not None else 0,
+                   dy3.ptr if dy3 is not None else None, dy3.ld if dy3 is not None else 0, dt, w7.data_ptr(), w3.data_ptr(),
+                   dx.data_ptr(), N, H, W, stem3.H, stem3.W)
+        return dx
 
     # ------------------------------------------------------------------ the step as two CUDA graphs
     def _addresses(self) -> tuple:
@@ -919,13 +945,13 @@ class TrainEngine:
                 tuple(b.data_ptr() for b in self.model.buffers()),
                 tuple(m.training for m in self.model.modules() if isinstance(m, torch.nn.BatchNorm2d)))
 
-    def step_forward(self, x: torch.Tensor, logits_dtype=torch.float32):
+    def step_forward(self, x: torch.Tensor, logits_dtype=torch.float32, input_grad: bool = False):
         """``forward`` for the autograd hand-off: eager for the first ``graph_after`` steps of a geometry, graph replay after."""
         self._active = None
         if not self.use_graph or self.trace is not None or torch.cuda.is_current_stream_capturing():
-            return self.forward(x, logits_dtype)
+            return self.forward(x, logits_dtype, input_grad)
         key = (tuple(x.shape), logits_dtype, self.use_tc, self.wgrad_tc, self.stem_gemm, self.dgrad_s2_tc, self.attn_tc,
-               self.wgrad_overlap, self.branch_overlap)
+               self.wgrad_overlap, self.branch_overlap) + ((True,) if input_grad else ())
         addr = self._addresses()
         st = self._gsteps.get(key)
         if st is not None and st.fwd is not None and st.addr != addr:
@@ -935,12 +961,12 @@ class TrainEngine:
         if st.fwd is None:
             st.seen += 1
             if st.seen <= self.graph_after:
-                return self.forward(x, logits_dtype)
+                return self.forward(x, logits_dtype, input_grad)
             captured = [k for k, v in self._gsteps.items() if v.fwd is not None]
             for k in captured[:max(0, len(captured) - self.max_graphs + 1)]:
                 del self._gsteps[k]  # oldest geometries first: each one pins its activations in its own pool
             try:
-                self._capture(st, x, logits_dtype, addr)
+                self._capture(st, x, logits_dtype, addr, input_grad)
             except Exception as e:  # e.g. out of memory for the pool: stay on the eager schedule, loudly
                 import warnings
 
@@ -948,29 +974,32 @@ class TrainEngine:
                 self.use_graph = False
                 self._gsteps.clear()
                 torch.cuda.synchronize(self.dev)
-                return self.forward(x, logits_dtype)
+                return self.forward(x, logits_dtype, input_grad)
         st.x.copy_(x)
         st.fwd.replay()
         self.launches, self.phase = st.n_fwd, "fwd"
         self._active = st
         return st.final.detach(), st.aux.detach()  # fresh tensor objects: autograd attaches this step's node to them
 
-    def step_backward(self, d_final: Optional[torch.Tensor], d_aux: Optional[torch.Tensor]) -> Dict[int, torch.Tensor]:
+    def step_backward(self, d_final: Optional[torch.Tensor],
+                      d_aux: Optional[torch.Tensor]) -> Tuple[Dict[int, torch.Tensor], Optional[torch.Tensor]]:
+        """-> (parameter gradients as ``backward`` returns them, the input gradient or None)."""
         st, self._active = self._active, None
         if st is None:
-            return self.backward(d_final, d_aux)
+            return self.backward(d_final, d_aux), self.dx
         if d_final is None or d_aux is None:
             # an unused output: the eager backward over the captured forward's tape (its saved activations are the static
             # buffers the replay just filled) leaves the parameters only that output reaches without a gradient
-            self.tape, self._out_bwd, self._branch = list(st.tape), st.out_bwd, st.branch
-            return self.backward(d_final, d_aux)
+            self.tape, self._out_bwd, self._branch, self._stems = list(st.tape), st.out_bwd, st.branch, st.stems
+            return self.backward(d_final, d_aux), self.dx
         st.d_final.copy_(d_final)
         st.d_aux.copy_(d_aux)
         st.bwd.replay()
         self.launches += st.n_bwd
-        return st.grads
+        # the next replay rewrites the static dx: hand autograd a copy, so a gradient the caller keeps stays as it is
+        return st.grads, st.dx.clone() if st.dx is not None else None
 
-    def _capture(self, st: "_GraphedStep", x: torch.Tensor, logits_dtype, addr: tuple):
+    def _capture(self, st: "_GraphedStep", x: torch.Tensor, logits_dtype, addr: tuple, input_grad: bool):
         dev = self.dev
         st.x = torch.empty(tuple(x.shape), dtype=torch.float32, device=dev)
         st.x.copy_(x)
@@ -982,12 +1011,14 @@ class TrainEngine:
         gc.disable()
         try:
             with torch.cuda.graph(fwd, pool=pool, capture_error_mode="thread_local"):
-                st.final, st.aux = self.forward(st.x, logits_dtype)
+                st.final, st.aux = self.forward(st.x, logits_dtype, input_grad)
             st.n_fwd = self.launches
             st.tape, st.out_bwd, st.branch = self.tape, self._out_bwd, self._branch  # keeps every saved activation alive
+            st.stems = self._stems
             st.d_final, st.d_aux = torch.empty_like(st.final), torch.empty_like(st.aux)
             with torch.cuda.graph(bwd, pool=pool, capture_error_mode="thread_local"):
                 st.grads = dict(self.backward(st.d_final, st.d_aux))
+                st.dx = self.dx
         finally:
             if gc_enabled:
                 gc.enable()
@@ -1002,17 +1033,18 @@ class _GraphedStep:
         self.seen = 0
         self.fwd = self.bwd = None
         self.x = self.final = self.aux = self.d_final = self.d_aux = None
-        self.tape = self.out_bwd = self.grads = self.addr = self.branch = None
+        self.tape = self.out_bwd = self.grads = self.addr = self.branch = self.stems = self.dx = None
         self.n_fwd = self.n_bwd = 0
 
 
 class TrainStep(torch.autograd.Function):
-    """Autograd hand-off: inputs = (engine, logits dtype, x, *parameters); outputs = the two logit tensors."""
+    """Autograd hand-off: inputs = (engine, logits dtype, x, *parameters); outputs = the two logit tensors.  The gradient
+    of ``x`` is computed when ``x`` requires grad (autograd casts the fp32 result to ``x``'s dtype)."""
 
     @staticmethod
     def forward(ctx, eng: TrainEngine, logits_dtype, x, *params):
         with torch.no_grad(), torch.cuda.device(eng.dev):
-            final, aux = eng.step_forward(x, logits_dtype)
+            final, aux = eng.step_forward(x, logits_dtype, bool(ctx.needs_input_grad[2]))
         ctx.eng, ctx.params = eng, params
         return final, aux
 
@@ -1020,9 +1052,9 @@ class TrainStep(torch.autograd.Function):
     def backward(ctx, d_final, d_aux):
         eng = ctx.eng
         with torch.no_grad(), torch.cuda.device(eng.dev):
-            grads = eng.step_backward(d_final, d_aux)
+            grads, dx = eng.step_backward(d_final, d_aux)
         out = []
         for p in ctx.params:
             gp = grads.get(id(p))
             out.append(gp.to(p.dtype) if gp is not None else None)
-        return (None, None, None, *out)
+        return (None, None, dx, *out)

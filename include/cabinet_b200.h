@@ -466,6 +466,15 @@ int cabinet_bn_frozen_backward(const void* dy, long long lddy, const void* z, lo
                                int act, float* dgamma, float* dbeta, void* dz, long long lddz, long long M, int C,
                                int accumulate, float* scratch, cabinet_stream_t stream);
 
+/* Data gradient of both stride-2 stems (sb.conv1 7x7 / pad 3, 64 outputs, src/models/cabinet.py:111; mobile.features.0.0
+ * 3x3 / pad 1, 16 outputs, src/models/mobilenetv3.py:86-91) into the fp32 NCHW network input: dx [N][3][H][W] = the sum
+ * of both transposed convolutions (overwritten, not accumulated).  dy7 / dy3: NHWC [N][OH][OW] with pixel strides ld7 /
+ * ld3, element type dtype (fp32, bf16 or fp16); either may be NULL (that stem received no gradient), not both.  w7 / w3:
+ * the raw fp32 filters [64][3][7][7] / [16][3][3][3], read (and for 2-byte dy rounded to dtype) on every call.  OH =
+ * (H - 1) / 2 + 1, OW = (W - 1) / 2 + 1.  2-byte dy runs on the tensor cores; fixed summation order, no atomics. */
+int cabinet_stem_dgrad(const void* dy7, long long ld7, const void* dy3, long long ld3, int dtype, const float* w7,
+                       const float* w3, float* dx, int N, int H, int W, int OH, int OW, cabinet_stream_t stream);
+
 /* Backward of y = act(v * (s[n][c] + plus)) (SE apply, mobilenetv3.py:83,143; FFM feat * atten + feat, cabinet.py:152):
  *   _scale_backward: ds[n][c] = sum_p dy * act'(v s') * v          (scratch: (HW, C, 1) * N floats)
  *   _apply_backward: dv (+)= dy * act'(v s') * s' + dm[n][c] * inv_hw  (dm = gradient of the pooled mean, may be NULL;
