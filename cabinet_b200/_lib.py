@@ -61,6 +61,7 @@ SIGNATURES = {
     "cabinet_psp_concat": ([_p, _ll, _p, _p, _ll, _i, _i, _i, _i, _i, _p], _i),
     "cabinet_softmax_rows": ([_p, _p, _i, _ll, _i, _p], _i),
     "cabinet_attention_tc": ([_p, _ll, _p, _ll, _p, _ll, _p, _p, _ll, _i, _i, _i, _f, _p], _i),
+    "cabinet_attention_tc_dkdv": ([_p, _ll, _p, _ll, _p, _ll, _p, _p, _ll, _i, _i, _i, _i, _f, _p], _i),
     "cabinet_cab_combine": ([_p, _p, _p, _p, _ll, _p, _i, _ll, _i, _p], _i),
     "cabinet_channel_sum": ([_p, _ll, _i, _i, _ll, _i, _p, _p, _ll, _p], _i),
     "cabinet_bilinear_nhwc": ([_p, _ll, _i, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _p], _i),

@@ -1,5 +1,6 @@
 // Fused global-context attention on tcgen05 (reference: src/models/cab.py:149-153):
-//     ctx = softmax(Q K^T / sqrt(d)) V        per image, d = 128, L = H/32 * W/32 tokens (1024 ... 8160)
+//     ctx = softmax(Q K^T / sqrt(dk)) V       per image, query / key width dk, value width dv, L tokens
+// (CABiNet: dk = dv = 128, L = H/32 * W/32 = 1024 ... 8160; a standalone ContextAggregationBlock(C, V): dk = C/2, dv = V)
 // The L x L score matrix never exists in memory: one CTA owns 128 queries of one image and streams the keys in
 // blocks of 128.  Two passes over the keys (QK^T is recomputed; the tensor work here is negligible):
 //   pass A  S = Q K_j^T (TMEM) -> row max m (registers; no exponentials)
@@ -7,19 +8,32 @@
 //           layout to shared memory; row sum l of the rounded values) -> O += P V_j (TMEM accumulator over all key
 //           blocks) -> ctx rows = O / l (bf16)
 // so no accumulator rescaling is needed.  V must be K-major (keys contiguous) for the P V product, hence the tiny
-// transpose pre-kernel v [L][128] -> vt [128][ceil8(L)].
+// transpose pre-kernel v [L][dv] -> vt [dv][ceil8(L)].
 // Warp roles (192 threads): warp 0 TMA producer, warp 1 TMEM allocator + MMA issuer, warps 2-5 softmax / epilogue
-// (thread = query row).  TMEM: S double-buffered (2 x 128 columns) + O (128 columns).
+// (thread = query row).  TMEM: S double-buffered (2 x 128 columns) + O (dv columns).
+// Instantiated for dk in {64, 128, 256} x dv in {64, 128}; dk <= 128 double-buffers the K / Vt stages, dk = 256 runs one
+// stage (the P V product of a key block is then issued before the next block's S, which reuses the stage).
 #include "tc_common.cuh"
 
 namespace {
 
-constexpr int D = 128;            // head dim (key / value channels)
 constexpr int BQ = 128, BKEY = 128;
 constexpr int TILE_BYTES = 128 * 128;  // one [128 rows x 64 elements] bf16 swizzled tile
 constexpr int NUM_THREADS = 192;
-// smem: Q (2 tiles) | 2 stages x { K (2 tiles) | Vt (2 tiles) } | P (2 tiles)
-constexpr int SMEM_BYTES = 2 * TILE_BYTES + 2 * 4 * TILE_BYTES + 2 * TILE_BYTES + 1024;
+
+// Query / key width DK, value / output width DV.  smem: Q (DK/64 tiles) | NST stages x { K (DK/64 tiles) | Vt (2 tiles of
+// DV rows x 64 keys) } | P (2 tiles).  Two stages wherever they fit; at DK = 256 one stage (Q 64 KB + 2 x 96 KB + P
+// 32 KB would exceed the 227 KB of shared memory).
+template <int DK, int DV>
+struct AttnCfg {
+    static constexpr int KT = DK / 64;                   // 64-element K tiles of Q and K
+    static constexpr int VT_TILE = DV * 128;             // one [DV rows x 64 keys] swizzled tile of Vt
+    static constexpr int STAGE = KT * TILE_BYTES + 2 * VT_TILE;
+    static constexpr int NST = DK >= 256 ? 1 : 2;
+    static constexpr int SMEM = KT * TILE_BYTES + NST * STAGE + 2 * TILE_BYTES + 1024;
+    static_assert(SMEM <= 227 * 1024, "attention_tc: shared memory");
+    static_assert(256 + DV <= 512, "attention_tc: TMEM");
+};
 
 struct AttnParams {
     int L, nkb;
@@ -28,16 +42,19 @@ struct AttnParams {
     long long ldc;
 };
 
+template <int DK, int DV>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                const __grid_constant__ CUtensorMap tmVt, const AttnParams p) {
+    using Cfg = AttnCfg<DK, DV>;
+    constexpr int KT = Cfg::KT, NST = Cfg::NST, STAGE = Cfg::STAGE, VT_TILE = Cfg::VT_TILE;
     extern __shared__ uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t q_full, kv_full[2], kv_empty[2], s_full[2], s_empty[2], p_full, p_empty, o_full;
+    __shared__ __align__(8) uint64_t q_full, kv_full[NST], kv_empty[NST], s_full[2], s_empty[2], p_full, p_empty, o_full;
     __shared__ uint32_t tmem_base_smem;
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t* sQ = smem;
-    uint8_t* sKV = sQ + 2 * TILE_BYTES;   // stage s: K at +s*4*TILE, Vt at +s*4*TILE + 2*TILE
-    uint8_t* sP = sKV + 8 * TILE_BYTES;
+    uint8_t* sKV = sQ + KT * TILE_BYTES;   // stage s: K at +s*STAGE, Vt at +s*STAGE + KT*TILE
+    uint8_t* sP = sKV + NST * STAGE;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int q0 = blockIdx.x * BQ, img = blockIdx.y;
@@ -48,9 +65,11 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
         tc::prefetch_tmap(&tmK);
         tc::prefetch_tmap(&tmVt);
         tc::mbar_init(&q_full, 1);
-        for (int s = 0; s < 2; ++s) {
+        for (int s = 0; s < NST; ++s) {
             tc::mbar_init(&kv_full[s], 1);
             tc::mbar_init(&kv_empty[s], 1);
+        }
+        for (int s = 0; s < 2; ++s) {
             tc::mbar_init(&s_full[s], 1);
             tc::mbar_init(&s_empty[s], 4);
         }
@@ -70,22 +89,23 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
     if (warp == 0) {
         if (lane == 0) {
             // ================= TMA producer =================
-            tc::mbar_expect_tx(&q_full, 2 * TILE_BYTES);
-            tc::tma_load_3d(sQ, &tmQ, &q_full, 0, q0, img);
-            tc::tma_load_3d(sQ + TILE_BYTES, &tmQ, &q_full, 64, q0, img);
+            tc::mbar_expect_tx(&q_full, KT * TILE_BYTES);
+#pragma unroll
+            for (int kb = 0; kb < KT; ++kb) tc::tma_load_3d(sQ + kb * TILE_BYTES, &tmQ, &q_full, 64 * kb, q0, img);
             for (int t = 0; t < T; ++t) {
-                const int s = t & 1;
-                const uint32_t ph = (t >> 1) & 1;
+                const int s = t % NST;
+                const uint32_t ph = (t / NST) & 1;
                 const int j = t < nkb ? t : t - nkb;
                 const bool pass_b = t >= nkb;
-                uint8_t* stage = sKV + s * 4 * TILE_BYTES;
+                uint8_t* stage = sKV + s * STAGE;
                 tc::mbar_wait(&kv_empty[s], ph ^ 1);
-                tc::mbar_expect_tx(&kv_full[s], (pass_b ? 4 : 2) * TILE_BYTES);
-                tc::tma_load_3d(stage, &tmK, &kv_full[s], 0, j * BKEY, img);
-                tc::tma_load_3d(stage + TILE_BYTES, &tmK, &kv_full[s], 64, j * BKEY, img);
+                tc::mbar_expect_tx(&kv_full[s], KT * TILE_BYTES + (pass_b ? 2 * VT_TILE : 0));
+#pragma unroll
+                for (int kb = 0; kb < KT; ++kb)
+                    tc::tma_load_3d(stage + kb * TILE_BYTES, &tmK, &kv_full[s], 64 * kb, j * BKEY, img);
                 if (pass_b) {
-                    tc::tma_load_3d(stage + 2 * TILE_BYTES, &tmVt, &kv_full[s], j * BKEY, 0, img);
-                    tc::tma_load_3d(stage + 3 * TILE_BYTES, &tmVt, &kv_full[s], j * BKEY + 64, 0, img);
+                    tc::tma_load_3d(stage + KT * TILE_BYTES, &tmVt, &kv_full[s], j * BKEY, 0, img);
+                    tc::tma_load_3d(stage + KT * TILE_BYTES + VT_TILE, &tmVt, &kv_full[s], j * BKEY + 64, 0, img);
                 }
             }
         }
@@ -93,41 +113,42 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
     } else if (warp == 1) {
         // ================= MMA issuer: warp-uniform control flow, one elected lane issues =================
         const uint32_t leader = tc::elect_one();
-        const uint32_t idesc = tc::make_idesc_bf16(128, 128);
+        const uint32_t idesc_s = tc::make_idesc_bf16(128, BKEY), idesc_o = tc::make_idesc_bf16(128, DV);
         const uint64_t q_desc = tc::make_desc_sw128(tc::smem_u32(sQ)), p_desc = tc::make_desc_sw128(tc::smem_u32(sP));
         const uint64_t kv_desc0 = tc::make_desc_sw128(tc::smem_u32(sKV));
-        constexpr uint32_t TILE16 = TILE_BYTES >> 4;
+        constexpr uint32_t TILE16 = TILE_BYTES >> 4, VT16 = VT_TILE >> 4, STAGE16 = STAGE >> 4;
         tc::mbar_wait(&q_full, 0);
         auto issue_pv = [&](int t) {  // O += P_t * V_t   (t is a pass-B index)
             const int kidx = t - nkb;
-            const uint64_t v_desc = kv_desc0 + static_cast<uint64_t>(((t & 1) * 4 + 2) * TILE16);
+            const uint64_t v_desc = kv_desc0 + static_cast<uint64_t>((t % NST) * STAGE16 + KT * TILE16);
             tc::mbar_wait(&p_full, kidx & 1);
             tc::tc_fence_after();
 #pragma unroll
             for (int kb = 0; kb < 2; ++kb)
 #pragma unroll
                 for (int k = 0; k < 4; ++k)
-                    tc::umma_bf16_if(leader, tmem_o, p_desc + (kb * TILE16 + 2 * k), v_desc + (kb * TILE16 + 2 * k), idesc,
+                    tc::umma_bf16_if(leader, tmem_o, p_desc + (kb * TILE16 + 2 * k), v_desc + (kb * VT16 + 2 * k), idesc_o,
                                      (kidx | kb | k) != 0 ? 1u : 0u);
             tc::umma_commit_if(leader, &p_empty);
-            tc::umma_commit_if(leader, &kv_empty[t & 1]);
+            tc::umma_commit_if(leader, &kv_empty[t % NST]);
         };
         for (int t = 0; t < T; ++t) {
-            const int s = t & 1;
-            const uint32_t ph = (t >> 1) & 1;
-            tc::mbar_wait(&kv_full[s], ph);
-            tc::mbar_wait(&s_empty[s], ph ^ 1);
+            const int s = t % NST, sb = t & 1;
+            // one stage: the previous block's P V must release the stage before the next K / Vt can land in it
+            if (NST == 1 && t > nkb) issue_pv(t - 1);
+            tc::mbar_wait(&kv_full[s], (t / NST) & 1);
+            tc::mbar_wait(&s_empty[sb], ((t >> 1) & 1) ^ 1);
             tc::tc_fence_after();
-            const uint64_t k_desc = kv_desc0 + static_cast<uint64_t>(s * 4 * TILE16);
+            const uint64_t k_desc = kv_desc0 + static_cast<uint64_t>(s * STAGE16);
 #pragma unroll
-            for (int kb = 0; kb < 2; ++kb)
+            for (int kb = 0; kb < KT; ++kb)
 #pragma unroll
                 for (int k = 0; k < 4; ++k)
-                    tc::umma_bf16_if(leader, tmem + s * 128, q_desc + (kb * TILE16 + 2 * k), k_desc + (kb * TILE16 + 2 * k),
-                                     idesc, (kb | k) ? 1u : 0u);
-            tc::umma_commit_if(leader, &s_full[s]);
+                    tc::umma_bf16_if(leader, tmem + sb * 128, q_desc + (kb * TILE16 + 2 * k), k_desc + (kb * TILE16 + 2 * k),
+                                     idesc_s, (kb | k) ? 1u : 0u);
+            tc::umma_commit_if(leader, &s_full[sb]);
             if (t < nkb) tc::umma_commit_if(leader, &kv_empty[s]);  // pass A: K block is free once S is computed
-            else if (t > nkb) issue_pv(t - 1);                       // pass B: P V of the previous block, lagging one S
+            else if (NST > 1 && t > nkb) issue_pv(t - 1);            // pass B: P V of the previous block, lagging one S
         }
         issue_pv(T - 1);
         tc::umma_commit_if(leader, &o_full);
@@ -222,7 +243,7 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
         const int qrow = q0 + row;
         bf16* out = p.ctx + (static_cast<long long>(img) * p.L + qrow) * p.ldc;
 #pragma unroll
-        for (int ch = 0; ch < 4; ++ch) {
+        for (int ch = 0; ch < DV / 32; ++ch) {
             uint32_t r[32];
             tc::tmem_ld32(tmem_o + lane_addr + ch * 32, r);
             tc::tmem_ld_wait();
@@ -247,9 +268,9 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
     }
 }
 
-// v [N][L][D] (pixel stride ldv) -> vt [N][D][Lp], zero padded keys L..Lp-1
+// v [N][L][dv] (pixel stride ldv) -> vt [N][dv][Lp], zero padded keys L..Lp-1
 __global__ void __launch_bounds__(256)
-transpose_v_kernel(const bf16* __restrict__ v, long long ldv, bf16* __restrict__ vt, int L, int Lp) {
+transpose_v_kernel(const bf16* __restrict__ v, long long ldv, bf16* __restrict__ vt, int L, int Lp, int dv) {
     __shared__ bf16 tile[32][33];
     const int n = blockIdx.z;
     const int k0 = blockIdx.x * 32, d0 = blockIdx.y * 32;
@@ -261,19 +282,33 @@ transpose_v_kernel(const bf16* __restrict__ v, long long ldv, bf16* __restrict__
     __syncthreads();
     for (int i = ty; i < 32; i += 8) {
         const int key = k0 + tx;
-        if (key < Lp) vt[(static_cast<long long>(n) * D + d0 + i) * Lp + key] = tile[tx][i];
+        if (key < Lp) vt[(static_cast<long long>(n) * dv + d0 + i) * Lp + key] = tile[tx][i];
     }
 }
 
-}  // namespace
+template <int DK, int DV>
+int launch_attention(const CUtensorMap& tmQ, const CUtensorMap& tmK, const CUtensorMap& tmVt, const AttnParams& p, int N,
+                     cudaStream_t s) {
+    constexpr int SMEM = AttnCfg<DK, DV>::SMEM;
+    static bool attr_done = false;
+    if (!attr_done) {
+        CAB_CUDA(cudaFuncSetAttribute(attn_tc_kernel<DK, DV>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+        attr_done = true;
+    }
+    dim3 grid((p.L + BQ - 1) / BQ, N);
+    attn_tc_kernel<DK, DV><<<grid, NUM_THREADS, SMEM, s>>>(tmQ, tmK, tmVt, p);
+    CAB_LAUNCH_CHECK();
+    return CABINET_OK;
+}
 
-extern "C" int cabinet_attention_tc(const void* q, long long ldq, const void* k, long long ldk, const void* v,
-                                    long long ldv, void* vt_workspace, void* ctx, long long ldc, int N, int L, int d,
-                                    float scale, cabinet_stream_t stream) {
+int attention_tc(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv,
+                 void* vt_workspace, void* ctx, long long ldc, int N, int L, int dk, int dv, float scale,
+                 cabinet_stream_t stream) {
     CAB_REQUIRE(q && k && v && vt_workspace && ctx, "attention_tc: null pointer");
-    CAB_REQUIRE(d == D, "attention_tc: head dim must be 128 (got %d)", d);
+    CAB_REQUIRE((dk == 64 || dk == 128 || dk == 256) && (dv == 64 || dv == 128),
+                "attention_tc: key width must be 64, 128 or 256 and value width 64 or 128 (got %d, %d)", dk, dv);
     CAB_REQUIRE(N >= 0 && L > 0 && N <= 65535, "attention_tc: bad sizes");
-    CAB_REQUIRE(ldq % 8 == 0 && ldk % 8 == 0 && ldc % 8 == 0 && ldq >= D && ldk >= D && ldv >= D && ldc >= D &&
+    CAB_REQUIRE(ldq % 8 == 0 && ldk % 8 == 0 && ldc % 8 == 0 && ldq >= dk && ldk >= dk && ldv >= dv && ldc >= dv &&
                     (reinterpret_cast<uintptr_t>(q) & 15) == 0 && (reinterpret_cast<uintptr_t>(k) & 15) == 0 &&
                     (reinterpret_cast<uintptr_t>(ctx) & 15) == 0 && (reinterpret_cast<uintptr_t>(vt_workspace) & 15) == 0,
                 "attention_tc: 16-byte aligned rows required");
@@ -281,24 +316,25 @@ extern "C" int cabinet_attention_tc(const void* q, long long ldq, const void* k,
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const int Lp = (L + 7) / 8 * 8;
     {
-        dim3 grid((Lp + 31) / 32, D / 32, N);
+        dim3 grid((Lp + 31) / 32, dv / 32, N);
         transpose_v_kernel<<<grid, 256, 0, s>>>(reinterpret_cast<const bf16*>(v), ldv, reinterpret_cast<bf16*>(vt_workspace),
-                                                L, Lp);
+                                                L, Lp, dv);
         CAB_LAUNCH_CHECK();
     }
     CUtensorMap tmQ, tmK, tmVt;
-    const uint32_t box[3] = {64, 128, 1};
     {
-        const uint64_t dims[3] = {(uint64_t)D, (uint64_t)L, (uint64_t)N};
+        const uint32_t box[3] = {64, 128, 1};
+        const uint64_t dims[3] = {(uint64_t)dk, (uint64_t)L, (uint64_t)N};
         const uint64_t sq[2] = {(uint64_t)ldq * 2, (uint64_t)ldq * 2 * L};
         const uint64_t sk[2] = {(uint64_t)ldk * 2, (uint64_t)ldk * 2 * L};
         int rc = cab_make_tmap_bf16(&tmQ, q, 3, dims, sq, box);
         if (rc) return rc;
         rc = cab_make_tmap_bf16(&tmK, k, 3, dims, sk, box);
         if (rc) return rc;
-        const uint64_t dv[3] = {(uint64_t)Lp, (uint64_t)D, (uint64_t)N};
-        const uint64_t sv[2] = {(uint64_t)Lp * 2, (uint64_t)Lp * 2 * D};
-        rc = cab_make_tmap_bf16(&tmVt, vt_workspace, 3, dv, sv, box);
+        const uint32_t vbox[3] = {64, (uint32_t)dv, 1};
+        const uint64_t dvt[3] = {(uint64_t)Lp, (uint64_t)dv, (uint64_t)N};
+        const uint64_t sv[2] = {(uint64_t)Lp * 2, (uint64_t)Lp * 2 * dv};
+        rc = cab_make_tmap_bf16(&tmVt, vt_workspace, 3, dvt, sv, vbox);
         if (rc) return rc;
     }
     AttnParams p;
@@ -307,13 +343,27 @@ extern "C" int cabinet_attention_tc(const void* q, long long ldq, const void* k,
     p.c = scale * 1.4426950408889634f;
     p.ctx = reinterpret_cast<bf16*>(ctx);
     p.ldc = ldc;
-    static bool attr_done = false;
-    if (!attr_done) {
-        CAB_CUDA(cudaFuncSetAttribute(attn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        attr_done = true;
+    switch (dk * 1000 + dv) {
+        case 64064: return launch_attention<64, 64>(tmQ, tmK, tmVt, p, N, s);
+        case 64128: return launch_attention<64, 128>(tmQ, tmK, tmVt, p, N, s);
+        case 128064: return launch_attention<128, 64>(tmQ, tmK, tmVt, p, N, s);
+        case 128128: return launch_attention<128, 128>(tmQ, tmK, tmVt, p, N, s);
+        case 256064: return launch_attention<256, 64>(tmQ, tmK, tmVt, p, N, s);
+        default: return launch_attention<256, 128>(tmQ, tmK, tmVt, p, N, s);
     }
-    dim3 grid((L + BQ - 1) / BQ, N);
-    attn_tc_kernel<<<grid, NUM_THREADS, SMEM_BYTES, s>>>(tmQ, tmK, tmVt, p);
-    CAB_LAUNCH_CHECK();
-    return CABINET_OK;
+}
+
+}  // namespace
+
+extern "C" int cabinet_attention_tc(const void* q, long long ldq, const void* k, long long ldk, const void* v,
+                                    long long ldv, void* vt_workspace, void* ctx, long long ldc, int N, int L, int d,
+                                    float scale, cabinet_stream_t stream) {
+    CAB_REQUIRE(d == 128, "attention_tc: head dim must be 128 (got %d)", d);
+    return attention_tc(q, ldq, k, ldk, v, ldv, vt_workspace, ctx, ldc, N, L, 128, 128, scale, stream);
+}
+
+extern "C" int cabinet_attention_tc_dkdv(const void* q, long long ldq, const void* k, long long ldk, const void* v,
+                                         long long ldv, void* vt_workspace, void* ctx, long long ldc, int N, int L, int dk,
+                                         int dv, float scale, cabinet_stream_t stream) {
+    return attention_tc(q, ldq, k, ldk, v, ldv, vt_workspace, ctx, ldc, N, L, dk, dv, scale, stream);
 }

@@ -179,6 +179,8 @@ class Engine:
     PACKED_ATTRS = ("stem", "blocks", "last", "stem_tc", "sb1", "sb2", "sb3", "sb4", "conva", "to_q", "to_k", "to_v",
                     "psp_k", "psp_v", "proj_out", "local", "gamma", "convb", "b1", "b4", "key_ch", "qkv", "ffm_blk",
                     "ffm_gate", "head_conv", "head_out", "ffm_sb", "low_fold", "stem_tc2")
+    # what ``_pack_cab`` produces: all an engine built over a standalone ContextAggregationBlock packs
+    CAB_ATTRS = ("to_q", "to_k", "to_v", "psp_k", "psp_v", "proj_out", "local", "gamma", "key_ch", "qkv")
 
     def __init__(self, model, precision: str = "bf16", packed: Optional[dict] = None):
         if precision not in ("bf16", "fp32"):
@@ -186,12 +188,16 @@ class Engine:
         p0 = next(model.parameters())
         if not p0.is_cuda:
             raise RuntimeError("cabinet_b200 engine needs the model on a CUDA device (no CPU path)")
+        from .modules import ContextAggregationBlock
+
         self.lib = _lib.load()
         self.dev = p0.device
         self.precision = precision
         self.tdt = torch.bfloat16 if precision == "bf16" else torch.float32
         self.dt = BF16 if precision == "bf16" else F32
-        self.n_classes = model.n_classes
+        # an engine over a standalone ContextAggregationBlock packs that block alone and runs ``forward_block``
+        self.block = isinstance(model, ContextAggregationBlock)
+        self.n_classes = 0 if self.block else model.n_classes
         self.stamp = None
         self.launches = 0  # kernels enqueued by the last forward
         self.use_tc = precision == "bf16"
@@ -227,6 +233,8 @@ class Engine:
         self.branch_overlap = True  # independent chains of the attention branch on side streams (fork / join by events)
         self._branch_streams, self._branch_events = [], {}
         self.sb_overlap = False     # experiment: spatial branch beside the backbone
+        if packed is not None and self.block:
+            raise ValueError("packed weights exist for CABiNet engines only")
         if packed is not None:  # cached fold + pack of exactly these weights (checkpoint.load_packed verified the digest)
             missing = [a for a in self.PACKED_ATTRS if a not in packed]
             if missing:
@@ -236,8 +244,8 @@ class Engine:
             self.gamma = model.ab.a2block.gamma.detach().float().contiguous()
         else:
             with torch.no_grad():
-                self._pack(model)  # on the host ...
-                for a in self.PACKED_ATTRS:  # ... then one upload per packed tensor
+                self._pack_cab(model) if self.block else self._pack(model)  # on the host ...
+                for a in self.CAB_ATTRS if self.block else self.PACKED_ATTRS:  # ... then one upload per packed tensor
                     setattr(self, a, _map_tensors(getattr(self, a), lambda t: t.to(self.dev)))
 
     def packed_state(self) -> dict:
@@ -329,27 +337,12 @@ class Engine:
         self.sb3 = ConvLayer(sb.conv3.conv, sb.conv3.bn, ACT_RELU, wd, "sb.conv3")
         self.sb4 = ConvLayer(sb.conv_out.conv, sb.conv_out.bn, ACT_RELU, wd, "sb.conv_out")
 
-        ab, ga = m.ab, m.ab.a2block.global_attn
+        ab = m.ab
         self.conva = ConvLayer(ab.conva[0], ab.conva[1], ACT_RELU, wd, "ab.conva")
-        self.to_q = ConvLayer(ga.to_query[0], ga.to_query[1], ACT_RELU, wd, "cab.to_query")
-        self.to_k = ConvLayer(ga.to_key[0], ga.to_key[1], ACT_RELU, wd, "cab.to_key")
-        self.to_v = ConvLayer(ga.to_value, None, ACT_NONE, wd, "cab.to_value")
-        self.psp_k = ConvLayer(ga.psp_key.project, None, ACT_NONE, wd, "cab.psp_key")
-        self.psp_v = ConvLayer(ga.psp_value.project, None, ACT_NONE, wd, "cab.psp_value")
-        self.proj_out = ConvLayer(ga.project_out, None, ACT_NONE, wd, "cab.project_out")
-        self.local = [DwLayer(d.block[0], d.block[1], ACT_RELU, f"cab.local{i}")
-                      for i, d in enumerate(ab.a2block.local_attn.refine)]
-        self.gamma = _host(ab.a2block.gamma).contiguous()
+        self._pack_cab(ab.a2block)
         self.convb = ConvLayer(ab.convb, None, ACT_NONE, wd, "ab.convb")
         self.b1 = ConvLayer(ab.b1, ab.b2, ACT_RELU, wd, "ab.b1")
         self.b4 = ConvLayer(ab.b4, None, ACT_NONE, wd, "ab.b4")
-        self.key_ch = self.to_k.cout
-        # to_query | to_key | to_value read the same tensor: one 256 -> 3 x 128 GEMM, ReLU on the first 2 x 128 outputs
-        self.qkv = None
-        if (self.precision == "bf16" and all(L.tc is not None and L.kh == 1 for L in (self.to_q, self.to_k, self.to_v))
-                and self.to_q.cout == self.to_k.cout == self.to_v.cout and self.to_q.cout % 16 == 0):
-            self.qkv = (torch.cat([L.tc[: L.cout] for L in (self.to_q, self.to_k, self.to_v)], 0).contiguous(),
-                        torch.cat([self.to_q.b, self.to_k.b, self.to_v.b]).contiguous())
 
         ffm = m.ffm
         self.ffm_blk = ConvLayer(ffm.convblk.conv, ffm.convblk.bn, ACT_RELU, wd, "ffm.convblk")
@@ -370,6 +363,27 @@ class Engine:
                                               (w_low @ bb.double()).float(), 1, 0))
         self.head_conv = ConvLayer(m.conv_out.conv.conv, m.conv_out.conv.bn, ACT_RELU, wd, "conv_out.conv")
         self.head_out = ConvLayer(m.conv_out.conv_out, None, ACT_NONE, wd, "conv_out.conv_out")
+
+    def _pack_cab(self, cab):
+        """The ContextAggregationBlock's layers (reference: cab.py:84-129,170-184,192-216), BN folded."""
+        wd = self.tdt
+        ga = cab.global_attn
+        self.to_q = ConvLayer(ga.to_query[0], ga.to_query[1], ACT_RELU, wd, "cab.to_query")
+        self.to_k = ConvLayer(ga.to_key[0], ga.to_key[1], ACT_RELU, wd, "cab.to_key")
+        self.to_v = ConvLayer(ga.to_value, None, ACT_NONE, wd, "cab.to_value")
+        self.psp_k = ConvLayer(ga.psp_key.project, None, ACT_NONE, wd, "cab.psp_key")
+        self.psp_v = ConvLayer(ga.psp_value.project, None, ACT_NONE, wd, "cab.psp_value")
+        self.proj_out = ConvLayer(ga.project_out, None, ACT_NONE, wd, "cab.project_out")
+        self.local = [DwLayer(d.block[0], d.block[1], ACT_RELU, f"cab.local{i}")
+                      for i, d in enumerate(cab.local_attn.refine)]
+        self.gamma = _host(cab.gamma).contiguous()
+        self.key_ch = self.to_k.cout
+        # to_query | to_key | to_value read the same tensor: one 256 -> 3 x 128 GEMM, ReLU on the first 2 x 128 outputs
+        self.qkv = None
+        if (self.precision == "bf16" and all(L.tc is not None and L.kh == 1 for L in (self.to_q, self.to_k, self.to_v))
+                and self.to_q.cout == self.to_k.cout == self.to_v.cout and self.to_q.cout % 16 == 0):
+            self.qkv = (torch.cat([L.tc[: L.cout] for L in (self.to_q, self.to_k, self.to_v)], 0).contiguous(),
+                        torch.cat([self.to_q.b, self.to_k.b, self.to_v.b]).contiguous())
 
     # ------------------------------------------------------------------ kernel wrappers
     @property
@@ -640,19 +654,27 @@ class Engine:
         return self.conv(cat, L)
 
     def attention(self, q: Map, k: Map, v: Map) -> Map:
-        """softmax(q k^T / sqrt(d)) v per image (reference: cab.py:149-153).  q,k,v: [N, L, d] dense."""
-        N, Lq, d = q.N, q.H * q.W, q.C
+        """softmax(q k^T / sqrt(dk)) v per image (reference: cab.py:149-153).  q, k: [N, L, dk], v: [N, L, dv] dense;
+        -> ctx [N, L, dv].  The tensor-core kernel takes dk in {64, 128, 256} x dv in {64, 128} (bf16, 16-byte rows);
+        every other width / the fp32 parity mode runs the CUDA-core GEMMs + softmax."""
+        N, Lq, d, dv = q.N, q.H * q.W, q.C, v.C
         es = q.t.element_size()
-        ctx = self.new(q.N, q.H, q.W, d)
-        if self.use_tc and d == 128 and q.dt == BF16 and all(m.ld % 8 == 0 and m.off % 8 == 0 for m in (q, k, v)):
-            vt = torch.empty((N, d, -(-Lq // 8) * 8), dtype=torch.bfloat16, device=self.dev)
-            self._run("attention_tc", "cab.attention", 4 * N * Lq * d * es, 4 * N * Lq * Lq * d,
-                      self.lib.cabinet_attention_tc, q.ptr, q.ld, k.ptr, k.ld, v.ptr, v.ld, vt.data_ptr(), ctx.ptr,
-                      ctx.ld, N, Lq, d, float(d) ** -0.5, self.stream)
+        ctx = self.new(q.N, q.H, q.W, dv)
+        if (self.use_tc and d in (64, 128, 256) and dv in (64, 128) and q.dt == BF16
+                and all(m.ld % 8 == 0 and m.off % 8 == 0 for m in (q, k, v))):
+            vt = torch.empty((N, dv, -(-Lq // 8) * 8), dtype=torch.bfloat16, device=self.dev)
+            nbytes, flops = 2 * N * Lq * (d + dv) * es, 2 * N * Lq * Lq * (d + dv)
+            if d == dv == 128:  # CABiNet's attention: the original entry point
+                self._run("attention_tc", "cab.attention", nbytes, flops, self.lib.cabinet_attention_tc, q.ptr, q.ld,
+                          k.ptr, k.ld, v.ptr, v.ld, vt.data_ptr(), ctx.ptr, ctx.ld, N, Lq, d, float(d) ** -0.5, self.stream)
+            else:
+                self._run("attention_tc", "cab.attention", nbytes, flops, self.lib.cabinet_attention_tc_dkdv, q.ptr, q.ld,
+                          k.ptr, k.ld, v.ptr, v.ld, vt.data_ptr(), ctx.ptr, ctx.ld, N, Lq, d, dv, float(d) ** -0.5,
+                          self.stream)
             self.launches += 1  # the V transpose pre-kernel
             return ctx
         s = torch.empty((N, Lq, Lq), dtype=torch.float32, device=self.dev)
-        # S[b][i][j] = alpha * sum_c q[b][i][c] k[b][j][c]   (k acts as the [Cout=L][K=d] "weights")
+        # S[b][i][j] = alpha * sum_c q[b][i][c] k[b][j][c]   (k acts as the [Cout=L][K=dk] "weights")
         self._run("conv2d_simt", "cab.qk", 2 * N * Lq * d * es, 2 * N * Lq * Lq * d, self.lib.cabinet_conv2d_simt,
                   q.ptr, q.dt, 0, 0, q.ld, 1, Lq * q.ld, k.ptr, k.dt, k.ld, 1, Lq * k.ld, None, None, 0,
                   s.data_ptr(), F32, Lq, Lq * Lq, N, 1, 1, Lq, d, Lq, 1, 1, 1, 0, 1, Lq, ACT_NONE, float(d) ** -0.5,
@@ -660,12 +682,76 @@ class Engine:
         p = torch.empty((N, Lq, Lq), dtype=self.tdt, device=self.dev)
         self._run("softmax_rows", "cab.softmax", 0, 0, self.lib.cabinet_softmax_rows, s.data_ptr(), p.data_ptr(),
                   self.dt, N * Lq, Lq, self.stream)
-        # ctx[b][i][c] = sum_j P[b][i][j] v[b][j][c]   (v read as [Cout=d][K=L] with strides (1, ld))
-        self._run("conv2d_simt", "cab.pv", 2 * N * Lq * d * es, 2 * N * Lq * Lq * d, self.lib.cabinet_conv2d_simt,
+        # ctx[b][i][c] = sum_j P[b][i][j] v[b][j][c]   (v read as [Cout=dv][K=L] with strides (1, ld))
+        self._run("conv2d_simt", "cab.pv", 2 * N * Lq * dv * es, 2 * N * Lq * Lq * dv, self.lib.cabinet_conv2d_simt,
                   p.data_ptr(), self.dt, 0, 0, Lq, 1, Lq * Lq, v.ptr, v.dt, 1, v.ld, Lq * v.ld, None, None, 0,
-                  ctx.ptr, ctx.dt, ctx.ld, Lq * ctx.ld, N, 1, 1, Lq, Lq, d, 1, 1, 1, 0, 1, Lq, ACT_NONE, 1.0,
+                  ctx.ptr, ctx.dt, ctx.ld, Lq * ctx.ld, N, 1, 1, Lq, Lq, dv, 1, 1, 1, 0, 1, Lq, ACT_NONE, 1.0,
                   self.stream)
         return ctx
+
+    def cab(self, feat: Map, out: Map):
+        """ContextAggregationBlock: out = gamma * global(feat) + local(feat) (reference: cab.py:131-162,175-184,213-216).
+        ``feat`` dense; ``out`` may be a channel slice of a wider buffer."""
+        N, h, w = feat.N, feat.H, feat.W
+        if self.qkv is not None and self.use_tc and feat.dt == BF16:
+            kc = self.key_ch
+            qkv = self.new(N, h, w, 3 * kc)
+            M = N * h * w
+            self._run("conv_tc", "cab.to_query|key|value", (M * (feat.C + 3 * kc) + self.qkv[0].numel()) * 2,
+                      2 * M * 3 * kc * feat.C, self.lib.cabinet_conv_tc_split_act, feat.ptr, feat.ld, N, h, w, feat.C,
+                      self.qkv[0].data_ptr(), 3 * kc, 1, 1, 1, 0, self.qkv[1].data_ptr(), qkv.ptr, qkv.dt, qkv.ld, h, w,
+                      ACT_RELU, 2 * kc, self.stream)
+            q = qkv.slice(0, kc)
+            with self._branch(1) as joined:     # value PSP chain beside the key PSP chain
+                v = self.psp(qkv.slice(2 * kc, kc), self.psp_v)
+                joined(v.t)
+            k = self.psp(qkv.slice(kc, kc), self.psp_k)
+        else:
+            q = self.conv(feat, self.to_q)
+            k = self.psp(self.conv(feat, self.to_k), self.psp_k)
+            v = self.psp(self.conv(feat, self.to_v), self.psp_v)
+        with self._branch(0) as joined:         # local attention (three depthwise convs) beside the global attention
+            r = feat
+            for L in self.local:
+                r, _ = self.dwconv(r, L)
+            joined(r.t)
+        self._join(1)
+        ctx = self.attention(q, k, v)
+        g = self.conv(ctx, self.proj_out)
+        self._join(0)
+        es = feat.t.element_size()
+        self._run("cab_combine", "cab", 2 * N * h * w * feat.C * es, 0, self.lib.cabinet_cab_combine, g.ptr, feat.ptr,
+                  r.ptr, out.ptr, out.ld, self.gamma.data_ptr(), self.dt, N * h * w, feat.C, self.stream)
+
+    def relayout(self, src: torch.Tensor, src_strides, dst: torch.Tensor, dst_strides, N, H, W, C, name: str):
+        """dst = src element for element, between two (N, H, W, C) stride patterns and any two float dtypes (NCHW <->
+        NHWC at a standalone block's boundary): cabinet_resample_sep with identity row operators."""
+        from .train_engine import _Tables
+
+        if getattr(self, "_tables", None) is None:
+            self._tables = _Tables(self.dev)
+        ty, tx = self._tables.get("identity", H, H, False), self._tables.get("identity", W, W, False)
+        self._run("resample_sep", name, N * H * W * C * (src.element_size() + dst.element_size()), 0,
+                  self.lib.cabinet_resample_sep, src.data_ptr(), dtype_code(src.dtype), *src_strides, dst.data_ptr(),
+                  dtype_code(dst.dtype), *dst_strides, N, H, W, C, *(t.data_ptr() for t in ty), *(t.data_ptr() for t in tx),
+                  0, self.stream)
+
+    @torch.no_grad()
+    def forward_block(self, x: torch.Tensor) -> torch.Tensor:
+        """Standalone ContextAggregationBlock: (N, C, H, W) fp32 / bf16 / fp16 -> the same shape and dtype."""
+        N, C, H, W = x.shape
+        y = torch.empty_like(x, memory_format=torch.contiguous_format)
+        self.launches = 0
+        if N == 0 or H * W == 0:
+            return y
+        nchw = lambda t: (t.stride(0), t.stride(2), t.stride(3), t.stride(1))  # noqa: E731  (n, y, x, c) strides
+        with self._guard():
+            self._scratch = []  # the PSP pools take freshly zeroed scratch
+            feat, out = self.new(N, H, W, C), self.new(N, H, W, C)
+            self.relayout(x, nchw(x), feat.t, (H * W * C, W * C, C, 1), N, H, W, C, "cab.in")
+            self.cab(feat, out)
+            self.relayout(out.t, (H * W * C, W * C, C, 1), y, nchw(y), N, H, W, C, "cab.out")
+        return y
 
     def bilinear(self, x: Map, out: Map, name: str):
         nbytes = x.N * x.C * (x.H * x.W * x.t.element_size() + out.H * out.W * out.t.element_size())
@@ -824,36 +910,8 @@ class Engine:
 
         # ---- attention branch (reference: cabinet.py:75-94, cab.py:131-162,175-184,213-216)
         feat = self.conv(mf, self.conva)
-        if self.qkv is not None and self.use_tc and feat.dt == BF16:
-            kc = self.key_ch
-            qkv = self.new(N, h32, w32, 3 * kc)
-            M = N * h32 * w32
-            self._run("conv_tc", "cab.to_query|key|value", (M * (feat.C + 3 * kc) + self.qkv[0].numel()) * 2,
-                      2 * M * 3 * kc * feat.C, self.lib.cabinet_conv_tc_split_act, feat.ptr, feat.ld, N, h32, w32, feat.C,
-                      self.qkv[0].data_ptr(), 3 * kc, 1, 1, 1, 0, self.qkv[1].data_ptr(), qkv.ptr, qkv.dt, qkv.ld, h32, w32,
-                      ACT_RELU, 2 * kc, self.stream)
-            q = qkv.slice(0, kc)
-            with self._branch(1) as joined:     # value PSP chain beside the key PSP chain
-                v = self.psp(qkv.slice(2 * kc, kc), self.psp_v)
-                joined(v.t)
-            k = self.psp(qkv.slice(kc, kc), self.psp_k)
-        else:
-            q = self.conv(feat, self.to_q)
-            k = self.psp(self.conv(feat, self.to_k), self.psp_k)
-            v = self.psp(self.conv(feat, self.to_v), self.psp_v)
-        with self._branch(0) as joined:         # local attention (three depthwise convs) beside the global attention
-            r = feat
-            for L in self.local:
-                r, _ = self.dwconv(r, L)
-            joined(r.t)
-        self._join(1)
-        ctx = self.attention(q, k, v)
-        g = self.conv(ctx, self.proj_out)
-        self._join(0)
         feat2 = cat_b1.slice(self.last.cout, 256)
-        es = feat.t.element_size()
-        self._run("cab_combine", "cab", 2 * N * h32 * w32 * 256 * es, 0, self.lib.cabinet_cab_combine, g.ptr, feat.ptr,
-                  r.ptr, feat2.ptr, feat2.ld, self.gamma.data_ptr(), self.dt, N * h32 * w32, 256, self.stream)
+        self.cab(feat, feat2)
         aux8 = high = low = None
 
         def low_path():

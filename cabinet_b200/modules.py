@@ -120,6 +120,62 @@ class MobileNetV3(nn.Module):
                 m.bias.data.zero_()
 
 
+class _EngineCache:
+    """Lazily built engines kept in ``__dict__`` (not module state): dropped by ``.to()`` / ``.cuda()`` / ``.half()``,
+    left out of ``deepcopy`` and pickling; a weight change is seen through the parameters' addresses and versions."""
+
+    def _weights_stamp(self):
+        return tuple((t.data_ptr(), t._version) for t in list(self.parameters()) + list(self.buffers()))
+
+    def engine(self):
+        """The packed-weight execution engine for the current weights/device/precision (lazy, cached)."""
+        from .engine import Engine
+
+        eng = self.__dict__.get("_engine")
+        stamp = (self.precision, self._weights_stamp())
+        if eng is None or eng.stamp != stamp:
+            eng = Engine(self, precision=self.precision)
+            eng.stamp = stamp
+            self.__dict__["_engine"] = eng
+        return eng
+
+    def train_engine(self):
+        """The training-step engine (train-mode forward + backward kernels) for the current device / precision."""
+        from .train_engine import TrainEngine
+
+        eng = self.__dict__.get("_train_engine")
+        dev = next(self.parameters()).device
+        if eng is None or eng.dev != dev or eng.precision != self.train_precision:
+            eng = self.__dict__["_train_engine"] = TrainEngine(self, precision=self.train_precision)
+        return eng
+
+    def repack(self):
+        """Drop packed weights (call after mutating parameters through ``.data`` views the stamp cannot see)."""
+        self.__dict__["_engine"] = None
+
+    def _apply(self, fn, *a, **kw):
+        self.__dict__["_engine"] = None
+        self.__dict__["_train_engine"] = None
+        return super()._apply(fn, *a, **kw)
+
+    def __deepcopy__(self, memo):  # EMA deep-copies the model (reference: src/utils/ema.py:44)
+        eng, teng = self.__dict__.pop("_engine", None), self.__dict__.pop("_train_engine", None)
+        try:
+            cls = self.__class__
+            new = cls.__new__(cls)
+            memo[id(self)] = new
+            new.__dict__.update({k: copy.deepcopy(v, memo) for k, v in self.__dict__.items()})
+            new.__dict__["_engine"] = new.__dict__["_train_engine"] = None
+        finally:
+            self.__dict__["_engine"], self.__dict__["_train_engine"] = eng, teng
+        return new
+
+    def __getstate__(self):
+        d = dict(self.__dict__)
+        d["_engine"] = d["_train_engine"] = None
+        return d
+
+
 # --------------------------------------------------------------------------- CAB
 class DWConv(nn.Module):
     """``block.{0,1}``: depthwise 3x3 + BN (+ReLU) (reference: cab.py:18-38)."""
@@ -166,14 +222,50 @@ class LocalAttention(nn.Module):
         self.gate = _slot()
 
 
-class ContextAggregationBlock(nn.Module):
-    """gamma * global + local (reference: cab.py:192-211)."""
+class ContextAggregationBlock(_EngineCache, nn.Module):
+    """gamma * global + local (reference: cab.py:192-216), runnable on its own.
+
+    ``forward`` maps an (N, in_channels, H, W) CUDA tensor (fp32 / bf16 / fp16) to a tensor of the same shape and dtype
+    with the mode semantics of ``CABiNet.forward``: ``.eval()`` runs the inference schedule (BN folded) unless ``x``
+    requires grad with grad mode on, which runs the differentiable schedule with running-statistics BatchNorm;
+    ``.train()`` uses batch statistics (running statistics updated) and fills ``p.grad`` / ``x.grad`` on backward.
+    ``precision`` ("bf16" | "fp32") selects the inference schedule, ``train_precision`` ("fp32" | "bf16" | "fp16") the
+    differentiable one.  Widths: ``in_channels % 16 == 0`` (key width in_channels / 2 a multiple of 8) and
+    ``value_channels % 8 == 0`` (16-byte pixel rows for the kernels).
+    """
 
     def __init__(self, in_channels, value_channels):
         super().__init__()
+        self.in_channels, self.value_channels = in_channels, value_channels
         self.global_attn = GlobalContextAttention(in_channels, in_channels // 2, value_channels, in_channels, 1)
         self.local_attn = LocalAttention(in_channels)
         self.gamma = nn.Parameter(torch.zeros(1))
+        self.precision = "bf16"
+        self.train_precision = "fp32"
+        self.__dict__["_engine"] = None
+        self.__dict__["_train_engine"] = None
+
+    def _check_input(self, x):
+        C, V = self.in_channels, self.value_channels
+        if C <= 0 or C % 16 or V <= 0 or V % 8:
+            raise ValueError(f"ContextAggregationBlock({C}, {V}): the kernels need in_channels % 16 == 0 and "
+                             f"value_channels % 8 == 0")
+        if not isinstance(x, torch.Tensor) or x.dim() != 4 or x.shape[1] != C:
+            raise ValueError(f"expected an (N, {C}, H, W) tensor, got {getattr(x, 'shape', type(x))}")
+        if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
+            raise TypeError(f"ContextAggregationBlock takes float32, bfloat16 or float16 input, got {x.dtype}")
+        if not x.is_cuda:
+            raise RuntimeError("cabinet_b200.ContextAggregationBlock has no CPU path: move the block and the input to a "
+                               "CUDA device")
+
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        """(N, C, H, W) -> gamma * global(x) + local(x), same shape and dtype (reference: cab.py:213-216)."""
+        self._check_input(x)
+        if self.training or (torch.is_grad_enabled() and x.requires_grad):
+            from .train_engine import BlockStep
+
+            return BlockStep.apply(self.train_engine(), x, *self.parameters())
+        return self.engine().forward_block(x)
 
 
 # --------------------------------------------------------------------------- CABiNet heads
@@ -243,7 +335,7 @@ class CABiNetOutput(nn.Module):
         self.conv_out = _conv(mid_chan, n_classes)
 
 
-class CABiNet(nn.Module):
+class CABiNet(_EngineCache, nn.Module):
     """Drop-in for the reference ``CABiNet`` (reference: cabinet.py:175-300).
 
     Same constructor, same children (``mobile / ab / sb / ffm / conv_out``), same
@@ -282,47 +374,11 @@ class CABiNet(nn.Module):
         self.__dict__["_train_engine"] = None
 
     # ------------------------------------------------------------------ engine plumbing
-    def _weights_stamp(self):
-        return tuple((t.data_ptr(), t._version) for t in list(self.parameters()) + list(self.buffers()))
-
     def engine(self):
         """The packed-weight execution engine for the current weights/device/precision (lazy, cached)."""
-        from .engine import Engine
-
-        eng = self.__dict__.get("_engine")
-        stamp = (self.precision, self._weights_stamp())
-        if eng is None or eng.stamp != stamp:
-            eng = Engine(self, precision=self.precision)
-            eng.stamp = stamp
-            self.__dict__["_engine"] = eng
+        eng = super().engine()
         eng.use_cuda_graph, eng.sub_batch = bool(self.use_cuda_graph), int(self.sub_batch)
         return eng
-
-    def repack(self):
-        """Drop packed weights (call after mutating parameters through ``.data`` views the stamp cannot see)."""
-        self.__dict__["_engine"] = None
-
-    def _apply(self, fn, *a, **kw):
-        self.__dict__["_engine"] = None
-        self.__dict__["_train_engine"] = None
-        return super()._apply(fn, *a, **kw)
-
-    def __deepcopy__(self, memo):  # EMA deep-copies the model (reference: src/utils/ema.py:44)
-        eng, teng = self.__dict__.pop("_engine", None), self.__dict__.pop("_train_engine", None)
-        try:
-            cls = self.__class__
-            new = cls.__new__(cls)
-            memo[id(self)] = new
-            new.__dict__.update({k: copy.deepcopy(v, memo) for k, v in self.__dict__.items()})
-            new.__dict__["_engine"] = new.__dict__["_train_engine"] = None
-        finally:
-            self.__dict__["_engine"], self.__dict__["_train_engine"] = eng, teng
-        return new
-
-    def __getstate__(self):
-        d = dict(self.__dict__)
-        d["_engine"] = d["_train_engine"] = None
-        return d
 
     # ------------------------------------------------------------------ forward surface
     def _check_input(self, x, inference_only=True):
@@ -333,16 +389,6 @@ class CABiNet(nn.Module):
         if self.training and inference_only:
             raise RuntimeError("the fused mask / confusion-matrix / class-map calls are inference paths (eval-mode BN); "
                                "call .eval() first")
-
-    def train_engine(self):
-        """The training-step engine (train-mode forward + backward kernels) for the current device / precision."""
-        from .train_engine import TrainEngine
-
-        eng = self.__dict__.get("_train_engine")
-        dev = next(self.parameters()).device
-        if eng is None or eng.dev != dev or eng.precision != self.train_precision:
-            eng = self.__dict__["_train_engine"] = TrainEngine(self, precision=self.train_precision)
-        return eng
 
     def forward(self, x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
         """(N,3,H,W) -> (final_logit, high_res_logit_up), each (N, n_classes, H, W) NCHW.

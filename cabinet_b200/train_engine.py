@@ -142,7 +142,7 @@ class TrainEngine:
         # the activation dtype, in one place: every 2-byte buffer and operand of the schedule follows it
         self.tdt = {"bf16": torch.bfloat16, "fp16": torch.float16, "fp32": torch.float32}[precision]
         self.dt = dtype_code(self.tdt)
-        self.n_classes = model.n_classes
+        self.n_classes = getattr(model, "n_classes", 0)   # 0: a standalone ContextAggregationBlock (``block_forward``)
         self.tables = _Tables(self.dev)
         self.tape: List = []
         self.pgrads: Dict[int, torch.Tensor] = {}
@@ -661,14 +661,16 @@ class TrainEngine:
         return self.conv(cat, project)
 
     def attention(self, q: Map, k: Map, v: Map) -> Map:
-        """softmax(q k^T / sqrt(d)) v per image with the probabilities kept for the backward (cab.py:149-153)."""
-        N, L, d = q.N, q.H * q.W, q.C
+        """softmax(q k^T / sqrt(d)) v per image with the probabilities kept for the backward (cab.py:149-153).  q, k: [N, L, d]
+        (d = key width, which sets the scale), v: [N, L, dv]; -> ctx [N, L, dv]."""
+        N, L, d, dv = q.N, q.H * q.W, q.C, v.C
         alpha = float(d) ** -0.5
-        if (self.use_tc and self.attn_tc and L % 128 == 0 and d % 64 == 0 and all(self._tc_ok(t) and t.ld == d for t in (q, k, v))):
+        if (self.use_tc and self.attn_tc and L % 128 == 0 and d % 64 == 0 and dv % 64 == 0
+                and all(self._tc_ok(t) and t.ld == t.C for t in (q, k, v))):
             return self._attention_tc(q, k, v, alpha)
         s = torch.empty((N, L, L), dtype=torch.float32, device=self.dev)
         p = torch.empty((N, L, L), dtype=torch.float32, device=self.dev)
-        ctx = self.new(q.N, q.H, q.W, d)
+        ctx = self.new(q.N, q.H, q.W, dv)
 
         def gemm(xp, xdt, sxw, sxc, xbs, wpt, wdt, w_sco, w_sk, wbs, yp, ydt, ldy, ybs, Mr, Kd, Nc, al=1.0):
             # out[b][m][co] = al * sum_k x[b][m][k] w[b][co][k]
@@ -677,7 +679,7 @@ class TrainEngine:
 
         gemm(q.ptr, q.dt, q.ld, 1, L * q.ld, k.ptr, k.dt, k.ld, 1, L * k.ld, s.data_ptr(), F32, L, L * L, L, d, L, alpha)
         self._call("cabinet_softmax_rows", s.data_ptr(), p.data_ptr(), F32, N * L, L)
-        gemm(p.data_ptr(), F32, L, 1, L * L, v.ptr, v.dt, 1, v.ld, L * v.ld, ctx.ptr, ctx.dt, ctx.ld, L * ctx.ld, L, L, d)
+        gemm(p.data_ptr(), F32, L, 1, L * L, v.ptr, v.dt, 1, v.ld, L * v.ld, ctx.ptr, ctx.dt, ctx.ld, L * ctx.ld, L, L, dv)
         ctx.needs_grad = q.needs_grad or k.needs_grad or v.needs_grad
 
         def backward(g: _Grads):
@@ -686,16 +688,17 @@ class TrainEngine:
                 return
             dp = s  # the raw scores are not needed any more: reuse their buffer
             ds = torch.empty((N, L, L), dtype=torch.float32, device=self.dev)
-            dq, dk, dv = (self.new(q.N, q.H, q.W, d) for _ in range(3))
+            dq, dk = (self.new(q.N, q.H, q.W, d) for _ in range(2))
+            dV = self.new(q.N, q.H, q.W, dv)
             # dV[j][c] = sum_i P[i][j] dO[i][c]
-            gemm(p.data_ptr(), F32, 1, L, L * L, do.ptr, do.dt, 1, do.ld, L * do.ld, dv.ptr, dv.dt, d, L * d, L, L, d)
+            gemm(p.data_ptr(), F32, 1, L, L * L, do.ptr, do.dt, 1, do.ld, L * do.ld, dV.ptr, dV.dt, dv, L * dv, L, L, dv)
             # dP[i][j] = sum_c dO[i][c] V[j][c]
-            gemm(do.ptr, do.dt, do.ld, 1, L * do.ld, v.ptr, v.dt, v.ld, 1, L * v.ld, dp.data_ptr(), F32, L, L * L, L, d, L)
+            gemm(do.ptr, do.dt, do.ld, 1, L * do.ld, v.ptr, v.dt, v.ld, 1, L * v.ld, dp.data_ptr(), F32, L, L * L, L, dv, L)
             self._call("cabinet_softmax_backward", p.data_ptr(), dp.data_ptr(), ds.data_ptr(), N * L, L, alpha)
             # dQ[i][c] = sum_j dS[i][j] K[j][c];  dK[j][c] = sum_i dS[i][j] Q[i][c]
             gemm(ds.data_ptr(), F32, L, 1, L * L, k.ptr, k.dt, 1, k.ld, L * k.ld, dq.ptr, dq.dt, d, L * d, L, L, d)
             gemm(ds.data_ptr(), F32, 1, L, L * L, q.ptr, q.dt, 1, q.ld, L * q.ld, dk.ptr, dk.dt, d, L * d, L, L, d)
-            for tgt, src in ((q, dq), (k, dk), (v, dv)):
+            for tgt, src in ((q, dq), (k, dk), (v, dV)):
                 if tgt.needs_grad:
                     self.add_grad(g, tgt, src)
 
@@ -707,14 +710,14 @@ class TrainEngine:
         of an image IS a cabinet_conv_tc weight matrix (rows = tokens, k = channels), so S = Q K^T and dP = dO V^T are 1x1
         convolutions with per-image weights K / V, P V and dQ = dS K the same with K^T / V^T ([d][L], one small transpose
         each), and dV = P^T dO, dK = dS^T Q reduce over the token ("pixel") index: the weight-gradient GEMM, batched per image."""
-        N, L, d, H, W = q.N, q.H * q.W, q.C, q.H, q.W
+        N, L, d, dv, H, W = q.N, q.H * q.W, q.C, v.C, q.H, q.W
         dev, bf = self.dev, self.tdt
         s = torch.empty((N, L, L), dtype=torch.float32, device=dev)
         p = torch.empty((N, L, L), dtype=torch.float32, device=dev)
         p16 = torch.empty((N, L, L), dtype=bf, device=dev)
-        vt = torch.empty((N, d, L), dtype=bf, device=dev)
-        ctx = self.new(N, H, W, d)
-        zL, zd = self._zeros(L), self._zeros(d)
+        vt = torch.empty((N, dv, L), dtype=bf, device=dev)
+        ctx = self.new(N, H, W, dv)
+        zL, zd, zv = self._zeros(L), self._zeros(d), self._zeros(dv)
 
         def gemm(x_ptr, ldx, cin, w_ptr, cout, bias, y_ptr, ydt, ldy):
             # y[n][l][co] = sum_k x[n][l][k] w[n][co][k]   (w: [N][cout][cin] 2-byte, dense)
@@ -723,8 +726,8 @@ class TrainEngine:
 
         gemm(q.ptr, q.ld, d, k.ptr, L, zL, s.data_ptr(), F32, L)
         self._call_tc("cabinet_attn_softmax", s.data_ptr(), alpha, p.data_ptr(), p16.data_ptr(), N * L, L)
-        self._call_tc("cabinet_transpose_tokens", v.ptr, v.ld, vt.data_ptr(), N, L, d)
-        gemm(p16.data_ptr(), L, L, vt.data_ptr(), d, zd, ctx.ptr, ctx.dt, ctx.ld)
+        self._call_tc("cabinet_transpose_tokens", v.ptr, v.ld, vt.data_ptr(), N, L, dv)
+        gemm(p16.data_ptr(), L, L, vt.data_ptr(), dv, zv, ctx.ptr, ctx.dt, ctx.ld)
         ctx.needs_grad = q.needs_grad or k.needs_grad or v.needs_grad
 
         def backward(g: _Grads):
@@ -735,27 +738,42 @@ class TrainEngine:
             ds16 = torch.empty((N, L, L), dtype=bf, device=dev)
             kt = torch.empty((N, d, L), dtype=bf, device=dev)
             dq = self.new(N, H, W, d)
-            dkv = torch.empty((2, N, L, d), dtype=torch.float32, device=dev)
+            dk32 = torch.empty((N, L, d), dtype=torch.float32, device=dev)
+            dv32 = torch.empty((N, L, dv), dtype=torch.float32, device=dev)
 
             def wgrad(a, x_map, out):  # out[n][j][c] = sum_i a[n][i][j] x[n][i][c]
-                self._call_tc("cabinet_conv_wgrad_tc_batched", a.data_ptr(), L, x_map.ptr, x_map.ld, out.data_ptr(), N, H, W, d, L)
+                self._call_tc("cabinet_conv_wgrad_tc_batched", a.data_ptr(), L, x_map.ptr, x_map.ld, out.data_ptr(), N, H, W,
+                              x_map.C, L)
 
-            wgrad(p16, do, dkv[1])                                                # dV[j][c] = sum_i P[i][j] dO[i][c]
-            gemm(do.ptr, do.ld, d, v.ptr, L, zL, dp.data_ptr(), F32, L)           # dP[i][j] = sum_c dO[i][c] V[j][c]
+            wgrad(p16, do, dv32)                                                  # dV[j][c] = sum_i P[i][j] dO[i][c]
+            gemm(do.ptr, do.ld, dv, v.ptr, L, zL, dp.data_ptr(), F32, L)          # dP[i][j] = sum_c dO[i][c] V[j][c]
             self._call_tc("cabinet_attn_softmax_backward", p.data_ptr(), dp.data_ptr(), ds16.data_ptr(), N * L, L, alpha)
             self._call_tc("cabinet_transpose_tokens", k.ptr, k.ld, kt.data_ptr(), N, L, d)
             gemm(ds16.data_ptr(), L, L, kt.data_ptr(), d, zd, dq.ptr, dq.dt, dq.ld)  # dQ[i][c] = sum_j dS[i][j] K[j][c]
-            wgrad(ds16, q, dkv[0])                                                # dK[j][c] = sum_i dS[i][j] Q[i][c]
-            dk, dv = self.new(N, H, W, d), self.new(N, H, W, d)
-            for src, dst in ((dkv[0], dk), (dkv[1], dv)):  # fp32 -> the activation dtype
-                self._call("cabinet_affine_act", src.data_ptr(), d, F32, None, None, None, 0.0, None, 0, dst.ptr, dst.ld,
-                           dst.dt, N * L, L, d, ACT_NONE)
-            for tgt, src in ((q, dq), (k, dk), (v, dv)):
+            wgrad(ds16, q, dk32)                                                  # dK[j][c] = sum_i dS[i][j] Q[i][c]
+            dk, dV = self.new(N, H, W, d), self.new(N, H, W, dv)
+            for src, dst in ((dk32, dk), (dv32, dV)):  # fp32 -> the activation dtype
+                self._call("cabinet_affine_act", src.data_ptr(), dst.C, F32, None, None, None, 0.0, None, 0, dst.ptr, dst.ld,
+                           dst.dt, N * L, L, dst.C, ACT_NONE)
+            for tgt, src in ((q, dq), (k, dk), (v, dV)):
                 if tgt.needs_grad:
                     self.add_grad(g, tgt, src)
 
         self.tape.append(backward)
         return ctx
+
+    def cab(self, feat: Map, block, out: Map):
+        """ContextAggregationBlock ``block``: out = gamma * global(feat) + local(feat) (cab.py:131-162,175-184,213-216)."""
+        ga = block.global_attn
+        q = self.bn(self.conv(feat, ga.to_query[0]), ga.to_query[1], ACT_RELU)
+        k = self.psp(self.bn(self.conv(feat, ga.to_key[0]), ga.to_key[1], ACT_RELU), ga.psp_key.project)
+        v = self.psp(self.conv(feat, ga.to_value), ga.psp_value.project)
+        ctx = self.attention(q, k, v)
+        gl = self.conv(ctx, ga.project_out)
+        r = feat
+        for dwb in block.local_attn.refine:
+            r = self.bn(self.dwconv(r, dwb.block[0]), dwb.block[1], ACT_RELU)
+        self.cab_combine(gl, feat, r, block.gamma, out)
 
     def cab_combine(self, gmap: Map, x: Map, r: Map, gamma, out: Map):
         """out = gamma * global + x + x * sigmoid(r) (cab.py:175-184,213-216)."""
@@ -810,7 +828,6 @@ class TrainEngine:
         self._pflat, self._bn_seen = None, []
         self._stems = (None, None, tuple(x.shape)) if input_grad else None
         mob, sb, ab, ffm, head = m.mobile, m.sb, m.ab, m.ffm, m.conv_out
-        ga, cab = ab.a2block.global_attn, ab.a2block
 
         # ---- spatial branch (cabinet.py:108-129)
         xcol = self.stem_im2col(x) if (self.use_tc and self.stem_gemm) else None
@@ -858,16 +875,8 @@ class TrainEngine:
 
         # ---- attention branch (cabinet.py:75-94, cab.py:131-162,175-184,213-216)
         feat = self.bn(self.conv(mf, ab.conva[0]), ab.conva[1], ACT_RELU)
-        q = self.bn(self.conv(feat, ga.to_query[0]), ga.to_query[1], ACT_RELU)
-        k = self.psp(self.bn(self.conv(feat, ga.to_key[0]), ga.to_key[1], ACT_RELU), ga.psp_key.project)
-        v = self.psp(self.conv(feat, ga.to_value), ga.psp_value.project)
-        ctx = self.attention(q, k, v)
-        gl = self.conv(ctx, ga.project_out)
-        r = feat
-        for dwb in cab.local_attn.refine:
-            r = self.bn(self.dwconv(r, dwb.block[0]), dwb.block[1], ACT_RELU)
         feat2 = cat_b1.slice(n_mf, 256)
-        self.cab_combine(gl, feat, r, cab.gamma, feat2)
+        self.cab(feat, ab.a2block, feat2)
         low = self.conv(feat2, ab.convb)
         low_up = self.resample(low, "bilinear", H8, W8, out=cat_ffm.slice(n_sb, low.C))         # cabinet.py:228-233
         cat_b1.needs_grad = mf.needs_grad or feat2.needs_grad
@@ -936,6 +945,54 @@ class TrainEngine:
                    dy3.ptr if dy3 is not None else None, dy3.ld if dy3 is not None else 0, dt, w7.data_ptr(), w3.data_ptr(),
                    dx.data_ptr(), N, H, W, stem3.H, stem3.W)
         return dx
+
+    # ------------------------------------------------------------------ a standalone ContextAggregationBlock
+    def _relayout(self, src: torch.Tensor, src_strides, dst: torch.Tensor, dst_strides, N, H, W, C):
+        """dst = src between two (N, H, W, C) stride patterns and float dtypes (NCHW <-> NHWC at the block's boundary)."""
+        ty, tx = self.tables.get("identity", H, H, False), self.tables.get("identity", W, W, False)
+        self._call("cabinet_resample_sep", src.data_ptr(), self._dt(src), *src_strides, dst.data_ptr(), self._dt(dst),
+                   *dst_strides, N, H, W, C, *(t.data_ptr() for t in ty), *(t.data_ptr() for t in tx), 0)
+
+    def block_forward(self, x: torch.Tensor, input_grad: bool) -> torch.Tensor:
+        """``self.model`` is a ContextAggregationBlock: its train-mode (or differentiable eval-mode) forward on the
+        (N, C, H, W) ``x`` -> y of x's shape and dtype; the tape is kept for ``block_backward``."""
+        N, C, H, W = x.shape
+        self.tape, self.launches, self.pgrads, self.phase = [], 0, {}, "fwd"
+        self._pflat, self._bn_seen, self._stems = None, [], None
+        nchw = lambda t: (t.stride(0), t.stride(2), t.stride(3), t.stride(1))  # noqa: E731  (n, y, x, c) strides
+        feat, out = self.new(N, H, W, C), self.new(N, H, W, C)
+        self._relayout(x, nchw(x), feat.t, (H * W * C, W * C, C, 1), N, H, W, C)
+        feat.needs_grad = input_grad
+        self.cab(feat, self.model, out)
+        y = torch.empty_like(x, memory_format=torch.contiguous_format)
+        self._relayout(out.t, (H * W * C, W * C, C, 1), y, nchw(y), N, H, W, C)
+        self._block = (feat, out)
+        if self._bn_seen:
+            torch._foreach_add_(self._bn_seen, 1)
+        return y
+
+    def block_backward(self, dy: torch.Tensor) -> Tuple[Dict[int, torch.Tensor], Optional[torch.Tensor]]:
+        """Gradient of ``block_forward``'s output -> ({id(parameter): fp32 gradient}, gradient of x in x's dtype or None)."""
+        feat, out = self._block
+        N, H, W, C = out.N, out.H, out.W, out.C
+        g = _Grads(self)
+        self.pgrads, self.phase, self._pflat, self._side_used = {}, "bwd", None, False
+        self._ensure_pflat()
+        dx = None
+        if out.needs_grad:
+            dout, _ = g.out(out)
+            self._relayout(dy, (dy.stride(0), dy.stride(2), dy.stride(3), dy.stride(1)), dout.t, (H * W * C, W * C, C, 1),
+                           N, H, W, C)
+            for i in range(len(self.tape) - 1, -1, -1):
+                self.tape[i](g)
+            dfeat = g.get(feat) if feat.needs_grad else None
+            if dfeat is not None:
+                dx = torch.empty((N, C, H, W), dtype=dy.dtype, device=self.dev)
+                self._relayout(dfeat.t, (H * W * C, W * C, C, 1), dx, (C * H * W, W, 1, H * W), N, H, W, C)
+        if self._side_used:  # join: the parameter gradients are complete when the caller's stream continues
+            torch.cuda.current_stream(self.dev).wait_stream(self._side)
+        self.tape, self._block = [], None
+        return self.pgrads, dx
 
     # ------------------------------------------------------------------ the step as two CUDA graphs
     def _addresses(self) -> tuple:
@@ -1058,3 +1115,21 @@ class TrainStep(torch.autograd.Function):
             gp = grads.get(id(p))
             out.append(gp.to(p.dtype) if gp is not None else None)
         return (None, None, dx, *out)
+
+
+class BlockStep(torch.autograd.Function):
+    """Autograd hand-off of a standalone ContextAggregationBlock: inputs = (engine, x, *parameters); output = y."""
+
+    @staticmethod
+    def forward(ctx, eng: TrainEngine, x, *params):
+        with torch.no_grad(), torch.cuda.device(eng.dev):
+            y = eng.block_forward(x, bool(ctx.needs_input_grad[1]))
+        ctx.eng, ctx.params = eng, params
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        eng = ctx.eng
+        with torch.no_grad(), torch.cuda.device(eng.dev):
+            grads, dx = eng.block_backward(dy)
+        return (None, dx, *(grads[id(p)].to(p.dtype) if id(p) in grads else None for p in ctx.params))

@@ -305,6 +305,14 @@ int cabinet_attention_tc(const void* q, long long ldq, const void* k, long long 
                          void* vt_workspace, void* ctx, long long ldc, int N, int L, int d, float scale,
                          cabinet_stream_t stream);
 
+/* The same with separate query / key width dk and value / output width dv (a ContextAggregationBlock(C, V) has dk = C / 2,
+ * dv = V): q, k bf16 [N][L][dk], v bf16 [N][L][dv], ctx bf16 [N][L][dv], vt_workspace bf16 [N][dv][ceil8(L)].
+ * dk in {64, 128, 256}, dv in {64, 128}; scale is the caller's (the reference's dk^-0.5).  At dk = dv = 128 it computes
+ * exactly what cabinet_attention_tc computes. */
+int cabinet_attention_tc_dkdv(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv,
+                              void* vt_workspace, void* ctx, long long ldc, int N, int L, int dk, int dv, float scale,
+                              cabinet_stream_t stream);
+
 /* out[p][0:C] = gamma * g + x + x * sigmoid(r)   (src/models/cab.py:182-184,213-216).  g, x, r are dense
  * [n_pixels][C]; out has pixel stride ldo (it is written straight into the b1 concat buffer,
  * src/models/cabinet.py:87).  gamma is a DEVICE scalar (the nn.Parameter itself). */
