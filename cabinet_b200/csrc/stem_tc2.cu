@@ -314,3 +314,262 @@ extern "C" int cabinet_stem_tc2(const float* x, int N, int H, int W, const void*
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
 }
+
+// ===================================================================================================================
+// The backbone stem alone (a standalone MobileNetV3): 3x3 s2 p1, 3 -> 16, BN folded, HardSwish, in the formulation
+// above.  The window starts one aligned pixel group left of the footprint (input column 2 ow0 - 4), so tap row ky of
+// output (oy, ox) reads the copy at pixels 2 ox + 2 .. 2 ox + 5: slot 0 carries no weight (its constant-1 channel carries
+// the bias), slots 1..3 are kx = 0..2.  That is ONE K16 slice per tap row: 3 MMAs of M128 N16 K16 per 128 pixels, over a
+// 33 x 20 window.  Per tile the kernel moves ~8 KB in and 4 KB out against 6 tiny MMAs, so it keeps more windows in
+// flight (6 stages) than the fused kernel.
+namespace {
+namespace s3 {
+
+constexpr int TH = 16, TW = 8;
+constexpr int WIN_H = 2 * TH + 1, WIN_W = 20;       // rows 2 oh0 - 1 .. 2 oh0 + 31, cols 2 ow0 - 4 .. 2 ow0 + 15
+constexpr int WIN_BYTES = 3 * WIN_H * WIN_W * 4;    // 7920
+constexpr int WIN_STRIDE = 7936;
+constexpr int WIN_STAGES = 6;
+constexpr int PITCH = WIN_W * 8;                    // 160
+constexpr int WINB_STRIDE = 5376;                   // >= WIN_H * PITCH = 5280
+constexpr int WINB_STAGES = 3;
+constexpr int NOUT = 16;
+constexpr int NMMA = 3;                             // one K16 slice per tap row
+constexpr int W_MMA_BYTES = 2 * (NOUT / 8) * 128;   // 512
+constexpr int W_BYTES = NMMA * W_MMA_BYTES;         // 1536
+constexpr int ACC_STAGES = 2, ACC_COLS = 32;
+constexpr int CONV_WARPS = 8, CONV_THREADS = 32 * CONV_WARPS;
+constexpr int EPI_WARP0 = 2 + CONV_WARPS;
+constexpr int NUM_THREADS = 64 + CONV_THREADS + 128;
+constexpr int CST_BYTES = 128 * 32;
+constexpr int W_RESERVE = 2048;
+constexpr int SMEM_BYTES = W_RESERVE + 2 * CST_BYTES + WIN_STAGES * WIN_STRIDE + WINB_STAGES * WINB_STRIDE + 1024;
+
+__global__ void __launch_bounds__(NUM_THREADS, 1)
+stem3_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmY, const Stem2Params p) {
+    extern __shared__ uint8_t smem_raw[];
+    __shared__ __align__(8) uint64_t w_bar, win_full[WIN_STAGES], win_empty[WIN_STAGES], a_full[WINB_STAGES],
+        a_empty[WINB_STAGES], acc_full[ACC_STAGES], acc_empty[ACC_STAGES];
+    __shared__ uint32_t tmem_base_smem;
+
+    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+    uint8_t* sW = smem;                                   // 3 x [16 x 16] bf16 core-matrix tiles
+    uint8_t* sCst = sW + W_RESERVE;                       // 2 x staged output tile [128 px][16]
+    uint8_t* sWin = sCst + 2 * CST_BYTES;                 // 6 x [3][33][20] fp32
+    uint8_t* sWinB = sWin + WIN_STAGES * WIN_STRIDE;      // 3 x [33][20][4] bf16: the A operand of the 3 MMAs
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+
+    if (threadIdx.x == 0) {
+        tc::prefetch_tmap(&tmX);
+        tc::prefetch_tmap(&tmY);
+        tc::mbar_init(&w_bar, 1);
+        for (int s = 0; s < WIN_STAGES; ++s) {
+            tc::mbar_init(&win_full[s], 1);
+            tc::mbar_init(&win_empty[s], CONV_WARPS);
+        }
+        for (int s = 0; s < WINB_STAGES; ++s) {
+            tc::mbar_init(&a_full[s], CONV_WARPS);
+            tc::mbar_init(&a_empty[s], 1);
+        }
+        for (int s = 0; s < ACC_STAGES; ++s) {
+            tc::mbar_init(&acc_full[s], 1);
+            tc::mbar_init(&acc_empty[s], 4);
+        }
+        tc::mbar_fence_init();
+        tc::fence_proxy_async();
+    }
+    if (warp == 1) tc::tmem_alloc(&tmem_base_smem, ACC_STAGES * ACC_COLS);
+    tc::tc_fence_before();
+    __syncthreads();
+    tc::tc_fence_after();
+    const uint32_t tmem = tmem_base_smem;
+    const int tiles_per_img = p.tiles_w * p.tiles_h;
+
+    if (warp == 0) {
+        if (lane == 0) {
+            // ================= TMA producer =================
+            tc::mbar_expect_tx(&w_bar, W_BYTES);
+            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                             tc::smem_u32(sW)),
+                         "l"(reinterpret_cast<uint64_t>(p.w)), "r"(W_BYTES), "r"(tc::smem_u32(&w_bar))
+                         : "memory");
+            int it = 0;
+            for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+                const int s = it % WIN_STAGES;
+                const uint32_t ph = (it / WIN_STAGES) & 1;
+                const int img = tile / tiles_per_img, r = tile - img * tiles_per_img;
+                const int oh0 = (r / p.tiles_w) * TH, ow0 = (r % p.tiles_w) * TW;
+                tc::mbar_wait(&win_empty[s], ph ^ 1);
+                tc::mbar_expect_tx(&win_full[s], WIN_BYTES);
+                tc::tma_load_3d(sWin + s * WIN_STRIDE, &tmX, &win_full[s], 2 * ow0 - 4, 2 * oh0 - 1, 3 * img);
+            }
+        }
+        __syncwarp();
+    } else if (warp == 1) {
+        // ================= MMA issuer =================
+        const uint32_t leader = tc::elect_one();
+        const uint32_t idesc = tc::make_idesc_bf16(128, NOUT);
+        tc::mbar_wait(&w_bar, 0);
+        int it = 0;
+        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+            const int as = it % WINB_STAGES, cs = it % ACC_STAGES;
+            const uint32_t aph = (it / WINB_STAGES) & 1, cph = (it / ACC_STAGES) & 1;
+            tc::mbar_wait(&acc_empty[cs], cph ^ 1);
+            tc::mbar_wait(&a_full[as], aph);
+            tc::tc_fence_after();
+            const uint32_t a0 = tc::smem_u32(sWinB) + as * WINB_STRIDE;
+            const uint32_t d = tmem + cs * ACC_COLS;
+#pragma unroll
+            for (int ky = 0; ky < NMMA; ++ky) {  // A row (oy, ox) of tap row ky: copy row 2 oy + ky, pixel 2 ox + 2
+                const uint64_t a_desc = make_desc_nosw(a0 + ky * PITCH + 16, 16, 2 * PITCH);
+                const uint64_t w_desc = make_desc_nosw(tc::smem_u32(sW) + ky * W_MMA_BYTES, (NOUT / 8) * 128, 128);
+                tc::umma_bf16_if(leader, d, a_desc, w_desc, idesc, ky ? 1u : 0u);
+            }
+            tc::umma_commit_if(leader, &a_empty[as]);
+            tc::umma_commit_if(leader, &acc_full[cs]);
+        }
+        __syncwarp();
+    } else if (warp < EPI_WARP0) {
+        // ================= converters: fp32 planar window -> (r, g, b, 1.0) bf16 pixels =================
+        const int ct = threadIdx.x - 64;
+        int it = 0;
+        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+            const int ws = it % WIN_STAGES, as = it % WINB_STAGES;
+            const uint32_t wph = (it / WIN_STAGES) & 1, aph = (it / WINB_STAGES) & 1;
+            tc::mbar_wait(&win_full[ws], wph);
+            tc::mbar_wait(&a_empty[as], aph ^ 1);
+            const uint32_t win = tc::smem_u32(sWin) + ws * WIN_STRIDE;
+            const uint32_t winb = tc::smem_u32(sWinB) + as * WINB_STRIDE;
+#pragma unroll
+            for (int k = 0; k < (WIN_H * WIN_W + CONV_THREADS - 1) / CONV_THREADS; ++k) {
+                const int pidx = ct + CONV_THREADS * k;
+                if (pidx < WIN_H * WIN_W) {
+                    float f0, f1, f2;
+                    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(f0) : "r"(win + pidx * 4));
+                    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(f1) : "r"(win + (WIN_H * WIN_W + pidx) * 4));
+                    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(f2) : "r"(win + (2 * WIN_H * WIN_W + pidx) * 4));
+                    asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(winb + pidx * 8), "r"(pack2(f0, f1)), "r"(pack2(f2, 1.0f))
+                                 : "memory");
+                }
+            }
+            tc::fence_proxy_async();
+            __syncwarp();
+            if (lane == 0) {
+                tc::mbar_arrive(&win_empty[ws]);
+                tc::mbar_arrive(&a_full[as]);
+            }
+        }
+    } else {
+        // ================= epilogue: HardSwish, one 16 x 8 x 16 TMA store per tile =================
+        const int q = warp & 3;
+        const int r = q * 32 + lane;
+        const bool leader = warp == EPI_WARP0 && lane == 0;
+        int it = 0;
+        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+            const int cs = it % ACC_STAGES;
+            const uint32_t cph = (it / ACC_STAGES) & 1;
+            const int img = tile / tiles_per_img, rr = tile - img * tiles_per_img;
+            const int oh0 = (rr / p.tiles_w) * TH, ow0 = (rr % p.tiles_w) * TW;
+            uint8_t* bst = sCst + (it & 1) * CST_BYTES;
+            tc::mbar_wait(&acc_full[cs], cph);
+            tc::tc_fence_after();
+            uint32_t a[16];
+            tc::tmem_ld16(tmem + cs * ACC_COLS + (static_cast<uint32_t>(q * 32) << 16), a);
+            tc::tmem_ld_wait();
+            tc::tc_fence_before();
+            __syncwarp();
+            if (lane == 0) tc::mbar_arrive(&acc_empty[cs]);
+            if (leader) tc::bulk_wait_read<1>();  // the store that read this staging buffer two tiles ago is done
+            tc::named_bar_sync(1, 128);
+#pragma unroll
+            for (int g = 0; g < 2; ++g) {
+                float v[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const float t = __uint_as_float(a[8 * g + j]);
+                    v[j] = t * __saturatef(fmaf(t, 1.f / 6.f, 0.5f));
+                }
+                Vec16<bf16> o;
+                o.pack(v);
+                tc::sts128(tc::smem_u32(bst) + r * 32 + g * 16, o.raw);
+            }
+            tc::fence_proxy_async();
+            tc::named_bar_sync(1, 128);
+            if (leader) {
+                tc::tma_store_4d(&tmY, bst, 0, ow0, oh0, img);
+                tc::bulk_commit();
+            }
+        }
+        if (leader) tc::bulk_wait_read<0>();
+    }
+    tc::tc_fence_before();
+    __syncthreads();
+    if (warp == 1) {
+        tc::tc_fence_after();
+        tc::tmem_dealloc(tmem, ACC_STAGES * ACC_COLS);
+    }
+}
+
+int g_attr_set3 = 0;
+
+int launch(const float* x, int N, int H, int W, const void* w_packed3, void* y, long long ld_y, int OH, int OW,
+           cabinet_stream_t stream) {
+    CAB_REQUIRE(x && w_packed3 && y, "stem3_tc: null pointer");
+    CAB_REQUIRE(N >= 0 && H > 0 && W > 0 && W % 4 == 0, "stem3_tc: W must be a multiple of 4 (TMA row pitch)");
+    CAB_REQUIRE(OH == (H - 1) / 2 + 1 && OW == (W - 1) / 2 + 1, "stem3_tc: inconsistent output size");
+    CAB_REQUIRE(ld_y >= 16 && ld_y % 8 == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0 &&
+                    (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(w_packed3) & 15) == 0,
+                "stem3_tc: alignment (ld_y a multiple of 8 >= 16, 16-byte aligned pointers)");
+    if (N == 0) return CABINET_OK;
+    cab_encode_tiled_fn enc = cab_get_encode_tiled();
+    CAB_REQUIRE(enc != nullptr, "stem3_tc: cuTensorMapEncodeTiled unavailable");
+    CUtensorMap tmX;
+    {
+        cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)3 * N};
+        cuuint64_t strides[2] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4};
+        cuuint32_t box[3] = {WIN_W, WIN_H, 3};
+        cuuint32_t estr[3] = {1, 1, 1};
+        CUresult r = enc(&tmX, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(x), dims, strides, box, estr,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) {
+            cabinet_set_error("stem3_tc: input tensor map encode failed (CUresult %d)", (int)r);
+            return CABINET_ERR_CUDA;
+        }
+    }
+    Stem2Params p;
+    p.N = N; p.OH = OH; p.OW = OW; p.w = w_packed3;
+    p.tiles_w = (OW + TW - 1) / TW;
+    p.tiles_h = (OH + TH - 1) / TH;
+    const long long nt = static_cast<long long>(N) * p.tiles_w * p.tiles_h;
+    CAB_REQUIRE(nt < (1LL << 31), "stem3_tc: too many tiles");
+    p.num_tiles = static_cast<int>(nt);
+    CUtensorMap tmY;
+    {
+        const uint64_t d[4] = {16, (uint64_t)OW, (uint64_t)OH, (uint64_t)N};
+        const uint64_t s[3] = {(uint64_t)ld_y * 2, (uint64_t)ld_y * 2 * OW, (uint64_t)ld_y * 2 * OW * OH};
+        const uint32_t b[4] = {16, TW, TH, 1};
+        int rc = cab_make_tmap_bf16(&tmY, y, 4, d, s, b, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_SWIZZLE_NONE);
+        if (rc) return rc;
+    }
+    if (!g_attr_set3) {
+        CAB_CUDA(cudaFuncSetAttribute(stem3_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        g_attr_set3 = 1;
+    }
+    int dev = 0, sms = 148;
+    CAB_CUDA(cudaGetDevice(&dev));
+    CAB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int grid = static_cast<int>(std::min<long long>(nt, sms));
+    stem3_tc_kernel<<<grid, NUM_THREADS, SMEM_BYTES, static_cast<cudaStream_t>(stream)>>>(tmX, tmY, p);
+    CAB_LAUNCH_CHECK();
+    return CABINET_OK;
+}
+
+}  // namespace s3
+}  // namespace
+
+extern "C" int cabinet_stem3_tc(const float* x, int N, int H, int W, const void* w_packed3, void* y, long long ld_y, int OH,
+                                int OW, cabinet_stream_t stream) {
+    return s3::launch(x, N, H, W, w_packed3, y, ld_y, OH, OW, stream);
+}

@@ -15,7 +15,7 @@ from __future__ import annotations
 
 import math
 from dataclasses import dataclass
-from typing import Optional
+from typing import Optional, Tuple
 
 import torch
 
@@ -174,6 +174,15 @@ def _out_size(n, k, s, p):
     return (n + 2 * p - k) // s + 1
 
 
+def backbone_hw(specs, H: int, W: int) -> Tuple[int, int]:
+    """(h, w) of the backbone's output for a stem output of H x W: the stride-2 depthwise convolutions of the blocks
+    (``MBConv.spec`` dicts; padding (k - 1) / 2)."""
+    for s in specs:
+        if s["s"] == 2:
+            H, W = _out_size(H, s["k"], 2, (s["k"] - 1) // 2), _out_size(W, s["k"], 2, (s["k"] - 1) // 2)
+    return H, W
+
+
 class Engine:
     # everything ``_pack`` produces (what ``checkpoint.save_packed`` caches)
     PACKED_ATTRS = ("stem", "blocks", "last", "stem_tc", "sb1", "sb2", "sb3", "sb4", "conva", "to_q", "to_k", "to_v",
@@ -181,6 +190,8 @@ class Engine:
                     "ffm_gate", "head_conv", "head_out", "ffm_sb", "low_fold", "stem_tc2")
     # what ``_pack_cab`` produces: all an engine built over a standalone ContextAggregationBlock packs
     CAB_ATTRS = ("to_q", "to_k", "to_v", "psp_k", "psp_v", "proj_out", "local", "gamma", "key_ch", "qkv")
+    # what ``_pack_mobilenet`` produces: all an engine built over a standalone MobileNetV3 packs
+    BACKBONE_ATTRS = ("stem", "blocks", "last", "stem_tc3")
 
     def __init__(self, model, precision: str = "bf16", packed: Optional[dict] = None):
         if precision not in ("bf16", "fp32"):
@@ -188,7 +199,7 @@ class Engine:
         p0 = next(model.parameters())
         if not p0.is_cuda:
             raise RuntimeError("cabinet_b200 engine needs the model on a CUDA device (no CPU path)")
-        from .modules import ContextAggregationBlock
+        from .modules import ContextAggregationBlock, MobileNetV3
 
         self.lib = _lib.load()
         self.dev = p0.device
@@ -197,7 +208,9 @@ class Engine:
         self.dt = BF16 if precision == "bf16" else F32
         # an engine over a standalone ContextAggregationBlock packs that block alone and runs ``forward_block``
         self.block = isinstance(model, ContextAggregationBlock)
-        self.n_classes = 0 if self.block else model.n_classes
+        # ... and one over a standalone MobileNetV3 packs the backbone alone and runs ``forward_backbone``
+        self.backbone = isinstance(model, MobileNetV3)
+        self.n_classes = 0 if self.block or self.backbone else model.n_classes
         self.stamp = None
         self.launches = 0  # kernels enqueued by the last forward
         self.use_tc = precision == "bf16"
@@ -207,6 +220,7 @@ class Engine:
         self.fuse_mbconv = True     # expand + depthwise (+ project) in one kernel (blocks whose tiles fit the shared memory)
         self.se_from_sums = True    # stride-1 SE blocks: gate from sums of the expanded activation, whole block in one kernel
         self.use_stem2 = True       # stems without the im2col tile (cabinet_stem_tc2)
+        self.use_stem3 = True       # standalone backbone: its stem on the tensor cores (cabinet_stem3_tc), not conv2d_simt
         self.t_small_s2 = False     # stride-2 blocks with <= 64 expanded channels (Large f2) through cabinet_mbconv_t too
         self.t_k5s2 = True          # k5 stride-2 SE blocks (Large f4, f13) through cabinet_mbconv_t as well
         self.use_mbconv_t = True    # ... in the channel-major formulation (cabinet_mbconv_t) where it supports the block
@@ -233,7 +247,7 @@ class Engine:
         self.branch_overlap = True  # independent chains of the attention branch on side streams (fork / join by events)
         self._branch_streams, self._branch_events = [], {}
         self.sb_overlap = False     # experiment: spatial branch beside the backbone
-        if packed is not None and self.block:
+        if packed is not None and (self.block or self.backbone):
             raise ValueError("packed weights exist for CABiNet engines only")
         if packed is not None:  # cached fold + pack of exactly these weights (checkpoint.load_packed verified the digest)
             missing = [a for a in self.PACKED_ATTRS if a not in packed]
@@ -244,8 +258,14 @@ class Engine:
             self.gamma = model.ab.a2block.gamma.detach().float().contiguous()
         else:
             with torch.no_grad():
-                self._pack_cab(model) if self.block else self._pack(model)  # on the host ...
-                for a in self.CAB_ATTRS if self.block else self.PACKED_ATTRS:  # ... then one upload per packed tensor
+                if self.block:  # on the host ...
+                    self._pack_cab(model)
+                elif self.backbone:
+                    self._pack_mobilenet(model)
+                else:
+                    self._pack(model)
+                attrs = self.CAB_ATTRS if self.block else self.BACKBONE_ATTRS if self.backbone else self.PACKED_ATTRS
+                for a in attrs:  # ... then one upload per packed tensor
                     setattr(self, a, _map_tensors(getattr(self, a), lambda t: t.to(self.dev)))
 
     def packed_state(self) -> dict:
@@ -258,57 +278,7 @@ class Engine:
         wd = self.tdt
         f32 = torch.float32
         mob = m.mobile
-        # stems read the fp32 NCHW input directly; their (tiny) weights stay fp32
-        self.stem = ConvLayer(mob.features[0][0], mob.features[0][1], ACT_HSWISH, f32, "mobile.stem")
-        self.blocks = []
-        for bi, blk in enumerate(list(mob.features)[1:], 1):
-            s, c = blk.spec, blk.conv
-            act = ACT_HSWISH if s["hs"] else ACT_RELU
-            e = dict(spec=s, act=act)
-            if s["expand"]:
-                e["pw1"] = ConvLayer(c[0], c[1], act, wd, f"mobile.f{bi}.expand")
-                e["dw"] = DwLayer(c[3], c[4], ACT_NONE if s["se"] else act, f"mobile.f{bi}.dw")
-                se, pw2, bn2 = c[5], c[7], c[8]
-                if self.precision == "bf16":
-                    # fused-block side table: fp32 [chunks][k*k + 2][64] = depthwise taps, expand bias, depthwise bias
-                    dwl, kk, nc = e["dw"], e["dw"].k ** 2, -(-e["dw"].c // 64)
-                    aux = torch.zeros((nc * 64, kk + 2), dtype=f32, device=dwl.w.device)
-                    aux[: dwl.c, :kk] = dwl.w.t()
-                    aux[: dwl.c, kk + 1] = dwl.b
-                    e["aux"] = aux.view(nc, 64, kk + 2).permute(0, 2, 1).contiguous()
-                    p1 = e["pw1"]
-                    if p1.cin % 8 == 0 and p1.cin % 64 <= 56 and p1.cin <= 248:
-                        # expand weights with the bias as two extra K columns (bf16 hi + lo; the kernel feeds 1.0 there);
-                        # K = Cin + 2 padded to whole 64-channel K blocks
-                        wb = torch.zeros((-(-p1.cout // 16) * 16, (p1.cin // 64 + 1) * 64), dtype=f32, device=dwl.w.device)
-                        wb[: p1.cout, : p1.cin] = p1.tc[: p1.cout, 0, : p1.cin].float()
-                        hi = p1.b.to(torch.bfloat16).float()
-                        wb[: p1.cout, p1.cin], wb[: p1.cout, p1.cin + 1] = hi, p1.b - hi
-                        e["w1b"] = wb.to(torch.bfloat16).contiguous()
-                        # channel-major kernel (cabinet_mbconv_t): chunks of 128 TMEM lanes; widths <= 64 are replicated
-                        # twice along the lanes.  Same columns as w1b; taps + depthwise bias in the same row order.
-                        ch = 64 if dwl.c <= 64 else 128
-                        nct = 1 if dwl.c <= 64 else -(-dwl.c // 128)
-                        flat = torch.zeros((nct * ch, wb.shape[1]), dtype=f32, device=dwl.w.device)
-                        flat[: dwl.c] = wb[: dwl.c]
-                        e["w1t"] = (flat.view(nct, ch, -1).repeat(1, 128 // ch, 1).reshape(nct * 128, -1)
-                                    .to(torch.bfloat16).contiguous())
-                        fa = torch.zeros((nct * ch, kk + 1), dtype=f32, device=dwl.w.device)
-                        fa[: dwl.c, :kk] = dwl.w.t()
-                        fa[: dwl.c, kk] = dwl.b
-                        e["auxt"] = fa.view(nct, ch, kk + 1).repeat(1, 128 // ch, 1).permute(0, 2, 1).contiguous()
-            else:
-                e["dw"] = DwLayer(c[0], c[1], act, f"mobile.f{bi}.dw")
-                se, pw2, bn2 = c[3], c[4], c[5]
-            if s["se"]:
-                e["se"] = GateLayer(se.fc[0].weight, se.fc[0].bias, se.fc[2].weight, se.fc[2].bias, ACT_HSIGMOID)
-            e["pw2"] = ConvLayer(pw2, bn2, ACT_NONE, wd, f"mobile.f{bi}.project")
-            if (not s["expand"] and not s["se"] and s["identity"] and s["k"] == 3 and s["exp"] in (8, 16, 32)
-                    and self.precision == "bf16"):
-                w2, b2 = _fold(pw2.weight, pw2.bias, bn2)  # fused whole-block kernel keeps the pointwise in fp32
-                e["fused_pw"] = (w2.reshape(w2.shape[0], -1).contiguous(), b2.contiguous())
-            self.blocks.append(e)
-        self.last = ConvLayer(mob.conv[0], mob.conv[1], ACT_HSWISH, wd, "mobile.conv")
+        self._pack_backbone(mob)
 
         sb = m.sb
         self.stem_tc = self.stem_tc2 = None
@@ -363,6 +333,76 @@ class Engine:
                                               (w_low @ bb.double()).float(), 1, 0))
         self.head_conv = ConvLayer(m.conv_out.conv.conv, m.conv_out.conv.bn, ACT_RELU, wd, "conv_out.conv")
         self.head_out = ConvLayer(m.conv_out.conv_out, None, ACT_NONE, wd, "conv_out.conv_out")
+
+    def _pack_backbone(self, mob):
+        """The MobileNetV3's stem, blocks and last conv (reference: mobilenetv3.py:86-159,173-205), BN folded."""
+        wd = self.tdt
+        f32 = torch.float32
+        # stems read the fp32 NCHW input directly; their (tiny) weights stay fp32
+        self.stem = ConvLayer(mob.features[0][0], mob.features[0][1], ACT_HSWISH, f32, "mobile.stem")
+        self.blocks = []
+        for bi, blk in enumerate(list(mob.features)[1:], 1):
+            s, c = blk.spec, blk.conv
+            act = ACT_HSWISH if s["hs"] else ACT_RELU
+            e = dict(spec=s, act=act)
+            if s["expand"]:
+                e["pw1"] = ConvLayer(c[0], c[1], act, wd, f"mobile.f{bi}.expand")
+                e["dw"] = DwLayer(c[3], c[4], ACT_NONE if s["se"] else act, f"mobile.f{bi}.dw")
+                se, pw2, bn2 = c[5], c[7], c[8]
+                if self.precision == "bf16":
+                    # fused-block side table: fp32 [chunks][k*k + 2][64] = depthwise taps, expand bias, depthwise bias
+                    dwl, kk, nc = e["dw"], e["dw"].k ** 2, -(-e["dw"].c // 64)
+                    aux = torch.zeros((nc * 64, kk + 2), dtype=f32, device=dwl.w.device)
+                    aux[: dwl.c, :kk] = dwl.w.t()
+                    aux[: dwl.c, kk + 1] = dwl.b
+                    e["aux"] = aux.view(nc, 64, kk + 2).permute(0, 2, 1).contiguous()
+                    p1 = e["pw1"]
+                    if p1.cin % 8 == 0 and p1.cin % 64 <= 56 and p1.cin <= 248:
+                        # expand weights with the bias as two extra K columns (bf16 hi + lo; the kernel feeds 1.0 there);
+                        # K = Cin + 2 padded to whole 64-channel K blocks
+                        wb = torch.zeros((-(-p1.cout // 16) * 16, (p1.cin // 64 + 1) * 64), dtype=f32, device=dwl.w.device)
+                        wb[: p1.cout, : p1.cin] = p1.tc[: p1.cout, 0, : p1.cin].float()
+                        hi = p1.b.to(torch.bfloat16).float()
+                        wb[: p1.cout, p1.cin], wb[: p1.cout, p1.cin + 1] = hi, p1.b - hi
+                        e["w1b"] = wb.to(torch.bfloat16).contiguous()
+                        # channel-major kernel (cabinet_mbconv_t): chunks of 128 TMEM lanes; widths <= 64 are replicated
+                        # twice along the lanes.  Same columns as w1b; taps + depthwise bias in the same row order.
+                        ch = 64 if dwl.c <= 64 else 128
+                        nct = 1 if dwl.c <= 64 else -(-dwl.c // 128)
+                        flat = torch.zeros((nct * ch, wb.shape[1]), dtype=f32, device=dwl.w.device)
+                        flat[: dwl.c] = wb[: dwl.c]
+                        e["w1t"] = (flat.view(nct, ch, -1).repeat(1, 128 // ch, 1).reshape(nct * 128, -1)
+                                    .to(torch.bfloat16).contiguous())
+                        fa = torch.zeros((nct * ch, kk + 1), dtype=f32, device=dwl.w.device)
+                        fa[: dwl.c, :kk] = dwl.w.t()
+                        fa[: dwl.c, kk] = dwl.b
+                        e["auxt"] = fa.view(nct, ch, kk + 1).repeat(1, 128 // ch, 1).permute(0, 2, 1).contiguous()
+            else:
+                e["dw"] = DwLayer(c[0], c[1], act, f"mobile.f{bi}.dw")
+                se, pw2, bn2 = c[3], c[4], c[5]
+            if s["se"]:
+                e["se"] = GateLayer(se.fc[0].weight, se.fc[0].bias, se.fc[2].weight, se.fc[2].bias, ACT_HSIGMOID)
+            e["pw2"] = ConvLayer(pw2, bn2, ACT_NONE, wd, f"mobile.f{bi}.project")
+            if (not s["expand"] and not s["se"] and s["identity"] and s["k"] == 3 and s["exp"] in (8, 16, 32)
+                    and self.precision == "bf16"):
+                w2, b2 = _fold(pw2.weight, pw2.bias, bn2)  # fused whole-block kernel keeps the pointwise in fp32
+                e["fused_pw"] = (w2.reshape(w2.shape[0], -1).contiguous(), b2.contiguous())
+            self.blocks.append(e)
+        self.last = ConvLayer(mob.conv[0], mob.conv[1], ACT_HSWISH, wd, "mobile.conv")
+
+    def _pack_mobilenet(self, mob):
+        """A standalone MobileNetV3: the backbone's layers + the weights of the backbone-only tensor-core stem."""
+        self._pack_backbone(mob)
+        self.stem_tc3 = None
+        if self.precision == "bf16":
+            # cabinet_stem3_tc: W[o][ky][s][c], slot s = kx + 1 (slot 0: no tap; its constant-1 channel c = 3 carries
+            # the bias, hi part at ky 1, lo part at ky 0) as UMMA core matrices [ky][k chunk][o][8]
+            w3, b3 = _fold(mob.features[0][0].weight, None, mob.features[0][1])
+            wn = torch.zeros((16, 3, 4, 4), dtype=torch.float32, device=w3.device)
+            wn[:, :, 1:, :3] = w3.permute(0, 2, 3, 1)
+            b_hi = b3.to(torch.bfloat16).float()
+            wn[:, 1, 0, 3], wn[:, 0, 0, 3] = b_hi, b3 - b_hi
+            self.stem_tc3 = wn.view(16, 3, 2, 8).permute(1, 2, 0, 3).contiguous().to(torch.bfloat16)
 
     def _pack_cab(self, cab):
         """The ContextAggregationBlock's layers (reference: cab.py:84-129,170-184,192-216), BN folded."""
@@ -753,72 +793,11 @@ class Engine:
             self.relayout(out.t, (H * W * C, W * C, C, 1), y, nchw(y), N, H, W, C, "cab.out")
         return y
 
-    def bilinear(self, x: Map, out: Map, name: str):
-        nbytes = x.N * x.C * (x.H * x.W * x.t.element_size() + out.H * out.W * out.t.element_size())
-        self._run("bilinear_nhwc", name, nbytes, 0, self.lib.cabinet_bilinear_nhwc, x.ptr, x.ld, x.dt, out.ptr, out.ld,
-                  out.dt, x.N, x.H, x.W, x.C, out.H, out.W, self.stream)
-
-    # ------------------------------------------------------------------ the forward schedule
-    def _trunk(self, x: torch.Tensor, need_aux: bool = True):
-        """Everything up to the two fp32 class-logit maps: (final8 [N,H/8,W/8,C], aux8 [N,H/8,W/8,C]).
-
-        ``need_aux=False`` (mask / confusion-matrix / probability callers, which only read ``model(x)[0]``,
-        evaluate.py:76-78): the auxiliary head ``b1 -> b4 -> x4 upsample`` (cabinet.py:88-93,234-239) is not launched
-        and ``aux8`` is None -- it feeds nothing but the second output."""
-        if x.dtype != torch.float32 or not x.is_contiguous():
-            x = x.float().contiguous()
-        if x.device != self.dev:
-            raise RuntimeError(f"input on {x.device}, model on {self.dev}")
-        N, _, H, W = x.shape
-        self.launches = 0
-        dev, C = self.dev, self.n_classes
-        n_se = sum(1 for b in self.blocks if "se" in b)
-        # ONE memset per forward: the SE / FFM pooling sums, and the scratch areas (tickets + parked partial sums) of the
-        # deterministic reductions (cabinet_channel_sum, 2 x cabinet_psp_pool)
-        kc = self.key_ch
-        # (every SE block owns N x 1024 8-byte slots: int64 fixed-point accumulators on the bf16 path, fp32 sums in the
-        # parity mode; the FFM pooling row sits behind them)
-        n_gap, n_psp, n_ffm = (2 * n_se + 1) * N * 1024, 128 + N * (110 + 256 * kc), 128 + N * 64 * 256
-        zeros_all = torch.zeros(n_gap + 2 * n_psp + n_ffm, dtype=torch.float32, device=dev)
-        gap_all = zeros_all[:n_gap].view(2 * n_se + 1, N * 1024)
-        self._scratch = [zeros_all[n_gap + i * n_psp: n_gap + (i + 1) * n_psp] for i in range(2)]
-        ffm_scratch = zeros_all[n_gap + 2 * n_psp:]
-        self.launches += 1
-
-        # ---- spatial branch (reference: cabinet.py:108-129) -> channels [0:128] of the FFM concat buffer
-        fused_stems = self.use_tc and self.stem_tc is not None and W % 4 == 0
-        if fused_stems:
-            OH2, OW2 = (H - 1) // 2 + 1, (W - 1) // 2 + 1
-            s1, f0 = self.new(N, OH2, OW2, 64), self.new(N, OH2, OW2, 16)
-            nbytes = x.numel() * 4 + (s1.t.numel() + f0.t.numel()) * 2 + 80 * 192 * 2
-            if self.use_stem2 and self.stem_tc2 is not None:
-                self._run("stem_tc", "sb.conv1+mobile.stem", nbytes, 2 * N * OH2 * OW2 * (64 * 147 + 16 * 27),
-                          self.lib.cabinet_stem_tc2, x.data_ptr(), N, H, W, self.stem_tc2.data_ptr(), s1.ptr, s1.ld,
-                          f0.ptr, f0.ld, OH2, OW2, self.stream)
-            else:
-                self._run("stem_tc", "sb.conv1+mobile.stem", nbytes, 2 * N * OH2 * OW2 * (64 * 147 + 16 * 27),
-                          self.lib.cabinet_stem_tc, x.data_ptr(), N, H, W, self.stem_tc[0].data_ptr(),
-                          self.stem_tc[1].data_ptr(), s1.ptr, s1.ld, f0.ptr, f0.ld, OH2, OW2, self.stream)
-        else:
-            s1 = self.conv(None, self.sb1, nchw_input=x)
-        H8, W8 = _out_size(_out_size(s1.H, 3, 2, 1), 3, 2, 1), _out_size(_out_size(s1.W, 3, 2, 1), 3, 2, 1)
-        fold_low = (self.fold_low_up and self.use_tc and not self.debug and self.ffm_sb is not None
-                    and self.ffm_sb.tc is not None and self.low_fold.tc is not None and self.sb4.cout == self.ffm_sb.cin)
-        cat_ffm = self.new(N, H8, W8, self.sb4.cout if fold_low else 128 + 256)
-        if self.sb_overlap:  # experiment: the rest of the spatial branch beside the backbone (joined before the FFM)
-            with self._branch(2) as joined:
-                s2 = self.conv(s1, self.sb2)
-                s3 = self.conv(s2, self.sb3)
-                self.conv(s3, self.sb4, out=cat_ffm.slice(0, 128))
-                joined(s1.t)
-        else:
-            s2 = self.conv(s1, self.sb2)
-            s3 = self.conv(s2, self.sb3)
-            self.conv(s3, self.sb4, out=cat_ffm.slice(0, 128))
-        assert (s3.H, s3.W) == (H8, W8)
-
-        # ---- backbone (reference: mobilenetv3.py:202-205)
-        f = f0 if fused_stems else self.conv(None, self.stem, nchw_input=x)
+    def mobilenet(self, f: Map, gap_all: torch.Tensor, out: Optional[Map] = None) -> Map:
+        """The backbone after its stem: the inverted-residual blocks and ``mobile.conv`` (reference: mobilenetv3.py:
+        102-159,202-205).  ``f``: the stem's output; ``gap_all``: zeroed [>= 2 x SE blocks][N * 1024] fp32 (the SE pooling
+        sums); ``out``: where ``mobile.conv`` writes (a channel slice of CABiNet's b1 concat buffer) or None."""
+        N, dev = f.N, self.dev
         gi = 0
         for e in self.blocks:
             s = e["spec"]
@@ -904,9 +883,106 @@ class Engine:
             else:
                 d, _ = self.dwconv(h, e["dw"])
             f = self.conv(d, e["pw2"], res=f if s["identity"] else None)
-        h32, w32 = f.H, f.W
+        return self.conv(f, self.last, out=out)
+
+    @torch.no_grad()
+    def forward_backbone(self, x: torch.Tensor) -> torch.Tensor:
+        """Standalone MobileNetV3: (N, 3, H, W) fp32 / bf16 / fp16 -> (N, out_channels, h32, w32) NCHW in x's dtype."""
+        N, _, H, W = x.shape
+        OH, OW = _out_size(H, 3, 2, 1), _out_size(W, 3, 2, 1)
+        h32, w32 = backbone_hw([e["spec"] for e in self.blocks], OH, OW)
+        C = self.last.cout
+        y = torch.empty((N, C, h32, w32), dtype=x.dtype, device=x.device)
+        self.launches = 0
+        if N == 0:
+            return y
+        with self._guard():
+            xf = x if x.dtype == torch.float32 and x.is_contiguous() else x.float().contiguous()
+            n_se = sum(1 for b in self.blocks if "se" in b)
+            gap_all = torch.zeros((max(2 * n_se, 1), N * 1024), dtype=torch.float32, device=self.dev)
+            self.launches += 1
+            if (self.use_tc and self.use_stem3 and self.stem_tc3 is not None and W % 4 == 0
+                    and xf.data_ptr() % 16 == 0):
+                f = self.new(N, OH, OW, 16)
+                self._run("stem3_tc", "mobile.stem", xf.numel() * 4 + f.t.numel() * 2 + self.stem_tc3.numel() * 2,
+                          2 * N * OH * OW * 16 * 27, self.lib.cabinet_stem3_tc, xf.data_ptr(), N, H, W,
+                          self.stem_tc3.data_ptr(), f.ptr, f.ld, OH, OW, self.stream)
+            else:
+                f = self.conv(None, self.stem, nchw_input=xf)
+            mf = self.mobilenet(f, gap_all)
+            self.relayout(mf.t, (h32 * w32 * C, w32 * C, C, 1), y, (y.stride(0), y.stride(2), y.stride(3), y.stride(1)),
+                          N, h32, w32, C, "mobile.out")
+        return y
+
+    def bilinear(self, x: Map, out: Map, name: str):
+        nbytes = x.N * x.C * (x.H * x.W * x.t.element_size() + out.H * out.W * out.t.element_size())
+        self._run("bilinear_nhwc", name, nbytes, 0, self.lib.cabinet_bilinear_nhwc, x.ptr, x.ld, x.dt, out.ptr, out.ld,
+                  out.dt, x.N, x.H, x.W, x.C, out.H, out.W, self.stream)
+
+    # ------------------------------------------------------------------ the forward schedule
+    def _trunk(self, x: torch.Tensor, need_aux: bool = True):
+        """Everything up to the two fp32 class-logit maps: (final8 [N,H/8,W/8,C], aux8 [N,H/8,W/8,C]).
+
+        ``need_aux=False`` (mask / confusion-matrix / probability callers, which only read ``model(x)[0]``,
+        evaluate.py:76-78): the auxiliary head ``b1 -> b4 -> x4 upsample`` (cabinet.py:88-93,234-239) is not launched
+        and ``aux8`` is None -- it feeds nothing but the second output."""
+        if x.dtype != torch.float32 or not x.is_contiguous():
+            x = x.float().contiguous()
+        if x.device != self.dev:
+            raise RuntimeError(f"input on {x.device}, model on {self.dev}")
+        N, _, H, W = x.shape
+        self.launches = 0
+        dev, C = self.dev, self.n_classes
+        n_se = sum(1 for b in self.blocks if "se" in b)
+        # ONE memset per forward: the SE / FFM pooling sums, and the scratch areas (tickets + parked partial sums) of the
+        # deterministic reductions (cabinet_channel_sum, 2 x cabinet_psp_pool)
+        kc = self.key_ch
+        # (every SE block owns N x 1024 8-byte slots: int64 fixed-point accumulators on the bf16 path, fp32 sums in the
+        # parity mode; the FFM pooling row sits behind them)
+        n_gap, n_psp, n_ffm = (2 * n_se + 1) * N * 1024, 128 + N * (110 + 256 * kc), 128 + N * 64 * 256
+        zeros_all = torch.zeros(n_gap + 2 * n_psp + n_ffm, dtype=torch.float32, device=dev)
+        gap_all = zeros_all[:n_gap].view(2 * n_se + 1, N * 1024)
+        self._scratch = [zeros_all[n_gap + i * n_psp: n_gap + (i + 1) * n_psp] for i in range(2)]
+        ffm_scratch = zeros_all[n_gap + 2 * n_psp:]
+        self.launches += 1
+
+        # ---- spatial branch (reference: cabinet.py:108-129) -> channels [0:128] of the FFM concat buffer
+        fused_stems = self.use_tc and self.stem_tc is not None and W % 4 == 0
+        if fused_stems:
+            OH2, OW2 = (H - 1) // 2 + 1, (W - 1) // 2 + 1
+            s1, f0 = self.new(N, OH2, OW2, 64), self.new(N, OH2, OW2, 16)
+            nbytes = x.numel() * 4 + (s1.t.numel() + f0.t.numel()) * 2 + 80 * 192 * 2
+            if self.use_stem2 and self.stem_tc2 is not None:
+                self._run("stem_tc", "sb.conv1+mobile.stem", nbytes, 2 * N * OH2 * OW2 * (64 * 147 + 16 * 27),
+                          self.lib.cabinet_stem_tc2, x.data_ptr(), N, H, W, self.stem_tc2.data_ptr(), s1.ptr, s1.ld,
+                          f0.ptr, f0.ld, OH2, OW2, self.stream)
+            else:
+                self._run("stem_tc", "sb.conv1+mobile.stem", nbytes, 2 * N * OH2 * OW2 * (64 * 147 + 16 * 27),
+                          self.lib.cabinet_stem_tc, x.data_ptr(), N, H, W, self.stem_tc[0].data_ptr(),
+                          self.stem_tc[1].data_ptr(), s1.ptr, s1.ld, f0.ptr, f0.ld, OH2, OW2, self.stream)
+        else:
+            s1 = self.conv(None, self.sb1, nchw_input=x)
+        H8, W8 = _out_size(_out_size(s1.H, 3, 2, 1), 3, 2, 1), _out_size(_out_size(s1.W, 3, 2, 1), 3, 2, 1)
+        fold_low = (self.fold_low_up and self.use_tc and not self.debug and self.ffm_sb is not None
+                    and self.ffm_sb.tc is not None and self.low_fold.tc is not None and self.sb4.cout == self.ffm_sb.cin)
+        cat_ffm = self.new(N, H8, W8, self.sb4.cout if fold_low else 128 + 256)
+        if self.sb_overlap:  # experiment: the rest of the spatial branch beside the backbone (joined before the FFM)
+            with self._branch(2) as joined:
+                s2 = self.conv(s1, self.sb2)
+                s3 = self.conv(s2, self.sb3)
+                self.conv(s3, self.sb4, out=cat_ffm.slice(0, 128))
+                joined(s1.t)
+        else:
+            s2 = self.conv(s1, self.sb2)
+            s3 = self.conv(s2, self.sb3)
+            self.conv(s3, self.sb4, out=cat_ffm.slice(0, 128))
+        assert (s3.H, s3.W) == (H8, W8)
+
+        # ---- backbone (reference: mobilenetv3.py:202-205) -> channels [0:960 | 576] of the b1 concat buffer
+        f = f0 if fused_stems else self.conv(None, self.stem, nchw_input=x)
+        h32, w32 = backbone_hw([e["spec"] for e in self.blocks], f.H, f.W)
         cat_b1 = self.new(N, h32, w32, self.last.cout + 256)  # [mobile_feat | CAB feat] (reference: cabinet.py:87)
-        mf = self.conv(f, self.last, out=cat_b1.slice(0, self.last.cout))
+        mf = self.mobilenet(f, gap_all, out=cat_b1.slice(0, self.last.cout))
 
         # ---- attention branch (reference: cabinet.py:75-94, cab.py:131-162,175-184,213-216)
         feat = self.conv(mf, self.conva)

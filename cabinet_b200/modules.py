@@ -68,58 +68,6 @@ class MBConv(nn.Module):
         self.conv = nn.Sequential(*seq)
 
 
-class MobileNetV3(nn.Module):
-    """Backbone parameter tree (reference: mobilenetv3.py:162-235)."""
-
-    def __init__(self, cfgs, mode, num_classes=1000, width_mult=1.0, weights=None):
-        super().__init__()
-        self.cfgs = cfgs
-        self.weights = weights
-        if mode not in ("large", "small"):
-            raise ValueError(f"mode must be 'large' or 'small', got '{mode}'")
-        stem, blocks, last_exp = resolve_blocks(cfgs, width_mult)
-        feats = [nn.Sequential(_conv(3, stem, 3, 2, 1), nn.BatchNorm2d(stem), _slot())]
-        for b in blocks:
-            feats.append(MBConv(b["inp"], b["exp"], b["out"], b["k"], b["s"], b["se"], b["hs"]))
-        self.features = nn.Sequential(*feats)
-        last_in = blocks[-1]["out"] if blocks else stem
-        self.conv = nn.Sequential(_conv(last_in, last_exp), nn.BatchNorm2d(last_exp), _slot())
-        self.avgpool = _slot()  # parameter-free in the reference as well; unused by forward (F9)
-        head = MODEL_CONFIG[mode]["output_channel"]
-        if width_mult > 1.0:
-            head = make_divisible(head * width_mult, 8)
-        # classifier.{0,3}: in the state_dict, never used by the forward path (F9)
-        self.classifier = nn.Sequential(nn.Linear(last_exp, head), _slot(), _slot(), nn.Linear(head, num_classes))
-        self.out_channels = last_exp
-        self._initialize_weights()
-
-    def _initialize_weights(self):
-        """Pretrained load (minus classifier) or the MobileNetV3 init (reference: mobilenetv3.py:207-235)."""
-        if self.weights is not None and Path(self.weights).is_file():
-            try:
-                blob = torch.load(self.weights, map_location="cpu", weights_only=True)
-                merged = self.state_dict()
-                merged.update({k: v for k, v in blob.items() if "classifier" not in k})
-                self.load_state_dict(merged)
-                print(f"Loaded pretrained weights from {self.weights}")
-                return
-            except Exception as e:  # non-fatal in the reference too (mobilenetv3.py:221-223)
-                print(f"Failed to load backbone weights from {self.weights}: {e}")
-                print("Proceeding with random weight initialization.")
-        for m in self.modules():
-            if isinstance(m, nn.Conv2d):
-                fan = m.kernel_size[0] * m.kernel_size[1] * m.out_channels
-                m.weight.data.normal_(0, math.sqrt(2.0 / fan))
-                if m.bias is not None:
-                    m.bias.data.zero_()
-            elif isinstance(m, nn.BatchNorm2d):
-                m.weight.data.fill_(1)
-                m.bias.data.zero_()
-            elif isinstance(m, nn.Linear):
-                m.weight.data.normal_(0, 0.01)
-                m.bias.data.zero_()
-
-
 class _EngineCache:
     """Lazily built engines kept in ``__dict__`` (not module state): dropped by ``.to()`` / ``.cuda()`` / ``.half()``,
     left out of ``deepcopy`` and pickling; a weight change is seen through the parameters' addresses and versions."""
@@ -174,6 +122,92 @@ class _EngineCache:
         d = dict(self.__dict__)
         d["_engine"] = d["_train_engine"] = None
         return d
+
+
+class MobileNetV3(_EngineCache, nn.Module):
+    """Backbone (reference: mobilenetv3.py:162-235), runnable on its own.
+
+    ``forward`` maps an (N, 3, H, W) CUDA tensor (fp32 / bf16 / fp16) to the (N, out_channels, H/32, W/32) feature map
+    in x's dtype: the stem, the inverted-residual blocks and ``conv`` (reference: mobilenetv3.py:202-205); the classifier
+    is not on this path.  Mode semantics are ``CABiNet.forward``'s: ``.eval()`` runs the inference schedule (BN folded)
+    unless ``x`` requires grad with grad mode on, which runs the differentiable schedule with running-statistics
+    BatchNorm; ``.train()`` uses batch statistics (running statistics updated) and fills ``p.grad`` / ``x.grad`` on
+    backward.  ``precision`` ("bf16" | "fp32") selects the inference schedule, ``train_precision`` ("fp32" | "bf16" |
+    "fp16") the differentiable one.  Only ``width_mult == 1.0`` runs.
+    """
+
+    def __init__(self, cfgs, mode, num_classes=1000, width_mult=1.0, weights=None):
+        super().__init__()
+        self.cfgs = cfgs
+        self.weights = weights
+        self.width_mult = width_mult
+        self.precision = "bf16"
+        self.train_precision = "fp32"
+        self.__dict__["_engine"] = None
+        self.__dict__["_train_engine"] = None
+        if mode not in ("large", "small"):
+            raise ValueError(f"mode must be 'large' or 'small', got '{mode}'")
+        stem, blocks, last_exp = resolve_blocks(cfgs, width_mult)
+        feats = [nn.Sequential(_conv(3, stem, 3, 2, 1), nn.BatchNorm2d(stem), _slot())]
+        for b in blocks:
+            feats.append(MBConv(b["inp"], b["exp"], b["out"], b["k"], b["s"], b["se"], b["hs"]))
+        self.features = nn.Sequential(*feats)
+        last_in = blocks[-1]["out"] if blocks else stem
+        self.conv = nn.Sequential(_conv(last_in, last_exp), nn.BatchNorm2d(last_exp), _slot())
+        self.avgpool = _slot()  # parameter-free in the reference as well; unused by forward (F9)
+        head = MODEL_CONFIG[mode]["output_channel"]
+        if width_mult > 1.0:
+            head = make_divisible(head * width_mult, 8)
+        # classifier.{0,3}: in the state_dict, never used by the forward path (F9)
+        self.classifier = nn.Sequential(nn.Linear(last_exp, head), _slot(), _slot(), nn.Linear(head, num_classes))
+        self.out_channels = last_exp
+        self._initialize_weights()
+
+    def _initialize_weights(self):
+        """Pretrained load (minus classifier) or the MobileNetV3 init (reference: mobilenetv3.py:207-235)."""
+        if self.weights is not None and Path(self.weights).is_file():
+            try:
+                blob = torch.load(self.weights, map_location="cpu", weights_only=True)
+                merged = self.state_dict()
+                merged.update({k: v for k, v in blob.items() if "classifier" not in k})
+                self.load_state_dict(merged)
+                print(f"Loaded pretrained weights from {self.weights}")
+                return
+            except Exception as e:  # non-fatal in the reference too (mobilenetv3.py:221-223)
+                print(f"Failed to load backbone weights from {self.weights}: {e}")
+                print("Proceeding with random weight initialization.")
+        for m in self.modules():
+            if isinstance(m, nn.Conv2d):
+                fan = m.kernel_size[0] * m.kernel_size[1] * m.out_channels
+                m.weight.data.normal_(0, math.sqrt(2.0 / fan))
+                if m.bias is not None:
+                    m.bias.data.zero_()
+            elif isinstance(m, nn.BatchNorm2d):
+                m.weight.data.fill_(1)
+                m.bias.data.zero_()
+            elif isinstance(m, nn.Linear):
+                m.weight.data.normal_(0, 0.01)
+                m.bias.data.zero_()
+
+    def _check_input(self, x):
+        if self.width_mult != 1.0:
+            raise ValueError(f"MobileNetV3 runs at width_mult 1.0 only, got {self.width_mult}")
+        if not isinstance(x, torch.Tensor) or x.dim() != 4 or x.shape[1] != 3:
+            raise ValueError(f"expected an (N, 3, H, W) tensor, got {getattr(x, 'shape', type(x))}")
+        if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
+            raise TypeError(f"MobileNetV3 takes float32, bfloat16 or float16 input, got {x.dtype}")
+        if not x.is_cuda:
+            raise RuntimeError("cabinet_b200.MobileNetV3 has no CPU path: move the backbone and the input to a CUDA device")
+
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        """(N, 3, H, W) -> (N, out_channels, h32, w32) NCHW in x's dtype (reference: mobilenetv3.py:202-205)."""
+        self._check_input(x)
+        if self.training or (torch.is_grad_enabled() and x.requires_grad):
+            from .train_engine import BackboneStep
+
+            params = [p for n, p in self.named_parameters() if not n.startswith("classifier")]
+            return BackboneStep.apply(self.train_engine(), x, *params)
+        return self.engine().forward_backbone(x)
 
 
 # --------------------------------------------------------------------------- CAB

@@ -39,7 +39,7 @@ import torch
 from . import _lib
 from ._lib import ACT_HSIGMOID, ACT_HSWISH, ACT_NONE, ACT_RELU, ACT_SIGMOID, BF16, F16, F32, check
 from .constants import BN_EPS
-from .engine import Map, _out_size, dtype_code
+from .engine import Map, _out_size, backbone_hw, dtype_code
 
 BN_MOMENTUM = 0.1  # nn.BatchNorm2d default (the reference never overrides it)
 PSP_SIZES = (1, 3, 6, 8)  # reference: src/models/cab.py:49
@@ -142,7 +142,8 @@ class TrainEngine:
         # the activation dtype, in one place: every 2-byte buffer and operand of the schedule follows it
         self.tdt = {"bf16": torch.bfloat16, "fp16": torch.float16, "fp32": torch.float32}[precision]
         self.dt = dtype_code(self.tdt)
-        self.n_classes = getattr(model, "n_classes", 0)   # 0: a standalone ContextAggregationBlock (``block_forward``)
+        # 0: a standalone ContextAggregationBlock (``block_forward``) or MobileNetV3 (``backbone_forward``)
+        self.n_classes = getattr(model, "n_classes", 0)
         self.tables = _Tables(self.dev)
         self.tape: List = []
         self.pgrads: Dict[int, torch.Tensor] = {}
@@ -389,31 +390,39 @@ class TrainEngine:
         p0, p1 = cls._parity_geom(k, pad, 0)[1], cls._parity_geom(k, pad, 1)[1]
         return p0 if p0 == p1 else None
 
-    STEM_K, STEM_LD = 7, 152   # im2col footprint of the stems: 3 x 7 x 7 = 147 columns, pixel stride padded to 8
+    # im2col footprint of CABiNet's stems: 3 x 7 x 7 = 147 columns (a standalone MobileNetV3 uses its stem's 3 x 3 x 3)
+    STEM_K = 7
 
-    def stem_im2col(self, x: torch.Tensor) -> Map:
-        """2-byte (bf16 / fp16) im2col [N, H/2, W/2, 152] of the fp32 NCHW input over the 7x7 / stride-2 / pad-3 footprint shared by both
-        stem convolutions (the 3x3 / pad-1 backbone stem is its centre): read once, used by two forward GEMMs and two
-        weight-gradient GEMMs on the tensor cores."""
+    @staticmethod
+    def stem_ld(k: int) -> int:
+        """Pixel stride of the im2col over a k x k footprint: 3 k^2 columns padded to 8 (7: 152, 3: 32)."""
+        return -(-3 * k * k // 8) * 8
+
+    def stem_im2col(self, x: torch.Tensor, k: int = STEM_K) -> Map:
+        """2-byte (bf16 / fp16) im2col [N, H/2, W/2, stem_ld(k)] of the fp32 NCHW input over the k x k / stride-2 /
+        pad-(k-1)/2 footprint.  CABiNet's 7x7 one is shared by both stem convolutions (the 3x3 / pad-1 backbone stem is
+        its centre): read once, used by two forward GEMMs and two weight-gradient GEMMs on the tensor cores."""
         N, _, H, W = x.shape
-        OH, OW = _out_size(H, 7, 2, 3), _out_size(W, 7, 2, 3)
-        xcol = Map(torch.empty((N, OH, OW, self.STEM_LD), dtype=self.tdt, device=self.dev), N, OH, OW, self.STEM_LD,
-                   self.STEM_LD)
-        self._call_tc("cabinet_im2col_nchw", x.data_ptr(), N, 3, H, W, 7, 2, 3, xcol.ptr, xcol.ld)
+        pad, ld = (k - 1) // 2, self.stem_ld(k)
+        OH, OW = _out_size(H, k, 2, pad), _out_size(W, k, 2, pad)
+        xcol = Map(torch.empty((N, OH, OW, ld), dtype=self.tdt, device=self.dev), N, OH, OW, ld, ld)
+        self._call_tc("cabinet_im2col_nchw", x.data_ptr(), N, 3, H, W, k, 2, pad, xcol.ptr, xcol.ld)
         return xcol
 
-    def conv_stem(self, xcol: Map, conv) -> Map:
-        """A stem convolution (7x7 s2 p3, or 3x3 s2 p1 embedded in the same footprint) as a 1x1 GEMM on the im2col matrix."""
+    def conv_stem(self, xcol: Map, conv, K: int = STEM_K) -> Map:
+        """A stem convolution (7x7 s2 p3, or 3x3 s2 p1 embedded in the same footprint) as a 1x1 GEMM on the im2col matrix
+        of the K x K footprint."""
         w = conv.weight
         cout, cin, k, _ = w.shape
         assert cin == 3 and conv.stride[0] == 2 and (k, conv.padding[0]) in ((7, 3), (3, 1)) and conv.bias is None
-        N, OH, OW, LD = xcol.N, xcol.H, xcol.W, self.STEM_LD
+        assert k <= K and xcol.ld == self.stem_ld(K)
+        N, OH, OW, LD = xcol.N, xcol.H, xcol.W, xcol.ld
         out = self.new(N, OH, OW, cout)
         r16, k64 = -(-cout // 16) * 16, -(-LD // 64) * 64
         wbig = torch.zeros((cout, LD), dtype=torch.float32, device=self.dev)
         self.launches += 1
         wp = torch.empty((r16, 1, k64), dtype=self.tdt, device=self.dev)
-        self._call("cabinet_embed_filter", w.data_ptr(), cout, 3, k, self.STEM_K, wbig.data_ptr(), LD, 0)
+        self._call("cabinet_embed_filter", w.data_ptr(), cout, 3, k, K, wbig.data_ptr(), LD, 0)
         self._call("cabinet_pack_conv_weight", wbig.data_ptr(), cout, LD, 1, 1, wp.data_ptr(), self.dt, r16, k64, 0)
         self._call_tc("cabinet_conv_tc", xcol.ptr, xcol.ld, N, OH, OW, LD, wp.data_ptr(), cout, 1, 1, 1, 0,
                       self._zeros(cout).data_ptr(), None, 0, out.ptr, out.dt, out.ld, OH, OW, ACT_NONE)
@@ -430,7 +439,7 @@ class TrainEngine:
                 sc = torch.empty(n, dtype=torch.float32, device=self.dev)
                 self._call_tc("cabinet_conv_wgrad_tc", dy.ptr, dy.ld, xcol.ptr, xcol.ld, dwbig.data_ptr(), N, OH, OW, LD, cout,
                               1, 1, 1, 0, sc.data_ptr())
-                self._call("cabinet_embed_filter", self.pgrad(w).data_ptr(), cout, 3, k, self.STEM_K, dwbig.data_ptr(), LD, 1)
+                self._call("cabinet_embed_filter", self.pgrad(w).data_ptr(), cout, 3, k, K, dwbig.data_ptr(), LD, 1)
 
         self.tape.append(backward)
         return out
@@ -816,6 +825,32 @@ class TrainEngine:
 
         return y, backward
 
+    def mobilenet(self, f: Map, mob, out: Optional[Map] = None) -> Map:
+        """The MobileNetV3 ``mob`` after its stem: the inverted-residual blocks and ``mobile.conv`` (mobilenetv3.py:102-159,
+        202-205).  ``f``: the stem's output; ``out``: where ``mobile.conv`` writes (a channel slice of CABiNet's b1 concat
+        buffer) or None."""
+        for blk in list(mob.features)[1:]:
+            s, c = blk.spec, blk.conv
+            act = ACT_HSWISH if s["hs"] else ACT_RELU
+            res = f if s["identity"] else None
+            if s["expand"]:
+                h = self.bn(self.conv(f, c[0]), c[1], act)
+                z = self.dwconv(h, c[3])
+                if s["se"]:
+                    u = self.bn(z, c[4], ACT_NONE)
+                    se = c[5]
+                    y = self.gate(u, se.fc[0].weight, se.fc[0].bias, se.fc[2].weight, se.fc[2].bias, ACT_HSIGMOID, act, 0.0)
+                else:
+                    y = self.bn(z, c[4], act)
+                f = self.bn(self.conv(y, c[7]), c[8], ACT_NONE, res=res)
+            else:
+                y = self.bn(self.dwconv(f, c[0]), c[1], act)
+                if s["se"]:  # no-expand form: activation first, then SE (SURVEY F10)
+                    se = c[3]
+                    y = self.gate(y, se.fc[0].weight, se.fc[0].bias, se.fc[2].weight, se.fc[2].bias, ACT_HSIGMOID, ACT_NONE, 0.0)
+                f = self.bn(self.conv(y, c[4]), c[5], ACT_NONE, res=res)
+        return self.bn(self.conv(f, mob.conv[0]), mob.conv[1], ACT_HSWISH, out=out)
+
     # ------------------------------------------------------------------ the step
     def forward(self, x: torch.Tensor, logits_dtype=torch.float32, input_grad: bool = False):
         """Train-mode ``CABiNet.forward`` (cabinet.py:207-247) -> (final_logit, high_res_logit_up), NCHW.  ``input_grad``:
@@ -848,30 +883,10 @@ class TrainEngine:
         f = self.bn(stem3, mob.features[0][1], ACT_HSWISH)
         if input_grad:
             self._stems = (stem7, stem3, tuple(x.shape))
-        for blk in list(mob.features)[1:]:
-            s, c = blk.spec, blk.conv
-            act = ACT_HSWISH if s["hs"] else ACT_RELU
-            res = f if s["identity"] else None
-            if s["expand"]:
-                h = self.bn(self.conv(f, c[0]), c[1], act)
-                z = self.dwconv(h, c[3])
-                if s["se"]:
-                    u = self.bn(z, c[4], ACT_NONE)
-                    se = c[5]
-                    y = self.gate(u, se.fc[0].weight, se.fc[0].bias, se.fc[2].weight, se.fc[2].bias, ACT_HSIGMOID, act, 0.0)
-                else:
-                    y = self.bn(z, c[4], act)
-                f = self.bn(self.conv(y, c[7]), c[8], ACT_NONE, res=res)
-            else:
-                y = self.bn(self.dwconv(f, c[0]), c[1], act)
-                if s["se"]:  # no-expand form: activation first, then SE (SURVEY F10)
-                    se = c[3]
-                    y = self.gate(y, se.fc[0].weight, se.fc[0].bias, se.fc[2].weight, se.fc[2].bias, ACT_HSIGMOID, ACT_NONE, 0.0)
-                f = self.bn(self.conv(y, c[4]), c[5], ACT_NONE, res=res)
-        h32, w32 = f.H, f.W
+        h32, w32 = backbone_hw([blk.spec for blk in list(mob.features)[1:]], f.H, f.W)
         n_mf = mob.conv[0].out_channels
         cat_b1 = self.new(N, h32, w32, n_mf + 256)
-        mf = self.bn(self.conv(f, mob.conv[0]), mob.conv[1], ACT_HSWISH, out=cat_b1.slice(0, n_mf))
+        mf = self.mobilenet(f, mob, out=cat_b1.slice(0, n_mf))
 
         # ---- attention branch (cabinet.py:75-94, cab.py:131-162,175-184,213-216)
         feat = self.bn(self.conv(mf, ab.conva[0]), ab.conva[1], ACT_RELU)
@@ -934,16 +949,17 @@ class TrainEngine:
     def _stem_dgrad(self, g: _Grads) -> Optional[torch.Tensor]:
         """dx of the network input: both stems' data gradients in one cabinet_stem_dgrad call, on the main stream once the
         spatial branch (sb.conv1's output gradient) has joined it.  None when neither stem received a gradient."""
-        stem7, stem3, (N, _, H, W) = self._stems
-        dy7, dy3 = g.get(stem7), g.get(stem3)
+        stem7, stem3, (N, _, H, W) = self._stems   # stem7 None: a standalone MobileNetV3
+        dy7, dy3 = g.get(stem7) if stem7 is not None else None, g.get(stem3)
         if dy7 is None and dy3 is None:
             return None
         dx = torch.empty((N, 3, H, W), dtype=torch.float32, device=self.dev)
-        w7, w3 = self.model.sb.conv1.conv.weight, self.model.mobile.features[0][0].weight
+        mob = self.model if stem7 is None else self.model.mobile
+        w7 = self.model.sb.conv1.conv.weight.data_ptr() if stem7 is not None else None
         dt = (dy7 if dy7 is not None else dy3).dt
         self._call("cabinet_stem_dgrad", dy7.ptr if dy7 is not None else None, dy7.ld if dy7 is not None else 0,
-                   dy3.ptr if dy3 is not None else None, dy3.ld if dy3 is not None else 0, dt, w7.data_ptr(), w3.data_ptr(),
-                   dx.data_ptr(), N, H, W, stem3.H, stem3.W)
+                   dy3.ptr if dy3 is not None else None, dy3.ld if dy3 is not None else 0, dt, w7,
+                   mob.features[0][0].weight.data_ptr(), dx.data_ptr(), N, H, W, stem3.H, stem3.W)
         return dx
 
     # ------------------------------------------------------------------ a standalone ContextAggregationBlock
@@ -992,6 +1008,52 @@ class TrainEngine:
         if self._side_used:  # join: the parameter gradients are complete when the caller's stream continues
             torch.cuda.current_stream(self.dev).wait_stream(self._side)
         self.tape, self._block = [], None
+        return self.pgrads, dx
+
+    # ------------------------------------------------------------------ a standalone MobileNetV3
+    def backbone_forward(self, x: torch.Tensor, input_grad: bool) -> torch.Tensor:
+        """``self.model`` is a MobileNetV3: its train-mode (or differentiable eval-mode) forward on the (N, 3, H, W) ``x``
+        -> (N, out_channels, h32, w32) NCHW in x's dtype; the tape is kept for ``backbone_backward``."""
+        mob, xdt = self.model, x.dtype
+        if x.dtype != torch.float32 or not x.is_contiguous():
+            x = x.float().contiguous()
+        self.tape, self.launches, self.pgrads, self.phase = [], 0, {}, "fwd"
+        self._pflat, self._bn_seen = None, []
+        self._stems = (None, None, tuple(x.shape)) if input_grad else None
+        stem = mob.features[0][0]
+        k = stem.kernel_size[0]
+        stem3 = (self.conv_stem(self.stem_im2col(x, k), stem, k) if self.use_tc and self.stem_gemm
+                 else self.conv(None, stem, nchw=x))
+        f = self.bn(stem3, mob.features[0][1], ACT_HSWISH)
+        if input_grad:
+            self._stems = (None, stem3, tuple(x.shape))
+        out = self.mobilenet(f, mob)
+        N, C, h, w = out.N, out.C, out.H, out.W
+        y = torch.empty((N, C, h, w), dtype=xdt, device=self.dev)
+        self._relayout(out.t, (h * w * C, w * C, C, 1), y, (C * h * w, w, 1, h * w), N, h, w, C)
+        self._block = out
+        if self._bn_seen:
+            torch._foreach_add_(self._bn_seen, 1)
+        return y
+
+    def backbone_backward(self, dy: torch.Tensor) -> Tuple[Dict[int, torch.Tensor], Optional[torch.Tensor]]:
+        """Gradient of ``backbone_forward``'s output -> ({id(parameter): fp32 gradient}, fp32 gradient of x or None)."""
+        out = self._block
+        N, H, W, C = out.N, out.H, out.W, out.C
+        g = _Grads(self)
+        self.pgrads, self.phase, self._pflat, self._side_used = {}, "bwd", None, False
+        self._ensure_pflat()
+        dx = None
+        if out.needs_grad:
+            dout, _ = g.out(out)
+            self._relayout(dy, (dy.stride(0), dy.stride(2), dy.stride(3), dy.stride(1)), dout.t, (H * W * C, W * C, C, 1),
+                           N, H, W, C)
+            for i in range(len(self.tape) - 1, -1, -1):
+                self.tape[i](g)
+            dx = self._stem_dgrad(g) if self._stems is not None else None
+        if self._side_used:  # join: the parameter gradients are complete when the caller's stream continues
+            torch.cuda.current_stream(self.dev).wait_stream(self._side)
+        self.tape, self._block, self._stems = [], None, None
         return self.pgrads, dx
 
     # ------------------------------------------------------------------ the step as two CUDA graphs
@@ -1132,4 +1194,24 @@ class BlockStep(torch.autograd.Function):
         eng = ctx.eng
         with torch.no_grad(), torch.cuda.device(eng.dev):
             grads, dx = eng.block_backward(dy)
+        return (None, dx, *(grads[id(p)].to(p.dtype) if id(p) in grads else None for p in ctx.params))
+
+
+class BackboneStep(torch.autograd.Function):
+    """Autograd hand-off of a standalone MobileNetV3: inputs = (engine, x, *parameters); output = the feature map.  The
+    gradient of ``x`` is computed when ``x`` requires grad and returned in x's dtype."""
+
+    @staticmethod
+    def forward(ctx, eng: TrainEngine, x, *params):
+        with torch.no_grad(), torch.cuda.device(eng.dev):
+            y = eng.backbone_forward(x, bool(ctx.needs_input_grad[1]))
+        ctx.eng, ctx.params, ctx.xdt = eng, params, x.dtype
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        eng = ctx.eng
+        with torch.no_grad(), torch.cuda.device(eng.dev):
+            grads, dx = eng.backbone_backward(dy)
+        dx = dx.to(ctx.xdt) if dx is not None else None
         return (None, dx, *(grads[id(p)].to(p.dtype) if id(p) in grads else None for p in ctx.params))

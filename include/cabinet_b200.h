@@ -130,6 +130,15 @@ int cabinet_stem_tc(const float* x, int N, int H, int W, const void* w_packed, c
 int cabinet_stem_tc2(const float* x, int N, int H, int W, const void* w_packed2, void* y_sb, long long ld_sb, void* y_stem,
                      long long ld_stem, int OH, int OW, cabinet_stream_t stream);
 
+/* The backbone stem alone (a standalone MobileNetV3: 3x3 s2 p1, 3 -> 16, BN folded, HardSwish) in the formulation of
+ * cabinet_stem_tc2, one K16 slice per tap row.  x fp32 NCHW [N][3][H][W] (W % 4 == 0); y bf16 NHWC [N][OH][OW] with pixel
+ * stride ld_y (a multiple of 8, >= 16).
+ * w_packed3: bf16 [3 ky][2 k chunks][16 out][8] = UMMA core matrices of W[o][ky][s][c], s = 0..3, c = 0..3: slot s = kx + 1
+ * holds the filter tap kx (c < 3), slot 0 is zero except the bias on the constant-1 channel c = 3 (hi part at ky 1, lo
+ * part at ky 0); element e = (s % 2) * 4 + c of chunk s / 2. */
+int cabinet_stem3_tc(const float* x, int N, int H, int W, const void* w_packed3, void* y, long long ld_y, int OH, int OW,
+                     cabinet_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Depthwise k x k (k in {3,5}, stride in {1,2}, pad (k-1)/2) + folded-BN bias + activation,
  * optional per-(image, channel) sum of the written values for the SE / GAP consumers.
