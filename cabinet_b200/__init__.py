@@ -2,7 +2,8 @@
 
 from .constants import BACKBONE_CFGS, DEFAULT_EVAL_SCALES, EVAL_STRIDE_RATE, MODEL_CONFIG  # noqa: F401
 from .loss import OhemCELoss  # noqa: F401
-from .modules import CABiNet, ContextAggregationBlock, MobileNetV3  # noqa: F401
+from .modules import (AttentionBranch, CABiNet, CABiNetOutput, ContextAggregationBlock, FeatureFusionModule,  # noqa: F401
+                      MobileNetV3, SpatialBranch)
 
-__all__ = ["CABiNet", "ContextAggregationBlock", "MobileNetV3", "OhemCELoss", "MODEL_CONFIG", "BACKBONE_CFGS",
-           "EVAL_STRIDE_RATE", "DEFAULT_EVAL_SCALES"]
+__all__ = ["CABiNet", "ContextAggregationBlock", "MobileNetV3", "SpatialBranch", "AttentionBranch", "FeatureFusionModule",
+           "CABiNetOutput", "OhemCELoss", "MODEL_CONFIG", "BACKBONE_CFGS", "EVAL_STRIDE_RATE", "DEFAULT_EVAL_SCALES"]

@@ -46,6 +46,7 @@ SIGNATURES = {
     "cabinet_stem_tc": ([_p, _i, _i, _i, _p, _p, _p, _ll, _p, _ll, _i, _i, _p], _i),
     "cabinet_stem_tc2": ([_p, _i, _i, _i, _p, _p, _ll, _p, _ll, _i, _i, _p], _i),
     "cabinet_stem3_tc": ([_p, _i, _i, _i, _p, _p, _ll, _i, _i, _p], _i),
+    "cabinet_stem7_tc": ([_p, _i, _i, _i, _p, _p, _ll, _i, _i, _p], _i),
     "cabinet_dwconv": ([_p, _ll, _p, _p, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p], _i),
     "cabinet_dwconv_tma": ([_p, _ll, _p, _p, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p], _i),
     "cabinet_dwconv_tma_dt": ([_p, _ll, _p, _p, _p, _ll, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _i, _p], _i),

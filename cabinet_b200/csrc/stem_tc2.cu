@@ -32,11 +32,15 @@ constexpr int PITCH = WIN_W * 8;             // bytes per row of the bf16 x 4 co
 constexpr int WINB_BYTES = WIN_H * PITCH;    // 7104
 constexpr int WINB_STRIDE = 7168;
 constexpr int WINB_STAGES = 3;
-constexpr int NOUT = 80;
 constexpr int NMMA = 14;                     // 7 tap rows x 2 K halves
-constexpr int W_MMA_BYTES = 2 * (NOUT / 8) * 128;    // one [80 x 16] bf16 operand as 2 x 10 core matrices = 2560
-constexpr int W_BYTES = NMMA * W_MMA_BYTES;  // 35840
-constexpr int ACC_STAGES = 2, ACC_COLS = 128;
+// NOUT = 80: sb.conv1 (64) + the backbone stem (16), CABiNet's fused stems; NOUT = 64: sb.conv1 alone
+template <int NOUT>
+struct Stem2Shape {
+    static constexpr int W_MMA_BYTES = 2 * (NOUT / 8) * 128;  // one [NOUT x 16] bf16 operand (80: 2 x 10 core matrices)
+    static constexpr int W_BYTES = NMMA * W_MMA_BYTES;        // 80: 35840 (<= the 36 KB reserved), 64: 28672
+    static constexpr int ACC_COLS = NOUT > 64 ? 128 : 64;     // TMEM columns per accumulator stage (a power of 2)
+};
+constexpr int ACC_STAGES = 2;
 constexpr int CONV_WARPS = 8, CONV_THREADS = 32 * CONV_WARPS;
 constexpr int EPI_WARP0 = 2 + CONV_WARPS;
 constexpr int NUM_THREADS = 64 + CONV_THREADS + 128;
@@ -64,9 +68,14 @@ __device__ __forceinline__ uint32_t pack2(float lo, float hi) {
     return *reinterpret_cast<uint32_t*>(&h);
 }
 
+// NOUT = 64 stores the sb tile only (tmYst is not read).
+template <int NOUT>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 stem_tc2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmYsb,
                 const __grid_constant__ CUtensorMap tmYst, const Stem2Params p) {
+    constexpr int W_MMA_BYTES = Stem2Shape<NOUT>::W_MMA_BYTES, W_BYTES = Stem2Shape<NOUT>::W_BYTES;
+    constexpr int ACC_COLS = Stem2Shape<NOUT>::ACC_COLS;
+    constexpr bool kStem = NOUT == 80;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t w_bar, win_full[WIN_STAGES], win_empty[WIN_STAGES], a_full[WINB_STAGES],
         a_empty[WINB_STAGES], acc_full[ACC_STAGES], acc_empty[ACC_STAGES];
@@ -84,7 +93,7 @@ stem_tc2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     if (threadIdx.x == 0) {
         tc::prefetch_tmap(&tmX);
         tc::prefetch_tmap(&tmYsb);
-        tc::prefetch_tmap(&tmYst);
+        if constexpr (kStem) tc::prefetch_tmap(&tmYst);
         tc::mbar_init(&w_bar, 1);
         for (int s = 0; s < WIN_STAGES; ++s) {
             tc::mbar_init(&win_full[s], 1);
@@ -202,7 +211,7 @@ stem_tc2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
             uint32_t a0[32], a1[32], a2[16];
             tc::tmem_ld32(taddr, a0);
             tc::tmem_ld32(taddr + 32, a1);
-            tc::tmem_ld16(taddr + 64, a2);
+            if constexpr (kStem) tc::tmem_ld16(taddr + 64, a2);
             tc::tmem_ld_wait();
             tc::tc_fence_before();
             __syncwarp();
@@ -221,23 +230,25 @@ stem_tc2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
                 }
                 tc::sts128(rowp + ((g ^ (r & 7)) << 4), make_uint4(w[0], w[1], w[2], w[3]));
             }
+            if constexpr (kStem) {
 #pragma unroll
-            for (int g = 0; g < 2; ++g) {
-                float v[8];
+                for (int g = 0; g < 2; ++g) {
+                    float v[8];
 #pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float t = __uint_as_float(a2[8 * g + j]);
-                    v[j] = t * __saturatef(fmaf(t, 1.f / 6.f, 0.5f));
+                    for (int j = 0; j < 8; ++j) {
+                        const float t = __uint_as_float(a2[8 * g + j]);
+                        v[j] = t * __saturatef(fmaf(t, 1.f / 6.f, 0.5f));
+                    }
+                    Vec16<bf16> o;
+                    o.pack(v);
+                    tc::sts128(tc::smem_u32(bst) + r * 32 + g * 16, o.raw);
                 }
-                Vec16<bf16> o;
-                o.pack(v);
-                tc::sts128(tc::smem_u32(bst) + r * 32 + g * 16, o.raw);
             }
             tc::fence_proxy_async();
             tc::named_bar_sync(1, 128);
             if (leader) {
                 tc::tma_store_4d(&tmYsb, bsb, 0, ow0, oh0, img);
-                tc::tma_store_4d(&tmYst, bst, 0, ow0, oh0, img);
+                if constexpr (kStem) tc::tma_store_4d(&tmYst, bst, 0, ow0, oh0, img);
                 tc::bulk_commit();
             }
         }
@@ -251,22 +262,24 @@ stem_tc2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     }
 }
 
+template <int NOUT>
 int g_attr_set2 = 0;
 
-}  // namespace
-
-extern "C" int cabinet_stem_tc2(const float* x, int N, int H, int W, const void* w_packed2, void* y_sb, long long ld_sb,
-                                void* y_stem, long long ld_stem, int OH, int OW, cabinet_stream_t stream) {
-    CAB_REQUIRE(x && w_packed2 && y_sb && y_stem, "stem_tc2: null pointer");
-    CAB_REQUIRE(N >= 0 && H > 0 && W > 0 && W % 4 == 0, "stem_tc2: W must be a multiple of 4 (TMA row pitch)");
-    CAB_REQUIRE(OH == (H - 1) / 2 + 1 && OW == (W - 1) / 2 + 1, "stem_tc2: inconsistent output size");
-    CAB_REQUIRE(ld_sb >= 64 && ld_sb % 8 == 0 && ld_stem >= 16 && ld_stem % 8 == 0 &&
+// Host side of both instantiations.  y_stem == nullptr: NOUT = 64, sb.conv1 alone.
+template <int NOUT>
+int launch_stem2(const char* name, const float* x, int N, int H, int W, const void* w_packed, void* y_sb, long long ld_sb,
+                 void* y_stem, long long ld_stem, int OH, int OW, cabinet_stream_t stream) {
+    constexpr bool kStem = NOUT == 80;
+    CAB_REQUIRE(x && w_packed && y_sb && (y_stem || !kStem), "%s: null pointer", name);
+    CAB_REQUIRE(N >= 0 && H > 0 && W > 0 && W % 4 == 0, "%s: W must be a multiple of 4 (TMA row pitch)", name);
+    CAB_REQUIRE(OH == (H - 1) / 2 + 1 && OW == (W - 1) / 2 + 1, "%s: inconsistent output size", name);
+    CAB_REQUIRE(ld_sb >= 64 && ld_sb % 8 == 0 && (!kStem || (ld_stem >= 16 && ld_stem % 8 == 0)) &&
                     (reinterpret_cast<uintptr_t>(y_sb) & 15) == 0 && (reinterpret_cast<uintptr_t>(y_stem) & 15) == 0 &&
-                    (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(w_packed2) & 15) == 0,
-                "stem_tc2: alignment");
+                    (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(w_packed) & 15) == 0,
+                kStem ? "%s: alignment" : "%s: alignment (ld_y a multiple of 8 >= 64, 16-byte aligned pointers)", name);
     if (N == 0) return CABINET_OK;
     cab_encode_tiled_fn enc = cab_get_encode_tiled();
-    CAB_REQUIRE(enc != nullptr, "stem_tc2: cuTensorMapEncodeTiled unavailable");
+    CAB_REQUIRE(enc != nullptr, "%s: cuTensorMapEncodeTiled unavailable", name);
     CUtensorMap tmX;
     {
         cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)3 * N};
@@ -277,16 +290,16 @@ extern "C" int cabinet_stem_tc2(const float* x, int N, int H, int W, const void*
                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) {
-            cabinet_set_error("stem_tc2: input tensor map encode failed (CUresult %d)", (int)r);
+            cabinet_set_error("%s: input tensor map encode failed (CUresult %d)", name, (int)r);
             return CABINET_ERR_CUDA;
         }
     }
     Stem2Params p;
-    p.N = N; p.OH = OH; p.OW = OW; p.w = w_packed2;
+    p.N = N; p.OH = OH; p.OW = OW; p.w = w_packed;
     p.tiles_w = (OW + TW - 1) / TW;
     p.tiles_h = (OH + TH - 1) / TH;
     const long long nt = static_cast<long long>(N) * p.tiles_w * p.tiles_h;
-    CAB_REQUIRE(nt < (1LL << 31), "stem_tc2: too many tiles");
+    CAB_REQUIRE(nt < (1LL << 31), "%s: too many tiles", name);
     p.num_tiles = static_cast<int>(nt);
     CUtensorMap tmYsb, tmYst;
     {
@@ -295,24 +308,41 @@ extern "C" int cabinet_stem_tc2(const float* x, int N, int H, int W, const void*
         const uint32_t bsb[4] = {64, TW, TH, 1};
         int rc = cab_make_tmap_bf16(&tmYsb, y_sb, 4, dsb, ssb, bsb);
         if (rc) return rc;
-        const uint64_t dst[4] = {16, (uint64_t)OW, (uint64_t)OH, (uint64_t)N};
-        const uint64_t sst[3] = {(uint64_t)ld_stem * 2, (uint64_t)ld_stem * 2 * OW, (uint64_t)ld_stem * 2 * OW * OH};
-        const uint32_t bst[4] = {16, TW, TH, 1};
-        rc = cab_make_tmap_bf16(&tmYst, y_stem, 4, dst, sst, bst, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_SWIZZLE_NONE);
-        if (rc) return rc;
+        if (kStem) {
+            const uint64_t dst[4] = {16, (uint64_t)OW, (uint64_t)OH, (uint64_t)N};
+            const uint64_t sst[3] = {(uint64_t)ld_stem * 2, (uint64_t)ld_stem * 2 * OW, (uint64_t)ld_stem * 2 * OW * OH};
+            const uint32_t bst[4] = {16, TW, TH, 1};
+            rc = cab_make_tmap_bf16(&tmYst, y_stem, 4, dst, sst, bst, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                                    CU_TENSOR_MAP_SWIZZLE_NONE);
+            if (rc) return rc;
+        } else {
+            tmYst = tmYsb;  // not read by the NOUT = 64 kernel
+        }
     }
-    if (!g_attr_set2) {
-        CAB_CUDA(cudaFuncSetAttribute(stem_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        g_attr_set2 = 1;
+    if (!g_attr_set2<NOUT>) {
+        CAB_CUDA(cudaFuncSetAttribute(stem_tc2_kernel<NOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        g_attr_set2<NOUT> = 1;
     }
     int dev = 0, sms = 148;
     CAB_CUDA(cudaGetDevice(&dev));
     CAB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const int grid = static_cast<int>(std::min<long long>(nt, sms));
-    stem_tc2_kernel<<<grid, NUM_THREADS, SMEM_BYTES, static_cast<cudaStream_t>(stream)>>>(tmX, tmYsb, tmYst, p);
+    stem_tc2_kernel<NOUT><<<grid, NUM_THREADS, SMEM_BYTES, static_cast<cudaStream_t>(stream)>>>(tmX, tmYsb, tmYst, p);
     CAB_LAUNCH_CHECK();
     return CABINET_OK;
+}
+
+}  // namespace
+
+extern "C" int cabinet_stem_tc2(const float* x, int N, int H, int W, const void* w_packed2, void* y_sb, long long ld_sb,
+                                void* y_stem, long long ld_stem, int OH, int OW, cabinet_stream_t stream) {
+    return launch_stem2<80>("stem_tc2", x, N, H, W, w_packed2, y_sb, ld_sb, y_stem, ld_stem, OH, OW, stream);
+}
+
+// sb.conv1 alone (a standalone SpatialBranch): the N = 64 instantiation, one TMA store per tile.
+extern "C" int cabinet_stem7_tc(const float* x, int N, int H, int W, const void* w_packed7, void* y, long long ld_y, int OH,
+                                int OW, cabinet_stream_t stream) {
+    return launch_stem2<64>("stem7_tc", x, N, H, W, w_packed7, y, ld_y, nullptr, 0, OH, OW, stream);
 }
 
 // ===================================================================================================================

@@ -170,6 +170,11 @@ def _from_plain(o):
     return o
 
 
+def _nchw_strides(t: torch.Tensor):
+    """(n, y, x, c) element strides of an NCHW tensor, in the order ``Engine.relayout`` takes them."""
+    return (t.stride(0), t.stride(2), t.stride(3), t.stride(1))
+
+
 def _out_size(n, k, s, p):
     return (n + 2 * p - k) // s + 1
 
@@ -183,6 +188,17 @@ def backbone_hw(specs, H: int, W: int) -> Tuple[int, int]:
     return H, W
 
 
+def _stem_tc2_pack(pk, bias, b_hi):
+    """cabinet_stem_tc2 / cabinet_stem7_tc weights from ``pk`` [n][3][7 ky][8 kx] fp32 (kx = 0 zero): W[o][ky][kx][c] (c = 3:
+    the constant-1 channel, carrying the bias -- ``b_hi`` its bf16 part -- at the centre pixel) as UMMA core matrices
+    [ky][K half][k chunk][o][8]."""
+    n = pk.shape[0]
+    wn = torch.zeros((n, 7, 8, 4), dtype=torch.float32, device=pk.device)
+    wn[..., :3] = pk.permute(0, 2, 3, 1)
+    wn[:, 3, 4, 3], wn[:, 3, 5, 3] = b_hi, bias - b_hi
+    return wn.view(n, 7, 2, 2, 8).permute(1, 2, 3, 0, 4).contiguous().to(torch.bfloat16)
+
+
 class Engine:
     # everything ``_pack`` produces (what ``checkpoint.save_packed`` caches)
     PACKED_ATTRS = ("stem", "blocks", "last", "stem_tc", "sb1", "sb2", "sb3", "sb4", "conva", "to_q", "to_k", "to_v",
@@ -192,6 +208,11 @@ class Engine:
     CAB_ATTRS = ("to_q", "to_k", "to_v", "psp_k", "psp_v", "proj_out", "local", "gamma", "key_ch", "qkv")
     # what ``_pack_mobilenet`` produces: all an engine built over a standalone MobileNetV3 packs
     BACKBONE_ATTRS = ("stem", "blocks", "last", "stem_tc3")
+    # ... and what an engine over a standalone SpatialBranch / AttentionBranch / FeatureFusionModule / CABiNetOutput packs
+    SB_ATTRS = ("sb1", "sb2", "sb3", "sb4", "stem_tc7")
+    AB_ATTRS = ("conva", "convb", "b1", "b4") + CAB_ATTRS
+    FFM_ATTRS = ("ffm_blk", "ffm_gate")
+    HEAD_ATTRS = ("head_conv", "head_out")
 
     def __init__(self, model, precision: str = "bf16", packed: Optional[dict] = None):
         if precision not in ("bf16", "fp32"):
@@ -199,18 +220,30 @@ class Engine:
         p0 = next(model.parameters())
         if not p0.is_cuda:
             raise RuntimeError("cabinet_b200 engine needs the model on a CUDA device (no CPU path)")
-        from .modules import ContextAggregationBlock, MobileNetV3
+        from . import modules
 
         self.lib = _lib.load()
         self.dev = p0.device
         self.precision = precision
         self.tdt = torch.bfloat16 if precision == "bf16" else torch.float32
         self.dt = BF16 if precision == "bf16" else F32
-        # an engine over a standalone ContextAggregationBlock packs that block alone and runs ``forward_block``
-        self.block = isinstance(model, ContextAggregationBlock)
-        # ... and one over a standalone MobileNetV3 packs the backbone alone and runs ``forward_backbone``
-        self.backbone = isinstance(model, MobileNetV3)
-        self.n_classes = 0 if self.block or self.backbone else model.n_classes
+        # an engine over a standalone module packs that module alone (``attrs``) and runs its ``forward_*`` method:
+        # ContextAggregationBlock -> forward_block, MobileNetV3 -> forward_backbone, SpatialBranch -> forward_sb,
+        # AttentionBranch -> forward_ab, FeatureFusionModule -> forward_ffm, CABiNetOutput -> forward_head
+        # (subclasses included: a user's subclass with its own forward packs and runs as its base class)
+        standalone = None
+        for cls, v in ((modules.ContextAggregationBlock, (self._pack_cab, self.CAB_ATTRS)),
+                       (modules.MobileNetV3, (self._pack_mobilenet, self.BACKBONE_ATTRS)),
+                       (modules.SpatialBranch, (self._pack_spatial, self.SB_ATTRS)),
+                       (modules.AttentionBranch, (self._pack_ab, self.AB_ATTRS)),
+                       (modules.FeatureFusionModule, (self._pack_ffm, self.FFM_ATTRS)),
+                       (modules.CABiNetOutput, (self._pack_head, self.HEAD_ATTRS))):
+            if isinstance(model, cls):
+                standalone = v
+                break
+        self.block = isinstance(model, modules.ContextAggregationBlock)
+        self.backbone = isinstance(model, modules.MobileNetV3)
+        self.n_classes = model.n_classes if standalone is None else 0
         self.stamp = None
         self.launches = 0  # kernels enqueued by the last forward
         self.use_tc = precision == "bf16"
@@ -247,7 +280,7 @@ class Engine:
         self.branch_overlap = True  # independent chains of the attention branch on side streams (fork / join by events)
         self._branch_streams, self._branch_events = [], {}
         self.sb_overlap = False     # experiment: spatial branch beside the backbone
-        if packed is not None and (self.block or self.backbone):
+        if packed is not None and standalone is not None:
             raise ValueError("packed weights exist for CABiNet engines only")
         if packed is not None:  # cached fold + pack of exactly these weights (checkpoint.load_packed verified the digest)
             missing = [a for a in self.PACKED_ATTRS if a not in packed]
@@ -258,13 +291,8 @@ class Engine:
             self.gamma = model.ab.a2block.gamma.detach().float().contiguous()
         else:
             with torch.no_grad():
-                if self.block:  # on the host ...
-                    self._pack_cab(model)
-                elif self.backbone:
-                    self._pack_mobilenet(model)
-                else:
-                    self._pack(model)
-                attrs = self.CAB_ATTRS if self.block else self.BACKBONE_ATTRS if self.backbone else self.PACKED_ATTRS
+                pack, attrs = standalone if standalone is not None else (self._pack, self.PACKED_ATTRS)
+                pack(model)  # on the host ...
                 for a in attrs:  # ... then one upload per packed tensor
                     setattr(self, a, _map_tensors(getattr(self, a), lambda t: t.to(self.dev)))
 
@@ -276,7 +304,6 @@ class Engine:
     # ------------------------------------------------------------------ packing
     def _pack(self, m):
         wd = self.tdt
-        f32 = torch.float32
         mob = m.mobile
         self._pack_backbone(mob)
 
@@ -296,27 +323,12 @@ class Engine:
             b_hi = bias.to(torch.bfloat16).float()
             wk[:, 168], wk[:, 169] = b_hi, bias - b_hi  # bias rides in two spare K slots (A feeds 1.0 there)
             self.stem_tc = (wk.to(torch.bfloat16).contiguous(), bias)
-            # cabinet_stem_tc2: W[o][ky][kx][c] (c = 3: the constant-1 channel, carrying the bias at the centre pixel) as
-            # UMMA core matrices [ky][K half][k chunk][o][8]
-            wn = torch.zeros((80, 7, 8, 4), dtype=torch.float32, device=w7.device)
-            wn[..., :3] = pk.permute(0, 2, 3, 1)
-            wn[:, 3, 4, 3], wn[:, 3, 5, 3] = b_hi, bias - b_hi
-            self.stem_tc2 = wn.view(80, 7, 2, 2, 8).permute(1, 2, 3, 0, 4).contiguous().to(torch.bfloat16)
-        self.sb1 = ConvLayer(sb.conv1.conv, sb.conv1.bn, ACT_RELU, f32, "sb.conv1")
-        self.sb2 = ConvLayer(sb.conv2.conv, sb.conv2.bn, ACT_RELU, wd, "sb.conv2")
-        self.sb3 = ConvLayer(sb.conv3.conv, sb.conv3.bn, ACT_RELU, wd, "sb.conv3")
-        self.sb4 = ConvLayer(sb.conv_out.conv, sb.conv_out.bn, ACT_RELU, wd, "sb.conv_out")
-
+            self.stem_tc2 = _stem_tc2_pack(pk, bias, b_hi)
+        self._pack_sb(sb)
         ab = m.ab
-        self.conva = ConvLayer(ab.conva[0], ab.conva[1], ACT_RELU, wd, "ab.conva")
-        self._pack_cab(ab.a2block)
-        self.convb = ConvLayer(ab.convb, None, ACT_NONE, wd, "ab.convb")
-        self.b1 = ConvLayer(ab.b1, ab.b2, ACT_RELU, wd, "ab.b1")
-        self.b4 = ConvLayer(ab.b4, None, ACT_NONE, wd, "ab.b4")
-
+        self._pack_ab(ab)
         ffm = m.ffm
-        self.ffm_blk = ConvLayer(ffm.convblk.conv, ffm.convblk.bn, ACT_RELU, wd, "ffm.convblk")
-        self.ffm_gate = GateLayer(ffm.conv1.weight, None, ffm.conv2.weight, None, ACT_SIGMOID)
+        self._pack_ffm(ffm)
         # A 1x1 conv commutes with bilinear interpolation: convblk(cat[sb, up(low)]) = W_sb sb + up(W_low low) + b, and
         # low = convb(feat) is itself a 1x1 conv -> one 256 -> 256 conv at 1/32 resolution (W_low W_convb, bias
         # W_low b_convb) whose fp32 output the convblk epilogue upsamples and adds (cabinet_conv_tc_up).  The x4-upsampled
@@ -331,8 +343,45 @@ class Engine:
             self.low_fold = ConvLayer(None, None, ACT_NONE, wd, "ab.convb*ffm.low",
                                       folded=((w_low @ wb[:, :, 0, 0].double()).float()[:, :, None, None].contiguous(),
                                               (w_low @ bb.double()).float(), 1, 0))
-        self.head_conv = ConvLayer(m.conv_out.conv.conv, m.conv_out.conv.bn, ACT_RELU, wd, "conv_out.conv")
-        self.head_out = ConvLayer(m.conv_out.conv_out, None, ACT_NONE, wd, "conv_out.conv_out")
+        self._pack_head(m.conv_out)
+
+    def _pack_sb(self, sb):
+        """The SpatialBranch's four ConvBNReLU layers (reference: cabinet.py:108-129), BN folded."""
+        wd = self.tdt
+        self.sb1 = ConvLayer(sb.conv1.conv, sb.conv1.bn, ACT_RELU, torch.float32, "sb.conv1")  # reads the fp32 NCHW input
+        self.sb2 = ConvLayer(sb.conv2.conv, sb.conv2.bn, ACT_RELU, wd, "sb.conv2")
+        self.sb3 = ConvLayer(sb.conv3.conv, sb.conv3.bn, ACT_RELU, wd, "sb.conv3")
+        self.sb4 = ConvLayer(sb.conv_out.conv, sb.conv_out.bn, ACT_RELU, wd, "sb.conv_out")
+
+    def _pack_spatial(self, sb):
+        """A standalone SpatialBranch: its layers + the weights of the sb.conv1-only tensor-core stem."""
+        self._pack_sb(sb)
+        self.stem_tc7 = None
+        if self.precision == "bf16":
+            # cabinet_stem7_tc: rows 0..63 of the cabinet_stem_tc2 pack (kx = 0 is the zero-weight alignment slot)
+            w7, b7 = _fold(sb.conv1.conv.weight, None, sb.conv1.bn)
+            pk = torch.zeros((64, 3, 7, 8), dtype=torch.float32, device=w7.device)
+            pk[:, :, :, 1:8] = w7
+            self.stem_tc7 = _stem_tc2_pack(pk, b7, b7.to(torch.bfloat16).float())
+
+    def _pack_ab(self, ab):
+        """The AttentionBranch (reference: cabinet.py:54-94), BN folded; b2 is b1's BatchNorm."""
+        wd = self.tdt
+        self.conva = ConvLayer(ab.conva[0], ab.conva[1], ACT_RELU, wd, "ab.conva")
+        self._pack_cab(ab.a2block)
+        self.convb = ConvLayer(ab.convb, None, ACT_NONE, wd, "ab.convb")
+        self.b1 = ConvLayer(ab.b1, ab.b2, ACT_RELU, wd, "ab.b1")
+        self.b4 = ConvLayer(ab.b4, None, ACT_NONE, wd, "ab.b4")
+
+    def _pack_ffm(self, ffm):
+        """The FeatureFusionModule's convblk and its channel gate (reference: cabinet.py:132-153), BN folded."""
+        self.ffm_blk = ConvLayer(ffm.convblk.conv, ffm.convblk.bn, ACT_RELU, self.tdt, "ffm.convblk")
+        self.ffm_gate = GateLayer(ffm.conv1.weight, None, ffm.conv2.weight, None, ACT_SIGMOID)
+
+    def _pack_head(self, head):
+        """CABiNetOutput (reference: cabinet.py:156-172), BN folded."""
+        self.head_conv = ConvLayer(head.conv.conv, head.conv.bn, ACT_RELU, self.tdt, "conv_out.conv")
+        self.head_out = ConvLayer(head.conv_out, None, ACT_NONE, self.tdt, "conv_out.conv_out")
 
     def _pack_backbone(self, mob):
         """The MobileNetV3's stem, blocks and last conv (reference: mobilenetv3.py:86-159,173-205), BN folded."""
@@ -770,6 +819,10 @@ class Engine:
 
         if getattr(self, "_tables", None) is None:
             self._tables = _Tables(self.dev)
+        if {src.dtype, dst.dtype} == {torch.bfloat16, torch.float16}:  # no kernel for this pair: through fp32
+            tmp = torch.empty((N, H, W, C), dtype=torch.float32, device=self.dev)
+            self.relayout(src, src_strides, tmp, (H * W * C, W * C, C, 1), N, H, W, C, name)
+            src, src_strides = tmp, (H * W * C, W * C, C, 1)
         ty, tx = self._tables.get("identity", H, H, False), self._tables.get("identity", W, W, False)
         self._run("resample_sep", name, N * H * W * C * (src.element_size() + dst.element_size()), 0,
                   self.lib.cabinet_resample_sep, src.data_ptr(), dtype_code(src.dtype), *src_strides, dst.data_ptr(),
@@ -914,6 +967,164 @@ class Engine:
                           N, h32, w32, C, "mobile.out")
         return y
 
+    def spatial_branch(self, s1: Map, out: Optional[Map] = None) -> Map:
+        """The SpatialBranch after ``sb.conv1`` (reference: cabinet.py:108-129): sb.conv2, sb.conv3, sb.conv_out.  ``s1``:
+        sb.conv1's output; ``out``: where sb.conv_out writes (CABiNet: channels [0:128] of the FFM concat buffer) or None."""
+        s2 = self.conv(s1, self.sb2)
+        s3 = self.conv(s2, self.sb3)
+        return self.conv(s3, self.sb4, out=out)
+
+    def attention_branch(self, cat: Map, n_in: int, low_path=None, need_high: bool = True, high_path=None):
+        """AttentionBranch (reference: cabinet.py:75-94).  ``cat``: the b1 concat buffer [x | CAB feat] (cabinet.py:87)
+        with x in channels [0:n_in]; the CAB writes the rest.  -> (low, high): ``low_path(feat)`` (default: convb;
+        CABiNet's adds its x4 upsample) and b4's fp32 class logits, None unless ``need_high``.  The low path runs on a
+        side stream beside b1 -> b4; ``high_path(high)`` is enqueued before the join."""
+        feat = self.conv(cat.slice(0, n_in), self.conva)
+        feat2 = cat.slice(n_in, feat.C)
+        self.cab(feat, feat2)
+        if low_path is None:
+            low_path = lambda f: self.conv(f, self.convb)  # noqa: E731
+        if not need_high:
+            return low_path(feat2), None
+        with self._branch(0) as joined:  # low-level path beside b1 / b4
+            low = low_path(feat2)
+            joined(low.t)
+        fused = self.conv(cat, self.b1)
+        high = self.conv(fused, self.b4, out_dtype=torch.float32)  # class logits stay fp32
+        if high_path is not None:
+            high_path(high)
+        self._join(0)
+        return low, high
+
+    def ffm_feat(self, cat: Map, gap: torch.Tensor, scratch: torch.Tensor, low_fold: Optional[Map] = None) -> Map:
+        """FeatureFusionModule up to its gate (reference: cabinet.py:142-147): convblk over ``cat`` = [fsp | fcp], and the
+        per-(image, channel) sums of its output into ``gap`` [N, C] (``scratch``: zeroed, 128 + N * 64 * C floats).
+        ``low_fold``: CABiNet's fp32 1/32-resolution low map, upsampled and added in convblk's epilogue (``fold_low_up``);
+        ``cat`` then holds the spatial-branch half only."""
+        if low_fold is not None:
+            L, (N, H8, W8) = self.ffm_sb, (cat.N, cat.H, cat.W)
+            ff = self.new(N, H8, W8, L.cout)
+            M = N * H8 * W8
+            self._run("conv_tc", L.name, (M * (L.cin + L.cout) + L.w.numel()) * 2 + low_fold.t.numel() * 4,
+                      2 * M * L.cout * L.cin, self.lib.cabinet_conv_tc_up, cat.ptr, cat.ld, N, H8, W8, L.cin,
+                      L.tc.data_ptr(), L.cout, 1, 1, 1, 0, L.b.data_ptr(), low_fold.ptr, low_fold.H, low_fold.W, ff.ptr,
+                      ff.ld, H8, W8, L.act, self.stream)
+        else:
+            ff = self.conv(cat, self.ffm_blk)
+        self.channel_sum(ff, gap, "ffm.gap", scratch)
+        return ff
+
+    def ffm_gate_apply(self, ff: Map, gap: torch.Tensor):
+        """ff = ff * atten + ff in place, atten = sigmoid(conv2(relu(conv1(mean(ff))))) (reference: cabinet.py:148-153)."""
+        att = self.gate(gap, ff.H * ff.W, self.ffm_gate, "ffm.gate")
+        self.scale_act(ff, att, ACT_NONE, "ffm.gate", plus_one=True)
+
+    def head(self, f: Map, ffm_gap: Optional[torch.Tensor] = None) -> Map:
+        """CABiNetOutput (reference: cabinet.py:162-172) -> its fp32 class map.  ``ffm_gap``: ``f`` is the FFM's convblk
+        output with the gate still to apply, and these are its pooling sums (``ffm_feat``)."""
+        hcl = self.head_conv
+        N, H8, W8 = f.N, f.H, f.W
+        if (ffm_gap is not None and self.fold_ffm and self.use_tc and not self.debug and hcl.tc is not None
+                and f.dt == BF16 and hcl.kh * hcl.kw > 1):
+            # feat * atten + feat is a per-(image, channel) scale of the head conv's INPUT: fold it into per-image
+            # copies of the head weights (19 MB) instead of rewriting the 134 MB feature map; the gate MLP runs inside
+            # the same launch
+            wimg = torch.empty((N,) + tuple(hcl.tc.shape), dtype=torch.bfloat16, device=self.dev)
+            self.gate_scale_weights(ffm_gap, False, H8 * W8, self.ffm_gate, hcl.tc, wimg, hcl.cin, True, "ffm.gate")
+            hc = self.new(N, H8, W8, hcl.cout)
+            M = N * H8 * W8
+            self._run("conv_tc", hcl.name, (M * (hcl.cin + hcl.cout) + wimg.numel()) * 2,
+                      2 * M * hcl.cout * hcl.cin * hcl.kh * hcl.kw, self.lib.cabinet_conv_tc_imgw, f.ptr, f.ld, N, H8, W8,
+                      f.C, wimg.data_ptr(), hcl.tc[0].numel() * hcl.tc.shape[0], hcl.cout, hcl.kh, hcl.kw, hcl.stride,
+                      hcl.pad, hcl.b.data_ptr(), None, 0, hc.ptr, hc.dt, hc.ld, H8, W8, hcl.act, self.stream)
+        else:
+            if ffm_gap is not None:
+                self.ffm_gate_apply(f, ffm_gap)
+            hc = self.conv(f, hcl)
+        return self.conv(hc, self.head_out, out_dtype=torch.float32)
+
+    # ------------------------------------------------------------------ standalone branches and heads
+    def _to_map(self, x: torch.Tensor, m: Map, name: str):
+        """NCHW ``x`` -> the NHWC map ``m`` (a channel slice of a concat buffer, say), in m's dtype."""
+        self.relayout(x, _nchw_strides(x), m.t[..., m.off:m.off + m.C], (m.H * m.W * m.ld, m.W * m.ld, m.ld, 1), m.N, m.H,
+                      m.W, m.C, name)
+
+    def _from_map(self, m: Map, dtype: torch.dtype, name: str) -> torch.Tensor:
+        """The NHWC map ``m`` -> a new NCHW tensor of ``dtype``."""
+        y = torch.empty((m.N, m.C, m.H, m.W), dtype=dtype, device=self.dev)
+        self.relayout(m.t[..., m.off:m.off + m.C], (m.H * m.W * m.ld, m.W * m.ld, m.ld, 1), y, _nchw_strides(y), m.N, m.H,
+                      m.W, m.C, name)
+        return y
+
+    @torch.no_grad()
+    def forward_sb(self, x: torch.Tensor) -> torch.Tensor:
+        """Standalone SpatialBranch: (N, 3, H, W) fp32 / bf16 / fp16 -> (N, 128, h8, w8) NCHW in x's dtype.  sb.conv1 runs
+        on the tensor cores (cabinet_stem7_tc) when W % 4 == 0 in the bf16 precision, else on conv2d_simt."""
+        N, _, H, W = x.shape
+        OH, OW = _out_size(H, 7, 2, 3), _out_size(W, 7, 2, 3)
+        h8, w8 = _out_size(_out_size(OH, 3, 2, 1), 3, 2, 1), _out_size(_out_size(OW, 3, 2, 1), 3, 2, 1)
+        self.launches = 0
+        if N == 0 or H * W == 0:
+            return torch.empty((N, self.sb4.cout, h8, w8), dtype=x.dtype, device=x.device)
+        with self._guard():
+            xf = x if x.dtype == torch.float32 and x.is_contiguous() else x.float().contiguous()
+            if self.use_tc and self.stem_tc7 is not None and W % 4 == 0 and xf.data_ptr() % 16 == 0:
+                s1 = self.new(N, OH, OW, 64)
+                self._run("stem7_tc", "sb.conv1", xf.numel() * 4 + s1.t.numel() * 2 + self.stem_tc7.numel() * 2,
+                          2 * N * OH * OW * 64 * 147, self.lib.cabinet_stem7_tc, xf.data_ptr(), N, H, W,
+                          self.stem_tc7.data_ptr(), s1.ptr, s1.ld, OH, OW, self.stream)
+            else:
+                s1 = self.conv(None, self.sb1, nchw_input=xf)
+            return self._from_map(self.spatial_branch(s1), x.dtype, "sb.out")
+
+    @torch.no_grad()
+    def forward_ab(self, x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Standalone AttentionBranch: (N, inplanes, h, w) -> (low, high) = (N, outplanes, h, w), (N, num_classes, h, w)
+        NCHW in x's dtype.  x is written straight into the b1 concat buffer; high stays fp32 until the relayout."""
+        N, C, h, w = x.shape
+        self.launches = 0
+        if N == 0 or h * w == 0:
+            return tuple(torch.empty((N, L.cout, h, w), dtype=x.dtype, device=x.device) for L in (self.convb, self.b4))
+        with self._guard():
+            self._scratch = []  # the PSP pools take freshly zeroed scratch
+            cat = self.new(N, h, w, C + self.conva.cout)
+            self._to_map(x, cat.slice(0, C), "ab.in")
+            low, high = self.attention_branch(cat, C)
+            return self._from_map(low, x.dtype, "ab.low"), self._from_map(high, x.dtype, "ab.high")
+
+    @torch.no_grad()
+    def forward_ffm(self, fsp: torch.Tensor, fcp: torch.Tensor) -> torch.Tensor:
+        """Standalone FeatureFusionModule: (N, c1, h, w), (N, c2, h, w) -> (N, out_chan, h, w) = feat * atten + feat, NCHW
+        in fsp's dtype.  fsp / fcp are written straight into the two slices of convblk's input."""
+        N, c1, h, w = fsp.shape
+        c2, C = fcp.shape[1], self.ffm_blk.cout
+        self.launches = 0
+        if N == 0 or h * w == 0:
+            return torch.empty((N, C, h, w), dtype=fsp.dtype, device=fsp.device)
+        with self._guard():
+            zeros = torch.zeros(N * C + 128 + N * 64 * C, dtype=torch.float32, device=self.dev)  # gap sums + scratch
+            self.launches += 1
+            cat = self.new(N, h, w, c1 + c2)
+            self._to_map(fsp, cat.slice(0, c1), "ffm.in_sp")
+            self._to_map(fcp, cat.slice(c1, c2), "ffm.in_cp")
+            gap = zeros[: N * C].view(N, C)
+            ff = self.ffm_feat(cat, gap, zeros[N * C:])
+            self.ffm_gate_apply(ff, gap)
+            return self._from_map(ff, fsp.dtype, "ffm.out")
+
+    @torch.no_grad()
+    def forward_head(self, x: torch.Tensor) -> torch.Tensor:
+        """Standalone CABiNetOutput: (N, in_chan, h, w) -> (N, n_classes, h, w) class logits (not upsampled) in x's dtype;
+        fp32 inside until the relayout."""
+        N, C, h, w = x.shape
+        self.launches = 0
+        if N == 0 or h * w == 0:
+            return torch.empty((N, self.head_out.cout, h, w), dtype=x.dtype, device=x.device)
+        with self._guard():
+            f = self.new(N, h, w, C)
+            self._to_map(x, f, "conv_out.in")
+            return self._from_map(self.head(f), x.dtype, "conv_out.out")
+
     def bilinear(self, x: Map, out: Map, name: str):
         nbytes = x.N * x.C * (x.H * x.W * x.t.element_size() + out.H * out.W * out.t.element_size())
         self._run("bilinear_nhwc", name, nbytes, 0, self.lib.cabinet_bilinear_nhwc, x.ptr, x.ld, x.dt, out.ptr, out.ld,
@@ -968,15 +1179,10 @@ class Engine:
         cat_ffm = self.new(N, H8, W8, self.sb4.cout if fold_low else 128 + 256)
         if self.sb_overlap:  # experiment: the rest of the spatial branch beside the backbone (joined before the FFM)
             with self._branch(2) as joined:
-                s2 = self.conv(s1, self.sb2)
-                s3 = self.conv(s2, self.sb3)
-                self.conv(s3, self.sb4, out=cat_ffm.slice(0, 128))
+                self.spatial_branch(s1, cat_ffm.slice(0, 128))
                 joined(s1.t)
         else:
-            s2 = self.conv(s1, self.sb2)
-            s3 = self.conv(s2, self.sb3)
-            self.conv(s3, self.sb4, out=cat_ffm.slice(0, 128))
-        assert (s3.H, s3.W) == (H8, W8)
+            self.spatial_branch(s1, cat_ffm.slice(0, 128))
 
         # ---- backbone (reference: mobilenetv3.py:202-205) -> channels [0:960 | 576] of the b1 concat buffer
         f = f0 if fused_stems else self.conv(None, self.stem, nchw_input=x)
@@ -985,65 +1191,25 @@ class Engine:
         mf = self.mobilenet(f, gap_all, out=cat_b1.slice(0, self.last.cout))
 
         # ---- attention branch (reference: cabinet.py:75-94, cab.py:131-162,175-184,213-216)
-        feat = self.conv(mf, self.conva)
-        feat2 = cat_b1.slice(self.last.cout, 256)
-        self.cab(feat, feat2)
-        aux8 = high = low = None
-
-        def low_path():
+        def low_path(feat2):
             if fold_low:  # fp32 [N, h32, w32, 256] map that the convblk epilogue upsamples and adds
                 return self.conv(feat2, self.low_fold, out_dtype=torch.float32)
             lo = self.conv(feat2, self.convb)
             self.bilinear(lo, cat_ffm.slice(128, 256), "low_up")   # 1/32 -> 1/8 (reference: cabinet.py:228-233)
             return lo
 
-        if need_aux or self.debug:
-            aux8 = self.new(N, H8, W8, C, torch.float32)
-            with self._branch(0) as joined:  # low-level path beside b1 / b4
-                low = low_path()
-                joined(low.t)
-            fused = self.conv(cat_b1, self.b1)
-            high = self.conv(fused, self.b4, out_dtype=torch.float32)  # class logits stay fp32
-            self.bilinear(high, aux8, "high_up")
-            self._join(0)
-        else:
-            low = low_path()
+        need_high = need_aux or self.debug
+        aux8 = self.new(N, H8, W8, C, torch.float32) if need_high else None
+        low, high = self.attention_branch(cat_b1, self.last.cout, low_path, need_high,
+                                          lambda hi: self.bilinear(hi, aux8, "high_up"))
 
         # ---- feature fusion (reference: cabinet.py:142-153)
         self._join(2)
-        if fold_low:
-            L = self.ffm_sb
-            ff = self.new(N, H8, W8, L.cout)
-            M = N * H8 * W8
-            self._run("conv_tc", L.name, (M * (L.cin + L.cout) + L.w.numel()) * 2 + low.t.numel() * 4,
-                      2 * M * L.cout * L.cin, self.lib.cabinet_conv_tc_up, cat_ffm.ptr, cat_ffm.ld, N, H8, W8, L.cin,
-                      L.tc.data_ptr(), L.cout, 1, 1, 1, 0, L.b.data_ptr(), low.ptr, low.H, low.W, ff.ptr, ff.ld, H8, W8,
-                      L.act, self.stream)
-        else:
-            ff = self.conv(cat_ffm, self.ffm_blk)
         gap = gap_all[2 * n_se].view(-1)[: N * 256].view(N, 256)
-        self.channel_sum(ff, gap, "ffm.gap", ffm_scratch)
-        hcl = self.head_conv
-        if (self.fold_ffm and self.use_tc and not self.debug and hcl.tc is not None and ff.dt == BF16
-                and hcl.kh * hcl.kw > 1):
-            # feat * atten + feat is a per-(image, channel) scale of the head conv's INPUT: fold it into per-image
-            # copies of the head weights (19 MB) instead of rewriting the 134 MB feature map; the gate MLP runs inside
-            # the same launch
-            wimg = torch.empty((N,) + tuple(hcl.tc.shape), dtype=torch.bfloat16, device=dev)
-            self.gate_scale_weights(gap, False, H8 * W8, self.ffm_gate, hcl.tc, wimg, hcl.cin, True, "ffm.gate")
-            hc = self.new(N, H8, W8, hcl.cout)
-            M = N * H8 * W8
-            self._run("conv_tc", hcl.name, (M * (hcl.cin + hcl.cout) + wimg.numel()) * 2,
-                      2 * M * hcl.cout * hcl.cin * hcl.kh * hcl.kw, self.lib.cabinet_conv_tc_imgw, ff.ptr, ff.ld, N, H8, W8,
-                      ff.C, wimg.data_ptr(), hcl.tc[0].numel() * hcl.tc.shape[0], hcl.cout, hcl.kh, hcl.kw, hcl.stride,
-                      hcl.pad, hcl.b.data_ptr(), None, 0, hc.ptr, hc.dt, hc.ld, H8, W8, hcl.act, self.stream)
-        else:
-            att = self.gate(gap, H8 * W8, self.ffm_gate, "ffm.gate")
-            self.scale_act(ff, att, ACT_NONE, "ffm.gate", plus_one=True)
-            hc = self.conv(ff, hcl)
+        ff = self.ffm_feat(cat_ffm, gap, ffm_scratch, low if fold_low else None)
 
-        # ---- head (reference: cabinet.py:162-172)
-        final8 = self.conv(hc, self.head_out, out_dtype=torch.float32)
+        # ---- head (reference: cabinet.py:162-172), the FFM's gate folded into it or applied first
+        final8 = self.head(ff, gap)
         if self.debug:  # stage activations for the parity tests (keeps the buffers alive)
             self.stages = dict(feat_sb=cat_ffm.slice(0, 128), mobile_feat=mf, low=low, high=high, feat_fuse=ff,
                                final8=final8, aux8=aux8)

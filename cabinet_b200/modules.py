@@ -124,6 +124,40 @@ class _EngineCache:
         return d
 
 
+def _check_nchw(module, x, channels: int, name: str = "x"):
+    """A CPU tensor raises RuntimeError, a wrong shape ValueError, a dtype other than fp32 / bf16 / fp16 TypeError."""
+    cls = type(module).__name__
+    if not isinstance(x, torch.Tensor) or x.dim() != 4 or x.shape[1] != channels:
+        raise ValueError(f"{cls}: expected {name} of shape (N, {channels}, H, W), got {getattr(x, 'shape', type(x))}")
+    if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
+        raise TypeError(f"{cls} takes float32, bfloat16 or float16 input, got {x.dtype}")
+    if not x.is_cuda:
+        raise RuntimeError(f"cabinet_b200.{cls} has no CPU path: move the module and the input to a CUDA device")
+
+
+class _Standalone(_EngineCache):
+    """A child of CABiNet that runs on its own: ``forward`` with the mode semantics of ``CABiNet.forward`` -- ``.eval()``
+    runs the inference schedule (BN folded) unless an input requires grad with grad mode on, which runs the
+    differentiable schedule with running-statistics BatchNorm; ``.train()`` uses batch statistics (running statistics
+    updated) and fills ``p.grad`` and the inputs' ``.grad`` (in their dtypes) on backward.  ``precision`` ("bf16" |
+    "fp32") selects the inference schedule, ``train_precision`` ("fp32" | "bf16" | "fp16") the differentiable one.
+    Outputs have the first input's dtype."""
+
+    def _init_engines(self):
+        self.precision = "bf16"
+        self.train_precision = "fp32"
+        self.__dict__["_engine"] = None
+        self.__dict__["_train_engine"] = None
+
+    def _run(self, inference, *xs):
+        if self.training or (torch.is_grad_enabled() and any(x.requires_grad for x in xs)):
+            from .train_engine import ModuleStep
+
+            ys = ModuleStep.apply(self.train_engine(), len(xs), *xs, *self.parameters())
+            return ys if len(ys) > 1 else ys[0]
+        return inference(self.engine(), *xs)
+
+
 class MobileNetV3(_EngineCache, nn.Module):
     """Backbone (reference: mobilenetv3.py:162-235), runnable on its own.
 
@@ -314,11 +348,19 @@ class ConvBNReLU(nn.Module):
         nn.init.kaiming_normal_(self.conv.weight, a=1)
 
 
-class AttentionBranch(nn.Module):
-    """reference: cabinet.py:54-105."""
+class AttentionBranch(_Standalone, nn.Module):
+    """reference: cabinet.py:54-105, runnable on its own (mode semantics: ``_Standalone``).
+
+    ``forward`` maps an (N, inplanes, h, w) CUDA tensor to ``(low, high)``: convb's (N, outplanes, h, w) features and
+    b4's (N, num_classes, h, w) class logits (not upsampled).  Widths: ``interplanes == outplanes`` (b1 is built for
+    inplanes + outplanes channels but reads cat[x, CAB(conva(x))], which has inplanes + interplanes; the reference fails
+    there too), ``interplanes % 16 == 0`` (the ContextAggregationBlock's rule) and ``inplanes % 8 == 0`` (16-byte pixel
+    rows in the b1 concat buffer).  Checked at the first call.
+    """
 
     def __init__(self, inplanes, interplanes, outplanes, num_classes):
         super().__init__()
+        self._init_engines()
         self.conva = nn.Sequential(_conv(inplanes, interplanes, 3, 1, 1), nn.BatchNorm2d(interplanes), _slot())
         self.a2block = ContextAggregationBlock(interplanes, interplanes // 2)
         self.convb = _conv(interplanes, outplanes, bias=True)
@@ -335,23 +377,49 @@ class AttentionBranch(nn.Module):
                 nn.init.constant_(m.weight, 1)
                 nn.init.constant_(m.bias, 0)
 
+    def forward(self, x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(N, inplanes, h, w) -> (low, high) (reference: cabinet.py:84-94)."""
+        cin, inter, out = self.conva[0].in_channels, self.conva[0].out_channels, self.convb.out_channels
+        if inter != out or inter <= 0 or inter % 16 or cin <= 0 or cin % 8:
+            raise ValueError(f"AttentionBranch({cin}, {inter}, {out}, ...): the kernels need interplanes == outplanes, "
+                             f"interplanes % 16 == 0 and inplanes % 8 == 0")
+        _check_nchw(self, x, cin)
+        return self._run(lambda eng, t: eng.forward_ab(t), x)
 
-class SpatialBranch(nn.Module):
-    """reference: cabinet.py:108-114."""
+
+class SpatialBranch(_Standalone, nn.Module):
+    """reference: cabinet.py:108-129, runnable on its own (mode semantics: ``_Standalone``).
+
+    ``forward`` maps an (N, 3, H, W) CUDA tensor to the (N, 128, h8, w8) spatial features, h8 = H halved three times
+    rounding up.  In the bf16 precision, sb.conv1 runs on the tensor cores when W % 4 == 0 (else on the CUDA cores).
+    """
 
     def __init__(self):
         super().__init__()
+        self._init_engines()
         self.conv1 = ConvBNReLU(3, 64, 7, 2, 3)
         self.conv2 = ConvBNReLU(64, 64, 3, 2, 1)
         self.conv3 = ConvBNReLU(64, 64, 3, 2, 1)
         self.conv_out = ConvBNReLU(64, 128, 1, 1, 0)
 
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        """(N, 3, H, W) -> (N, 128, h8, w8) (reference: cabinet.py:116-121)."""
+        _check_nchw(self, x, 3)
+        return self._run(lambda eng, t: eng.forward_sb(t), x)
 
-class FeatureFusionModule(nn.Module):
-    """reference: cabinet.py:132-140."""
+
+class FeatureFusionModule(_Standalone, nn.Module):
+    """reference: cabinet.py:132-153, runnable on its own (mode semantics: ``_Standalone``).
+
+    ``forward(fsp, fcp)`` maps (N, c1, h, w) and (N, c2, h, w) CUDA tensors (same N / h / w / dtype / device, c1 + c2 ==
+    in_chan) to the (N, out_chan, h, w) ``feat * atten + feat``.  Widths: c1, c2 and out_chan multiples of 8 (16-byte
+    pixel rows; c1 is where fcp starts in convblk's input), out_chan <= 1024 (the gate's limit).  Checked at the first
+    call.
+    """
 
     def __init__(self, in_chan, out_chan):
         super().__init__()
+        self._init_engines()
         self.convblk = ConvBNReLU(in_chan, out_chan, 1, 1, 0)
         self.avg_pool = _slot()
         self.conv1 = _conv(out_chan, out_chan // 4)
@@ -359,14 +427,50 @@ class FeatureFusionModule(nn.Module):
         self.conv2 = _conv(out_chan // 4, out_chan)
         self.sigmoid = _slot()
 
+    def forward(self, fsp: torch.Tensor, fcp: torch.Tensor) -> torch.Tensor:
+        """(N, c1, h, w), (N, c2, h, w) -> (N, out_chan, h, w) (reference: cabinet.py:142-153)."""
+        cin, cout = self.convblk.conv.in_channels, self.convblk.conv.out_channels
+        if cout <= 0 or cout % 8 or cout > 1024:
+            raise ValueError(f"FeatureFusionModule({cin}, {cout}): the kernels need out_chan % 8 == 0 and out_chan <= 1024")
+        if not isinstance(fsp, torch.Tensor) or fsp.dim() != 4:
+            raise ValueError(f"FeatureFusionModule: expected fsp of shape (N, C, h, w), got {getattr(fsp, 'shape', type(fsp))}")
+        c1 = fsp.shape[1]
+        if c1 <= 0 or c1 % 8 or cin - c1 <= 0 or (cin - c1) % 8:
+            raise ValueError(f"FeatureFusionModule({cin}, {cout}): fsp and fcp must split in_chan into two multiples of 8, "
+                             f"got fsp with {c1} channels")
+        if not isinstance(fcp, torch.Tensor) or fcp.dim() != 4 or fcp.shape[1] != cin - c1:
+            raise ValueError(f"FeatureFusionModule: expected fcp of shape (N, {cin - c1}, h, w) beside fsp's {c1} "
+                             f"channels, got {getattr(fcp, 'shape', type(fcp))}")
+        if fcp.shape[0] != fsp.shape[0] or fcp.shape[2:] != fsp.shape[2:]:
+            raise ValueError(f"FeatureFusionModule: fsp {tuple(fsp.shape)} and fcp {tuple(fcp.shape)} differ in N / h / w")
+        if fcp.dtype != fsp.dtype or fcp.device != fsp.device:
+            raise ValueError(f"FeatureFusionModule: fsp ({fsp.dtype}, {fsp.device}) and fcp ({fcp.dtype}, {fcp.device}) "
+                             f"differ in dtype or device")
+        _check_nchw(self, fsp, c1, "fsp")
+        _check_nchw(self, fcp, cin - c1, "fcp")
+        return self._run(lambda eng, a, b: eng.forward_ffm(a, b), fsp, fcp)
 
-class CABiNetOutput(nn.Module):
-    """reference: cabinet.py:156-160."""
+
+class CABiNetOutput(_Standalone, nn.Module):
+    """reference: cabinet.py:156-172, runnable on its own (mode semantics: ``_Standalone``).
+
+    ``forward`` maps an (N, in_chan, h, w) CUDA tensor to the (N, n_classes, h, w) class logits, not upsampled.  Widths:
+    in_chan and mid_chan multiples of 8 (16-byte pixel rows).  Checked at the first call.
+    """
 
     def __init__(self, in_chan, mid_chan, n_classes):
         super().__init__()
+        self._init_engines()
         self.conv = ConvBNReLU(in_chan, mid_chan, 3, 1, 1)
         self.conv_out = _conv(mid_chan, n_classes)
+
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        """(N, in_chan, h, w) -> (N, n_classes, h, w) (reference: cabinet.py:162-172)."""
+        cin, mid = self.conv.conv.in_channels, self.conv.conv.out_channels
+        if cin <= 0 or cin % 8 or mid <= 0 or mid % 8:
+            raise ValueError(f"CABiNetOutput({cin}, {mid}, ...): the kernels need in_chan % 8 == 0 and mid_chan % 8 == 0")
+        _check_nchw(self, x, cin)
+        return self._run(lambda eng, t: eng.forward_head(t), x)
 
 
 class CABiNet(_EngineCache, nn.Module):

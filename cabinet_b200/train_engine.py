@@ -41,6 +41,11 @@ from ._lib import ACT_HSIGMOID, ACT_HSWISH, ACT_NONE, ACT_RELU, ACT_SIGMOID, BF1
 from .constants import BN_EPS
 from .engine import Map, _out_size, backbone_hw, dtype_code
 
+def _sb_hw(H: int, W: int) -> Tuple[int, int]:
+    """(h, w) of the spatial branch's output: three stride-2 convolutions (7x7 pad 3, then 3x3 pad 1 twice)."""
+    return tuple(_out_size(_out_size(_out_size(n, 7, 2, 3), 3, 2, 1), 3, 2, 1) for n in (H, W))
+
+
 BN_MOMENTUM = 0.1  # nn.BatchNorm2d default (the reference never overrides it)
 PSP_SIZES = (1, 3, 6, 8)  # reference: src/models/cab.py:49
 
@@ -851,6 +856,40 @@ class TrainEngine:
                 f = self.bn(self.conv(y, c[4]), c[5], ACT_NONE, res=res)
         return self.bn(self.conv(f, mob.conv[0]), mob.conv[1], ACT_HSWISH, out=out)
 
+    def spatial_branch(self, x: torch.Tensor, xcol: Optional[Map], sb, out: Optional[Map] = None) -> Tuple[Map, Map]:
+        """SpatialBranch ``sb`` (cabinet.py:108-129) on the fp32 NCHW ``x`` (``xcol``: its 7x7 im2col, or None for the
+        CUDA-core stem) -> (sb.conv1's convolution output, the branch's output).  ``out``: where sb.conv_out's BN writes
+        (CABiNet: channels [0:128] of the FFM concat buffer) or None."""
+        stem7 = self.conv_stem(xcol, sb.conv1.conv) if xcol is not None else self.conv(None, sb.conv1.conv, nchw=x)
+        s1 = self.bn(stem7, sb.conv1.bn, ACT_RELU)
+        s2 = self.bn(self.conv(s1, sb.conv2.conv), sb.conv2.bn, ACT_RELU)
+        s3 = self.bn(self.conv(s2, sb.conv3.conv), sb.conv3.bn, ACT_RELU)
+        return stem7, self.bn(self.conv(s3, sb.conv_out.conv), sb.conv_out.bn, ACT_RELU, out=out)
+
+    def attention_branch(self, cat: Map, x: Map, ab, low_path=None) -> Tuple[Map, Map]:
+        """AttentionBranch ``ab`` (cabinet.py:75-94).  ``cat``: the b1 concat buffer [x | CAB feat] (cabinet.py:87); ``x``:
+        its first channels, already written.  -> (low, high): convb's output and b4's fp32 class logits.  ``low_path(low)``
+        runs right after convb (CABiNet: its x4 upsample into the FFM concat buffer)."""
+        feat = self.bn(self.conv(x, ab.conva[0]), ab.conva[1], ACT_RELU)
+        feat2 = cat.slice(x.C, feat.C)
+        self.cab(feat, ab.a2block, feat2)
+        low = self.conv(feat2, ab.convb)
+        if low_path is not None:
+            low_path(low)
+        cat.needs_grad = x.needs_grad or feat2.needs_grad
+        fused = self.bn(self.conv(cat, ab.b1), ab.b2, ACT_RELU)
+        return low, self.conv(fused, ab.b4, out_dtype=torch.float32)
+
+    def ffm(self, cat: Map, ffm) -> Map:
+        """FeatureFusionModule ``ffm`` (cabinet.py:142-153) on ``cat`` = [fsp | fcp]: feat * atten + feat."""
+        ff = self.bn(self.conv(cat, ffm.convblk.conv), ffm.convblk.bn, ACT_RELU)
+        return self.gate(ff, ffm.conv1.weight, None, ffm.conv2.weight, None, ACT_SIGMOID, ACT_NONE, 1.0)
+
+    def head(self, f: Map, head) -> Map:
+        """CABiNetOutput ``head`` (cabinet.py:162-172) -> its fp32 class map."""
+        hc = self.bn(self.conv(f, head.conv.conv), head.conv.bn, ACT_RELU)
+        return self.conv(hc, head.conv_out, out_dtype=torch.float32)
+
     # ------------------------------------------------------------------ the step
     def forward(self, x: torch.Tensor, logits_dtype=torch.float32, input_grad: bool = False):
         """Train-mode ``CABiNet.forward`` (cabinet.py:207-247) -> (final_logit, high_res_logit_up), NCHW.  ``input_grad``:
@@ -864,17 +903,13 @@ class TrainEngine:
         self._stems = (None, None, tuple(x.shape)) if input_grad else None
         mob, sb, ab, ffm, head = m.mobile, m.sb, m.ab, m.ffm, m.conv_out
 
-        # ---- spatial branch (cabinet.py:108-129)
-        xcol = self.stem_im2col(x) if (self.use_tc and self.stem_gemm) else None
-        sb_lo = len(self.tape)
-        stem7 = self.conv_stem(xcol, sb.conv1.conv) if xcol is not None else self.conv(None, sb.conv1.conv, nchw=x)
-        s1 = self.bn(stem7, sb.conv1.bn, ACT_RELU)
-        s2 = self.bn(self.conv(s1, sb.conv2.conv), sb.conv2.bn, ACT_RELU)
-        s3 = self.bn(self.conv(s2, sb.conv3.conv), sb.conv3.bn, ACT_RELU)
-        H8, W8 = s3.H, s3.W
+        # ---- spatial branch (cabinet.py:108-129) -> channels [0:128] of the FFM concat buffer
+        H8, W8 = _sb_hw(H, W)
         n_sb = sb.conv_out.conv.out_channels
         cat_ffm = self.new(N, H8, W8, n_sb + ab.convb.out_channels)
-        sb_feat = self.bn(self.conv(s3, sb.conv_out.conv), sb.conv_out.bn, ACT_RELU, out=cat_ffm.slice(0, n_sb))
+        xcol = self.stem_im2col(x) if (self.use_tc and self.stem_gemm) else None
+        sb_lo = len(self.tape)
+        stem7, sb_feat = self.spatial_branch(x, xcol, sb, out=cat_ffm.slice(0, n_sb))
         sb_hi = len(self.tape)
 
         # ---- backbone (mobilenetv3.py:102-159,202-205)
@@ -889,25 +924,18 @@ class TrainEngine:
         mf = self.mobilenet(f, mob, out=cat_b1.slice(0, n_mf))
 
         # ---- attention branch (cabinet.py:75-94, cab.py:131-162,175-184,213-216)
-        feat = self.bn(self.conv(mf, ab.conva[0]), ab.conva[1], ACT_RELU)
-        feat2 = cat_b1.slice(n_mf, 256)
-        self.cab(feat, ab.a2block, feat2)
-        low = self.conv(feat2, ab.convb)
-        low_up = self.resample(low, "bilinear", H8, W8, out=cat_ffm.slice(n_sb, low.C))         # cabinet.py:228-233
-        cat_b1.needs_grad = mf.needs_grad or feat2.needs_grad
-        cat_ffm.needs_grad = sb_feat.needs_grad or low_up.needs_grad
-        fused = self.bn(self.conv(cat_b1, ab.b1), ab.b2, ACT_RELU)
-        high = self.conv(fused, ab.b4, out_dtype=torch.float32)
+        def low_path(low):
+            low_up = self.resample(low, "bilinear", H8, W8, out=cat_ffm.slice(n_sb, low.C))     # cabinet.py:228-233
+            cat_ffm.needs_grad = sb_feat.needs_grad or low_up.needs_grad
+
+        _, high = self.attention_branch(cat_b1, mf, ab, low_path)
         aux8 = self.resample(high, "bilinear", H8, W8)                                          # cabinet.py:234-239
 
         # ---- feature fusion + head (cabinet.py:142-153,162-172)
         # backward: once this convolution's data gradient exists, the spatial branch (tape[sb_lo:sb_hi]: big, bandwidth-
         # bound kernels) is independent of the attention branch / backbone (many small kernels): a branch of its own
         self._branch = (sb_lo, sb_hi, len(self.tape))
-        ff = self.bn(self.conv(cat_ffm, ffm.convblk.conv), ffm.convblk.bn, ACT_RELU)
-        ffo = self.gate(ff, ffm.conv1.weight, None, ffm.conv2.weight, None, ACT_SIGMOID, ACT_NONE, 1.0)
-        hc = self.bn(self.conv(ffo, head.conv.conv), head.conv.bn, ACT_RELU)
-        final8 = self.conv(hc, head.conv_out, out_dtype=torch.float32)
+        final8 = self.head(self.ffm(cat_ffm, ffm), head)
         final, bwd_final = self.logits_up(final8, H, W, logits_dtype)
         aux, bwd_aux = self.logits_up(aux8, H, W, logits_dtype)
         self._out_bwd = (bwd_final, bwd_aux)
@@ -949,22 +977,29 @@ class TrainEngine:
     def _stem_dgrad(self, g: _Grads) -> Optional[torch.Tensor]:
         """dx of the network input: both stems' data gradients in one cabinet_stem_dgrad call, on the main stream once the
         spatial branch (sb.conv1's output gradient) has joined it.  None when neither stem received a gradient."""
-        stem7, stem3, (N, _, H, W) = self._stems   # stem7 None: a standalone MobileNetV3
-        dy7, dy3 = g.get(stem7) if stem7 is not None else None, g.get(stem3)
+        # stem7 None: a standalone MobileNetV3; stem3 None: a standalone SpatialBranch
+        stem7, stem3, (N, _, H, W) = self._stems
+        dy7 = g.get(stem7) if stem7 is not None else None
+        dy3 = g.get(stem3) if stem3 is not None else None
         if dy7 is None and dy3 is None:
             return None
         dx = torch.empty((N, 3, H, W), dtype=torch.float32, device=self.dev)
-        mob = self.model if stem7 is None else self.model.mobile
-        w7 = self.model.sb.conv1.conv.weight.data_ptr() if stem7 is not None else None
-        dt = (dy7 if dy7 is not None else dy3).dt
+        m = self.model
+        w7 = getattr(m, "sb", m).conv1.conv.weight.data_ptr() if stem7 is not None else None
+        w3 = getattr(m, "mobile", m).features[0][0].weight.data_ptr() if stem3 is not None else None
+        dy = dy7 if dy7 is not None else dy3
         self._call("cabinet_stem_dgrad", dy7.ptr if dy7 is not None else None, dy7.ld if dy7 is not None else 0,
-                   dy3.ptr if dy3 is not None else None, dy3.ld if dy3 is not None else 0, dt, w7,
-                   mob.features[0][0].weight.data_ptr(), dx.data_ptr(), N, H, W, stem3.H, stem3.W)
+                   dy3.ptr if dy3 is not None else None, dy3.ld if dy3 is not None else 0, dy.dt, w7, w3, dx.data_ptr(),
+                   N, H, W, dy.H, dy.W)
         return dx
 
     # ------------------------------------------------------------------ a standalone ContextAggregationBlock
     def _relayout(self, src: torch.Tensor, src_strides, dst: torch.Tensor, dst_strides, N, H, W, C):
         """dst = src between two (N, H, W, C) stride patterns and float dtypes (NCHW <-> NHWC at the block's boundary)."""
+        if {src.dtype, dst.dtype} == {torch.bfloat16, torch.float16}:  # no kernel for this pair: through fp32
+            tmp = torch.empty((N, H, W, C), dtype=torch.float32, device=self.dev)
+            self._relayout(src, src_strides, tmp, (H * W * C, W * C, C, 1), N, H, W, C)
+            src, src_strides = tmp, (H * W * C, W * C, C, 1)
         ty, tx = self.tables.get("identity", H, H, False), self.tables.get("identity", W, W, False)
         self._call("cabinet_resample_sep", src.data_ptr(), self._dt(src), *src_strides, dst.data_ptr(), self._dt(dst),
                    *dst_strides, N, H, W, C, *(t.data_ptr() for t in ty), *(t.data_ptr() for t in tx), 0)
@@ -1055,6 +1090,97 @@ class TrainEngine:
             torch.cuda.current_stream(self.dev).wait_stream(self._side)
         self.tape, self._block, self._stems = [], None, None
         return self.pgrads, dx
+
+    # ------------------------------------------------------------------ a standalone branch or head
+    def _to_map(self, x: torch.Tensor, m: Map):
+        """NCHW ``x`` -> the NHWC map ``m`` (a channel slice of a concat buffer, say), in m's dtype."""
+        self._relayout(x, (x.stride(0), x.stride(2), x.stride(3), x.stride(1)), m.t[..., m.off:m.off + m.C],
+                       (m.H * m.W * m.ld, m.W * m.ld, m.ld, 1), m.N, m.H, m.W, m.C)
+
+    def _from_map(self, m: Map, dtype: torch.dtype) -> torch.Tensor:
+        """The NHWC map ``m`` -> a new NCHW tensor of ``dtype``."""
+        y = torch.empty((m.N, m.C, m.H, m.W), dtype=dtype, device=self.dev)
+        self._relayout(m.t[..., m.off:m.off + m.C], (m.H * m.W * m.ld, m.W * m.ld, m.ld, 1), y,
+                       (y.stride(0), y.stride(2), y.stride(3), y.stride(1)), m.N, m.H, m.W, m.C)
+        return y
+
+    def module_forward(self, xs, needs_grad) -> Tuple[List[torch.Tensor], tuple]:
+        """``self.model`` is a standalone SpatialBranch, AttentionBranch, FeatureFusionModule or CABiNetOutput: its
+        train-mode (or differentiable eval-mode) forward on the NCHW inputs ``xs`` -> its NCHW outputs in the first
+        input's dtype, and the call's record (tape, boundary maps, stems) that ``module_backward`` takes.  The record belongs
+        to the call, not the engine: several calls of one module before a backward (two inputs into one loss, activation
+        checkpointing) each keep their own.  ``needs_grad[i]``: ``module_backward`` computes the gradient of ``xs[i]``.
+        Inputs are written straight into the buffers the first layers read (the b1 / convblk concat buffers)."""
+        from . import modules
+
+        m, xdt = self.model, xs[0].dtype
+        self.tape, self.launches, self.pgrads, self.phase = [], 0, {}, "fwd"
+        self._pflat, self._bn_seen, self._stems = None, [], None
+        N, _, H, W = xs[0].shape
+        ins = []
+        if isinstance(m, modules.SpatialBranch):
+            x = xs[0] if xdt == torch.float32 and xs[0].is_contiguous() else xs[0].float().contiguous()
+            self._stems = (None, None, tuple(x.shape)) if needs_grad[0] else None
+            xcol = self.stem_im2col(x) if (self.use_tc and self.stem_gemm) else None
+            stem7, out = self.spatial_branch(x, xcol, m)
+            if needs_grad[0]:
+                self._stems = (stem7, None, tuple(x.shape))
+            outs = [out]
+        elif isinstance(m, modules.AttentionBranch):
+            cat = self.new(N, H, W, xs[0].shape[1] + m.conva[0].out_channels)
+            x = cat.slice(0, xs[0].shape[1])
+            self._to_map(xs[0], x)
+            x.needs_grad = needs_grad[0]
+            ins, outs = [x], list(self.attention_branch(cat, x, m))
+        elif isinstance(m, modules.FeatureFusionModule):
+            c1, c2 = xs[0].shape[1], xs[1].shape[1]
+            cat = self.new(N, H, W, c1 + c2)
+            ins = [cat.slice(0, c1), cat.slice(c1, c2)]
+            for t, mp, rg in zip(xs, ins, needs_grad):
+                self._to_map(t, mp)
+                mp.needs_grad = rg
+            cat.needs_grad = any(needs_grad)
+            outs = [self.ffm(cat, m)]
+        elif isinstance(m, modules.CABiNetOutput):
+            f = self.new(N, H, W, xs[0].shape[1])
+            self._to_map(xs[0], f)
+            f.needs_grad = needs_grad[0]
+            ins, outs = [f], [self.head(f, m)]
+        else:
+            raise TypeError(f"module_forward runs the branches and heads of CABiNet, not {type(m).__name__}")
+        ys = [self._from_map(o, xdt) for o in outs]
+        record = (self.tape, ins, outs, self._stems)
+        self.tape, self._stems = [], None
+        if self._bn_seen:
+            torch._foreach_add_(self._bn_seen, 1)
+        return ys, record
+
+    def module_backward(self, record, dys, xdts) -> Tuple[Dict[int, torch.Tensor], List[Optional[torch.Tensor]]]:
+        """Gradients of the outputs of the ``module_forward`` call that returned ``record`` (None: that output is unused,
+        and layers only it reaches run no backward) -> ({id(parameter): fp32 gradient}, [gradient of each input in
+        ``xdts[i]`` or None])."""
+        self.tape, ins, outs, self._stems = record
+        g = _Grads(self)
+        self.pgrads, self.phase, self._pflat, self._side_used = {}, "bwd", None, False
+        self._ensure_pflat()
+        dxs = [None] * len(xdts)
+        live = [(o, dy) for o, dy in zip(outs, dys) if dy is not None and o.needs_grad]
+        if live:
+            for o, dy in live:
+                do, _ = g.out(o)
+                self._to_map(dy, do)
+            for i in range(len(self.tape) - 1, -1, -1):
+                self.tape[i](g)
+            if self._stems is not None:
+                dx = self._stem_dgrad(g)
+                dxs[0] = dx.to(xdts[0]) if dx is not None else None
+            for i, mp in enumerate(ins):
+                d = g.get(mp) if mp.needs_grad else None
+                dxs[i] = self._from_map(d, xdts[i]) if d is not None else None
+        if self._side_used:  # join: the parameter gradients are complete when the caller's stream continues
+            torch.cuda.current_stream(self.dev).wait_stream(self._side)
+        self.tape, self._stems = [], None
+        return self.pgrads, dxs
 
     # ------------------------------------------------------------------ the step as two CUDA graphs
     def _addresses(self) -> tuple:
@@ -1195,6 +1321,32 @@ class BlockStep(torch.autograd.Function):
         with torch.no_grad(), torch.cuda.device(eng.dev):
             grads, dx = eng.block_backward(dy)
         return (None, dx, *(grads[id(p)].to(p.dtype) if id(p) in grads else None for p in ctx.params))
+
+
+class ModuleStep(torch.autograd.Function):
+    """Autograd hand-off of a standalone module (``TrainEngine.module_forward``): inputs = (engine, k, k NCHW tensors,
+    *parameters); outputs = the module's NCHW outputs in the first input's dtype.  An unused output's gradient stays None
+    (no materialised zeros), and a gradient is returned for each input that requires one, in that input's dtype."""
+
+    @staticmethod
+    def forward(ctx, eng: TrainEngine, k: int, *args):
+        xs, params = args[:k], args[k:]
+        ctx.set_materialize_grads(False)
+        with torch.no_grad(), torch.cuda.device(eng.dev):
+            ys, ctx.record = eng.module_forward(xs, [bool(ctx.needs_input_grad[2 + i]) for i in range(k)])
+        ctx.eng, ctx.params, ctx.xdts = eng, params, [x.dtype for x in xs]
+        return tuple(ys)
+
+    @staticmethod
+    def backward(ctx, *dys):
+        eng = ctx.eng
+        if ctx.record is None:  # freed by the first backward, as PyTorch frees a node's saved tensors
+            raise RuntimeError("Trying to backward through a cabinet_b200 module's graph a second time: its saved "
+                               "activations were freed by the first backward")
+        with torch.no_grad(), torch.cuda.device(eng.dev):
+            grads, dxs = eng.module_backward(ctx.record, dys, ctx.xdts)
+        ctx.record = None
+        return (None, None, *dxs, *(grads[id(p)].to(p.dtype) if id(p) in grads else None for p in ctx.params))
 
 
 class BackboneStep(torch.autograd.Function):

@@ -130,6 +130,13 @@ int cabinet_stem_tc(const float* x, int N, int H, int W, const void* w_packed, c
 int cabinet_stem_tc2(const float* x, int N, int H, int W, const void* w_packed2, void* y_sb, long long ld_sb, void* y_stem,
                      long long ld_stem, int OH, int OW, cabinet_stream_t stream);
 
+/* sb.conv1 alone (a standalone SpatialBranch: 7x7 s2 p3, 3 -> 64, BN folded, ReLU): the kernel of cabinet_stem_tc2 at
+ * N = 64, one TMA store per tile.  x fp32 NCHW [N][3][H][W] (W % 4 == 0); y bf16 NHWC [N][OH][OW] with pixel stride ld_y
+ * (a multiple of 8, >= 64; channels 64.. of a pixel are not written).
+ * w_packed7: rows 0..63 of the cabinet_stem_tc2 pack, bf16 [7 ky][2 K halves][2 k chunks][64 out][8]. */
+int cabinet_stem7_tc(const float* x, int N, int H, int W, const void* w_packed7, void* y, long long ld_y, int OH, int OW,
+                     cabinet_stream_t stream);
+
 /* The backbone stem alone (a standalone MobileNetV3: 3x3 s2 p1, 3 -> 16, BN folded, HardSwish) in the formulation of
  * cabinet_stem_tc2, one K16 slice per tap row.  x fp32 NCHW [N][3][H][W] (W % 4 == 0); y bf16 NHWC [N][OH][OW] with pixel
  * stride ld_y (a multiple of 8, >= 16).
